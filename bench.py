@@ -2,7 +2,7 @@
 """Benchmark of the iALS hot path (BASELINE.json metric: iALS epochs/sec &
 interactions/sec at k=128).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one iALS epoch (Gram(item) -> solve users -> Gram(user) -> solve
 items) over a synthetic interaction matrix.  N=1 runs BASELINE.json configs[1]
@@ -25,6 +25,11 @@ line is printed by rank 0 (see DESIGN.md "Measurement" for every field).
 
 `--impl reference` times that CPU port alone with all host threads (the real
 irspack cannot be built offline: Eigen 5.0.1 / nanobind are not in the image).
+
+`--dump-outputs DIR` (N=1 only) writes the factors the timed epochs produced (after
+the last one) to DIR/<name>.npy, so that two builds can be compared output for
+output: the inputs are seeded and identical for identical arguments.  The sharded
+N>1 run keeps each rank's factor rows on its own GPU and has no such dump.
 """
 from __future__ import annotations
 
@@ -151,6 +156,19 @@ def make_inputs(w):
     return X, init_factors(w["n_users"], w["K"], 1), init_factors(w["n_items"], w["K"], 2)
 
 
+DUMP_USER_ROWS = 65536  # all 138493 user rows (71 MB) and the item factors would exceed the 64 MB dump budget
+
+
+def dump_outputs(out_dir, user, item):
+    """What a caller of the timed path receives after its last epoch: the item factors whole and a
+    fixed, seeded sample of user rows (ascending), float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = user.shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_USER_ROWS), replace=False))
+    np.save(os.path.join(out_dir, "user_factors_sample.npy"), np.ascontiguousarray(user[rows], dtype=np.float32))
+    np.save(os.path.join(out_dir, "item_factors.npy"), np.ascontiguousarray(item, dtype=np.float32))
+
+
 def solve_bytes(w):
     """Algorithmic bytes of the two row-solve launches of one epoch (DESIGN.md):
     every neighbour's K-vector + int32 index + f32 value once per half-epoch,
@@ -217,6 +235,8 @@ def run_reference(args):
     for _ in range(args.steps):
         o.epoch_native(oracle.SOLVER_CG, HYPER["max_cg_steps"], nt)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, o.user, o.item)
     value = w["nnz"] * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT,
@@ -302,6 +322,8 @@ def run_ours(args):
     ms = ev0.elapsed_time(ev1)
     phase_ms, n_prof = tr.get_timings()
     tr.set_profiling(False)
+    if args.dump_outputs:  # before the e2e leg below trains the same factors further
+        dump_outputs(args.dump_outputs, tr.user, tr.item)
     value = w["nnz"] * args.steps / (ms / 1e3)
 
     # ---- end to end through the reference-facing API, host buffers ----
@@ -422,7 +444,13 @@ def main():
     ap.add_argument("--cpu-epochs", type=int, default=5)
     ap.add_argument("--c4", choices=["auto", "off"], default="auto",
                     help="N=1 only: also time configs[3] (1 B interactions) on the one GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--gpus 1 only: write the factors of the last timed epoch to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus != 1:
+        ap.error("--dump-outputs is implemented for --gpus 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

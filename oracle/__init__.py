@@ -19,7 +19,10 @@ import ctypes
 import hashlib
 import math
 import os
+import shutil
+import stat
 import subprocess
+import tempfile
 from typing import Dict, List, Optional, Tuple
 
 import numpy as np
@@ -30,7 +33,6 @@ _SRC = os.path.join(_HERE, "ials_oracle.cpp")
 _SRC_RNG = os.path.join(_HERE, "ials_oracle_rng.cpp")
 _BUILD = os.path.join(_HERE, "_build")
 _SO = os.path.join(_BUILD, "libials_oracle.so")
-_STAMP = os.path.join(_BUILD, "cpu.stamp")
 # A toolchain that links libstdc++ statically (this image's /opt/gcc wrapper) must keep that copy
 # private: a Python process already holds another libstdc++, and a half-interposed static one
 # crashes on the first throw.  Harmless with a dynamic libstdc++.
@@ -59,29 +61,58 @@ def _cpu_stamp() -> str:
     return "unknown"
 
 
+def _fresh(build_dir: str) -> bool:
+    """The library in ``build_dir`` is newer than both sources and was built for this CPU."""
+    so, stamp = os.path.join(build_dir, "libials_oracle.so"), os.path.join(build_dir, "cpu.stamp")
+    if not (os.path.exists(so) and os.path.exists(stamp)):
+        return False
+    if any(os.path.getmtime(so) < os.path.getmtime(p) for p in (_SRC, _SRC_RNG)):
+        return False
+    with open(stamp) as f:
+        return f.read().strip() == _cpu_stamp()
+
+
+def _private_build_dir() -> str:
+    """Where a read-only checkout builds the oracle: one directory per user under the system's
+    temporary directory, reused by that user's later processes."""
+    d = os.path.join(tempfile.gettempdir(), f"ials_oracle_{os.getuid()}")
+    os.makedirs(d, mode=0o700, exist_ok=True)
+    st = os.lstat(d)
+    if not stat.S_ISDIR(st.st_mode) or st.st_uid != os.getuid() or st.st_mode & 0o077:
+        raise RuntimeError(f"{d} is not a directory private to this user; not loading a library from it")
+    return d
+
+
 def build(force: bool = False) -> str:
     """Compile the oracle with g++ -O3 (a few seconds): ``ials_oracle.cpp`` for this host
     (``-march=native``), ``ials_oracle_rng.cpp`` -- the libstdc++ random-number helpers -- for the
-    x86-64 baseline without FMA contraction, like the reference's portable wheels."""
-    srcs = (_SRC, _SRC_RNG)
-    stale = (
-        force
-        or not os.path.exists(_SO)
-        or any(os.path.getmtime(_SO) < os.path.getmtime(p) for p in srcs)
-        or not os.path.exists(_STAMP)
-        or open(_STAMP).read().strip() != _cpu_stamp()
-    )
-    if stale:
-        os.makedirs(_BUILD, exist_ok=True)
+    x86-64 baseline without FMA contraction, like the reference's portable wheels.  A read-only
+    checkout whose ``oracle/_build`` is missing or stale builds into ``_private_build_dir()``."""
+    if not force and _fresh(_BUILD):
+        return _SO
+    writable = os.access(_BUILD if os.path.isdir(_BUILD) else _HERE, os.W_OK)
+    out = _BUILD if writable else _private_build_dir()
+    so = os.path.join(out, "libials_oracle.so")
+    if not force and _fresh(out):
+        return so
+    os.makedirs(out, exist_ok=True)
+    # objects and library are made in a scratch directory and the library moved into place, so that
+    # processes building at the same time never load a half-written file
+    work = tempfile.mkdtemp(dir=out)
+    try:
         cxx = os.environ.get("CXX", "g++")
         common = ["-O3", "-std=c++17", "-fPIC", "-pthread", "-fvisibility=hidden"]
-        obj, obj_rng = os.path.join(_BUILD, "ials_oracle.o"), os.path.join(_BUILD, "ials_oracle_rng.o")
+        obj, obj_rng = os.path.join(work, "ials_oracle.o"), os.path.join(work, "ials_oracle_rng.o")
         subprocess.run([cxx, *common, "-march=native", "-c", _SRC, "-o", obj], check=True)
         subprocess.run([cxx, *common, "-ffp-contract=off", "-c", _SRC_RNG, "-o", obj_rng], check=True)
-        subprocess.run([cxx, "-shared", "-pthread", _PRIVATE_RUNTIME, "-o", _SO, obj, obj_rng], check=True)
-        with open(_STAMP, "w") as f:
-            f.write(_cpu_stamp())
-    return _SO
+        subprocess.run([cxx, "-shared", "-pthread", _PRIVATE_RUNTIME, "-o", os.path.join(work, "lib.so"),
+                        obj, obj_rng], check=True)
+        os.replace(os.path.join(work, "lib.so"), so)
+    finally:
+        shutil.rmtree(work, ignore_errors=True)
+    with open(os.path.join(out, "cpu.stamp"), "w") as f:
+        f.write(_cpu_stamp())
+    return so
 
 
 # ---- oracle/_ref: the reference's own sources, compiled where they lie ----
