@@ -4,182 +4,26 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
-#include <cstring>
 #include <random>
 #include <string>
 #include <vector>
 
-#include "common.cuh"
+#include "trainer.cuh"
 
 using namespace ials;
 
-namespace ials {  // cholesky_ll.cu: Cholesky rows whose Gram blocks are in a workspace
-size_t cholesky_ll_scratch_bytes();
-void launch_solve_cholesky_from_gram(const SolveArgs &a, const int32_t *first_job, int job0, int job_cap,
-                                     const float *workspace, float *scratch, cudaStream_t s);
-}  // namespace ials
-
-struct ials_trainer {
-  ials_model_config cfg{};
-  int device = 0;
-  cudaStream_t stream = nullptr;
-  int64_t U = 0, I = 0;
-  int K = 0, ld = 0;
-  float *factor[2] = {nullptr, nullptr};  // [0] user U x ld, [1] item I x ld
-  DeviceCsr X, Xt;
-  bool has_X = false;
-  float *P[2] = {nullptr, nullptr};  // P[0]: user_solver.P = alpha0 item^T item; P[1]: item_solver.P
-  float *gram_scratch = nullptr;
-  GramWorkspace gws;  // tensor-core Gram (ld == 128)
-  // heavy-row path of the CG solver: per-job Gram partials from wgram.cu
-  float *heavy_W = nullptr, *heavy_b = nullptr;
-  int64_t heavy_jobs_cap = 0;
-  int *err_flags = nullptr;
-  unsigned long long *work_counter = nullptr;
-  double *d_loss = nullptr;
-  float *score_buf = nullptr;
-  size_t score_buf_bytes = 0;
-  // ials_trainer_recommend: result and mask staging buffers, kept between calls (grow-only) --
-  // an Evaluator calls it once per block of users, and five cudaMalloc / cudaFree pairs per call
-  // cost as much as the kernel itself at 128 .. 4096 users per block
-  struct GrowBuf {
-    void *p = nullptr;
-    size_t cap = 0;
-    void *get(size_t bytes) {
-      if (bytes > cap) {
-        if (p) CUDA_CHECK(cudaFree(p));
-        p = nullptr;
-        cap = 0;
-        CUDA_CHECK(cudaMalloc(&p, bytes));
-        cap = bytes;
-      }
-      return p;
-    }
-    void release() {
-      if (p) cudaFree(p);
-      p = nullptr;
-      cap = 0;
-    }
-  } rec_idx, rec_score, rec_count, rec_mindptr, rec_mindices, rec_aindptr, rec_aindices, rec_uidx, rec_users, rec_emb;
-  std::vector<uint32_t> rec_abitmap_host;  // shared allow-list as a bitmap, staged for the upload
-  // shard (multi-GPU): rows owned (solved) by this rank, per side; X / Xt then hold only
-  // those rows (DeviceCsr::row_base = shard begin) while both factor matrices are full replicas
-  bool sharded = false;
-  int64_t shard[2][2] = {{0, 0}, {0, 0}};
-  int n_peers[2] = {0, 0};
-  float *peers[2][8] = {};
-  // phase timing: 5 events per profiled epoch (before, after each of the 4 phases)
-  bool profiling = false;
-  std::vector<cudaEvent_t> prof_events;
-  // ials_trainer_step_io: second stream + event for the overlapped read-back of the user factors
-  cudaStream_t copy_stream = nullptr;
-  cudaEvent_t users_done = nullptr;
-  int *ready_flags = nullptr;  // step_io: one flag per chunk of user rows arriving from the host
-  int *ready_host = nullptr;   // pinned source of the flag copies
-  int32_t *order_io = nullptr; // step_io: the light user rows by (arrival chunk, descending degree)
-  int ready_cap = 0, ready_token = 0;
-  bool ready_pending = false;          // a flagged upload is in flight for the next user solve
-  cudaEvent_t upload_done = nullptr;   // behind its last chunk, on the copy stream
-  // Cholesky with 256-column factors: a job plan over EVERY non-empty row of each side (shares
-  // the CSR arrays of X / Xt, owns only its job arrays), the host copy of its row -> job map, and
-  // the per-chunk workspace of Gram blocks
-  DeviceCsr chol_plan[2];
-  bool chol_plan_ready[2] = {false, false};
-  std::vector<int32_t> chol_first[2];
-  float *chol_ws = nullptr;
-  int64_t chol_cap = 0;  // jobs the workspace holds = jobs per chunk
-  float *gs_ws = nullptr;  // iALS++ route: W [gs_cap][128][128] | b [gs_cap][kWGramBParts][128]
-  int64_t gs_cap = 0;
-  float *chol_scratch = nullptr;  // cholesky_ll_kernel: the factor of every resident CTA
-  // feature-aware iALS (IALSTrainer(config, X, user_feature, item_feature), IALSTrainer.hpp:722-743)
-  struct FeatureSide {
-    bool given = false;       // the trainer was built with features for this side
-    bool weight_set = false;  // a weight matrix exists (given, or restored by set_feature_weight)
-    bool has_empty_row = false;
-    ials::FeatureDev F;       // views of the owned device arrays below
-    float *d_dense = nullptr, *d_data = nullptr;
-    int64_t *d_indptr = nullptr;
-    int32_t *d_indices = nullptr;
-    int64_t n_w = 0;          // rows of the weight (= feature columns)
-    float *weight = nullptr;  // [n_w x ld]
-    float *prior = nullptr;   // [n_rows x ld]
-    float *rw = nullptr;      // [n_rows]   compute_reg of every row (FeatureWeightCache::row_weights)
-    float *llt = nullptr;     // [n_w x n_w] Cholesky factor of F^T D F + lambda I (FeatureWeightCache::llt)
-    float *rhs = nullptr;     // [n_w x ld]
-    bool cache_ready = false;
-    float lambda = 0.f;
-    void free_features() {
-      if (d_dense) cudaFree(d_dense);
-      if (d_data) cudaFree(d_data);
-      if (d_indptr) cudaFree(d_indptr);
-      if (d_indices) cudaFree(d_indices);
-      d_dense = d_data = nullptr;
-      d_indptr = nullptr;
-      d_indices = nullptr;
-      F = ials::FeatureDev{};
-    }
-    void free_all() {
-      free_features();
-      for (float **p : {&weight, &prior, &rw, &llt, &rhs}) {
-        if (*p) cudaFree(*p);
-        *p = nullptr;
-      }
-    }
-  } feat[2];
-  bool feature_aware = false;
-  int64_t epoch = 0, feature_warmup = 0;  // epoch_, config_.feature_warmup_epochs
-  int64_t n_rows(int side) const { return side == 0 ? U : I; }
-};
-
 namespace ials {
+
 int64_t g_kernel_launches = 0;
-}
-
-namespace {
-
 thread_local std::string g_last_error;
 
-struct DeviceGuard {
-  int prev = -1;
-  explicit DeviceGuard(int dev) {
-    CUDA_CHECK(cudaGetDevice(&prev));
-    if (prev != dev) CUDA_CHECK(cudaSetDevice(dev));
-    else prev = -1;
+void require_device(int device) {
+  int n_dev = 0;
+  if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
+    cudaGetLastError();
+    throw CudaError("no CUDA device available: the B200 backend has no CPU fallback");
   }
-  ~DeviceGuard() {
-    if (prev >= 0) cudaSetDevice(prev);
-  }
-};
-
-template <typename F>
-int guarded(F &&fn) {
-  try {
-    fn();
-    return IALS_OK;
-  } catch (const InvalidArgument &e) {
-    g_last_error = e.what();
-    return IALS_ERR_INVALID_ARGUMENT;
-  } catch (const NotImplemented &e) {
-    g_last_error = e.what();
-    return IALS_ERR_NOT_IMPLEMENTED;
-  } catch (const CudaError &e) {
-    g_last_error = e.what();
-    cudaGetLastError();  // clear the sticky-less error state
-    return IALS_ERR_CUDA;
-  } catch (const std::invalid_argument &e) {
-    g_last_error = e.what();
-    return IALS_ERR_INVALID_ARGUMENT;
-  } catch (const std::exception &e) {
-    g_last_error = e.what();
-    return IALS_ERR_RUNTIME;
-  } catch (...) {  // nothing may unwind through the C ABI
-    g_last_error = "unknown C++ exception";
-    return IALS_ERR_RUNTIME;
-  }
-}
-
-void require(bool cond, const char *msg) {
-  if (!cond) throw InvalidArgument(msg);
+  require(device >= 0 && device < n_dev, "invalid CUDA device index");
 }
 
 void check_solver(const ials_solver_config *sc) {
@@ -201,35 +45,28 @@ void alloc_common(ials_trainer *t) {
   const int64_t ld = t->ld;
   for (int side = 0; side < 2; side++) {
     const int64_t n = t->n_rows(side);
-    CUDA_CHECK(cudaMalloc(&t->factor[side], sizeof(float) * std::max<int64_t>(n * ld, 1)));
-    CUDA_CHECK(cudaMemset(t->factor[side], 0, sizeof(float) * std::max<int64_t>(n * ld, 1)));
-    CUDA_CHECK(cudaMalloc(&t->P[side], sizeof(float) * ld * ld));
-    CUDA_CHECK(cudaMemset(t->P[side], 0, sizeof(float) * ld * ld));
+    CUDA_CHECK(cudaMemset(t->factor[side].alloc(std::max<int64_t>(n * ld, 1)), 0,
+                          sizeof(float) * std::max<int64_t>(n * ld, 1)));
+    CUDA_CHECK(cudaMemset(t->P[side].alloc(ld * ld), 0, sizeof(float) * ld * ld));
   }
-  CUDA_CHECK(cudaMalloc(&t->gram_scratch, sizeof(float) * ld * ld));
+  t->gram_scratch.alloc(ld * ld);
   if (ld == 128) t->gws.alloc(kNumSMsB200);
-  CUDA_CHECK(cudaMalloc(&t->err_flags, sizeof(int) * kNumErrFlags));
-  CUDA_CHECK(cudaMemset(t->err_flags, 0, sizeof(int) * kNumErrFlags));
-  CUDA_CHECK(cudaMalloc(&t->work_counter, sizeof(unsigned long long)));
-  CUDA_CHECK(cudaMalloc(&t->d_loss, sizeof(double)));
+  CUDA_CHECK(cudaMemset(t->err_flags.alloc(kNumErrFlags), 0, sizeof(int) * kNumErrFlags));
+  t->work_counter.alloc(1);
+  t->d_loss.alloc(1);
 }
 
-int64_t env_int(const char *name, int64_t dflt);
-
-ials_trainer *new_trainer(const ials_model_config *cfg, int64_t U, int64_t I, int device) {
+// Validates the model and the device; the trainer holds no device memory yet.  Its deleter is
+// ials_trainer_destroy, which frees on the trainer's device after a synchronise.
+TrainerPtr new_trainer(const ials_model_config *cfg, int64_t U, int64_t I, int device) {
   require(cfg != nullptr, "model_config is null");
   require(cfg->K >= 1 && cfg->K <= 512, "K must be in [1, 512]");
   require(U >= 0 && I >= 0, "negative matrix shape");
   require(U < (1ll << 31) && I < (1ll << 31), "matrix dimensions must fit int32");
   require(cfg->loss_type == IALS_LOSS_ORIGINAL || cfg->loss_type == IALS_LOSS_IALSPP,
           "unknown loss_type");
-  int n_dev = 0;
-  if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-    cudaGetLastError();
-    throw CudaError("no CUDA device available: the B200 backend has no CPU fallback");
-  }
-  require(device >= 0 && device < n_dev, "invalid CUDA device index");
-  auto *t = new ials_trainer();
+  require_device(device);
+  TrainerPtr t(new ials_trainer(), ials_trainer_destroy);
   t->cfg = *cfg;
   t->device = device;
   t->U = U;
@@ -243,9 +80,19 @@ ials_trainer *new_trainer(const ials_model_config *cfg, int64_t U, int64_t I, in
   return t;
 }
 
-// Solver::initialize, IALSTrainer.hpp:64-76: a fresh mt19937(seed) per matrix.
-void init_factors_host_rng(ials_trainer *t) {
+// Solver::initialize, IALSTrainer.hpp:64-76: a fresh mt19937(seed) per matrix; on_device: the
+// counter-based device fill (for factor matrices too large for the serial host RNG)
+void init_factors(ials_trainer *t, bool on_device) {
   if (!(t->cfg.init_stdev > 0)) return;  // matrices stay zero
+  if (on_device) {
+    const float sd = (float)(t->cfg.init_stdev / std::sqrt((double)t->K));
+    // same seed for both matrices, like the reference's two fresh generators
+    for (int side = 0; side < 2; side++)
+      launch_init_normal(t->factor[side].get(), t->n_rows(side), t->K, t->ld, sd,
+                         (uint64_t)(uint32_t)t->cfg.random_seed, t->stream);
+    CUDA_CHECK(cudaStreamSynchronize(t->stream));
+    return;
+  }
   for (int side = 0; side < 2; side++) {
     const int64_t n = t->n_rows(side);
     if (n == 0) continue;
@@ -253,8 +100,7 @@ void init_factors_host_rng(ials_trainer *t) {
     std::normal_distribution<float> dist(0.0, t->cfg.init_stdev / std::sqrt((double)t->K));
     std::vector<float> h((size_t)n * t->K);
     for (auto &v : h) v = dist(gen);
-    CUDA_CHECK(cudaMemcpy2D(t->factor[side], sizeof(float) * t->ld, h.data(), sizeof(float) * t->K,
-                            sizeof(float) * t->K, n, cudaMemcpyHostToDevice));
+    rows_to_device(t->factor[side].get(), t->ld, h.data(), t->K, n);
   }
 }
 
@@ -274,22 +120,16 @@ int64_t env_int(const char *name, int64_t dflt) {
 }
 void plan_csr(ials_trainer *t, DeviceCsr &csr) {
   build_row_order(csr, t->stream);
+  csr.has_negative = csr_has_negative(csr, t->stream);
   if (t->ld == 128) {
     const int64_t heavy = std::max<int64_t>(env_int("IALS_HEAVY_THRESHOLD", 2048), 1);
-    build_heavy_plan(csr, heavy, env_int("IALS_HEAVY_JOB_LEN", 4096), t->stream);
+    build_heavy_plan(csr, heavy, env_int("IALS_HEAVY_JOB_LEN", 4096), csr.heavy, t->stream);
   }
-}
-
-void finish_csr(ials_trainer *t) {
-  build_transpose(t->X, t->Xt, t->stream);
-  plan_csr(t, t->X);
-  plan_csr(t, t->Xt);
-  t->has_X = true;
 }
 
 // Copies a CSR (host or device arrays) into device memory owned by `d`.
 void upload_csr(DeviceCsr &d, int64_t n_rows, int64_t n_cols, const int64_t *indptr,
-                const int32_t *indices, const float *data, bool on_device = false) {
+                const int32_t *indices, const float *data, bool on_device) {
   require(indptr != nullptr, "indptr is null");
   int64_t nnz = 0;
   if (on_device) {
@@ -305,17 +145,23 @@ void upload_csr(DeviceCsr &d, int64_t n_rows, int64_t n_cols, const int64_t *ind
   if (!on_device)
     for (int64_t j = 0; j < nnz; j++)
       require(indices[j] >= 0 && indices[j] < n_cols, "column index out of range");
+  copy_csr(d, n_rows, n_cols, nnz, indptr, indices, data,
+           on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice);
+}
+
+// Copies the arrays of a validated CSR into device memory owned by `d`.
+void copy_csr(DeviceCsr &d, int64_t n_rows, int64_t n_cols, int64_t nnz, const int64_t *indptr,
+              const int32_t *indices, const float *data, cudaMemcpyKind kind) {
   d.n_rows = n_rows;
   d.n_cols = n_cols;
   d.nnz = nnz;
-  const cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-  CUDA_CHECK(cudaMalloc(&d.indptr, sizeof(int64_t) * (n_rows + 1)));
-  CUDA_CHECK(cudaMalloc(&d.indices, sizeof(int32_t) * std::max<int64_t>(nnz, 1)));
-  CUDA_CHECK(cudaMalloc(&d.data, sizeof(float) * std::max<int64_t>(nnz, 1)));
-  CUDA_CHECK(cudaMemcpy(d.indptr, indptr, sizeof(int64_t) * (n_rows + 1), kind));
+  d.indptr.alloc(n_rows + 1);
+  d.indices.alloc(std::max<int64_t>(nnz, 1));
+  d.data.alloc(std::max<int64_t>(nnz, 1));
+  CUDA_CHECK(cudaMemcpy(d.indptr.get(), indptr, sizeof(int64_t) * (n_rows + 1), kind));
   if (nnz) {
-    CUDA_CHECK(cudaMemcpy(d.indices, indices, sizeof(int32_t) * nnz, kind));
-    CUDA_CHECK(cudaMemcpy(d.data, data, sizeof(float) * nnz, kind));
+    CUDA_CHECK(cudaMemcpy(d.indices.get(), indices, sizeof(int32_t) * nnz, kind));
+    CUDA_CHECK(cudaMemcpy(d.data.get(), data, sizeof(float) * nnz, kind));
   }
 }
 
@@ -324,9 +170,9 @@ bool gram_use_tensor_cores(const ials_trainer *t) { return t->ld == 128 && t->gw
 
 void gram_rows(ials_trainer *t, int src, int64_t begin, int64_t end, float *dst) {
   if (gram_use_tensor_cores(t))
-    launch_gram_tc(t->factor[src], begin, end, t->cfg.alpha0, t->gws, dst, t->stream);
+    launch_gram_tc(t->factor[src].get(), begin, end, t->cfg.alpha0, t->gws, dst, t->stream);
   else
-    launch_gram(t->factor[src], begin, end, t->ld, t->cfg.alpha0, t->gram_scratch, dst, t->stream);
+    launch_gram(t->factor[src].get(), begin, end, t->ld, t->cfg.alpha0, t->gram_scratch.get(), dst, t->stream);
 }
 
 // Phase timing: one event per mark; an epoch records kMarksPerEpoch marks
@@ -343,406 +189,69 @@ void prof_mark(ials_trainer *t) {
 void gram_side(ials_trainer *t, int solver_side) {
   // solver_side 0 (users) needs alpha0 * item^T item, and vice versa
   const int src = 1 - solver_side;
-  gram_rows(t, src, 0, t->n_rows(src), t->P[solver_side]);
+  gram_rows(t, src, 0, t->n_rows(src), t->P[solver_side].get());
 }
 
-SolveArgs make_args(ials_trainer *t, int side, float *target, const DeviceCsr &csr,
-                    const ials_solver_config *sc) {
-  SolveArgs a{};
-  a.target = target;
-  a.other = t->factor[1 - side];
-  a.P = t->P[side];
-  a.indptr = csr.indptr;
-  a.indices = csr.indices;
-  a.data = csr.data;
-  a.order = csr.order;
-  a.n_rows = csr.n_rows;
-  a.n_sched = csr.n_rows;
-  a.row_base = csr.row_base;
-  a.n_other = t->n_rows(1 - side);
-  a.K = t->K;
-  a.ld = t->ld;
-  a.alpha0 = t->cfg.alpha0;
-  a.reg = t->cfg.reg;
-  a.nu = t->cfg.nu;
-  a.bias = t->cfg.loss_type == IALS_LOSS_IALSPP ? 0.f : t->cfg.alpha0;  // IALSTrainer.hpp:190-191
-  a.max_cg_steps = sc->max_cg_steps == 0 ? t->K : (int)sc->max_cg_steps;  // :232-234
-  a.err_flags = t->err_flags;
-  a.work_counter = t->work_counter;
-  a.n_peers = 0;
-  return a;
-}
-
-// Solver::step_cholesky for 256-column factors with the rank updates (IALSTrainer.hpp:37-58,
-// 301-308) on the tensor cores.  Per chunk of <= chol_cap jobs one launch of wgram256_kernel
-// fills  W [JC][256][256] | b [JC][8][256]  (G = W + W^T) and the left-looking Cholesky
-// (cholesky_ll.cu) starts its block rows from P + G.  Rows without
-// interactions are left to the plain kernel (their solution is zero).  Returns false when the
-// route does not apply (negative stored values: the sqrt-weighted Gram does not exist).
-// jobs per chunk: the factorisation kernel runs 592 rows at a time, so a chunk of 4096 rows ends in a
-// seventh, half-empty wave (7 % of its time); 16384 jobs = 4.4 GB of workspace, fewer for smaller sides
-constexpr int64_t kCholJobCapMax = 16384;
-// Every row with interactions as a list of Gram jobs (<= IALS_HEAVY_JOB_LEN entries each), in the
-// degree-sorted order: the schedule of the routes that form the normal equations on the tensor cores.
-DeviceCsr &all_rows_plan(ials_trainer *t, const DeviceCsr &csr, int side, cudaStream_t s) {
-  DeviceCsr &plan = t->chol_plan[side];
-  if (!t->chol_plan_ready[side]) {
-    plan = csr;  // shares indptr / indices / data / order with the trainer's CSR
-    plan.job_begin = plan.job_end = nullptr;
-    plan.heavy_first_job = nullptr;
-    build_heavy_plan(plan, /*threshold=*/0, env_int("IALS_HEAVY_JOB_LEN", 4096), s);
-    t->chol_first[side].assign((size_t)plan.n_heavy + 1, 0);
-    if (plan.n_heavy > 0)
-      CUDA_CHECK(cudaMemcpy(t->chol_first[side].data(), plan.heavy_first_job,
-                            sizeof(int32_t) * (plan.n_heavy + 1), cudaMemcpyDeviceToHost));
-    t->chol_plan_ready[side] = true;
-  }
-  return plan;
-}
-
-bool solve_cholesky_tensor(ials_trainer *t, const SolveArgs &a, const DeviceCsr &csr, int side,
-                           cudaStream_t s) {
-  DeviceCsr &plan = all_rows_plan(t, csr, side, s);
-  if (plan.has_negative) return false;
-  const std::vector<int32_t> &first = t->chol_first[side];
-  const int64_t want = std::min<int64_t>(kCholJobCapMax, std::max<int64_t>(plan.n_jobs, 1));
-  if (want > t->chol_cap) {
-    if (t->chol_ws) CUDA_CHECK(cudaFree(t->chol_ws));
-    t->chol_ws = nullptr;
-    t->chol_cap = 0;
-    CUDA_CHECK(cudaMalloc(&t->chol_ws, sizeof(float) * (size_t)want * (256 * 256 + kWGram256BParts * 256)));
-    t->chol_cap = want;
-  }
-  const int kCholJobCap = (int)t->chol_cap;
-  const size_t blk = (size_t)kCholJobCap * 256 * 256;
-  if (t->chol_scratch == nullptr) {
-    CUDA_CHECK(cudaMalloc(&t->chol_scratch, cholesky_ll_scratch_bytes()));
-    CUDA_CHECK(cudaMemsetAsync(t->chol_scratch, 0, cholesky_ll_scratch_bytes(), s));  // the padding words stay finite
-  }
-  float *ws = t->chol_ws;
-  for (int64_t h0 = 0; h0 < plan.n_heavy;) {
-    int64_t h1 = h0 + 1;  // at least one row (a row has at most max_degree / job_len + 1 jobs)
-    while (h1 < plan.n_heavy && first[h1 + 1] - first[h0] <= kCholJobCap) h1++;
-    const int j0 = first[h0], nj = first[h1] - first[h0];
-    if (nj > kCholJobCap) throw NotImplemented("Cholesky on tensor cores: a row with more jobs than the workspace holds");
-    WGramArgs w{};
-    w.ld = a.ld;
-    w.indices = plan.indices;
-    w.weights = plan.data;
-    w.job_begin = plan.job_begin + j0;
-    w.job_end = plan.job_end + j0;
-    w.n_jobs = nj;
-    w.bias = a.bias;
-    w.Y = a.other;
-    w.W = ws;
-    w.bpart = ws + blk;
-    launch_wgram256(w, s);
-    SolveArgs g = a;
-    g.order = plan.order + h0;
-    g.n_sched = h1 - h0;
-    launch_solve_cholesky_from_gram(g, plan.heavy_first_job + h0, j0, kCholJobCap, ws, t->chol_scratch, s);
-    h0 = h1;
-  }
-  if (plan.n_heavy < a.n_sched) {  // rows without interactions: A = P + reg I, b = 0
-    SolveArgs rest = a;
-    rest.order = plan.order + plan.n_heavy;
-    rest.n_sched = a.n_sched - plan.n_heavy;
-    launch_solve_cholesky_tile(rest, s);
-  }
-  return true;
-}
-
-// Solver::step_ialspp (IALSTrainer.hpp:387-535) for 128-column factors: per chunk of <= gs_cap jobs
-// one wgram_kernel launch forms G = sum c y y^T and b of every row of the chunk on the tensor cores
-// (one pass over the neighbours), ialspp_dense_kernel runs the block Gauss-Seidel sweeps on
-// A = P + G + reg I (ialspp_dense.cu has the algebra).  Returns false when the route does not apply.
-bool solve_ialspp_tensor(ials_trainer *t, const SolveArgs &a, const DeviceCsr &csr, int side, int S, int iters,
-                         cudaStream_t s) {
-  if (!ialspp_dense_supported(a, S)) return false;
-  DeviceCsr &plan = all_rows_plan(t, csr, side, s);
-  if (plan.has_negative) return false;
-  const std::vector<int32_t> &first = t->chol_first[side];
-  // jobs per chunk (64 KB of W per job): 4096 measured 46.5 ms per ML-20M epoch against 58.5 with
-  // 1024 (whose W round trip stays inside the L2, but whose launches end in half-empty waves) and
-  // 46.5 with 16384 (r02al / r02am)
-  const int64_t cap = 4096;
-  if (cap != t->gs_cap) {
-    if (t->gs_ws) CUDA_CHECK(cudaFree(t->gs_ws));
-    t->gs_ws = nullptr;
-    t->gs_cap = 0;
-    CUDA_CHECK(cudaMalloc(&t->gs_ws, sizeof(float) * (size_t)cap * (128 * 128 + kWGramBParts * 128)));
-    t->gs_cap = cap;
-  }
-  float *W = t->gs_ws, *bpart = t->gs_ws + (size_t)cap * 128 * 128;
-  DenseSolveArgs d{};
-  d.base = a;
-  d.W = W;
-  d.bpart = bpart;
-  for (int64_t h0 = 0; h0 < plan.n_heavy;) {
-    int64_t h1 = h0 + 1;
-    while (h1 < plan.n_heavy && first[h1 + 1] - first[h0] <= cap) h1++;
-    const int j0 = first[h0], nj = first[h1] - first[h0];
-    if (nj > cap) throw NotImplemented("iALS++ on tensor cores: a row with more jobs than the workspace holds");
-    WGramArgs w{};
-    w.Y = a.other;
-    w.ld = a.ld;
-    w.indices = plan.indices;
-    w.weights = plan.data;
-    w.job_begin = plan.job_begin + j0;
-    w.job_end = plan.job_end + j0;
-    w.n_jobs = nj;
-    w.bias = a.bias;
-    w.W = W;
-    w.bpart = bpart;
-    launch_wgram(w, s);
-    d.base.order = plan.order + h0;
-    d.n_heavy = h1 - h0;
-    d.heavy_first_job = plan.heavy_first_job + h0;
-    d.job0 = j0;
-    launch_ialspp_dense(d, S, iters, s);
-    h0 = h1;
-  }
-  if (plan.n_heavy < a.n_sched) {  // rows without interactions: A = P + reg I, b = 0
-    d.base.order = plan.order + plan.n_heavy;
-    d.n_heavy = a.n_sched - plan.n_heavy;
-    d.heavy_first_job = nullptr;
-    d.job0 = 0;
-    launch_ialspp_dense(d, S, iters, s);
-  }
-  return true;
-}
-
-void run_solver(ials_trainer *t, const SolveArgs &a, const DeviceCsr &csr,
-                const ials_solver_config *sc, cudaStream_t s) {
-  if (a.n_sched == 0) {
-    prof_mark(t);
-    prof_mark(t);
-    prof_mark(t);
-    return;
-  }
-  if (a.prior != nullptr) {
-    // feature-aware rows (step_cg with a prior / step_cholesky_with_prior, :170-271, :333-385):
-    // the generic kernels, which take the prior
-    prof_mark(t);
-    prof_mark(t);
-    if (sc->solver_type == IALS_SOLVER_CG) {
-      launch_solve_cg_simple(a, s);
-    } else if (sc->solver_type == IALS_SOLVER_CHOLESKY) {
-      if (!cholesky_tile_supported(a)) throw NotImplemented("Cholesky solver: n_components > 256 not supported");
-      launch_solve_cholesky_tile(a, s);
-    } else {
-      throw InvalidArgument("Feature-aware iALS does not support IALSPP.");  // :660-662
-    }
-    prof_mark(t);
-    return;
-  }
-  if (sc->solver_type == IALS_SOLVER_IALSPP) {  // Solver::step_ialspp, IALSTrainer.hpp:520-535
-    prof_mark(t);
-    prof_mark(t);
-    const int64_t S = std::min<int64_t>(sc->ialspp_subspace_dimension, a.K);
-    if (!ialspp_block_supported((int)S))
-      throw NotImplemented("iALS++: subspace blocks of more than 256 dimensions are not supported");
-    // 128-column factors, blocks of <= 64 dimensions, the trainer's own matrix: Gram on the tensor
-    // cores + block Gauss-Seidel; the per-block SIMT kernels below keep the other cases (wider
-    // factors or blocks, fold-in matrices, negative stored values).  r02aj A/B on a quarter of
-    // ML-20M: 139.4 ms per epoch below, 24.5 ms here (now 6.5).
-    if ((&csr == &t->X || &csr == &t->Xt) &&
-        solve_ialspp_tensor(t, a, csr, &csr == &t->X ? 0 : 1, (int)S, (int)sc->ialspp_iteration, s)) {
-      prof_mark(t);
-      return;
-    }
-    float *pred = nullptr;
-    CUDA_CHECK(cudaMallocAsync(&pred, sizeof(float) * std::max<int64_t>(csr.nnz, 1), s));
-    try {
-      for (int64_t iter = 0; iter < sc->ialspp_iteration; iter++) {
-        launch_ialspp_predict(a, pred, s);
-        for (int64_t d0 = 0; d0 < a.K; d0 += S)
-          launch_ialspp_block(a, pred, (int)d0, (int)std::min<int64_t>(S, a.K - d0), s);
-      }
-    } catch (...) {
-      cudaFreeAsync(pred, s);
-      throw;
-    }
-    CUDA_CHECK(cudaFreeAsync(pred, s));
-    prof_mark(t);
-    return;
-  }
-  if (sc->solver_type != IALS_SOLVER_CG) {
-    prof_mark(t);
-    prof_mark(t);
-    // 256-column factors: rank updates on the tensor cores + left-looking factorisation
-    // (IALS_CHOL=simt keeps the register-tiled SIMT kernel, for A/B runs)
-    static const bool tensor_chol = [] {
-      const char *e = std::getenv("IALS_CHOL");
-      return e == nullptr || std::string(e) != "simt";
-    }();
-    if (tensor_chol && a.ld == 256 && (&csr == &t->X || &csr == &t->Xt) &&
-        solve_cholesky_tensor(t, a, csr, &csr == &t->X ? 0 : 1, s)) {
-      prof_mark(t);
-      return;
-    }
-    if (!cholesky_tile_supported(a)) throw NotImplemented("Cholesky solver: n_components > 256 not supported");
-    launch_solve_cholesky_tile(a, s);
-    prof_mark(t);
-    return;
-  }
-  if (a.ld != 128) {  // ranks above 128: the generic warp-per-row kernel
-    prof_mark(t);
-    prof_mark(t);
-    launch_solve_cg_simple(a, s);
-    prof_mark(t);
-    return;
-  }
-  const int64_t n_heavy = (csr.n_heavy > 0 && !csr.has_negative) ? csr.n_heavy : 0;
-  auto run_heavy = [&] {
-    if (n_heavy == 0) {
-      prof_mark(t);
-      prof_mark(t);
-      return;
-    }
-    // heavy rows: tensor-core Gram of the gathered neighbours + dense CG
-    if (csr.n_jobs > t->heavy_jobs_cap) {
-      if (t->heavy_W) CUDA_CHECK(cudaFree(t->heavy_W));
-      if (t->heavy_b) CUDA_CHECK(cudaFree(t->heavy_b));
-      t->heavy_W = t->heavy_b = nullptr;
-      t->heavy_jobs_cap = 0;
-      CUDA_CHECK(cudaMalloc(&t->heavy_W, sizeof(float) * (size_t)csr.n_jobs * 128 * 128));
-      CUDA_CHECK(cudaMalloc(&t->heavy_b, sizeof(float) * (size_t)csr.n_jobs * kWGramBParts * 128));
-      t->heavy_jobs_cap = csr.n_jobs;
-    }
-    WGramArgs w{};
-    w.Y = a.other;
-    w.ld = a.ld;
-    w.indices = csr.indices;
-    w.weights = csr.data;
-    w.job_begin = csr.job_begin;
-    w.job_end = csr.job_end;
-    w.n_jobs = csr.n_jobs;
-    w.bias = a.bias;
-    w.W = t->heavy_W;
-    w.bpart = t->heavy_b;
-    DenseSolveArgs d{};
-    d.base = a;
-    d.n_heavy = csr.n_heavy;
-    d.heavy_first_job = csr.heavy_first_job;
-    d.W = t->heavy_W;
-    d.bpart = t->heavy_b;
-    launch_wgram(w, s);
-    prof_mark(t);
-    launch_dense_cg(d, s);
-    prof_mark(t);
-  };
-  auto run_light = [&] {
-    SolveArgs light = a;  // everything else (all rows when a stored value is negative)
-    light.order = csr.order + n_heavy;
-    light.n_sched = csr.n_rows - n_heavy;
-    // rows whose warm starts are still arriving (step_io) are taken in arrival order
-    if (a.ready_flags != nullptr && t->order_io != nullptr && &csr == &t->X) light.order = t->order_io;
-    launch_solve_cg_rows(light, s);
-    prof_mark(t);
-  };
-  if (a.ready_flags != nullptr) {
-    // the few heavy rows sit in arbitrary chunks of the upload: after the light rows every chunk
-    // is there (the phase marks keep their count, not their labels, in this order)
-    run_light();
-    run_heavy();
-  } else {
-    run_heavy();
-    run_light();
+void sync_and_check(ials_trainer *t) {
+  if (t->ready_pending && t->copy_stream) CUDA_CHECK(cudaStreamSynchronize(t->copy_stream));  // an upload nobody consumed
+  int flags[kNumErrFlags];
+  CUDA_CHECK(cudaMemcpyAsync(flags, t->err_flags.get(), sizeof(flags), cudaMemcpyDeviceToHost, t->stream));
+  CUDA_CHECK(cudaStreamSynchronize(t->stream));
+  if (flags[kErrCgSingular] || flags[kErrCholDecomp] || flags[kErrCholSolve] || flags[kErrInternal] ||
+      flags[kErrFeatureLlt] || flags[kErrFeatureSolve]) {
+    CUDA_CHECK(cudaMemsetAsync(t->err_flags.get(), 0, sizeof(flags), t->stream));
+    // messages of IALSTrainer.hpp:252-253, 318, 322
+    if (flags[kErrInternal]) throw std::runtime_error("internal error: a row was scheduled on a kernel that cannot hold it");
+    if (flags[kErrFeatureLlt]) throw std::runtime_error("Feature ridge Cholesky decomposition failed.");  // :1107
+    if (flags[kErrFeatureSolve]) throw std::runtime_error("Feature ridge solve failed.");                  // :1171
+    if (flags[kErrCgSingular]) throw std::runtime_error("Conjugate-gradient solver encountered a singular system.");
+    if (flags[kErrCholDecomp]) throw std::runtime_error("Cholesky decomposition failed.");
+    throw std::runtime_error("Cholesky solve failed.");
   }
 }
 
-
-// ---------------- feature-aware iALS (IALSTrainer.hpp:634-662, 758-789, 1001-1209) ----------------
-
-// host features -> device (dense row-major when indptr == nullptr, else CSR); `owner` keeps the arrays
-void upload_features(ials_trainer::FeatureSide &owner, int64_t n_rows, int64_t n_cols, const float *dense,
-                     const int64_t *indptr, const int32_t *indices, const float *data) {
-  owner.free_features();
-  FeatureDev &F = owner.F;
-  F.n_rows = n_rows;
-  F.n_cols = n_cols;
-  if (indptr == nullptr) {
-    require(dense != nullptr || n_rows * n_cols == 0, "feature matrix is null");
-    CUDA_CHECK(cudaMalloc(&owner.d_dense, sizeof(float) * std::max<int64_t>(n_rows * n_cols, 1)));
-    if (n_rows * n_cols)
-      CUDA_CHECK(cudaMemcpy(owner.d_dense, dense, sizeof(float) * n_rows * n_cols, cudaMemcpyHostToDevice));
-    F.dense = owner.d_dense;
-    return;
+// Fold-in (Solver::X_to_vector, IALSTrainer.hpp:123-140, :791-801): solves the rows of the host CSR
+// (side 0) or of its transpose (side 1) against the trainer's other factor matrix, starting from zero.
+// stage_prior (X_to_vector_with_prior, :142-167) is given the planned CSR of the new rows and returns
+// device rows [n_new x ld] that the solve starts from and is regularised towards.
+void fold_in(ials_trainer *t, int side, int64_t n_rows, int64_t n_cols, const int64_t *indptr,
+             const int32_t *indices, const float *data, const ials_solver_config *solver, float *out_host,
+             const std::function<const float *(const DeviceCsr &)> &stage_prior) {
+  DeviceCsr given, transposed;
+  DeviceBuffer<float> target;
+  StreamSyncOnExit sync{t->stream};
+  upload_csr(given, n_rows, n_cols, indptr, indices, data);
+  if (side == 1) build_transpose(given, transposed, t->stream);  // X.transpose(), :800
+  DeviceCsr &csr = side == 1 ? transposed : given;
+  plan_csr(t, csr);
+  const int64_t n_new = csr.n_rows;
+  const float *prior = stage_prior ? stage_prior(csr) : nullptr;
+  const size_t bytes = sizeof(float) * std::max<int64_t>(n_new * t->ld, 1);
+  target.alloc(std::max<int64_t>(n_new * t->ld, 1));
+  if (prior)
+    CUDA_CHECK(cudaMemcpyAsync(target.get(), prior, bytes, cudaMemcpyDeviceToDevice, t->stream));  // result = prior, :156
+  else
+    CUDA_CHECK(cudaMemsetAsync(target.get(), 0, bytes, t->stream));  // DenseMatrix::Zero, :132
+  gram_side(t, side);  // prepare_p, :793 / :799
+  SolveArgs a = make_args(t, side, target.get(), csr, solver);
+  a.prior = prior;
+  run_solver(t, a, csr, solver, t->stream);
+  if (n_new) {
+    require(out_host != nullptr, "out is null");
+    rows_to_host(out_host, t->K, target.get(), t->ld, n_new, t->stream);
   }
-  require(indptr[0] == 0, "feature indptr must start at 0");
-  const int64_t nnz = indptr[n_rows];
-  require(nnz == 0 || (indices != nullptr && data != nullptr), "feature indices / data are null");
-  for (int64_t j = 0; j < nnz; j++) require(indices[j] >= 0 && indices[j] < n_cols, "feature column out of range");
-  CUDA_CHECK(cudaMalloc(&owner.d_indptr, sizeof(int64_t) * (n_rows + 1)));
-  CUDA_CHECK(cudaMalloc(&owner.d_indices, sizeof(int32_t) * std::max<int64_t>(nnz, 1)));
-  CUDA_CHECK(cudaMalloc(&owner.d_data, sizeof(float) * std::max<int64_t>(nnz, 1)));
-  CUDA_CHECK(cudaMemcpy(owner.d_indptr, indptr, sizeof(int64_t) * (n_rows + 1), cudaMemcpyHostToDevice));
-  if (nnz) {
-    CUDA_CHECK(cudaMemcpy(owner.d_indices, indices, sizeof(int32_t) * nnz, cudaMemcpyHostToDevice));
-    CUDA_CHECK(cudaMemcpy(owner.d_data, data, sizeof(float) * nnz, cudaMemcpyHostToDevice));
-  }
-  F.nnz = nnz;
-  F.indptr = owner.d_indptr;
-  F.indices = owner.d_indices;
-  F.data = owner.d_data;
+  sync_and_check(t);
 }
 
-const char *side_name(int side) { return side == 0 ? "user" : "item"; }
-const char *side_Name(int side) { return side == 0 ? "User" : "Item"; }
+}  // namespace ials
 
-// validate_user_feature_matrix / validate_item_feature_matrix (:1016-1042)
-void validate_feature_cols(const ials_trainer *t, int side, int64_t cols) {
-  const ials_trainer::FeatureSide &f = t->feat[side];
-  if (!f.weight_set) throw InvalidArgument(std::string(side_Name(side)) + " feature weights are not initialized.");
-  if (cols != f.n_w)
-    throw InvalidArgument(std::string("Shape mismatch: ") + side_name(side) + " feature matrix has " +
-                          std::to_string(cols) + " columns but " + side_name(side) + "_feature_weight has " +
-                          std::to_string(f.n_w) + " rows.");
-}
+namespace {
 
-// step_with_prior's guard (:639-652): with alpha0 = 0 and a vanishing ridge an empty row has no
-// unique solution
-void check_prior_defined(const ials_trainer *t, int side, bool has_empty_row) {
-  if (t->cfg.alpha0 != 0.f) return;
-  const float r0 = t->cfg.reg * std::pow(t->cfg.alpha0 * (float)t->n_rows(1 - side) + 0.f, t->cfg.nu);
-  if ((!(r0 > 0.f) || !std::isfinite(r0)) && has_empty_row)
-    throw InvalidArgument("Feature-prior embedding is not uniquely defined for an empty interaction row when "
-                          "alpha0 and its regularization are zero.");
-}
-
-bool side_uses_features(const ials_trainer *t, int side) {
-  return t->feature_aware && t->epoch >= t->feature_warmup && t->feat[side].n_w > 0;
-}
-
-// stored_user_feature_prior / stored_item_feature_prior (:1044-1050) into feat[side].prior
-const float *stored_prior(ials_trainer *t, int side) {
-  ials_trainer::FeatureSide &f = t->feat[side];
-  const int64_t n = t->n_rows(side);
-  if (f.prior == nullptr) CUDA_CHECK(cudaMalloc(&f.prior, sizeof(float) * std::max<int64_t>(n * t->ld, 1)));
-  launch_feature_prior(f.F, f.weight, t->ld, f.prior, t->stream);
-  return f.prior;
-}
-
-// update_stored_*_feature_weight -> update_feature_weight (:1052-1064, 1182-1209)
-void update_feature_weight(ials_trainer *t, int side) {
-  ials_trainer::FeatureSide &f = t->feat[side];
-  if (f.n_w == 0) return;
-  const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
-  const int64_t n = t->n_rows(side);
-  if (!f.cache_ready) {  // initialize_feature_weight_cache (:1083-1132): once per trainer
-    if (f.rw == nullptr) CUDA_CHECK(cudaMalloc(&f.rw, sizeof(float) * std::max<int64_t>(n, 1)));
-    if (f.llt == nullptr) CUDA_CHECK(cudaMalloc(&f.llt, sizeof(float) * f.n_w * f.n_w));
-    if (f.rhs == nullptr) CUDA_CHECK(cudaMalloc(&f.rhs, sizeof(float) * f.n_w * t->ld));
-    launch_feature_row_weights(csr.indptr, n, t->n_rows(1 - side), t->cfg.alpha0, t->cfg.reg, t->cfg.nu, f.rw,
-                               t->stream);
-    launch_feature_gram_llt(f.F, f.rw, f.lambda, f.llt, t->err_flags + kErrFeatureLlt, t->stream);
-    f.cache_ready = true;
-  }
-  // solve_feature_weight (:1134-1180); the solution replaces the weight
-  launch_feature_ridge_solve(f.F, f.rw, t->factor[side], t->ld, f.llt, f.rhs, t->err_flags + kErrFeatureSolve,
-                             t->stream);
-  CUDA_CHECK(cudaMemcpyAsync(f.weight, f.rhs, sizeof(float) * f.n_w * t->ld, cudaMemcpyDeviceToDevice, t->stream));
+void finish_csr(ials_trainer *t) {
+  build_transpose(t->X, t->Xt, t->stream);
+  plan_csr(t, t->X);
+  plan_csr(t, t->Xt);
+  t->has_X = true;
 }
 
 // One half-epoch of IALSTrainer::step (:758-789) on the trainer's own matrices: Gram, solve
@@ -751,7 +260,7 @@ void epoch_side(ials_trainer *t, int side, const ials_solver_config *sc, SolveAr
   gram_side(t, side);
   prof_mark(t);
   const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
-  SolveArgs a = io_args ? *io_args : make_args(t, side, t->factor[side], csr, sc);
+  SolveArgs a = io_args ? *io_args : make_args(t, side, t->factor[side].get(), csr, sc);
   const bool with_features = side_uses_features(t, side);
   if (with_features) {
     check_prior_defined(t, side, t->feat[side].has_empty_row);
@@ -759,90 +268,6 @@ void epoch_side(ials_trainer *t, int side, const ials_solver_config *sc, SolveAr
   }
   run_solver(t, a, csr, sc, t->stream);  // records three marks
   if (with_features) update_feature_weight(t, side);
-}
-
-void check_feature_solver(const ials_trainer *t, const ials_solver_config *sc) {
-  if (t->feature_aware && sc->solver_type == IALS_SOLVER_IALSPP)
-    throw InvalidArgument("Feature-aware iALS does not support IALSPP.");  // :759-761
-}
-
-
-constexpr int kReadyShift = 12;  // 4096 rows = 2 MB per chunk of a flagged upload
-
-void ensure_copy_stream(ials_trainer *t) {
-  if (t->copy_stream == nullptr) {
-    CUDA_CHECK(cudaStreamCreateWithFlags(&t->copy_stream, cudaStreamNonBlocking));
-    CUDA_CHECK(cudaEventCreateWithFlags(&t->users_done, cudaEventDisableTiming));
-    CUDA_CHECK(cudaEventCreateWithFlags(&t->upload_done, cudaEventDisableTiming));
-  }
-}
-
-// The user rows [row_begin, row_begin + n_rows) (the whole matrix, or this rank's shard) arrive from
-// the host in chunks on the copy stream WHILE the user half-epoch runs: a 4-byte copy behind every
-// chunk raises its flag (the copy engine does; a flag KERNEL found no SM to run on -- cg_rows_kernel
-// holds every register of every SM while its warps wait for exactly that flag: r02t, 1.7 s per
-// step), a row waits for its chunk before it reads its warm start (and therefore also before it
-// writes its solution, which a late chunk would overwrite), and the light rows are taken in
-// (arrival chunk, descending degree) order -- in the degree-sorted order every warp blocked on a
-// row of a late chunk (r02u).  Only the CG kernels of the 128-column layout wait for flags; any
-// other solve first waits for upload_done.
-void enqueue_flagged_user_upload(ials_trainer *t, int64_t row_begin, int64_t n_rows, const float *rows_host) {
-  ensure_copy_stream(t);
-  const size_t hp = sizeof(float) * t->K, dp = sizeof(float) * t->ld;
-  const int n_chunks = (int)((n_rows + (1ll << kReadyShift) - 1) >> kReadyShift);
-  if (n_chunks > t->ready_cap) {
-    if (t->ready_flags) CUDA_CHECK(cudaFree(t->ready_flags));
-    if (t->ready_host) CUDA_CHECK(cudaFreeHost(t->ready_host));
-    t->ready_flags = t->ready_host = nullptr;
-    CUDA_CHECK(cudaMalloc(&t->ready_flags, sizeof(int) * n_chunks));
-    CUDA_CHECK(cudaHostAlloc(&t->ready_host, sizeof(int) * n_chunks, cudaHostAllocDefault));
-    CUDA_CHECK(cudaMemsetAsync(t->ready_flags, 0, sizeof(int) * n_chunks, t->stream));
-    t->ready_cap = n_chunks;
-    t->ready_token = 0;
-  }
-  if (t->order_io == nullptr) {  // once: the light rows by (chunk of the upload, descending degree)
-    const DeviceCsr &X = t->X;
-    const int64_t nh = (X.n_heavy > 0 && !X.has_negative) ? X.n_heavy : 0, nl = X.n_rows - nh;
-    std::vector<int32_t> ord((size_t)std::max<int64_t>(nl, 1));
-    if (nl) CUDA_CHECK(cudaMemcpyAsync(ord.data(), X.order + nh, sizeof(int32_t) * nl, cudaMemcpyDeviceToHost, t->stream));
-    CUDA_CHECK(cudaStreamSynchronize(t->stream));
-    ord.resize((size_t)nl);
-    // X.order is by descending degree: a stable sort by chunk keeps that order inside a chunk
-    // (CSR row u is factor row X.row_base + u, and the upload starts at X.row_base)
-    std::stable_sort(ord.begin(), ord.end(),
-                     [&](int32_t x, int32_t y) { return (x >> kReadyShift) < (y >> kReadyShift); });
-    CUDA_CHECK(cudaMalloc(&t->order_io, sizeof(int32_t) * std::max<int64_t>(nl, 1)));
-    if (nl) CUDA_CHECK(cudaMemcpy(t->order_io, ord.data(), sizeof(int32_t) * nl, cudaMemcpyHostToDevice));
-  }
-  t->ready_token++;  // never 0; a stale flag of an earlier step never matches
-  // the flags' reset (first use) and every kernel enqueued so far precede the copies
-  CUDA_CHECK(cudaEventRecord(t->users_done, t->stream));
-  CUDA_CHECK(cudaStreamWaitEvent(t->copy_stream, t->users_done, 0));
-  for (int c = 0; c < n_chunks; c++) {
-    const int64_t r0 = (int64_t)c << kReadyShift, nr = std::min<int64_t>(1ll << kReadyShift, n_rows - r0);
-    CUDA_CHECK(cudaMemcpy2DAsync(t->factor[0] + (row_begin + r0) * t->ld, dp, rows_host + r0 * t->K, hp, hp, nr,
-                                 cudaMemcpyHostToDevice, t->copy_stream));
-    t->ready_host[c] = t->ready_token;
-    CUDA_CHECK(cudaMemcpyAsync(t->ready_flags + c, t->ready_host + c, sizeof(int), cudaMemcpyHostToDevice,
-                               t->copy_stream));
-  }
-  CUDA_CHECK(cudaEventRecord(t->upload_done, t->copy_stream));
-  t->ready_pending = true;
-}
-
-// Give the pending flagged upload to the user solve `a` (if its kernels can wait for flags), or make
-// the stream wait for the whole upload.
-void consume_flagged_upload(ials_trainer *t, const ials_solver_config *sc, SolveArgs &a, int64_t row_begin) {
-  if (!t->ready_pending) return;
-  t->ready_pending = false;
-  if (sc->solver_type == IALS_SOLVER_CG && t->ld == 128 && a.prior == nullptr) {
-    a.ready_flags = t->ready_flags;
-    a.ready_token = t->ready_token;
-    a.ready_shift = kReadyShift;
-    a.ready_base = row_begin;
-  } else {
-    CUDA_CHECK(cudaStreamWaitEvent(t->stream, t->upload_done, 0));
-  }
 }
 
 void half_step(ials_trainer *t, int side, const ials_solver_config *sc) {
@@ -856,35 +281,6 @@ void half_step(ials_trainer *t, int side, const ials_solver_config *sc) {
   if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix; it cannot train");
   check_feature_solver(t, sc);
   epoch_side(t, side, sc);  // (a test entry: the epoch counter is not advanced)
-}
-
-void sync_and_check(ials_trainer *t) {
-  if (t->ready_pending && t->copy_stream) CUDA_CHECK(cudaStreamSynchronize(t->copy_stream));  // an upload nobody consumed
-  int flags[kNumErrFlags];
-  CUDA_CHECK(cudaMemcpyAsync(flags, t->err_flags, sizeof(flags), cudaMemcpyDeviceToHost, t->stream));
-  CUDA_CHECK(cudaStreamSynchronize(t->stream));
-  if (flags[kErrCgSingular] || flags[kErrCholDecomp] || flags[kErrCholSolve] || flags[kErrInternal] ||
-      flags[kErrFeatureLlt] || flags[kErrFeatureSolve]) {
-    CUDA_CHECK(cudaMemsetAsync(t->err_flags, 0, sizeof(flags), t->stream));
-    // messages of IALSTrainer.hpp:252-253, 318, 322
-    if (flags[kErrInternal]) throw std::runtime_error("internal error: a row was scheduled on a kernel that cannot hold it");
-    if (flags[kErrFeatureLlt]) throw std::runtime_error("Feature ridge Cholesky decomposition failed.");  // :1107
-    if (flags[kErrFeatureSolve]) throw std::runtime_error("Feature ridge solve failed.");                  // :1171
-    if (flags[kErrCgSingular]) throw std::runtime_error("Conjugate-gradient solver encountered a singular system.");
-    if (flags[kErrCholDecomp]) throw std::runtime_error("Cholesky decomposition failed.");
-    throw std::runtime_error("Cholesky solve failed.");
-  }
-}
-
-float *ensure_score_buf(ials_trainer *t, size_t bytes) {
-  if (bytes > t->score_buf_bytes) {
-    if (t->score_buf) CUDA_CHECK(cudaFree(t->score_buf));
-    t->score_buf = nullptr;
-    t->score_buf_bytes = 0;
-    CUDA_CHECK(cudaMalloc(&t->score_buf, bytes));
-    t->score_buf_bytes = bytes;
-  }
-  return t->score_buf;
 }
 
 }  // namespace
@@ -908,18 +304,13 @@ int ials_trainer_create(const ials_model_config *config, int64_t n_users, int64_
   return guarded([&] {
     require(out != nullptr, "out is null");
     *out = nullptr;
-    ials_trainer *t = new_trainer(config, n_users, n_items, device);
-    try {
-      DeviceGuard g(device);
-      alloc_common(t);
-      upload_csr(t->X, n_users, n_items, indptr, indices, data);
-      finish_csr(t);
-      init_factors_host_rng(t);
-    } catch (...) {
-      ials_trainer_destroy(t);
-      throw;
-    }
-    *out = t;
+    TrainerPtr t = new_trainer(config, n_users, n_items, device);
+    DeviceGuard g(device);
+    alloc_common(t.get());
+    upload_csr(t->X, n_users, n_items, indptr, indices, data);
+    finish_csr(t.get());
+    init_factors(t.get(), false);
+    *out = t.release();
   });
 }
 
@@ -930,29 +321,13 @@ int ials_trainer_create_from_device_csr(const ials_model_config *config, int64_t
   return guarded([&] {
     require(out != nullptr, "out is null");
     *out = nullptr;
-    ials_trainer *t = new_trainer(config, n_users, n_items, device);
-    try {
-      DeviceGuard g(device);
-      alloc_common(t);
-      upload_csr(t->X, n_users, n_items, d_indptr, d_indices, d_data, /*on_device=*/true);
-      finish_csr(t);
-      if (init_on_device) {
-        if (t->cfg.init_stdev > 0) {
-          const float sd = (float)(t->cfg.init_stdev / std::sqrt((double)t->K));
-          // same seed for both matrices, like the reference's two fresh generators
-          for (int side = 0; side < 2; side++)
-            launch_init_normal(t->factor[side], t->n_rows(side), t->K, t->ld, sd,
-                               (uint64_t)(uint32_t)t->cfg.random_seed, t->stream);
-          CUDA_CHECK(cudaStreamSynchronize(t->stream));
-        }
-      } else {
-        init_factors_host_rng(t);
-      }
-    } catch (...) {
-      ials_trainer_destroy(t);
-      throw;
-    }
-    *out = t;
+    TrainerPtr t = new_trainer(config, n_users, n_items, device);
+    DeviceGuard g(device);
+    alloc_common(t.get());
+    upload_csr(t->X, n_users, n_items, d_indptr, d_indices, d_data, /*on_device=*/true);
+    finish_csr(t.get());
+    init_factors(t.get(), init_on_device != 0);
+    *out = t.release();
   });
 }
 
@@ -962,26 +337,18 @@ int ials_trainer_create_from_factors(const ials_model_config *config, int64_t n_
   return guarded([&] {
     require(out != nullptr, "out is null");
     *out = nullptr;
-    ials_trainer *t = new_trainer(config, n_users, n_items, device);
-    try {
-      DeviceGuard g(device);
-      alloc_common(t);
-      require((n_users == 0 || user) && (n_items == 0 || item), "factor pointer is null");
-      const float *src[2] = {user, item};
-      for (int side = 0; side < 2; side++)
-        if (t->n_rows(side))
-          CUDA_CHECK(cudaMemcpy2D(t->factor[side], sizeof(float) * t->ld, src[side],
-                                  sizeof(float) * t->K, sizeof(float) * t->K, t->n_rows(side),
-                                  cudaMemcpyHostToDevice));
-      // the reference rebuilds both P matrices on unpickle (IALSTrainer.hpp:751-755)
-      gram_side(t, 0);
-      gram_side(t, 1);
-      CUDA_CHECK(cudaStreamSynchronize(t->stream));
-    } catch (...) {
-      ials_trainer_destroy(t);
-      throw;
-    }
-    *out = t;
+    TrainerPtr t = new_trainer(config, n_users, n_items, device);
+    DeviceGuard g(device);
+    alloc_common(t.get());
+    require((n_users == 0 || user) && (n_items == 0 || item), "factor pointer is null");
+    const float *src[2] = {user, item};
+    for (int side = 0; side < 2; side++)
+      if (t->n_rows(side)) rows_to_device(t->factor[side].get(), t->ld, src[side], t->K, t->n_rows(side));
+    // the reference rebuilds both P matrices on unpickle (IALSTrainer.hpp:751-755)
+    gram_side(t.get(), 0);
+    gram_side(t.get(), 1);
+    CUDA_CHECK(cudaStreamSynchronize(t->stream));
+    *out = t.release();
   });
 }
 
@@ -991,46 +358,16 @@ void ials_trainer_destroy(ials_trainer *t) {
   cudaGetDevice(&prev);
   cudaSetDevice(t->device);
   cudaDeviceSynchronize();
-  for (int side = 0; side < 2; side++) {
+  for (int side = 0; side < 2; side++)
     for (int p = 0; p < t->n_peers[side]; p++)
       if (t->peers[side][p]) cudaIpcCloseMemHandle(t->peers[side][p]);
-    if (t->factor[side]) cudaFree(t->factor[side]);
-    if (t->P[side]) cudaFree(t->P[side]);
-  }
-  t->X.free_all();
-  t->Xt.free_all();
-  if (t->gram_scratch) cudaFree(t->gram_scratch);
-  t->gws.free_all();
-  if (t->heavy_W) cudaFree(t->heavy_W);
-  if (t->heavy_b) cudaFree(t->heavy_b);
-  for (int side = 0; side < 2; side++) {  // the plans only own their job arrays
-    if (t->chol_plan[side].job_begin) cudaFree(t->chol_plan[side].job_begin);
-    if (t->chol_plan[side].job_end) cudaFree(t->chol_plan[side].job_end);
-    if (t->chol_plan[side].heavy_first_job) cudaFree(t->chol_plan[side].heavy_first_job);
-  }
-  if (t->chol_ws) cudaFree(t->chol_ws);
-  if (t->gs_ws) cudaFree(t->gs_ws);
-  if (t->chol_scratch) cudaFree(t->chol_scratch);
-  if (t->err_flags) cudaFree(t->err_flags);
-  if (t->work_counter) cudaFree(t->work_counter);
-  if (t->d_loss) cudaFree(t->d_loss);
-  if (t->score_buf) cudaFree(t->score_buf);
-  t->rec_idx.release(); t->rec_score.release(); t->rec_count.release();
-  t->rec_mindptr.release(); t->rec_mindices.release();
-  t->rec_aindptr.release(); t->rec_aindices.release();
-  t->rec_uidx.release(); t->rec_users.release(); t->rec_emb.release();
   for (auto e : t->prof_events) cudaEventDestroy(e);
   if (t->users_done) cudaEventDestroy(t->users_done);
   if (t->upload_done) cudaEventDestroy(t->upload_done);
   if (t->copy_stream) cudaStreamDestroy(t->copy_stream);
-  if (t->ready_flags) cudaFree(t->ready_flags);
-  t->feat[0].free_all();
-  t->feat[1].free_all();
-  if (t->ready_host) cudaFreeHost(t->ready_host);
-  if (t->order_io) cudaFree(t->order_io);
+  delete t;  // the buffers free themselves, with the trainer's device current
   cudaGetLastError();
   if (prev >= 0) cudaSetDevice(prev);
-  delete t;
 }
 
 int ials_trainer_set_stream(ials_trainer *t, void *cuda_stream) {
@@ -1083,13 +420,13 @@ int ials_trainer_get_timings(ials_trainer *t, double ms[8], int64_t *n_epochs) {
 int ials_trainer_plan_stats(ials_trainer *t, int side, int64_t out[8]) {
   return guarded([&] {
     require(t != nullptr && out != nullptr, "null argument");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     const DeviceCsr &c = side == 0 ? t->X : t->Xt;
     out[0] = c.n_rows;
     out[1] = c.nnz;
-    out[2] = c.n_heavy;
-    out[3] = c.nnz_heavy;
-    out[4] = c.n_jobs;
+    out[2] = c.heavy.n_heavy;
+    out[3] = c.heavy.nnz_heavy;
+    out[4] = c.heavy.n_jobs;
     out[5] = c.max_degree;
     out[6] = c.has_negative ? 1 : 0;
     out[7] = 0;
@@ -1123,9 +460,8 @@ int ials_trainer_step_io(ials_trainer *t, const ials_solver_config *solver, cons
     if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix; it cannot train");
     DeviceGuard g(t->device);
     ensure_copy_stream(t);
-    const size_t hp = sizeof(float) * t->K, dp = sizeof(float) * t->ld;
     // item first: the user half-epoch starts with Gram(item)
-    if (t->I) CUDA_CHECK(cudaMemcpy2DAsync(t->factor[1], dp, item_in, hp, hp, t->I, cudaMemcpyHostToDevice, t->stream));
+    if (t->I) rows_to_device(t->factor[1].get(), t->ld, item_in, t->K, t->I, t->stream);
     // the user factors are only the warm starts of the user rows: with the CG kernels of the
     // 128-column layout they arrive while the half-epoch runs (enqueue_flagged_user_upload)
     check_feature_solver(t, solver);
@@ -1134,12 +470,12 @@ int ials_trainer_step_io(ials_trainer *t, const ials_solver_config *solver, cons
     if (overlap_upload) {
       enqueue_flagged_user_upload(t, 0, t->U, user_in);
     } else if (t->U) {
-      CUDA_CHECK(cudaMemcpy2DAsync(t->factor[0], dp, user_in, hp, hp, t->U, cudaMemcpyHostToDevice, t->stream));
+      rows_to_device(t->factor[0].get(), t->ld, user_in, t->K, t->U, t->stream);
     }
     prof_mark(t);
     for (int side = 0; side < 2; side++) {  // IALSTrainer.hpp:784-787
       const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
-      SolveArgs a = make_args(t, side, t->factor[side], csr, solver);
+      SolveArgs a = make_args(t, side, t->factor[side].get(), csr, solver);
       if (side == 0) consume_flagged_upload(t, solver, a, 0);
       epoch_side(t, side, solver, &a);
       if (side == 1) t->epoch++;
@@ -1147,10 +483,10 @@ int ials_trainer_step_io(ials_trainer *t, const ials_solver_config *solver, cons
         // the new user factors are final: they travel back while the item half-epoch runs
         CUDA_CHECK(cudaEventRecord(t->users_done, t->stream));
         CUDA_CHECK(cudaStreamWaitEvent(t->copy_stream, t->users_done, 0));
-        CUDA_CHECK(cudaMemcpy2DAsync(user_out, hp, t->factor[0], dp, hp, t->U, cudaMemcpyDeviceToHost, t->copy_stream));
+        rows_to_host(user_out, t->K, t->factor[0].get(), t->ld, t->U, t->copy_stream);
       }
     }
-    if (t->I) CUDA_CHECK(cudaMemcpy2DAsync(item_out, hp, t->factor[1], dp, hp, t->I, cudaMemcpyDeviceToHost, t->stream));
+    if (t->I) rows_to_host(item_out, t->K, t->factor[1].get(), t->ld, t->I, t->stream);
     CUDA_CHECK(cudaStreamSynchronize(t->copy_stream));
     sync_and_check(t);
   });
@@ -1159,7 +495,7 @@ int ials_trainer_step_io(ials_trainer *t, const ials_solver_config *solver, cons
 int ials_trainer_half_step(ials_trainer *t, int side, const ials_solver_config *solver) {
   return guarded([&] {
     require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     check_solver(solver);
     DeviceGuard g(t->device);
     half_step(t, side, solver);
@@ -1170,57 +506,23 @@ int ials_trainer_half_step(ials_trainer *t, int side, const ials_solver_config *
 int ials_trainer_gram(ials_trainer *t, int side, float *out_host) {
   return guarded([&] {
     require(t != nullptr && out_host != nullptr, "null argument");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     DeviceGuard g(t->device);
     gram_side(t, side);
-    CUDA_CHECK(cudaMemcpy2DAsync(out_host, sizeof(float) * t->K, t->P[side], sizeof(float) * t->ld,
-                                 sizeof(float) * t->K, t->K, cudaMemcpyDeviceToHost, t->stream));
+    rows_to_host(out_host, t->K, t->P[side].get(), t->ld, t->K, t->stream);
     CUDA_CHECK(cudaStreamSynchronize(t->stream));
-  });
-}
-
-int ials_trainer_user_scores(ials_trainer *t, int64_t begin, int64_t end,
-                             const ials_solver_config *solver, float *out_host) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(solver != nullptr, "solver_config is null");
-    // IALSTrainer.hpp:944-951
-    require(solver->n_threads > 0, "n_threads must be strictly positive.");
-    require(end >= begin, "userblock_end must be greater than or equal to userblock_begin");
-    require(begin >= 0 && t->U >= end, "userblock_end must be smaller than or equal to n_users");
-    const int64_t rows = end - begin;
-    if (rows == 0 || t->I == 0) return;
-    require(out_host != nullptr, "out is null");
-    DeviceGuard g(t->device);
-    // bound the device staging buffer; large blocks are produced in slabs
-    const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 30) / (4 * t->I)));
-    float *buf = ensure_score_buf(t, sizeof(float) * slab * t->I);
-    for (int64_t b = 0; b < rows; b += slab) {
-      const int64_t m = std::min(slab, rows - b);
-      if (score_tc_supported(t->ld, 1))
-        launch_scores_tc(t->factor[0] + (begin + b) * t->ld, m, t->factor[1], t->I, t->ld, buf, t->I,
-                         t->stream);
-      else
-        launch_scores(t->factor[0] + (begin + b) * t->ld, m, t->factor[1], t->I, t->ld, buf, t->I,
-                      t->stream);
-      CUDA_CHECK(cudaMemcpyAsync(out_host + b * t->I, buf, sizeof(float) * m * t->I,
-                                 cudaMemcpyDeviceToHost, t->stream));
-      CUDA_CHECK(cudaStreamSynchronize(t->stream));
-    }
   });
 }
 
 int ials_trainer_get_factors(ials_trainer *t, int side, float *out_host) {
   return guarded([&] {
     require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     const int64_t n = t->n_rows(side);
     if (n == 0) return;
     require(out_host != nullptr, "out is null");
     DeviceGuard g(t->device);
-    CUDA_CHECK(cudaMemcpy2DAsync(out_host, sizeof(float) * t->K, t->factor[side],
-                                 sizeof(float) * t->ld, sizeof(float) * t->K, n,
-                                 cudaMemcpyDeviceToHost, t->stream));
+    rows_to_host(out_host, t->K, t->factor[side].get(), t->ld, n, t->stream);
     CUDA_CHECK(cudaStreamSynchronize(t->stream));
   });
 }
@@ -1228,14 +530,12 @@ int ials_trainer_get_factors(ials_trainer *t, int side, float *out_host) {
 int ials_trainer_set_factors(ials_trainer *t, int side, const float *in_host) {
   return guarded([&] {
     require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     const int64_t n = t->n_rows(side);
     if (n == 0) return;
     require(in_host != nullptr, "input is null");
     DeviceGuard g(t->device);
-    CUDA_CHECK(cudaMemcpy2DAsync(t->factor[side], sizeof(float) * t->ld, in_host,
-                                 sizeof(float) * t->K, sizeof(float) * t->K, n,
-                                 cudaMemcpyHostToDevice, t->stream));
+    rows_to_device(t->factor[side].get(), t->ld, in_host, t->K, n, t->stream);
     CUDA_CHECK(cudaStreamSynchronize(t->stream));
   });
 }
@@ -1244,14 +544,13 @@ int ials_trainer_set_factor_rows(ials_trainer *t, int side, int64_t row_begin, i
                                  const float *in_host, int push_to_peers) {
   return guarded([&] {
     require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     require(row_begin >= 0 && n_rows >= 0 && row_begin + n_rows <= t->n_rows(side), "row range out of bounds");
     if (n_rows == 0) return;
     require(in_host != nullptr, "input is null");
     DeviceGuard g(t->device);
-    float *dst = t->factor[side] + row_begin * t->ld;
-    CUDA_CHECK(cudaMemcpy2DAsync(dst, sizeof(float) * t->ld, in_host, sizeof(float) * t->K,
-                                 sizeof(float) * t->K, n_rows, cudaMemcpyHostToDevice, t->stream));
+    float *dst = t->factor[side].get() + row_begin * t->ld;
+    rows_to_device(dst, t->ld, in_host, t->K, n_rows, t->stream);
     if (push_to_peers)
       for (int p = 0; p < t->n_peers[side]; p++)
         CUDA_CHECK(cudaMemcpyAsync(t->peers[side][p] + row_begin * t->ld, dst, sizeof(float) * n_rows * t->ld,
@@ -1276,14 +575,12 @@ int ials_trainer_get_factor_rows(ials_trainer *t, int side, int64_t row_begin, i
                                  float *out_host) {
   return guarded([&] {
     require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     require(row_begin >= 0 && n_rows >= 0 && row_begin + n_rows <= t->n_rows(side), "row range out of bounds");
     if (n_rows == 0) return;
     require(out_host != nullptr, "out is null");
     DeviceGuard g(t->device);
-    CUDA_CHECK(cudaMemcpy2DAsync(out_host, sizeof(float) * t->K, t->factor[side] + row_begin * t->ld,
-                                 sizeof(float) * t->ld, sizeof(float) * t->K, n_rows,
-                                 cudaMemcpyDeviceToHost, t->stream));
+    rows_to_host(out_host, t->K, t->factor[side].get() + row_begin * t->ld, t->ld, n_rows, t->stream);
     CUDA_CHECK(cudaStreamSynchronize(t->stream));
   });
 }
@@ -1292,8 +589,8 @@ int ials_trainer_factors_device(ials_trainer *t, int side, float **d_ptr, int64_
                                 int64_t *K, int64_t *ld) {
   return guarded([&] {
     require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    if (d_ptr) *d_ptr = t->factor[side];
+    require_side(side);
+    if (d_ptr) *d_ptr = t->factor[side].get();
     if (n_rows) *n_rows = t->n_rows(side);
     if (K) *K = t->K;
     if (ld) *ld = t->ld;
@@ -1305,7 +602,7 @@ int ials_trainer_transform(ials_trainer *t, int side, int64_t n_rows, int64_t n_
                            const ials_solver_config *solver, float *out_host) {
   return guarded([&] {
     require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
+    require_side(side);
     check_solver(solver);
     require(n_rows >= 0 && n_cols >= 0, "negative shape");
     // Solver::X_to_vector shape check, IALSTrainer.hpp:126-131
@@ -1316,238 +613,7 @@ int ials_trainer_transform(ials_trainer *t, int side, int64_t n_rows, int64_t n_
       throw InvalidArgument("Shape mismatch: X.cols() = " + std::to_string(n_rows) +
                             " but other.factor.rows() = " + std::to_string(t->U) + ".");
     DeviceGuard g(t->device);
-    DeviceCsr given, transposed;
-    float *target = nullptr;
-    try {
-      upload_csr(given, n_rows, n_cols, indptr, indices, data);
-      DeviceCsr *solve_csr = &given;
-      if (side == 1) {  // X.transpose(), :800
-        build_transpose(given, transposed, t->stream);
-        solve_csr = &transposed;
-      }
-      plan_csr(t, *solve_csr);
-      const int64_t n_new = solve_csr->n_rows;
-      CUDA_CHECK(cudaMalloc(&target, sizeof(float) * std::max<int64_t>(n_new * t->ld, 1)));
-      CUDA_CHECK(cudaMemsetAsync(target, 0, sizeof(float) * std::max<int64_t>(n_new * t->ld, 1),
-                                 t->stream));  // DenseMatrix::Zero, :132
-      gram_side(t, side);  // prepare_p, :793 / :799
-      SolveArgs a = make_args(t, side, target, *solve_csr, solver);
-      run_solver(t, a, *solve_csr, solver, t->stream);
-      if (n_new) {
-        require(out_host != nullptr, "out is null");
-        CUDA_CHECK(cudaMemcpy2DAsync(out_host, sizeof(float) * t->K, target, sizeof(float) * t->ld,
-                                     sizeof(float) * t->K, n_new, cudaMemcpyDeviceToHost,
-                                     t->stream));
-      }
-      sync_and_check(t);
-    } catch (...) {
-      cudaStreamSynchronize(t->stream);
-      given.free_all();
-      transposed.free_all();
-      if (target) cudaFree(target);
-      throw;
-    }
-    given.free_all();
-    transposed.free_all();
-    cudaFree(target);
-  });
-}
-
-// ---- feature-aware iALS: the C ABI (wrapper.cpp:133-136, 144-155, 160-161) ----
-
-int ials_trainer_set_features(ials_trainer *t, int side, int64_t n_rows, int64_t n_cols, const float *dense,
-                              const int64_t *indptr, const int32_t *indices, const float *data,
-                              float lambda_feature, int64_t feature_warmup_epochs) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    require(n_rows >= 0 && n_cols >= 0 && feature_warmup_epochs >= 0, "negative shape");
-    if (t->sharded) throw NotImplemented("feature-aware iALS on a row-sharded trainer is not implemented");
-    if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix");
-    // initialize_feature_aware (:1001-1014)
-    if (n_rows != t->n_rows(side)) throw InvalidArgument("Feature matrix row count mismatch.");
-    if (n_cols > 0 && !(lambda_feature > 0.f))
-      throw InvalidArgument("Feature weight regularization must be positive.");
-    DeviceGuard g(t->device);
-    ials_trainer::FeatureSide &f = t->feat[side];
-    f.free_all();
-    upload_features(f, n_rows, n_cols, dense, indptr, indices, data);
-    f.given = f.weight_set = true;
-    f.n_w = n_cols;
-    f.lambda = lambda_feature;
-    f.cache_ready = false;
-    CUDA_CHECK(cudaMalloc(&f.weight, sizeof(float) * std::max<int64_t>(n_cols * t->ld, 1)));
-    CUDA_CHECK(cudaMemset(f.weight, 0, sizeof(float) * std::max<int64_t>(n_cols * t->ld, 1)));  // setZero, :1012
-    {  // does the side's interaction matrix have an empty row? (step_with_prior's guard)
-      const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
-      std::vector<int64_t> ip((size_t)csr.n_rows + 1);
-      CUDA_CHECK(cudaMemcpy(ip.data(), csr.indptr, sizeof(int64_t) * (csr.n_rows + 1), cudaMemcpyDeviceToHost));
-      f.has_empty_row = false;
-      for (int64_t r = 0; r < csr.n_rows; r++)
-        if (ip[r] == ip[r + 1]) {
-          f.has_empty_row = true;
-          break;
-        }
-    }
-    t->feature_aware = true;
-    t->feature_warmup = feature_warmup_epochs;
-  });
-}
-
-int ials_trainer_feature_weight_rows(ials_trainer *t, int side, int64_t *n_rows) {
-  return guarded([&] {
-    require(t != nullptr && n_rows != nullptr, "null argument");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    *n_rows = t->feat[side].weight_set ? t->feat[side].n_w : 0;
-  });
-}
-
-int ials_trainer_get_feature_weight(ials_trainer *t, int side, float *out_host) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    const ials_trainer::FeatureSide &f = t->feat[side];
-    if (!f.weight_set || f.n_w == 0) return;
-    require(out_host != nullptr, "out is null");
-    DeviceGuard g(t->device);
-    CUDA_CHECK(cudaStreamSynchronize(t->stream));
-    CUDA_CHECK(cudaMemcpy2D(out_host, sizeof(float) * t->K, f.weight, sizeof(float) * t->ld, sizeof(float) * t->K,
-                            f.n_w, cudaMemcpyDeviceToHost));
-  });
-}
-
-int ials_trainer_set_feature_weight(ials_trainer *t, int side, int64_t n_rows, const float *in_host) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    require(n_rows >= 0 && (n_rows == 0 || in_host != nullptr), "null argument");
-    DeviceGuard g(t->device);
-    ials_trainer::FeatureSide &f = t->feat[side];
-    CUDA_CHECK(cudaStreamSynchronize(t->stream));
-    if (n_rows != f.n_w || f.weight == nullptr) {  // def_rw assigns the whole matrix (wrapper.cpp:160-161)
-      if (f.weight) CUDA_CHECK(cudaFree(f.weight));
-      if (f.rhs) CUDA_CHECK(cudaFree(f.rhs));
-      if (f.llt) CUDA_CHECK(cudaFree(f.llt));
-      f.weight = f.rhs = f.llt = nullptr;
-      f.cache_ready = false;
-      CUDA_CHECK(cudaMalloc(&f.weight, sizeof(float) * std::max<int64_t>(n_rows * t->ld, 1)));
-      f.n_w = n_rows;
-    }
-    CUDA_CHECK(cudaMemset(f.weight, 0, sizeof(float) * std::max<int64_t>(n_rows * t->ld, 1)));
-    if (n_rows)
-      CUDA_CHECK(cudaMemcpy2D(f.weight, sizeof(float) * t->ld, in_host, sizeof(float) * t->K, sizeof(float) * t->K,
-                              n_rows, cudaMemcpyHostToDevice));
-    f.weight_set = true;
-  });
-}
-
-// transform_user_feature / transform_item_feature (:820-830): features x stored weight
-int ials_trainer_transform_feature(ials_trainer *t, int side, int64_t n_rows, int64_t n_cols, const float *dense,
-                                   const int64_t *indptr, const int32_t *indices, const float *data,
-                                   float *out_host) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    require(n_rows >= 0 && n_cols >= 0, "negative shape");
-    validate_feature_cols(t, side, n_cols);
-    if (n_rows == 0) return;
-    require(out_host != nullptr, "out is null");
-    DeviceGuard g(t->device);
-    ials_trainer::FeatureSide tmp;
-    float *prior = nullptr;
-    try {
-      upload_features(tmp, n_rows, n_cols, dense, indptr, indices, data);
-      CUDA_CHECK(cudaMalloc(&prior, sizeof(float) * n_rows * t->ld));
-      launch_feature_prior(tmp.F, t->feat[side].weight, t->ld, prior, t->stream);
-      CUDA_CHECK(cudaMemcpy2DAsync(out_host, sizeof(float) * t->K, prior, sizeof(float) * t->ld, sizeof(float) * t->K,
-                                   n_rows, cudaMemcpyDeviceToHost, t->stream));
-      CUDA_CHECK(cudaStreamSynchronize(t->stream));
-    } catch (...) {
-      cudaStreamSynchronize(t->stream);
-      tmp.free_all();
-      if (prior) cudaFree(prior);
-      throw;
-    }
-    tmp.free_all();
-    cudaFree(prior);
-  });
-}
-
-// transform_user_with_feature / transform_item_with_feature (:803-818): fold-in whose rows start from,
-// and are regularised towards, features x stored weight (X_to_vector_with_prior, :142-167)
-int ials_trainer_transform_with_feature(ials_trainer *t, int side, int64_t n_rows, int64_t n_cols,
-                                        const int64_t *indptr, const int32_t *indices, const float *data,
-                                        int64_t f_rows, int64_t f_cols, const float *f_dense,
-                                        const int64_t *f_indptr, const int32_t *f_indices, const float *f_data,
-                                        const ials_solver_config *solver, float *out_host) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    check_solver(solver);
-    require(n_rows >= 0 && n_cols >= 0 && f_rows >= 0 && f_cols >= 0, "negative shape");
-    validate_feature_cols(t, side, f_cols);
-    if (side == 0 && n_cols != t->I)
-      throw InvalidArgument("Shape mismatch: X.cols() = " + std::to_string(n_cols) +
-                            " but other.factor.rows() = " + std::to_string(t->I) + ".");
-    if (side == 1 && n_rows != t->U)
-      throw InvalidArgument("Shape mismatch: X.cols() = " + std::to_string(n_rows) +
-                            " but other.factor.rows() = " + std::to_string(t->U) + ".");
-    const int64_t n_new = side == 0 ? n_rows : n_cols;
-    if (f_rows != n_new) throw InvalidArgument("Feature prior shape does not match X.");  // :153-155
-    if (solver->solver_type == IALS_SOLVER_IALSPP)
-      throw InvalidArgument("Feature-aware iALS does not support IALSPP.");
-    DeviceGuard g(t->device);
-    DeviceCsr given, transposed;
-    ials_trainer::FeatureSide tmp;
-    float *target = nullptr, *prior = nullptr;
-    try {
-      upload_csr(given, n_rows, n_cols, indptr, indices, data);
-      DeviceCsr *solve_csr = &given;
-      if (side == 1) {
-        build_transpose(given, transposed, t->stream);
-        solve_csr = &transposed;
-      }
-      plan_csr(t, *solve_csr);
-      {  // the guard of step_with_prior needs to know whether a new row is empty
-        std::vector<int64_t> ip((size_t)n_new + 1);
-        CUDA_CHECK(cudaMemcpyAsync(ip.data(), solve_csr->indptr, sizeof(int64_t) * (n_new + 1), cudaMemcpyDeviceToHost,
-                                   t->stream));
-        CUDA_CHECK(cudaStreamSynchronize(t->stream));
-        bool empty = false;
-        for (int64_t r = 0; r < n_new && !empty; r++) empty = ip[r] == ip[r + 1];
-        check_prior_defined(t, side, empty);
-      }
-      upload_features(tmp, f_rows, f_cols, f_dense, f_indptr, f_indices, f_data);
-      const size_t bytes = sizeof(float) * std::max<int64_t>(n_new * t->ld, 1);
-      CUDA_CHECK(cudaMalloc(&prior, bytes));
-      CUDA_CHECK(cudaMalloc(&target, bytes));
-      CUDA_CHECK(cudaMemsetAsync(prior, 0, bytes, t->stream));
-      launch_feature_prior(tmp.F, t->feat[side].weight, t->ld, prior, t->stream);
-      CUDA_CHECK(cudaMemcpyAsync(target, prior, bytes, cudaMemcpyDeviceToDevice, t->stream));  // result = prior, :156
-      gram_side(t, side);  // prepare_p
-      SolveArgs a = make_args(t, side, target, *solve_csr, solver);
-      a.prior = prior;
-      run_solver(t, a, *solve_csr, solver, t->stream);
-      if (n_new) {
-        require(out_host != nullptr, "out is null");
-        CUDA_CHECK(cudaMemcpy2DAsync(out_host, sizeof(float) * t->K, target, sizeof(float) * t->ld,
-                                     sizeof(float) * t->K, n_new, cudaMemcpyDeviceToHost, t->stream));
-      }
-      sync_and_check(t);
-    } catch (...) {
-      cudaStreamSynchronize(t->stream);
-      given.free_all();
-      transposed.free_all();
-      tmp.free_all();
-      if (target) cudaFree(target);
-      if (prior) cudaFree(prior);
-      throw;
-    }
-    given.free_all();
-    transposed.free_all();
-    tmp.free_all();
-    cudaFree(target);
-    cudaFree(prior);
+    fold_in(t, side, n_rows, n_cols, indptr, indices, data, solver, out_host);
   });
 }
 
@@ -1566,721 +632,18 @@ int ials_trainer_compute_loss(ials_trainer *t, const ials_solver_config *solver,
     const float *prior[2] = {nullptr, nullptr};
     for (int side = 0; side < 2; side++)
       if (t->feature_aware && t->feat[side].n_w > 0) prior[side] = stored_prior(t, side);
-    launch_loss(t->factor[0], t->factor[1], t->U, t->I, t->K, t->ld, t->X, t->Xt, t->P[0], t->P[1],
-                t->cfg.alpha0, t->cfg.reg, t->cfg.nu, bias, prior[0], prior[1], t->d_loss, t->stream);
+    launch_loss(t->factor[0].get(), t->factor[1].get(), t->U, t->I, t->K, t->ld, t->X, t->Xt, t->P[0].get(),
+                t->P[1].get(), t->cfg.alpha0, t->cfg.reg, t->cfg.nu, bias, prior[0], prior[1], t->d_loss.get(),
+                t->stream);
     for (int side = 0; side < 2; side++)
       if (prior[side])
-        launch_loss_add_sumsq(t->feat[side].weight, t->feat[side].n_w * t->ld, t->feat[side].lambda, t->d_loss,
-                              t->stream);
-    launch_loss_halve(t->d_loss, t->stream);
+        launch_loss_add_sumsq(t->feat[side].weight.get(), t->feat[side].n_w * t->ld, t->feat[side].lambda,
+                              t->d_loss.get(), t->stream);
+    launch_loss_halve(t->d_loss.get(), t->stream);
     double h = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&h, t->d_loss, sizeof(double), cudaMemcpyDeviceToHost, t->stream));
+    CUDA_CHECK(cudaMemcpyAsync(&h, t->d_loss.get(), sizeof(double), cudaMemcpyDeviceToHost, t->stream));
     CUDA_CHECK(cudaStreamSynchronize(t->stream));
     *out = (float)h;
-  });
-}
-
-// user_idx != nullptr: the rows are users user_idx[0 .. end) (begin = 0), gathered on the device;
-// user_emb != nullptr: the rows are the host embeddings user_emb[end x K] (begin = 0; fold-in results)
-static int recommend_impl(ials_trainer *t, const int64_t *user_idx, const float *user_emb, int64_t begin,
-                          int64_t end, int64_t k, int mask_mode,
-                          const int64_t *mask_indptr, const int32_t *mask_indices, int64_t allow_n_lists,
-                          const int64_t *allow_indptr, const int32_t *allow_indices,
-                          int32_t *out_idx, float *out_score, int32_t *out_count) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(end >= begin && begin >= 0 && (user_idx != nullptr || user_emb != nullptr || end <= t->U),
-            "bad user block");
-    require(user_emb == nullptr || mask_mode != 0, "embeddings have no training rows: give the mask explicitly");
-    require(k >= 1 && k <= t->I, "cutoff must be in [1, n_items]");  // evaluator.cpp:265-266
-    require(k <= 1024, "k > 1024 is not supported");
-    require(mask_mode >= 0 && mask_mode <= 2, "mask_mode must be 0, 1 or 2");
-    const int64_t rows = end - begin;
-    if (rows == 0) return;
-    require(out_idx != nullptr && out_count != nullptr, "output pointer is null");
-    if (mask_mode == 0 && !t->has_X) throw std::runtime_error("no training matrix to mask with");
-    if (mask_mode == 0 && user_idx == nullptr && user_emb == nullptr)  // a sharded trainer only holds its own users' rows of X
-      require(begin >= t->X.row_base && end <= t->X.row_base + t->X.n_rows,
-              "mask='train' on a sharded trainer needs a user block inside the rank's shard");
-    if (user_idx != nullptr)
-      for (int64_t r = 0; r < rows; r++) {
-        require(user_idx[r] >= 0 && user_idx[r] < t->U, "user index out of range");
-        if (mask_mode == 0)
-          require(user_idx[r] >= t->X.row_base && user_idx[r] < t->X.row_base + t->X.n_rows,
-                  "mask='train' on a sharded trainer needs users inside the rank's shard");
-      }
-    DeviceGuard g(t->device);
-    int64_t *d_mindptr = nullptr;
-    int32_t *d_mindices = nullptr;
-    // the fused tensor-core kernel walks each mask row with a cursor: column ids must ascend
-    bool mask_sorted = true;
-    if (mask_mode == 0) {
-      if (t->X.sorted_state < 0)
-        t->X.sorted_state = csr_rows_strictly_sorted(t->X.indptr, t->X.indices, t->X.n_rows, t->stream) ? 1 : 0;
-      mask_sorted = t->X.sorted_state == 1;
-    }
-    try {
-      if (mask_mode == 2) {
-        require(mask_indptr != nullptr && mask_indptr[0] == 0, "mask indptr must start at 0");
-        const int64_t mnnz = mask_indptr[rows];
-        for (int64_t j = 0; j < mnnz; j++)
-          require(mask_indices[j] >= 0 && mask_indices[j] < t->I, "mask index out of range");
-        for (int64_t r = 0; r < rows && mask_sorted; r++)
-          for (int64_t j = mask_indptr[r] + 1; j < mask_indptr[r + 1]; j++)
-            if (mask_indices[j - 1] >= mask_indices[j]) {
-              mask_sorted = false;
-              break;
-            }
-        d_mindptr = static_cast<int64_t *>(t->rec_mindptr.get(sizeof(int64_t) * (rows + 1)));
-        d_mindices = static_cast<int32_t *>(t->rec_mindices.get(sizeof(int32_t) * std::max<int64_t>(mnnz, 1)));
-        CUDA_CHECK(cudaMemcpyAsync(d_mindptr, mask_indptr, sizeof(int64_t) * (rows + 1),
-                                   cudaMemcpyHostToDevice, t->stream));
-        if (mnnz)
-          CUDA_CHECK(cudaMemcpyAsync(d_mindices, mask_indices, sizeof(int32_t) * mnnz,
-                                     cudaMemcpyHostToDevice, t->stream));
-      }
-      int32_t *d_idx = static_cast<int32_t *>(t->rec_idx.get(sizeof(int32_t) * rows * k));
-      float *d_sc = static_cast<float *>(t->rec_score.get(sizeof(float) * rows * k));
-      int32_t *d_cnt = static_cast<int32_t *>(t->rec_count.get(sizeof(int32_t) * rows));
-      // allow-lists (recommendable items): strictly ascending int32 lists, one shared or one per row
-      int64_t *d_aindptr = nullptr;
-      int32_t *d_aindices = nullptr;
-      uint32_t *d_abitmap = nullptr;
-      if (allow_n_lists > 0) {
-        require(allow_n_lists == 1 || allow_n_lists == rows, "allow-lists: one shared list or one per row");
-        require(allow_indptr != nullptr && allow_indptr[0] == 0, "allow indptr must start at 0");
-        const int64_t annz = allow_indptr[allow_n_lists];
-        require(annz == 0 || allow_indices != nullptr, "allow indices are null");
-        for (int64_t r = 0; r < allow_n_lists; r++)
-          for (int64_t j = allow_indptr[r]; j < allow_indptr[r + 1]; j++) {
-            require(allow_indices[j] >= 0 && allow_indices[j] < t->I, "allowed item out of range");
-            require(j == allow_indptr[r] || allow_indices[j - 1] < allow_indices[j],
-                    "allow-lists must be strictly ascending");
-          }
-        if (allow_n_lists == 1) {  // a shared list goes to the kernel as a bitmap of the catalogue
-          std::vector<uint32_t> &words = t->rec_abitmap_host;  // outlives the asynchronous copy
-          words.assign((size_t)((t->I + 31) / 32), 0u);
-          for (int64_t j = 0; j < annz; j++) words[allow_indices[j] >> 5] |= 1u << (allow_indices[j] & 31);
-          d_abitmap = static_cast<uint32_t *>(t->rec_aindices.get(sizeof(uint32_t) * words.size()));
-          CUDA_CHECK(cudaMemcpyAsync(d_abitmap, words.data(), sizeof(uint32_t) * words.size(),
-                                     cudaMemcpyHostToDevice, t->stream));
-        } else {
-          d_aindptr = static_cast<int64_t *>(t->rec_aindptr.get(sizeof(int64_t) * (allow_n_lists + 1)));
-          d_aindices = static_cast<int32_t *>(t->rec_aindices.get(sizeof(int32_t) * std::max<int64_t>(annz, 1)));
-          CUDA_CHECK(cudaMemcpyAsync(d_aindptr, allow_indptr, sizeof(int64_t) * (allow_n_lists + 1),
-                                     cudaMemcpyHostToDevice, t->stream));
-          if (annz)
-            CUDA_CHECK(cudaMemcpyAsync(d_aindices, allow_indices, sizeof(int32_t) * annz, cudaMemcpyHostToDevice,
-                                       t->stream));
-        }
-      }
-      const bool fused = score_tc_supported(t->ld, k) && mask_sorted;
-      // users picked by index: their factor rows are gathered into a dense block first
-      const float *user_rows = t->factor[0] + begin * t->ld;
-      int64_t *d_uidx = nullptr;
-      if (user_idx != nullptr) {
-        d_uidx = static_cast<int64_t *>(t->rec_uidx.get(sizeof(int64_t) * rows));
-        float *gathered = static_cast<float *>(t->rec_users.get(sizeof(float) * rows * t->ld));
-        CUDA_CHECK(cudaMemcpyAsync(d_uidx, user_idx, sizeof(int64_t) * rows, cudaMemcpyHostToDevice, t->stream));
-        launch_gather_rows(t->factor[0], t->ld, d_uidx, rows, gathered, t->stream);
-        user_rows = gathered;
-        if (mask_mode == 0 && !fused)
-          throw NotImplemented("mask='train' for users picked by index needs the fused tensor-core kernel");
-      }
-      if (user_emb != nullptr) {  // host embeddings [rows x K] -> padded device rows [rows x ld]
-        float *staged = static_cast<float *>(t->rec_emb.get(sizeof(float) * rows * t->K));
-        float *padded = static_cast<float *>(t->rec_users.get(sizeof(float) * rows * t->ld));
-        CUDA_CHECK(cudaMemcpyAsync(staged, user_emb, sizeof(float) * rows * t->K, cudaMemcpyHostToDevice, t->stream));
-        launch_pad_copy(staged, rows, (int)t->K, padded, t->ld, t->stream);
-        user_rows = padded;
-      }
-      if (allow_n_lists > 0 && !fused)
-        throw NotImplemented("allow-lists need the fused tensor-core kernel (row stride <= 128, cutoff <= 128, "
-                             "sorted mask rows)");
-      if (fused) {
-        // scores + mask + top-k in one tcgen05 kernel; only candidate keys touch HBM
-        const int64_t slab_rows = std::max<int64_t>(128, ((1ll << 29) / (8 * 256)) / 128 * 128);
-        for (int64_t b = 0; b < rows; b += slab_rows) {
-          const int64_t m = std::min(slab_rows, rows - b);
-          void *scratch = ensure_score_buf(t, score_tc_scratch_bytes(m, t->I, k));
-          const int64_t *mip = nullptr;
-          const int32_t *mix = nullptr;
-          const float *mdt = nullptr;
-          int64_t mrow0 = 0;
-          const int64_t *mrowmap = nullptr;
-          if (mask_mode == 0) {
-            mip = t->X.indptr; mix = t->X.indices; mdt = t->X.data;
-            mrow0 = begin + b - t->X.row_base;
-            if (d_uidx) { mrowmap = d_uidx + b; mrow0 = -t->X.row_base; }
-          } else if (mask_mode == 2) {
-            mip = d_mindptr; mix = d_mindices; mrow0 = b;
-          }
-          launch_score_topk_tc(user_rows + b * t->ld, m, t->factor[1], t->I, t->ld, mip,
-                               mix, mdt, mrow0, (int)k, scratch, d_idx + b * k, d_sc + b * k,
-                               d_cnt + b, t->stream, (int)std::min<int64_t>(allow_n_lists, 2), d_aindptr,
-                               d_aindices, b, d_abitmap, mrowmap);
-        }
-      }
-      const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 29) / (4 * t->I)));
-      float *buf = fused ? nullptr : ensure_score_buf(t, sizeof(float) * slab * t->I);
-      for (int64_t b = 0; b < rows && !fused; b += slab) {
-        const int64_t m = std::min(slab, rows - b);
-        launch_scores(user_rows + b * t->ld, m, t->factor[1], t->I, t->ld, buf, t->I, t->stream);
-        if (mask_mode == 0)
-          launch_mask_rows(buf, t->I, t->X.indptr, t->X.indices, t->X.data,
-                           begin + b - t->X.row_base, m, 0, t->stream);
-        else if (mask_mode == 2)
-          launch_mask_rows(buf, t->I, d_mindptr, d_mindices, nullptr, b, m, 0, t->stream);
-        launch_topk_rows(buf, t->I, m, t->I, (int)k, d_idx + b * k, d_sc + b * k, d_cnt + b,
-                         t->stream);
-      }
-      CUDA_CHECK(cudaMemcpyAsync(out_idx, d_idx, sizeof(int32_t) * rows * k, cudaMemcpyDeviceToHost,
-                                 t->stream));
-      if (out_score)
-        CUDA_CHECK(cudaMemcpyAsync(out_score, d_sc, sizeof(float) * rows * k,
-                                   cudaMemcpyDeviceToHost, t->stream));
-      CUDA_CHECK(cudaMemcpyAsync(out_count, d_cnt, sizeof(int32_t) * rows, cudaMemcpyDeviceToHost,
-                                 t->stream));
-      CUDA_CHECK(cudaStreamSynchronize(t->stream));
-    } catch (...) {
-      cudaStreamSynchronize(t->stream);  // the staging buffers stay with the trainer
-      throw;
-    }
-  });
-}
-
-int ials_trainer_recommend(ials_trainer *t, int64_t begin, int64_t end, int64_t k, int mask_mode,
-                           const int64_t *mask_indptr, const int32_t *mask_indices,
-                           int32_t *out_idx, float *out_score, int32_t *out_count) {
-  return recommend_impl(t, nullptr, nullptr, begin, end, k, mask_mode, mask_indptr, mask_indices, 0, nullptr,
-                        nullptr, out_idx, out_score, out_count);
-}
-
-int ials_trainer_recommend_allowed(ials_trainer *t, int64_t begin, int64_t end, int64_t k, int mask_mode,
-                                   const int64_t *mask_indptr, const int32_t *mask_indices, int64_t allow_n_lists,
-                                   const int64_t *allow_indptr, const int32_t *allow_indices, int32_t *out_idx,
-                                   float *out_score, int32_t *out_count) {
-  return recommend_impl(t, nullptr, nullptr, begin, end, k, mask_mode, mask_indptr, mask_indices, allow_n_lists,
-                        allow_indptr, allow_indices, out_idx, out_score, out_count);
-}
-
-int ials_trainer_recommend_users(ials_trainer *t, const int64_t *user_indices, int64_t n_users, int64_t k,
-                                 int mask_mode, const int64_t *mask_indptr, const int32_t *mask_indices,
-                                 int64_t allow_n_lists, const int64_t *allow_indptr, const int32_t *allow_indices,
-                                 int32_t *out_idx, float *out_score, int32_t *out_count) {
-  if (n_users > 0 && user_indices == nullptr) return guarded([] { require(false, "user_indices is null"); });
-  static const int64_t none = 0;
-  return recommend_impl(t, user_indices ? user_indices : &none, nullptr, 0, n_users, k, mask_mode, mask_indptr,
-                        mask_indices, allow_n_lists, allow_indptr, allow_indices, out_idx, out_score, out_count);
-}
-
-int ials_trainer_recommend_embeddings(ials_trainer *t, const float *user_embeddings, int64_t n_rows, int64_t k,
-                                      int mask_mode, const int64_t *mask_indptr, const int32_t *mask_indices,
-                                      int64_t allow_n_lists, const int64_t *allow_indptr,
-                                      const int32_t *allow_indices, int32_t *out_idx, float *out_score,
-                                      int32_t *out_count) {
-  if (n_rows > 0 && user_embeddings == nullptr) return guarded([] { require(false, "user_embeddings is null"); });
-  static const float none = 0.f;
-  return recommend_impl(t, nullptr, user_embeddings ? user_embeddings : &none, 0, n_rows, k, mask_mode,
-                        mask_indptr, mask_indices, allow_n_lists, allow_indptr, allow_indices, out_idx, out_score,
-                        out_count);
-}
-
-int ials_metrics_accumulate(const int32_t *rec, const int32_t *count, int64_t rows, int64_t k,
-                            const int64_t *gt_indptr, const int32_t *gt_indices, int64_t n_items,
-                            int recall_with_cutoff, const double *discount, int device, void *cuda_stream,
-                            double *acc, int64_t *valid_user, int64_t *item_cnt) {
-  return guarded([&] {
-    require(rows >= 0 && k >= 1 && n_items >= 1, "bad shape");
-    if (rows == 0) return;
-    require(rec && count && gt_indptr && discount && acc && valid_user && item_cnt, "null pointer");
-    require(gt_indptr[0] == 0, "ground-truth indptr must start at 0");
-    const int64_t gnnz = gt_indptr[rows];
-    require(gnnz == 0 || gt_indices != nullptr, "ground-truth indices are null");
-    for (int64_t r = 0; r < rows; r++) {
-      require(gt_indptr[r + 1] >= gt_indptr[r], "ground-truth indptr must be non-decreasing");
-      for (int64_t j = gt_indptr[r] + 1; j < gt_indptr[r + 1]; j++)
-        require(gt_indices[j - 1] <= gt_indices[j], "ground-truth rows must be sorted");
-    }
-    for (int64_t j = 0; j < rows * k; j++) require(rec[j] >= -1 && rec[j] < n_items, "recommended item out of range");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-      cudaGetLastError();
-      throw CudaError("no CUDA device available: the B200 backend has no CPU fallback");
-    }
-    require(device >= 0 && device < n_dev, "invalid CUDA device index");
-    DeviceGuard g(device);
-    cudaStream_t s = (cudaStream_t)cuda_stream;
-    std::vector<double> cum((size_t)k);
-    double run = 0;
-    for (int64_t j = 0; j < k; j++) cum[j] = (run += discount[j]);
-    // one allocation: rec | count | gt indptr | gt indices | discount | cum | acc[5] | valid | item_cnt
-    size_t off = 0;
-    auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-    const size_t o_rec = take(sizeof(int32_t) * rows * k), o_cnt = take(sizeof(int32_t) * rows),
-                 o_ip = take(sizeof(int64_t) * (rows + 1)), o_ix = take(sizeof(int32_t) * std::max<int64_t>(gnnz, 1)),
-                 o_d = take(sizeof(double) * k), o_c = take(sizeof(double) * k), o_acc = take(sizeof(double) * 5),
-                 o_v = take(sizeof(unsigned long long)), o_ic = take(sizeof(unsigned long long) * n_items);
-    char *d = nullptr;
-    CUDA_CHECK(cudaMalloc(&d, off));
-    try {
-      CUDA_CHECK(cudaMemcpyAsync(d + o_rec, rec, sizeof(int32_t) * rows * k, cudaMemcpyHostToDevice, s));
-      CUDA_CHECK(cudaMemcpyAsync(d + o_cnt, count, sizeof(int32_t) * rows, cudaMemcpyHostToDevice, s));
-      CUDA_CHECK(cudaMemcpyAsync(d + o_ip, gt_indptr, sizeof(int64_t) * (rows + 1), cudaMemcpyHostToDevice, s));
-      if (gnnz) CUDA_CHECK(cudaMemcpyAsync(d + o_ix, gt_indices, sizeof(int32_t) * gnnz, cudaMemcpyHostToDevice, s));
-      CUDA_CHECK(cudaMemcpyAsync(d + o_d, discount, sizeof(double) * k, cudaMemcpyHostToDevice, s));
-      CUDA_CHECK(cudaMemcpyAsync(d + o_c, cum.data(), sizeof(double) * k, cudaMemcpyHostToDevice, s));
-      CUDA_CHECK(cudaMemsetAsync(d + o_acc, 0, off - o_acc, s));
-      launch_metrics_rows(reinterpret_cast<int32_t *>(d + o_rec), reinterpret_cast<int32_t *>(d + o_cnt), rows, (int)k,
-                          reinterpret_cast<int64_t *>(d + o_ip), reinterpret_cast<int32_t *>(d + o_ix),
-                          reinterpret_cast<double *>(d + o_d), reinterpret_cast<double *>(d + o_c),
-                          recall_with_cutoff, reinterpret_cast<double *>(d + o_acc),
-                          reinterpret_cast<unsigned long long *>(d + o_v),
-                          reinterpret_cast<unsigned long long *>(d + o_ic), s);
-      double h_acc[5];
-      unsigned long long h_valid = 0;
-      std::vector<unsigned long long> h_cnt((size_t)n_items);
-      CUDA_CHECK(cudaMemcpyAsync(h_acc, d + o_acc, sizeof(h_acc), cudaMemcpyDeviceToHost, s));
-      CUDA_CHECK(cudaMemcpyAsync(&h_valid, d + o_v, sizeof(h_valid), cudaMemcpyDeviceToHost, s));
-      CUDA_CHECK(cudaMemcpyAsync(h_cnt.data(), d + o_ic, sizeof(unsigned long long) * n_items, cudaMemcpyDeviceToHost, s));
-      CUDA_CHECK(cudaStreamSynchronize(s));
-      for (int i = 0; i < 5; i++) acc[i] += h_acc[i];
-      *valid_user += (int64_t)h_valid;
-      for (int64_t i = 0; i < n_items; i++) item_cnt[i] += (int64_t)h_cnt[i];
-    } catch (...) {
-      cudaStreamSynchronize(s);
-      cudaFree(d);
-      throw;
-    }
-    cudaFree(d);
-  });
-}
-
-int ials_topk_scores(const float *scores_host, int64_t rows, int64_t n_items, int64_t k,
-                     const int64_t *mask_indptr, const int32_t *mask_indices, int device,
-                     void *cuda_stream, int32_t *out_idx, float *out_score, int32_t *out_count) {
-  return guarded([&] {
-    require(rows >= 0 && n_items >= 0, "negative shape");
-    require(k >= 1 && k <= n_items, "cutoff must be in [1, n_items]");
-    require(k <= 1024, "k > 1024 is not supported");
-    if (rows == 0) return;
-    require(scores_host && out_idx && out_count, "null pointer");
-    require((mask_indptr == nullptr) == (mask_indices == nullptr) || mask_indptr[rows] == 0,
-            "mask indptr / indices must both be given");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-      cudaGetLastError();
-      throw CudaError("no CUDA device available: the B200 backend has no CPU fallback");
-    }
-    require(device >= 0 && device < n_dev, "invalid CUDA device index");
-    DeviceGuard g(device);
-    cudaStream_t s = (cudaStream_t)cuda_stream;
-    float *d_scores = nullptr, *d_sc = nullptr;
-    int64_t *d_mindptr = nullptr;
-    int32_t *d_mindices = nullptr, *d_idx = nullptr, *d_cnt = nullptr;
-    const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 29) / (4 * n_items)));
-    try {
-      CUDA_CHECK(cudaMalloc(&d_scores, sizeof(float) * slab * n_items));
-      CUDA_CHECK(cudaMalloc(&d_idx, sizeof(int32_t) * rows * k));
-      CUDA_CHECK(cudaMalloc(&d_sc, sizeof(float) * rows * k));
-      CUDA_CHECK(cudaMalloc(&d_cnt, sizeof(int32_t) * rows));
-      if (mask_indptr) {
-        require(mask_indptr[0] == 0, "mask indptr must start at 0");
-        const int64_t mnnz = mask_indptr[rows];
-        for (int64_t j = 0; j < mnnz; j++)
-          require(mask_indices[j] >= 0 && mask_indices[j] < n_items, "mask index out of range");
-        CUDA_CHECK(cudaMalloc(&d_mindptr, sizeof(int64_t) * (rows + 1)));
-        CUDA_CHECK(cudaMalloc(&d_mindices, sizeof(int32_t) * std::max<int64_t>(mnnz, 1)));
-        CUDA_CHECK(cudaMemcpyAsync(d_mindptr, mask_indptr, sizeof(int64_t) * (rows + 1),
-                                   cudaMemcpyHostToDevice, s));
-        if (mnnz)
-          CUDA_CHECK(cudaMemcpyAsync(d_mindices, mask_indices, sizeof(int32_t) * mnnz,
-                                     cudaMemcpyHostToDevice, s));
-      }
-      for (int64_t b = 0; b < rows; b += slab) {
-        const int64_t m = std::min(slab, rows - b);
-        CUDA_CHECK(cudaMemcpyAsync(d_scores, scores_host + b * n_items, sizeof(float) * m * n_items,
-                                   cudaMemcpyHostToDevice, s));
-        if (d_mindptr) launch_mask_rows(d_scores, n_items, d_mindptr, d_mindices, nullptr, b, m, 0, s);
-        launch_topk_rows(d_scores, n_items, m, n_items, (int)k, d_idx + b * k, d_sc + b * k,
-                         d_cnt + b, s);
-      }
-      CUDA_CHECK(cudaMemcpyAsync(out_idx, d_idx, sizeof(int32_t) * rows * k, cudaMemcpyDeviceToHost, s));
-      if (out_score)
-        CUDA_CHECK(cudaMemcpyAsync(out_score, d_sc, sizeof(float) * rows * k, cudaMemcpyDeviceToHost, s));
-      CUDA_CHECK(cudaMemcpyAsync(out_count, d_cnt, sizeof(int32_t) * rows, cudaMemcpyDeviceToHost, s));
-      CUDA_CHECK(cudaStreamSynchronize(s));
-    } catch (...) {
-      cudaStreamSynchronize(s);
-      cudaFree(d_scores); cudaFree(d_sc); cudaFree(d_mindptr); cudaFree(d_mindices);
-      cudaFree(d_idx); cudaFree(d_cnt);
-      throw;
-    }
-    cudaFree(d_scores); cudaFree(d_sc); cudaFree(d_mindptr); cudaFree(d_mindices);
-    cudaFree(d_idx); cudaFree(d_cnt);
-  });
-}
-
-int ials_retrieve_recommend(const float *scores_host, int64_t rows, int64_t n_items, int64_t cutoff,
-                            int64_t n_allowed_lists, const int64_t *allowed_indptr,
-                            const int64_t *allowed_indices, int device, void *cuda_stream,
-                            int32_t *out_idx, float *out_score, int32_t *out_count) {
-  return guarded([&] {
-    require(rows >= 0 && n_items >= 0 && cutoff >= 0, "negative shape");
-    require(n_allowed_lists == 0 || n_allowed_lists == 1 || n_allowed_lists == rows,
-            "allowed_indices, if not empty, must have a size equal to X.rows()");  // util.hpp:436-439
-    const int64_t k = std::min(cutoff, n_items);
-    if (k > 1024) throw NotImplemented("retrieve_recommend: cutoff > 1024 is not supported");
-    require(rows == 0 || out_count != nullptr, "null pointer");
-    if (rows == 0 || k == 0) {
-      for (int64_t r = 0; r < rows; r++) out_count[r] = 0;
-      return;
-    }
-    require(scores_host && out_idx && out_count, "null pointer");
-    require(n_allowed_lists == 0 || allowed_indptr != nullptr, "null allowed_indptr");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-      cudaGetLastError();
-      throw CudaError("no CUDA device available: the B200 backend has no CPU fallback");
-    }
-    require(device >= 0 && device < n_dev, "invalid CUDA device index");
-    DeviceGuard g(device);
-    cudaStream_t s = (cudaStream_t)cuda_stream;
-    float *d_scores = nullptr, *d_allowed = nullptr, *d_sc = nullptr;
-    int64_t *d_aindptr = nullptr, *d_aindices = nullptr;
-    int32_t *d_idx = nullptr, *d_cnt = nullptr;
-    const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 29) / (4 * n_items)));
-    auto free_all = [&] {
-      cudaFree(d_scores); cudaFree(d_allowed); cudaFree(d_sc); cudaFree(d_aindptr);
-      cudaFree(d_aindices); cudaFree(d_idx); cudaFree(d_cnt);
-    };
-    try {
-      CUDA_CHECK(cudaMalloc(&d_scores, sizeof(float) * slab * n_items));
-      CUDA_CHECK(cudaMalloc(&d_idx, sizeof(int32_t) * rows * k));
-      CUDA_CHECK(cudaMalloc(&d_sc, sizeof(float) * rows * k));
-      CUDA_CHECK(cudaMalloc(&d_cnt, sizeof(int32_t) * rows));
-      if (n_allowed_lists > 0) {
-        require(allowed_indptr[0] == 0, "allowed indptr must start at 0");
-        const int64_t annz = allowed_indptr[n_allowed_lists];
-        require(annz == 0 || allowed_indices != nullptr, "null allowed_indices");
-        CUDA_CHECK(cudaMalloc(&d_allowed, sizeof(float) * slab * n_items));
-        CUDA_CHECK(cudaMalloc(&d_aindptr, sizeof(int64_t) * (n_allowed_lists + 1)));
-        CUDA_CHECK(cudaMalloc(&d_aindices, sizeof(int64_t) * std::max<int64_t>(annz, 1)));
-        CUDA_CHECK(cudaMemcpyAsync(d_aindptr, allowed_indptr, sizeof(int64_t) * (n_allowed_lists + 1),
-                                   cudaMemcpyHostToDevice, s));
-        if (annz)
-          CUDA_CHECK(cudaMemcpyAsync(d_aindices, allowed_indices, sizeof(int64_t) * annz,
-                                     cudaMemcpyHostToDevice, s));
-      }
-      for (int64_t b = 0; b < rows; b += slab) {
-        const int64_t m = std::min(slab, rows - b);
-        CUDA_CHECK(cudaMemcpyAsync(d_scores, scores_host + b * n_items, sizeof(float) * m * n_items,
-                                   cudaMemcpyHostToDevice, s));
-        const float *cand = d_scores;
-        if (d_allowed) {
-          launch_allow_rows(d_scores, d_allowed, n_items, d_aindptr, d_aindices, n_allowed_lists, b, m,
-                            n_items, s);
-          cand = d_allowed;
-        }
-        launch_topk_rows(cand, n_items, m, n_items, (int)k, d_idx + b * k, d_sc + b * k, d_cnt + b, s);
-      }
-      CUDA_CHECK(cudaMemcpyAsync(out_idx, d_idx, sizeof(int32_t) * rows * k, cudaMemcpyDeviceToHost, s));
-      if (out_score)
-        CUDA_CHECK(cudaMemcpyAsync(out_score, d_sc, sizeof(float) * rows * k, cudaMemcpyDeviceToHost, s));
-      CUDA_CHECK(cudaMemcpyAsync(out_count, d_cnt, sizeof(int32_t) * rows, cudaMemcpyDeviceToHost, s));
-      CUDA_CHECK(cudaStreamSynchronize(s));
-    } catch (...) {
-      cudaStreamSynchronize(s);
-      free_all();
-      throw;
-    }
-    free_all();
-  });
-}
-
-// Standalone operator: G = sum_t w_t y_{i_t} y_{i_t}^T (and b = sum (bias + w_t) y_{i_t}) on the
-// tensor cores, host buffers in and out.
-int ials_weighted_gram(const float *Y_host, int64_t n, int64_t K, const int32_t *idx_host,
-                       const float *w_host, int64_t m, int64_t n_jobs, float bias, int device,
-                       float *G_host, float *b_host) {
-  return guarded([&] {
-    require(Y_host != nullptr && G_host != nullptr, "null pointer");
-    require(n >= 0 && K >= 1 && K <= 128, "K must be in [1, 128]");
-    require(n_jobs >= 1 && n_jobs <= 4096, "n_jobs must be in [1, 4096]");
-    const bool gathered = idx_host != nullptr;
-    if (!gathered) m = n;
-    require(m >= 0, "negative length");
-    if (gathered)
-      for (int64_t i = 0; i < m; i++) require(idx_host[i] >= 0 && idx_host[i] < n, "index out of range");
-    if (w_host)
-      for (int64_t i = 0; i < m; i++) require(w_host[i] >= 0.f, "weights must be non-negative");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-      cudaGetLastError();
-      throw CudaError("no CUDA device available: the B200 backend has no CPU fallback");
-    }
-    require(device >= 0 && device < n_dev, "invalid CUDA device index");
-    DeviceGuard g(device);
-    const int ld = 128;
-    float *d_Y = nullptr, *d_w = nullptr, *d_W = nullptr, *d_b = nullptr, *d_G = nullptr, *d_tmp = nullptr;
-    int32_t *d_idx = nullptr;
-    int64_t *d_jb = nullptr, *d_je = nullptr;
-    cudaStream_t s = nullptr;
-    auto cleanup = [&] {
-      cudaFree(d_Y); cudaFree(d_w); cudaFree(d_W); cudaFree(d_b); cudaFree(d_G); cudaFree(d_tmp);
-      cudaFree(d_idx); cudaFree(d_jb); cudaFree(d_je);
-    };
-    try {
-      CUDA_CHECK(cudaMalloc(&d_tmp, sizeof(float) * std::max<int64_t>(n * K, 1)));
-      CUDA_CHECK(cudaMalloc(&d_Y, sizeof(float) * std::max<int64_t>(n * ld, 1)));
-      CUDA_CHECK(cudaMemcpy(d_tmp, Y_host, sizeof(float) * n * K, cudaMemcpyHostToDevice));
-      launch_pad_copy(d_tmp, n, (int)K, d_Y, ld, s);
-      if (gathered) {
-        CUDA_CHECK(cudaMalloc(&d_idx, sizeof(int32_t) * std::max<int64_t>(m, 1)));
-        CUDA_CHECK(cudaMemcpy(d_idx, idx_host, sizeof(int32_t) * m, cudaMemcpyHostToDevice));
-      }
-      if (w_host) {
-        CUDA_CHECK(cudaMalloc(&d_w, sizeof(float) * std::max<int64_t>(m, 1)));
-        CUDA_CHECK(cudaMemcpy(d_w, w_host, sizeof(float) * m, cudaMemcpyHostToDevice));
-      }
-      std::vector<int64_t> jb(n_jobs), je(n_jobs);
-      const int64_t per = (m + n_jobs - 1) / n_jobs;
-      for (int64_t j = 0; j < n_jobs; j++) {
-        jb[j] = std::min(j * per, m);
-        je[j] = std::min(jb[j] + per, m);
-      }
-      CUDA_CHECK(cudaMalloc(&d_jb, sizeof(int64_t) * n_jobs));
-      CUDA_CHECK(cudaMalloc(&d_je, sizeof(int64_t) * n_jobs));
-      CUDA_CHECK(cudaMemcpy(d_jb, jb.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
-      CUDA_CHECK(cudaMemcpy(d_je, je.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
-      CUDA_CHECK(cudaMalloc(&d_W, sizeof(float) * n_jobs * ld * ld));
-      CUDA_CHECK(cudaMalloc(&d_b, sizeof(float) * n_jobs * kWGramBParts * ld));
-      CUDA_CHECK(cudaMalloc(&d_G, sizeof(float) * ld * ld));
-      WGramArgs a{};
-      a.Y = d_Y; a.ld = ld; a.indices = d_idx; a.weights = d_w;
-      a.job_begin = d_jb; a.job_end = d_je; a.n_jobs = n_jobs; a.bias = bias;
-      a.W = d_W; a.bpart = d_b;
-      launch_wgram(a, s);
-      launch_wgram_reduce_sym(d_W, (int)n_jobs, 1.0f, d_G, s);
-      CUDA_CHECK(cudaStreamSynchronize(s));
-      CUDA_CHECK(cudaMemcpy2D(G_host, sizeof(float) * K, d_G, sizeof(float) * ld, sizeof(float) * K, K,
-                              cudaMemcpyDeviceToHost));
-      if (b_host) {
-        std::vector<float> hb((size_t)n_jobs * kWGramBParts * ld);
-        CUDA_CHECK(cudaMemcpy(hb.data(), d_b, sizeof(float) * hb.size(), cudaMemcpyDeviceToHost));
-        for (int64_t k = 0; k < K; k++) {
-          float acc = 0.f;
-          for (int64_t p = 0; p < n_jobs * kWGramBParts; p++) acc += hb[p * ld + k];
-          b_host[k] = acc;
-        }
-      }
-      CUDA_CHECK(cudaDeviceSynchronize());
-    } catch (...) {
-      cudaDeviceSynchronize();
-      cleanup();
-      throw;
-    }
-    cleanup();
-  });
-}
-
-// Standalone operator for 256-column factors (K = 256 Cholesky, BASELINE configs[2]): the
-// tensor-core launch of solve_cholesky_tensor (wgram256_kernel) on host buffers, its per-job
-// W blocks assembled into G = sum w y y^T (256 x 256) and b = sum (bias + w) y.
-int ials_weighted_gram256(const float *Y_host, int64_t n, int64_t K, const int32_t *idx_host,
-                          const float *w_host, int64_t m, int64_t n_jobs, float bias, int device,
-                          float *G_host, float *b_host) {
-  return guarded([&] {
-    require(Y_host != nullptr && G_host != nullptr && idx_host != nullptr, "null pointer");
-    require(n >= 1 && K > 128 && K <= 256, "K must be in (128, 256]");
-    require(n_jobs >= 1 && n_jobs <= 1024 && m >= 0, "n_jobs must be in [1, 1024]");
-    for (int64_t i = 0; i < m; i++) require(idx_host[i] >= 0 && idx_host[i] < n, "index out of range");
-    if (w_host)
-      for (int64_t i = 0; i < m; i++) require(w_host[i] >= 0.f, "weights must be non-negative");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-      cudaGetLastError();
-      throw CudaError("no CUDA device available: the B200 backend has no CPU fallback");
-    }
-    require(device >= 0 && device < n_dev, "invalid CUDA device index");
-    DeviceGuard g(device);
-    const int ld = 256;
-    const size_t blk = (size_t)n_jobs * 256 * 256, bsz = (size_t)n_jobs * kWGram256BParts * 256;
-    float *d_Y = nullptr, *d_w = nullptr, *d_ws = nullptr;
-    int32_t *d_idx = nullptr;
-    int64_t *d_jb = nullptr, *d_je = nullptr;
-    cudaStream_t s = nullptr;
-    auto cleanup = [&] {
-      cudaFree(d_Y); cudaFree(d_w); cudaFree(d_ws); cudaFree(d_idx); cudaFree(d_jb); cudaFree(d_je);
-    };
-    try {
-      CUDA_CHECK(cudaMalloc(&d_Y, sizeof(float) * n * ld));
-      CUDA_CHECK(cudaMemset(d_Y, 0, sizeof(float) * n * ld));
-      CUDA_CHECK(cudaMemcpy2D(d_Y, sizeof(float) * ld, Y_host, sizeof(float) * K, sizeof(float) * K, n,
-                              cudaMemcpyHostToDevice));
-      CUDA_CHECK(cudaMalloc(&d_idx, sizeof(int32_t) * std::max<int64_t>(m, 1)));
-      CUDA_CHECK(cudaMemcpy(d_idx, idx_host, sizeof(int32_t) * m, cudaMemcpyHostToDevice));
-      if (w_host) {
-        CUDA_CHECK(cudaMalloc(&d_w, sizeof(float) * std::max<int64_t>(m, 1)));
-        CUDA_CHECK(cudaMemcpy(d_w, w_host, sizeof(float) * m, cudaMemcpyHostToDevice));
-      }
-      std::vector<int64_t> jb(n_jobs), je(n_jobs);
-      const int64_t per = (m + n_jobs - 1) / n_jobs;
-      for (int64_t j = 0; j < n_jobs; j++) {
-        jb[j] = std::min(j * per, m);
-        je[j] = std::min(jb[j] + per, m);
-      }
-      CUDA_CHECK(cudaMalloc(&d_jb, sizeof(int64_t) * n_jobs));
-      CUDA_CHECK(cudaMalloc(&d_je, sizeof(int64_t) * n_jobs));
-      CUDA_CHECK(cudaMemcpy(d_jb, jb.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
-      CUDA_CHECK(cudaMemcpy(d_je, je.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
-      CUDA_CHECK(cudaMalloc(&d_ws, sizeof(float) * (blk + bsz)));
-      WGramArgs a{};
-      a.ld = ld; a.indices = d_idx; a.weights = d_w;
-      a.job_begin = d_jb; a.job_end = d_je; a.n_jobs = n_jobs; a.bias = bias;
-      a.Y = d_Y; a.W = d_ws; a.bpart = d_ws + blk;
-      launch_wgram256(a, s);
-      std::vector<float> h(blk + bsz);
-      CUDA_CHECK(cudaMemcpy(h.data(), d_ws, sizeof(float) * h.size(), cudaMemcpyDeviceToHost));
-      std::vector<double> G((size_t)256 * 256, 0.0);
-      for (int64_t j = 0; j < n_jobs; j++) {
-        const float *W = h.data() + j * 65536;
-        for (int r = 0; r < 256; r++)
-          for (int c = 0; c < 256; c++) G[(size_t)r * 256 + c] += (double)W[r * 256 + c] + (double)W[c * 256 + r];
-      }
-      for (int64_t r = 0; r < K; r++)
-        for (int64_t c = 0; c < K; c++) G_host[r * K + c] = (float)G[(size_t)r * 256 + c];
-      if (b_host)
-        for (int64_t k = 0; k < K; k++) {
-          const float *bp = h.data() + blk + k;
-          double acc = 0.0;
-          for (int64_t q = 0; q < n_jobs * kWGram256BParts; q++) acc += bp[q * 256];
-          b_host[k] = (float)acc;
-        }
-    } catch (...) {
-      cudaDeviceSynchronize();
-      cleanup();
-      throw;
-    }
-    cleanup();
-  });
-}
-
-// ---------------- row-sharded multi-GPU ----------------
-
-int ials_trainer_create_sharded(const ials_model_config *config, int64_t n_users, int64_t n_items,
-                                int64_t user_begin, int64_t user_end, const int64_t *u_indptr,
-                                const int32_t *u_indices, const float *u_data, int64_t item_begin,
-                                int64_t item_end, const int64_t *i_indptr, const int32_t *i_indices,
-                                const float *i_data, int csr_on_device, int init_on_device,
-                                int device, ials_trainer **out) {
-  return guarded([&] {
-    require(out != nullptr, "out is null");
-    *out = nullptr;
-    require(0 <= user_begin && user_begin <= user_end && user_end <= n_users, "bad user shard");
-    require(0 <= item_begin && item_begin <= item_end && item_end <= n_items, "bad item shard");
-    ials_trainer *t = new_trainer(config, n_users, n_items, device);
-    try {
-      DeviceGuard g(device);
-      alloc_common(t);
-      // rows [user_begin, user_end) of X and rows [item_begin, item_end) of X^T
-      upload_csr(t->X, user_end - user_begin, n_items, u_indptr, u_indices, u_data, csr_on_device != 0);
-      upload_csr(t->Xt, item_end - item_begin, n_users, i_indptr, i_indices, i_data, csr_on_device != 0);
-      t->X.row_base = user_begin;
-      t->Xt.row_base = item_begin;
-      plan_csr(t, t->X);
-      plan_csr(t, t->Xt);
-      t->has_X = true;
-      t->sharded = true;
-      t->shard[0][0] = user_begin; t->shard[0][1] = user_end;
-      t->shard[1][0] = item_begin; t->shard[1][1] = item_end;
-      if (init_on_device) {
-        if (t->cfg.init_stdev > 0) {
-          const float sd = (float)(t->cfg.init_stdev / std::sqrt((double)t->K));
-          for (int side = 0; side < 2; side++)
-            launch_init_normal(t->factor[side], t->n_rows(side), t->K, t->ld, sd,
-                               (uint64_t)(uint32_t)t->cfg.random_seed, t->stream);
-          CUDA_CHECK(cudaStreamSynchronize(t->stream));
-        }
-      } else {
-        init_factors_host_rng(t);
-      }
-    } catch (...) {
-      ials_trainer_destroy(t);
-      throw;
-    }
-    *out = t;
-  });
-}
-
-int ials_trainer_gram_partial(ials_trainer *t, int factor_side, float **d_out, int64_t *count) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(factor_side == 0 || factor_side == 1, "side must be 0 or 1");
-    DeviceGuard g(t->device);
-    const int64_t b = t->sharded ? t->shard[factor_side][0] : 0;
-    const int64_t e = t->sharded ? t->shard[factor_side][1] : t->n_rows(factor_side);
-    float *dst = t->P[1 - factor_side];
-    gram_rows(t, factor_side, b, e, dst);
-    if (d_out) *d_out = dst;
-    if (count) *count = (int64_t)t->ld * t->ld;
-  });
-}
-
-int ials_trainer_solve_shard(ials_trainer *t, int side, const ials_solver_config *solver) {
-  return guarded([&] {
-    require(t != nullptr, "trainer is null");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    check_solver(solver);
-    if (!t->has_X) throw std::runtime_error("no interaction matrix");
-    DeviceGuard g(t->device);
-    const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
-    SolveArgs a = make_args(t, side, t->factor[side], csr, solver);
-    a.n_peers = t->n_peers[side];
-    for (int p = 0; p < a.n_peers; p++) a.peers[p] = t->peers[side][p];
-    if (side == 0) consume_flagged_upload(t, solver, a, csr.row_base);
-    run_solver(t, a, csr, solver, t->stream);
-  });
-}
-
-int ials_trainer_shard_range(ials_trainer *t, int side, int64_t *begin, int64_t *end) {
-  return guarded([&] {
-    require(t != nullptr && begin != nullptr && end != nullptr, "null argument");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    *begin = t->sharded ? t->shard[side][0] : 0;
-    *end = t->sharded ? t->shard[side][1] : t->n_rows(side);
-  });
-}
-
-int ials_trainer_ipc_handle(ials_trainer *t, int side, unsigned char handle_out[64]) {
-  return guarded([&] {
-    require(t != nullptr && handle_out != nullptr, "null argument");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
-    DeviceGuard g(t->device);
-    cudaIpcMemHandle_t h;
-    CUDA_CHECK(cudaIpcGetMemHandle(&h, t->factor[side]));
-    std::memcpy(handle_out, &h, 64);
-  });
-}
-
-int ials_trainer_ipc_open_peers(ials_trainer *t, int side, const unsigned char *handles, int world,
-                                int rank) {
-  return guarded([&] {
-    require(t != nullptr && handles != nullptr, "null argument");
-    require(side == 0 || side == 1, "side must be 0 or 1");
-    require(world >= 1 && world <= 9 && rank >= 0 && rank < world, "world must be <= 9");
-    DeviceGuard g(t->device);
-    for (int p = 0; p < t->n_peers[side]; p++) cudaIpcCloseMemHandle(t->peers[side][p]);
-    t->n_peers[side] = 0;
-    for (int r = 0; r < world; r++) {
-      if (r == rank) continue;
-      cudaIpcMemHandle_t h;
-      std::memcpy(&h, handles + 64 * r, 64);
-      void *p = nullptr;
-      CUDA_CHECK(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
-      t->peers[side][t->n_peers[side]++] = (float *)p;
-    }
   });
 }
 

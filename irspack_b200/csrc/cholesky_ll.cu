@@ -1,6 +1,6 @@
 // K3 Cholesky row solve for 256-column factors, after the tensor-core Gram (replaces
 // Solver::step_cholesky, /root/reference/cpp_source/als/IALSTrainer.hpp:273-331, for the rows whose
-// rank updates -- BatchedRankUpdater, :37-58 -- were done by wgram.cu; api.cu solve_cholesky_tensor).
+// rank updates -- BatchedRankUpdater, :37-58 -- were done by wgram.cu; solve.cu solve_cholesky_tensor).
 //
 // Per row:  A = P + G + reg_u I  (G = sum c y y^T from the Gram workspace),  A = U^T U,
 // U^T z = b,  U x = z.
@@ -95,7 +95,7 @@ struct LLSmem {
 };
 static_assert(2 * kStagePivots * kStripLd <= kNB * kRowLd0, "the strips alias the block row buffer");
 
-// Workspace of one chunk of Gram jobs (api.cu solve_cholesky_tensor, wgram.cu wgram256_kernel):
+// Workspace of one chunk of Gram jobs (solve.cu solve_cholesky_tensor, wgram.cu wgram256_kernel):
 //   W [JC][256][256] | b [JC][kWGram256BParts][256];   G = W + W^T
 struct LLArgs {
   const float *ws;

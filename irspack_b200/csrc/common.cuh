@@ -5,6 +5,7 @@
 
 #include <atomic>
 #include <stdint.h>
+#include <utility>
 
 #include <stdexcept>
 #include <string>
@@ -57,6 +58,70 @@ struct PerDeviceOnce {
   }
 };
 
+// Owning handles of device memory (and of the one pinned host array, the step_io flag source).
+// Each alloc() is one plain cudaMalloc and each release one cudaFree: allocation timing is part of
+// what the benchmarks measure, so there is no pool and no stream-ordered free.
+template <typename T, bool kPinnedHost = false>
+class Buffer {
+ public:
+  Buffer() = default;
+  Buffer(const Buffer &) = delete;
+  Buffer &operator=(const Buffer &) = delete;
+  Buffer(Buffer &&o) noexcept : p_(std::exchange(o.p_, nullptr)), n_(std::exchange(o.n_, 0)) {}
+  Buffer &operator=(Buffer &&o) noexcept {
+    if (this != &o) {
+      reset();
+      p_ = std::exchange(o.p_, nullptr);
+      n_ = std::exchange(o.n_, 0);
+    }
+    return *this;
+  }
+  ~Buffer() { reset(); }  // the status of the free is ignored, as in ials_trainer_destroy
+
+  // n elements, contents undefined; whatever was held is freed first
+  T *alloc(size_t n) {
+    if (p_) CUDA_CHECK(reset());
+    void *p = nullptr;
+    if (kPinnedHost)
+      CUDA_CHECK(cudaHostAlloc(&p, sizeof(T) * n, cudaHostAllocDefault));
+    else
+      CUDA_CHECK(cudaMalloc(&p, sizeof(T) * n));
+    p_ = static_cast<T *>(p);
+    n_ = n;
+    return p_;
+  }
+  // grow-only: reallocates (the contents are not kept) when fewer than n elements are held
+  T *ensure(size_t n) { return n > n_ ? alloc(n) : p_; }
+  cudaError_t reset() {
+    T *p = std::exchange(p_, nullptr);
+    n_ = 0;
+    if (!p) return cudaSuccess;
+    return kPinnedHost ? cudaFreeHost(p) : cudaFree(p);
+  }
+
+  T *get() const { return p_; }
+  size_t size() const { return n_; }
+
+ private:
+  T *p_ = nullptr;
+  size_t n_ = 0;
+};
+
+template <typename T>
+using DeviceBuffer = Buffer<T>;
+template <typename T>
+using PinnedBuffer = Buffer<T, true>;
+
+// Declared after the temporary buffers of a call, these run before the buffers are freed, on the
+// error path too: the work enqueued on them has finished (cudaFree is not relied on to wait for it).
+struct StreamSyncOnExit {
+  cudaStream_t s;
+  ~StreamSyncOnExit() { cudaStreamSynchronize(s); }
+};
+struct DeviceSyncOnExit {
+  ~DeviceSyncOnExit() { cudaDeviceSynchronize(); }
+};
+
 // Count of kernels launched by this library (bench.py reports it as gpu_launches).
 extern int64_t g_kernel_launches;
 inline void count_launch(int n = 1) { __atomic_fetch_add(&g_kernel_launches, (int64_t)n, __ATOMIC_RELAXED); }
@@ -64,25 +129,28 @@ inline void count_launch(int n = 1) { __atomic_fetch_add(&g_kernel_launches, (in
 __host__ __device__ inline int64_t round_up(int64_t x, int64_t m) { return (x + m - 1) / m * m; }
 __host__ __device__ inline int64_t ceil_div(int64_t x, int64_t m) { return (x + m - 1) / m; }
 
+// Rows of a CSR whose neighbour lists are cut into jobs of <= job_len entries for the tensor-core
+// Gram: the first n_heavy entries of the CSR's `order` (jobs of the h-th: [heavy_first_job[h],
+// heavy_first_job[h + 1]))
+struct JobPlan {
+  int64_t n_heavy = 0, n_jobs = 0, nnz_heavy = 0;
+  DeviceBuffer<int64_t> job_begin, job_end;  // [n_jobs]
+  DeviceBuffer<int32_t> heavy_first_job;     // [n_heavy + 1]
+};
+
 // CSR in device memory.
 struct DeviceCsr {
   int64_t n_rows = 0, n_cols = 0, nnz = 0;
   int64_t row_base = 0;  // global index of CSR row 0 (row shards; 0 for a full matrix)
-  int64_t *indptr = nullptr;
-  int32_t *indices = nullptr;
-  float *data = nullptr;
+  DeviceBuffer<int64_t> indptr;
+  DeviceBuffer<int32_t> indices;
+  DeviceBuffer<float> data;
   // rows sorted by descending degree (longest-processing-time-first schedule)
-  int32_t *order = nullptr;
+  DeviceBuffer<int32_t> order;
   int64_t max_degree = 0;
-  // "heavy" rows (degree > threshold) are the first n_heavy entries of `order`; their
-  // neighbour lists are cut into jobs of <= job_len entries for the tensor-core Gram
-  // (jobs of heavy row h: [heavy_first_job[h], heavy_first_job[h + 1]))
-  int64_t n_heavy = 0, n_jobs = 0, nnz_heavy = 0;
-  int64_t *job_begin = nullptr, *job_end = nullptr;
-  int32_t *heavy_first_job = nullptr;
+  JobPlan heavy;  // "heavy" rows (degree > threshold)
   bool has_negative = false;  // some stored value < 0: sqrt-weighted Gram not applicable
   int sorted_state = -1;      // column ids strictly ascending in every row? (-1: not checked yet)
-  void free_all();
 };
 
 // Arguments common to the per-row solvers (one half-epoch).
@@ -169,10 +237,9 @@ constexpr int kWGram256BParts = 8;  // producer warps of wgram256_kernel
 // Workspace of the tensor-core K1 Gram: block jobs over contiguous rows + their partials.
 struct GramWorkspace {
   int max_jobs = 0;
-  int64_t *job_begin = nullptr, *job_end = nullptr;  // [max_jobs]
-  float *W = nullptr;                                // [max_jobs x 128 x 128]
+  DeviceBuffer<int64_t> job_begin, job_end;  // [max_jobs]
+  DeviceBuffer<float> W;                     // [max_jobs x 128 x 128]
   void alloc(int jobs);
-  void free_all();
 };
 // P = alpha0 * Y[row_begin:row_end]^T Y[...] on tcgen05 (ld == 128 only)
 void launch_gram_tc(const float *Y, int64_t row_begin, int64_t row_end, float alpha0,
@@ -180,7 +247,9 @@ void launch_gram_tc(const float *Y, int64_t row_begin, int64_t row_end, float al
 
 void build_transpose(const DeviceCsr &X, DeviceCsr &Xt, cudaStream_t s);
 void build_row_order(DeviceCsr &X, cudaStream_t s);
-void build_heavy_plan(DeviceCsr &X, int64_t threshold, int64_t job_len, cudaStream_t s);
+bool csr_has_negative(const DeviceCsr &X, cudaStream_t s);
+// rows of X (in X.order) with more than `threshold` entries, cut into jobs of <= job_len entries
+void build_heavy_plan(const DeviceCsr &X, int64_t threshold, int64_t job_len, JobPlan &plan, cudaStream_t s);
 // Dense CG on explicitly formed normal equations (dense_cg.cu): heavy rows only.
 struct DenseSolveArgs {
   SolveArgs base;                 // target / P / CSR / order / hyper-parameters / peers
@@ -220,7 +289,7 @@ void launch_topk_rows(const float *scores, int64_t out_ld, int64_t n_rows, int64
                       int32_t *out_idx, float *out_score, int32_t *out_count, cudaStream_t s);
 
 // score_tc.cu: scores + seen mask + top-k fused on tcgen05 (ld in {32, 64, 96, 128}, k <= 128;
-// mask rows strictly ascending).  IALS_SCORE=simt keeps the three-kernel FP32 SIMT path.
+// mask rows strictly ascending).
 bool score_tc_supported(int ld, int64_t k);
 size_t score_tc_scratch_bytes(int64_t n_rows, int64_t n_items, int64_t k);
 bool csr_rows_strictly_sorted(const int64_t *indptr, const int32_t *indices, int64_t n_rows,

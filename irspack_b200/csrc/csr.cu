@@ -9,23 +9,6 @@
 
 namespace ials {
 
-void DeviceCsr::free_all() {
-  if (indptr) cudaFree(indptr);
-  if (indices) cudaFree(indices);
-  if (data) cudaFree(data);
-  if (order) cudaFree(order);
-  if (job_begin) cudaFree(job_begin);
-  if (job_end) cudaFree(job_end);
-  if (heavy_first_job) cudaFree(heavy_first_job);
-  job_begin = job_end = nullptr;
-  heavy_first_job = nullptr;
-  n_heavy = n_jobs = 0;
-  indptr = nullptr;
-  indices = nullptr;
-  data = nullptr;
-  order = nullptr;
-}
-
 namespace {
 
 // row id of every stored element: one warp per row, lanes stride the row.
@@ -151,102 +134,95 @@ void build_transpose(const DeviceCsr &X, DeviceCsr &Xt, cudaStream_t s) {
   Xt.n_rows = X.n_cols;
   Xt.n_cols = X.n_rows;
   Xt.nnz = X.nnz;
-  CUDA_CHECK(cudaMalloc(&Xt.indptr, sizeof(int64_t) * (Xt.n_rows + 1)));
-  CUDA_CHECK(cudaMalloc(&Xt.indices, sizeof(int32_t) * std::max<int64_t>(X.nnz, 1)));
-  CUDA_CHECK(cudaMalloc(&Xt.data, sizeof(float) * std::max<int64_t>(X.nnz, 1)));
+  Xt.indptr.alloc(Xt.n_rows + 1);
+  Xt.indices.alloc(std::max<int64_t>(X.nnz, 1));
+  Xt.data.alloc(std::max<int64_t>(X.nnz, 1));
   const int64_t nnz = X.nnz;
   if (nnz == 0) {
-    CUDA_CHECK(cudaMemsetAsync(Xt.indptr, 0, sizeof(int64_t) * (Xt.n_rows + 1), s));
+    CUDA_CHECK(cudaMemsetAsync(Xt.indptr.get(), 0, sizeof(int64_t) * (Xt.n_rows + 1), s));
     return;
   }
-  int32_t *row_of = nullptr, *cols_sorted = nullptr;
-  uint32_t *perm_in = nullptr, *perm_out = nullptr;
-  CUDA_CHECK(cudaMalloc(&row_of, sizeof(int32_t) * nnz));
-  CUDA_CHECK(cudaMalloc(&cols_sorted, sizeof(int32_t) * nnz));
-  CUDA_CHECK(cudaMalloc(&perm_in, sizeof(uint32_t) * nnz));
-  CUDA_CHECK(cudaMalloc(&perm_out, sizeof(uint32_t) * nnz));
+  DeviceBuffer<int32_t> row_of, cols_sorted;
+  DeviceBuffer<uint32_t> perm_in, perm_out;
+  DeviceBuffer<char> tmp;
+  StreamSyncOnExit sync{s};
+  row_of.alloc(nnz);
+  cols_sorted.alloc(nnz);
+  perm_in.alloc(nnz);
+  perm_out.alloc(nnz);
   const int T = 256;
   expand_rows_kernel<<<(unsigned)std::min<int64_t>(ceil_div(X.n_rows * kWarp, T), 65535 * 8), T, 0,
-                       s>>>(X.indptr, X.n_rows, row_of); count_launch();
-  iota_kernel<<<(unsigned)ceil_div(nnz, T), T, 0, s>>>(perm_in, nnz); count_launch();
+                       s>>>(X.indptr.get(), X.n_rows, row_of.get()); count_launch();
+  iota_kernel<<<(unsigned)ceil_div(nnz, T), T, 0, s>>>(perm_in.get(), nnz); count_launch();
   // stable LSD radix sort by column keeps rows ascending inside each column
   size_t tmp_bytes = 0;
   const int end_bit = bits_for(X.n_cols);
-  CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, X.indices, cols_sorted, perm_in,
-                                             perm_out, nnz, 0, end_bit, s));
-  void *tmp = nullptr;
-  CUDA_CHECK(cudaMalloc(&tmp, tmp_bytes));
-  CUDA_CHECK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, X.indices, cols_sorted, perm_in,
-                                             perm_out, nnz, 0, end_bit, s));
-  gather_transposed_kernel<<<(unsigned)ceil_div(nnz, T), T, 0, s>>>(perm_out, row_of, X.data, nnz,
-                                                                    Xt.indices, Xt.data); count_launch();
-  lower_bound_kernel<<<(unsigned)ceil_div(Xt.n_rows + 1, T), T, 0, s>>>(cols_sorted, nnz,
-                                                                        Xt.n_rows, Xt.indptr); count_launch();
+  CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, X.indices.get(), cols_sorted.get(), perm_in.get(),
+                                             perm_out.get(), nnz, 0, end_bit, s));
+  tmp.alloc(tmp_bytes);
+  CUDA_CHECK(cub::DeviceRadixSort::SortPairs(tmp.get(), tmp_bytes, X.indices.get(), cols_sorted.get(), perm_in.get(),
+                                             perm_out.get(), nnz, 0, end_bit, s));
+  gather_transposed_kernel<<<(unsigned)ceil_div(nnz, T), T, 0, s>>>(perm_out.get(), row_of.get(), X.data.get(), nnz,
+                                                                    Xt.indices.get(), Xt.data.get()); count_launch();
+  lower_bound_kernel<<<(unsigned)ceil_div(Xt.n_rows + 1, T), T, 0, s>>>(cols_sorted.get(), nnz,
+                                                                        Xt.n_rows, Xt.indptr.get()); count_launch();
   CUDA_CHECK(cudaGetLastError());
   CUDA_CHECK(cudaStreamSynchronize(s));
-  cudaFree(tmp);
-  cudaFree(row_of);
-  cudaFree(cols_sorted);
-  cudaFree(perm_in);
-  cudaFree(perm_out);
 }
 
 void build_row_order(DeviceCsr &X, cudaStream_t s) {
   const int64_t n = X.n_rows;
-  CUDA_CHECK(cudaMalloc(&X.order, sizeof(int32_t) * std::max<int64_t>(n, 1)));
+  X.order.alloc(std::max<int64_t>(n, 1));
   X.max_degree = 0;
   if (n == 0) return;
-  uint32_t *deg = nullptr, *deg_sorted = nullptr, *ids = nullptr;
-  CUDA_CHECK(cudaMalloc(&deg, sizeof(uint32_t) * n));
-  CUDA_CHECK(cudaMalloc(&deg_sorted, sizeof(uint32_t) * n));
-  CUDA_CHECK(cudaMalloc(&ids, sizeof(uint32_t) * n));
+  DeviceBuffer<uint32_t> deg, deg_sorted, ids;
+  DeviceBuffer<char> tmp;
+  StreamSyncOnExit sync{s};
+  deg.alloc(n);
+  deg_sorted.alloc(n);
+  ids.alloc(n);
   const int T = 256;
-  degree_kernel<<<(unsigned)ceil_div(n, T), T, 0, s>>>(X.indptr, n, deg, ids); count_launch();
+  degree_kernel<<<(unsigned)ceil_div(n, T), T, 0, s>>>(X.indptr.get(), n, deg.get(), ids.get()); count_launch();
   size_t tmp_bytes = 0;
-  CUDA_CHECK(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, deg, deg_sorted, ids,
-                                                       (uint32_t *)X.order, n, 0, 32, s));
-  void *tmp = nullptr;
-  CUDA_CHECK(cudaMalloc(&tmp, tmp_bytes));
-  CUDA_CHECK(cub::DeviceRadixSort::SortPairsDescending(tmp, tmp_bytes, deg, deg_sorted, ids,
-                                                       (uint32_t *)X.order, n, 0, 32, s));
+  CUDA_CHECK(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, deg.get(), deg_sorted.get(), ids.get(),
+                                                       (uint32_t *)X.order.get(), n, 0, 32, s));
+  tmp.alloc(tmp_bytes);
+  CUDA_CHECK(cub::DeviceRadixSort::SortPairsDescending(tmp.get(), tmp_bytes, deg.get(), deg_sorted.get(), ids.get(),
+                                                       (uint32_t *)X.order.get(), n, 0, 32, s));
   uint32_t maxdeg = 0;
-  CUDA_CHECK(cudaMemcpyAsync(&maxdeg, deg_sorted, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaMemcpyAsync(&maxdeg, deg_sorted.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
   CUDA_CHECK(cudaStreamSynchronize(s));
   X.max_degree = maxdeg;
-  cudaFree(tmp);
-  cudaFree(deg);
-  cudaFree(deg_sorted);
-  cudaFree(ids);
+}
+
+// Some stored value < 0 (or NaN)?  The rows of such a matrix all take the light path.
+bool csr_has_negative(const DeviceCsr &X, cudaStream_t s) {
+  if (X.nnz == 0) return false;
+  DeviceBuffer<float> d_min;
+  DeviceBuffer<char> tmp;
+  StreamSyncOnExit sync{s};
+  size_t tmp_bytes = 0;
+  d_min.alloc(1);
+  CUDA_CHECK(cub::DeviceReduce::Min(nullptr, tmp_bytes, X.data.get(), d_min.get(), X.nnz, s));
+  tmp.alloc(tmp_bytes);
+  CUDA_CHECK(cub::DeviceReduce::Min(tmp.get(), tmp_bytes, X.data.get(), d_min.get(), X.nnz, s));
+  float h_min = 0.f;
+  CUDA_CHECK(cudaMemcpyAsync(&h_min, d_min.get(), sizeof(float), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  return !(h_min >= 0.f);
 }
 
 // Host-side planning (once per matrix): which rows go to the tensor-core path and how
-// their neighbour lists are cut into jobs.  Also detects negative stored values.
-void build_heavy_plan(DeviceCsr &X, int64_t threshold, int64_t job_len, cudaStream_t s) {
-  X.n_heavy = X.n_jobs = X.nnz_heavy = 0;
-  X.has_negative = false;
+// their neighbour lists are cut into jobs.
+void build_heavy_plan(const DeviceCsr &X, int64_t threshold, int64_t job_len, JobPlan &plan, cudaStream_t s) {
+  plan = JobPlan{};
   const int64_t n = X.n_rows;
-  if (n == 0 || X.order == nullptr) return;
+  if (n == 0 || X.order.get() == nullptr) return;
   std::vector<int64_t> indptr(n + 1);
   std::vector<int32_t> order(n);
-  CUDA_CHECK(cudaMemcpyAsync(indptr.data(), X.indptr, sizeof(int64_t) * (n + 1), cudaMemcpyDeviceToHost, s));
-  CUDA_CHECK(cudaMemcpyAsync(order.data(), X.order, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, s));
-  if (X.nnz > 0) {  // min of the stored values
-    float *d_min = nullptr;
-    void *tmp = nullptr;
-    size_t tmp_bytes = 0;
-    CUDA_CHECK(cudaMalloc(&d_min, sizeof(float)));
-    CUDA_CHECK(cub::DeviceReduce::Min(nullptr, tmp_bytes, X.data, d_min, X.nnz, s));
-    CUDA_CHECK(cudaMalloc(&tmp, tmp_bytes));
-    CUDA_CHECK(cub::DeviceReduce::Min(tmp, tmp_bytes, X.data, d_min, X.nnz, s));
-    float h_min = 0.f;
-    CUDA_CHECK(cudaMemcpyAsync(&h_min, d_min, sizeof(float), cudaMemcpyDeviceToHost, s));
-    CUDA_CHECK(cudaStreamSynchronize(s));
-    cudaFree(tmp);
-    cudaFree(d_min);
-    X.has_negative = !(h_min >= 0.f);
-  } else {
-    CUDA_CHECK(cudaStreamSynchronize(s));
-  }
+  CUDA_CHECK(cudaMemcpyAsync(indptr.data(), X.indptr.get(), sizeof(int64_t) * (n + 1), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaMemcpyAsync(order.data(), X.order.get(), sizeof(int32_t) * n, cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
   std::vector<int64_t> jb, je;
   std::vector<int32_t> first;
   int64_t h = 0;
@@ -255,7 +231,7 @@ void build_heavy_plan(DeviceCsr &X, int64_t threshold, int64_t job_len, cudaStre
     const int64_t b = indptr[u], e = indptr[u + 1];
     if (e - b <= threshold) break;
     first.push_back((int32_t)jb.size());
-    X.nnz_heavy += e - b;
+    plan.nnz_heavy += e - b;
     const int64_t pieces = ceil_div(e - b, job_len);
     const int64_t per = round_up(ceil_div(e - b, pieces), 32);  // whole pipeline stages
     for (int64_t p = b; p < e; p += per) {
@@ -264,15 +240,16 @@ void build_heavy_plan(DeviceCsr &X, int64_t threshold, int64_t job_len, cudaStre
     }
   }
   first.push_back((int32_t)jb.size());
-  X.n_heavy = h;
-  X.n_jobs = (int64_t)jb.size();
-  if (X.n_heavy == 0) return;
-  CUDA_CHECK(cudaMalloc(&X.job_begin, sizeof(int64_t) * X.n_jobs));
-  CUDA_CHECK(cudaMalloc(&X.job_end, sizeof(int64_t) * X.n_jobs));
-  CUDA_CHECK(cudaMalloc(&X.heavy_first_job, sizeof(int32_t) * first.size()));
-  CUDA_CHECK(cudaMemcpy(X.job_begin, jb.data(), sizeof(int64_t) * X.n_jobs, cudaMemcpyHostToDevice));
-  CUDA_CHECK(cudaMemcpy(X.job_end, je.data(), sizeof(int64_t) * X.n_jobs, cudaMemcpyHostToDevice));
-  CUDA_CHECK(cudaMemcpy(X.heavy_first_job, first.data(), sizeof(int32_t) * first.size(), cudaMemcpyHostToDevice));
+  plan.n_heavy = h;
+  plan.n_jobs = (int64_t)jb.size();
+  if (plan.n_heavy == 0) return;
+  plan.job_begin.alloc(plan.n_jobs);
+  plan.job_end.alloc(plan.n_jobs);
+  plan.heavy_first_job.alloc(first.size());
+  CUDA_CHECK(cudaMemcpy(plan.job_begin.get(), jb.data(), sizeof(int64_t) * plan.n_jobs, cudaMemcpyHostToDevice));
+  CUDA_CHECK(cudaMemcpy(plan.job_end.get(), je.data(), sizeof(int64_t) * plan.n_jobs, cudaMemcpyHostToDevice));
+  CUDA_CHECK(cudaMemcpy(plan.heavy_first_job.get(), first.data(), sizeof(int32_t) * first.size(),
+                        cudaMemcpyHostToDevice));
 }
 
 void launch_gather_rows(const float *src, int ld, const int64_t *rows, int64_t n_rows, float *dst,

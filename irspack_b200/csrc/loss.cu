@@ -92,11 +92,11 @@ void launch_loss(const float *user, const float *item, int64_t U, int64_t I, int
   const int T = 256;
   if (U > 0)
     loss_rows_kernel<<<(unsigned)std::min<int64_t>(ceil_div(U * kWarp, T), kNumSMsB200 * 16), T, 0,
-                       s>>>(user, item, U, I, ld, X.indptr, X.indices, X.data, alpha0, reg, nu,
+                       s>>>(user, item, U, I, ld, X.indptr.get(), X.indices.get(), X.data.get(), alpha0, reg, nu,
                             bias, 1, prior_u, d_out); count_launch();
   if (I > 0)
     loss_rows_kernel<<<(unsigned)std::min<int64_t>(ceil_div(I * kWarp, T), kNumSMsB200 * 16), T, 0,
-                       s>>>(item, user, I, U, ld, Xt.indptr, Xt.indices, Xt.data, alpha0, reg, nu,
+                       s>>>(item, user, I, U, ld, Xt.indptr.get(), Xt.indices.get(), Xt.data.get(), alpha0, reg, nu,
                             bias, 0, prior_i, d_out); count_launch();
   CUDA_CHECK(cudaGetLastError());
 }

@@ -640,17 +640,17 @@ size_t score_tc_scratch_bytes(int64_t n_rows, int64_t n_items, int64_t k) {
 bool csr_rows_strictly_sorted(const int64_t *indptr, const int32_t *indices, int64_t n_rows,
                               cudaStream_t s) {
   if (n_rows == 0) return true;
-  int *d_flag = nullptr;
-  CUDA_CHECK(cudaMalloc(&d_flag, sizeof(int)));
-  CUDA_CHECK(cudaMemsetAsync(d_flag, 0, sizeof(int), s));
+  DeviceBuffer<int> d_flag;
+  StreamSyncOnExit sync{s};
+  d_flag.alloc(1);
+  CUDA_CHECK(cudaMemsetAsync(d_flag.get(), 0, sizeof(int), s));
   const int T = 256;
-  csr_sorted_kernel<<<(unsigned)ceil_div(n_rows * kWarp, T), T, 0, s>>>(indptr, indices, n_rows, d_flag);
+  csr_sorted_kernel<<<(unsigned)ceil_div(n_rows * kWarp, T), T, 0, s>>>(indptr, indices, n_rows, d_flag.get());
   count_launch();
   CUDA_CHECK(cudaGetLastError());
   int h = 0;
-  CUDA_CHECK(cudaMemcpyAsync(&h, d_flag, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaMemcpyAsync(&h, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost, s));
   CUDA_CHECK(cudaStreamSynchronize(s));
-  CUDA_CHECK(cudaFree(d_flag));
   return h == 0;
 }
 

@@ -295,7 +295,7 @@ __global__ void __launch_bounds__(kThreads, 1) wgram_kernel(WGramArgs a) {
 
 // ---------------------------------------------------------------------------------------------
 // Whole Gram of 256-column factor rows in ONE pass over the neighbours (K = 256 Cholesky,
-// BASELINE configs[2]; api.cu solve_cholesky_tensor).  A 256-float row is two halves y0 | y1;
+// BASELINE configs[2]; solve.cu solve_cholesky_tensor).  A 256-float row is two halves y0 | y1;
 // with u = sqrt(c) y = hi + lo as above,
 //     W = 1/2 hi (hi + 2 lo)^T      (256 x 256),        G = sum c y y^T = W + W^T + O(2^-22)
 // (W + W^T = hi hi^T + hi lo^T + lo hi^T; 2 lo is as exact in TF32 as lo).  A stage holds four
@@ -576,17 +576,9 @@ unsigned grid_for(int64_t n_jobs) {
 
 void GramWorkspace::alloc(int jobs) {
   max_jobs = jobs;
-  CUDA_CHECK(cudaMalloc(&job_begin, sizeof(int64_t) * jobs));
-  CUDA_CHECK(cudaMalloc(&job_end, sizeof(int64_t) * jobs));
-  CUDA_CHECK(cudaMalloc(&W, sizeof(float) * (size_t)jobs * KP * KP));
-}
-void GramWorkspace::free_all() {
-  if (job_begin) cudaFree(job_begin);
-  if (job_end) cudaFree(job_end);
-  if (W) cudaFree(W);
-  job_begin = job_end = nullptr;
-  W = nullptr;
-  max_jobs = 0;
+  job_begin.alloc(jobs);
+  job_end.alloc(jobs);
+  W.alloc((size_t)jobs * KP * KP);
 }
 
 void launch_gram_tc(const float *Y, int64_t row_begin, int64_t row_end, float alpha0,
@@ -598,17 +590,17 @@ void launch_gram_tc(const float *Y, int64_t row_begin, int64_t row_end, float al
   }
   // at least 8 stages of work per job, at most one job per workspace slot
   const int n_jobs = (int)std::max<int64_t>(1, std::min<int64_t>(ws.max_jobs, n / (8 * KT)));
-  block_jobs_kernel<<<1, 256, 0, s>>>(row_begin, row_end, n_jobs, ws.job_begin, ws.job_end);
+  block_jobs_kernel<<<1, 256, 0, s>>>(row_begin, row_end, n_jobs, ws.job_begin.get(), ws.job_end.get());
   count_launch();
   WGramArgs a{};
   a.Y = Y;
   a.ld = KP;
-  a.job_begin = ws.job_begin;
-  a.job_end = ws.job_end;
+  a.job_begin = ws.job_begin.get();
+  a.job_end = ws.job_end.get();
   a.n_jobs = n_jobs;
-  a.W = ws.W;
+  a.W = ws.W.get();
   launch_wgram(a, s);
-  launch_wgram_reduce_sym(ws.W, n_jobs, alpha0, P, s);
+  launch_wgram_reduce_sym(ws.W.get(), n_jobs, alpha0, P, s);
 }
 
 // One 128 x 128 block per job.  a.Y may point into a wider row (Y + 128 with a.ld = 256: the

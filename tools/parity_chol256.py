@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cholesky half-epochs at K in (224, 256] (row stride 256) against the oracle; prints one JSON
 line with the errors.  The tensor-core route is the default; run under IALS_CHOL=simt to check the register-tiled kernel of
-irspack_b200/csrc/api.cu solve_cholesky_tensor (tests/test_zz_experimental.py does)."""
+irspack_b200/csrc/solve.cu solve_cholesky_tensor (tests/test_zz_experimental.py does)."""
 import json
 import os
 import sys
