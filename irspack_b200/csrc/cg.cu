@@ -172,11 +172,16 @@ void launch_solve_cg_simple(const SolveArgs &a, cudaStream_t s) {
     case 6: launch_nv<6>(a, s); break;
     case 7: launch_nv<7>(a, s); break;
     case 8: launch_nv<8>(a, s); break;
+    case 9: launch_nv<9>(a, s); break;
     case 10: launch_nv<10>(a, s); break;
+    case 11: launch_nv<11>(a, s); break;
     case 12: launch_nv<12>(a, s); break;
+    case 13: launch_nv<13>(a, s); break;
+    case 14: launch_nv<14>(a, s); break;
+    case 15: launch_nv<15>(a, s); break;
     case 16: launch_nv<16>(a, s); break;
-    default:
-      throw NotImplemented("CG solver: n_components must pad to 32..256, 320, 384 or 512");
+    default:  // new_trainer accepts K <= 512, so every stride it produces has a case above
+      throw NotImplemented("CG solver: the row stride must be a multiple of 32 in [32, 512]");
   }
 }
 

@@ -23,6 +23,7 @@ import scipy.sparse as sps
 import oracle
 import invariants as inv
 from backends import GpuBackend
+from parity import assert_close, dump_observed, make_pair, observe, solver_cfg
 
 pytestmark = pytest.mark.gpu
 
@@ -42,31 +43,13 @@ def core():
     return _ials_core
 
 
-_OBSERVED = []
-
-
-def observe(**numbers):
-    """Record the observed error of a comparison (written to gpurun_out/parity_observed.json
-    at the end of the module, so that the stated tolerances can be read against what holds)."""
-    import os
-
-    name = os.environ.get("PYTEST_CURRENT_TEST", "?").split("::")[-1].split(" ")[0]
-    _OBSERVED.append({"test": name, **{k: float(v) for k, v in numbers.items()}})
-
-
 @pytest.fixture(scope="module", autouse=True)
 def _dump_observed():
     yield
-    import json
     import os
 
     out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpurun_out")
-    try:
-        os.makedirs(out, exist_ok=True)
-        with open(os.path.join(out, "parity_observed.json"), "w") as f:
-            json.dump(_OBSERVED, f, indent=0)
-    except OSError:
-        pass
+    dump_observed(out)
 
 
 @pytest.fixture(scope="module")
@@ -75,46 +58,6 @@ def X_ml20m():
 
     U, I, nnz, K = SHAPES["ml20m"]
     return synth_csr(U, I, nnz, seed=1002)
-
-
-def make_pair(core, X, K, alpha0=0.1, reg=0.05, nu=1.0, loss="IALSPP", seed=1):
-    """(gpu trainer, f32 oracle, f64 oracle) with identical X and initial factors."""
-    from irspack_b200.synth import init_factors
-
-    U, I = X.shape
-    u0, i0 = init_factors(U, K, seed), init_factors(I, K, seed + 1)
-    cfg = (core.IALSModelConfigBuilder().set_K(K).set_alpha0(alpha0).set_reg(reg).set_nu(nu)
-           .set_loss_type(getattr(core.LossType, loss)).build())
-    g = core.IALSTrainer(cfg, X)
-    g.user, g.item = u0, i0
-    lt = oracle.LOSS_ORIGINAL if loss == "ORIGINAL" else oracle.LOSS_IALSPP
-    o32 = oracle.OracleTrainer(X, K, alpha0, reg, nu, lt, dtype=np.float32)
-    o64 = oracle.OracleTrainer(X, K, alpha0, reg, nu, lt, dtype=np.float64)
-    o32.user, o32.item = u0.copy(), i0.copy()
-    o64.user, o64.item = u0.astype(np.float64), i0.astype(np.float64)
-    return g, o32, o64
-
-
-def solver_cfg(core, solver="CG", steps=3, n_threads=1):
-    st = core.SolverType.CG if solver == "CG" else core.SolverType.CHOLESKY
-    return (core.IALSSolverConfigBuilder().set_solver_type(st).set_max_cg_steps(steps)
-            .set_n_threads(n_threads).build())
-
-
-def assert_close(gpu, o32, o64, tol, guard=4, floor=1e-6):
-    """|gpu - f32 oracle| <= tol * scale, widened by twice the f32 oracle's own distance to
-    the float64 twin (two float32 evaluations of an ill-conditioned, unconverged CG can
-    only agree as well as each agrees with the exact arithmetic), and the GPU result must
-    be as close to the float64 twin as the f32 oracle is (factor ``guard``, plus ``floor`` of
-    the scale: 1e-6, or 1e-5 where the normal equations come from the 3xTF32 tensor-core Gram,
-    whose 2^-22 relative error is multiplied by the condition number of the row's system)."""
-    scale = np.abs(o32).max() + 1e-30
-    e_ref = np.abs(o32 - o64).max()
-    err = np.abs(gpu - o32).max()
-    e_gpu = np.abs(gpu - o64).max()
-    observe(gpu_vs_f32=err / scale, gpu_vs_f64=e_gpu / scale, f32_vs_f64=e_ref / scale, tol=tol)
-    assert err <= tol * scale + 2 * e_ref, f"max err {err:.3e} vs scale {scale:.3e} (f32-vs-f64 {e_ref:.3e})"
-    assert e_gpu <= guard * e_ref + floor * scale + 1e-9, (e_gpu, e_ref)
 
 
 # ---- the reference's own invariants, now on the CUDA backend ----
