@@ -21,7 +21,8 @@
  *     "device" pointers live on the trainer's CUDA device.
  *   - Dense matrices crossing the boundary are row-major float32 with exactly K
  *     columns (Eigen RowMajor DenseMatrix, cpp_source/als/definitions.hpp:9-10).
- *     Inside the library rows are padded to `ld = round_up(K, 32)` floats.
+ *     Inside the library rows are padded to `ld` floats: 128 for every K <= 128,
+ *     round_up(K, 32) above.
  *   - CSR: int64 indptr[n_rows + 1], int32 indices[nnz] (ascending within a
  *     row), float data[nnz]  (Eigen::SparseMatrix<float, RowMajor>).
  *   - Calls on one handle are synchronous and not re-entrant, like the

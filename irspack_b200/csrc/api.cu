@@ -280,6 +280,7 @@ void half_step(ials_trainer *t, int side, const ials_solver_config *sc) {
   if (t->sharded) throw std::runtime_error("sharded trainer: drive the epoch with gram_partial / solve_shard");
   if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix; it cannot train");
   check_feature_solver(t, sc);
+  check_feature_weight_shapes(t, false);
   epoch_side(t, side, sc);  // (a test entry: the epoch counter is not advanced)
 }
 
@@ -385,6 +386,7 @@ int ials_trainer_step_async(ials_trainer *t, const ials_solver_config *solver) {
     DeviceGuard g(t->device);
     if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix; it cannot train");
     check_feature_solver(t, solver);
+    check_feature_weight_shapes(t, false);
     prof_mark(t);
     for (int side = 0; side < 2; side++) epoch_side(t, side, solver);  // IALSTrainer.hpp:762-787
     t->epoch++;
@@ -458,13 +460,14 @@ int ials_trainer_step_io(ials_trainer *t, const ials_solver_config *solver, cons
             "factor pointer is null");
     if (t->sharded) throw std::runtime_error("sharded trainer: drive the epoch with gram_partial / solve_shard");
     if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix; it cannot train");
+    check_feature_solver(t, solver);
+    check_feature_weight_shapes(t, false);  // before the uploads: a rejected call leaves the factors as they were
     DeviceGuard g(t->device);
     ensure_copy_stream(t);
     // item first: the user half-epoch starts with Gram(item)
     if (t->I) rows_to_device(t->factor[1].get(), t->ld, item_in, t->K, t->I, t->stream);
     // the user factors are only the warm starts of the user rows: with the CG kernels of the
     // 128-column layout they arrive while the half-epoch runs (enqueue_flagged_user_upload)
-    check_feature_solver(t, solver);
     const bool overlap_upload = solver->solver_type == IALS_SOLVER_CG && t->ld == 128 && t->U > 0 &&
                                 !side_uses_features(t, 0);
     if (overlap_upload) {
@@ -623,6 +626,7 @@ int ials_trainer_compute_loss(ials_trainer *t, const ials_solver_config *solver,
     require(solver != nullptr && solver->n_threads > 0, "n_threads must be strictly positive.");
     if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix");
     if (t->sharded) throw NotImplemented("compute_loss on a row-sharded trainer is not implemented");
+    check_feature_weight_shapes(t, true);
     DeviceGuard g(t->device);
     gram_side(t, 0);
     gram_side(t, 1);

@@ -66,6 +66,18 @@ bool side_uses_features(const ials_trainer *t, int side) {
   return t->feature_aware && t->epoch >= t->feature_warmup && t->feat[side].n_w > 0;
 }
 
+// The stored features meet the stored weight in the prior F W and in the weight refit, which read
+// F.n_cols rows of the weight and of its cached Gram factor.  The setter accepts any row count (as
+// the reference's def_rw does), so the shape is checked where the two meet, before the first launch:
+// on the sides a step uses (`any_epoch` false) or on every side with a weight (compute_loss, which
+// does not look at the warm-up).
+void check_feature_weight_shapes(const ials_trainer *t, bool any_epoch) {
+  for (int side = 0; side < 2; side++) {
+    const bool used = any_epoch ? t->feature_aware && t->feat[side].n_w > 0 : side_uses_features(t, side);
+    if (used) validate_feature_cols(t, side, t->feat[side].F.n_cols);
+  }
+}
+
 // stored_user_feature_prior / stored_item_feature_prior (:1044-1050) into feat[side].prior
 const float *stored_prior(ials_trainer *t, int side) {
   ials_trainer::FeatureSide &f = t->feat[side];

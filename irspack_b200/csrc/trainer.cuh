@@ -181,6 +181,7 @@ void consume_flagged_upload(ials_trainer *t, const ials_solver_config *sc, Solve
 // api_features.cu
 void check_prior_defined(const ials_trainer *t, int side, bool has_empty_row);
 bool side_uses_features(const ials_trainer *t, int side);
+void check_feature_weight_shapes(const ials_trainer *t, bool any_epoch);
 const float *stored_prior(ials_trainer *t, int side);
 void update_feature_weight(ials_trainer *t, int side);
 void check_feature_solver(const ials_trainer *t, const ials_solver_config *sc);

@@ -23,8 +23,8 @@ import pytest
 import scipy.sparse as sps
 
 import oracle
-from parity import (assert_close, dump_observed, make_pair, np_cholesky_step, np_ialspp_step, observe,
-                    solver_cfg)
+from parity import (HSETS, assert_close, balanced_reg, dump_observed, hparams, make_data, make_pair,
+                    np_cholesky_step, np_ialspp_step, observe, solver_cfg, transpose)
 
 pytestmark = pytest.mark.gpu
 
@@ -58,99 +58,6 @@ def launches():
 def ialspp_cfg(core, S, iters):
     return (core.IALSSolverConfigBuilder().set_solver_type(core.SolverType.IALSPP)
             .set_ialspp_subspace_dimension(S).set_ialspp_iteration(iters).build())
-
-
-# ---- data ----
-
-def fill_empty(X, rng):
-    """One entry in every empty row and column (alpha0 = 0 leaves such a row singular)."""
-    X = sps.lil_matrix(X)
-    U, I = X.shape
-    for u in np.flatnonzero(np.diff(sps.csr_matrix(X).indptr) == 0):
-        X[u, rng.integers(I)] = 1.0
-    Xc = sps.csc_matrix(X)
-    for i in np.flatnonzero(np.diff(Xc.indptr) == 0):
-        X[rng.integers(U), i] = 1.0
-    X = sps.csr_matrix(X, dtype=np.float32)
-    X.sort_indices()
-    return X
-
-
-def add_long_rows(X, rng, degrees=(3000, 9000)):
-    """Rows 0 and 1 get ``degrees`` neighbours among a widened set of columns."""
-    U, I = X.shape
-    I2 = max(I, max(degrees) + 200)
-    X = sps.lil_matrix(sps.hstack([X, sps.csr_matrix((U, I2 - I), dtype=np.float32)]))
-    for u, d in enumerate(degrees):
-        X.rows[u] = []
-        X.data[u] = []
-        cols = np.sort(rng.choice(I2, d, replace=False))
-        X.rows[u] = list(cols)
-        X.data[u] = list(rng.integers(1, 4, d).astype(np.float32))
-    X = sps.csr_matrix(X, dtype=np.float32)
-    X.sort_indices()
-    return X
-
-
-def make_data(variant, long_rows=False, seed=3, nnz=12000):
-    """500 x 300 counts (1..5, ``nnz`` entries before filling), no empty row or column, in one of the variants:
-    counts | zeros: 5 % stored zeros and three rows of stored zeros only |
-    neg: 2 % of the values -0.25 | neg1: one value -0.25 | zeros+neg1."""
-    from irspack_b200.synth import synth_csr
-
-    rng = np.random.default_rng(seed)
-    X = fill_empty(synth_csr(500, 300, nnz, seed=seed, values="counts"), rng)
-    if long_rows:
-        X = add_long_rows(X, rng)
-    if "zeros" in variant:
-        X.data[rng.random(X.nnz) < 0.05] = 0.0
-        for u in (5, 6, 7):
-            X.data[X.indptr[u]:X.indptr[u + 1]] = 0.0
-    if variant == "neg":
-        X.data[rng.random(X.nnz) < 0.02] = -0.25
-    if variant.endswith("neg1"):
-        X.data[X.indptr[20] + 1] = -0.25
-    return X
-
-
-def transpose(X):
-    Xt = sps.csr_matrix(X.T)
-    Xt.sort_indices()
-    assert Xt.nnz == X.nnz  # stored zeros survive
-    return Xt
-
-
-# ---- hyper-parameter sets ----
-
-HSETS = {
-    # name: (nu, alpha0, reg, loss, perturbations that must move the answer)
-    "H0": (0.0, 0.1, 0.05, "IALSPP", ({"nu": 0.25},)),
-    "H1": (0.5, 2.0, 0.02, "ORIGINAL", ({"nu": 0.75}, {"loss": "IALSPP"})),
-    "H2": (2.0, 0.05, None, "IALSPP", ({"nu": 1.75},)),  # reg: see balanced_reg
-    "H3": (1.0, 0.0, 0.05, "ORIGINAL", ({"alpha0": 0.05},)),
-}
-
-
-def balanced_reg(X, K, alpha0, nu):
-    """reg at which reg_u of a median user row equals the mean diagonal of its Gram
-    alpha0 Y^T Y + sum c y y^T at the initial item factors, so neither the ridge nor the data
-    term dominates the row's system."""
-    from irspack_b200.synth import init_factors
-
-    Y = init_factors(X.shape[1], K, 2).astype(np.float64)
-    nnz = np.diff(X.indptr)
-    u = int(np.argsort(nnz)[len(nnz) // 2])
-    s, e = X.indptr[u], X.indptr[u + 1]
-    Yr = Y[X.indices[s:e]]
-    diag = alpha0 * (Y * Y).sum() / K + (np.abs(X.data[s:e])[:, None] * Yr * Yr).sum() / K
-    return float(diag / (alpha0 * X.shape[1] + (e - s)) ** nu)
-
-
-def hparams(name, X, K):
-    nu, alpha0, reg, loss, perturb = HSETS[name]
-    if reg is None:
-        reg = balanced_reg(X, K, alpha0, nu)
-    return dict(nu=nu, alpha0=alpha0, reg=reg, loss=loss), perturb
 
 
 # ---- references ----
