@@ -250,8 +250,8 @@ IALS_API int ials_trainer_recommend(ials_trainer *t, int64_t begin, int64_t end,
  * evaluator.py:115-136; allowed_item_indices of retrieve_recommend_from_score, util.hpp:426-504):
  * allow_n_lists = 1 (one list for every row) or end - begin (one per row), CSR with int32 item ids
  * strictly ascending inside a list.  Only items on a row's list can be returned (seen / masked items
- * are still dropped).  No score block ever leaves the device.  Needs the fused kernel (row stride
- * <= 128, k <= 128), otherwise IALS_ERR_NOT_IMPLEMENTED. */
+ * are still dropped).  No score block ever leaves the device.  Needs the fused kernel (any row
+ * stride, k <= 128, mask rows strictly ascending), otherwise IALS_ERR_NOT_IMPLEMENTED. */
 IALS_API int ials_trainer_recommend_allowed(ials_trainer *t, int64_t begin, int64_t end, int64_t k, int mask_mode,
                                             const int64_t *mask_indptr, const int32_t *mask_indices,
                                             int64_t allow_n_lists, const int64_t *allow_indptr,

@@ -163,7 +163,7 @@ static int recommend_impl(ials_trainer *t, const int64_t *user_idx, const float 
                                      t->stream));
       }
     }
-    const bool fused = score_tc_supported(t->ld, k) && mask_sorted;
+    const bool fused = score_topk_tc_supported(t->ld, k) && mask_sorted;
     // users picked by index: their factor rows are gathered into a dense block first
     const float *user_rows = t->factor[0].get() + begin * t->ld;
     int64_t *d_uidx = nullptr;
@@ -184,8 +184,7 @@ static int recommend_impl(ials_trainer *t, const int64_t *user_idx, const float 
       user_rows = padded;
     }
     if (allow_n_lists > 0 && !fused)
-      throw NotImplemented("allow-lists need the fused tensor-core kernel (row stride <= 128, cutoff <= 128, "
-                           "sorted mask rows)");
+      throw NotImplemented("allow-lists need the fused tensor-core kernel (cutoff <= 128, sorted mask rows)");
     if (fused) {
       // scores + mask + top-k in one tcgen05 kernel; only candidate keys touch HBM
       const int64_t slab_rows = std::max<int64_t>(128, ((1ll << 29) / (8 * 256)) / 128 * 128);

@@ -288,9 +288,11 @@ void launch_allow_rows(const float *src, float *dst, int64_t ld, const int64_t *
 void launch_topk_rows(const float *scores, int64_t out_ld, int64_t n_rows, int64_t n_items, int k,
                       int32_t *out_idx, float *out_score, int32_t *out_count, cudaStream_t s);
 
-// score_tc.cu: scores + seen mask + top-k fused on tcgen05 (ld in {32, 64, 96, 128}, k <= 128;
-// mask rows strictly ascending).
+// score_tc.cu: scores + seen mask + top-k fused on tcgen05 (ld a multiple of 32 in [32, 512],
+// k <= 128; mask rows strictly ascending).  The dense score block (launch_scores_tc) takes
+// ld <= 128 only: score_tc_supported(ld, 1).
 bool score_tc_supported(int ld, int64_t k);
+bool score_topk_tc_supported(int ld, int64_t k);
 size_t score_tc_scratch_bytes(int64_t n_rows, int64_t n_items, int64_t k);
 bool csr_rows_strictly_sorted(const int64_t *indptr, const int32_t *indices, int64_t n_rows,
                               cudaStream_t s);

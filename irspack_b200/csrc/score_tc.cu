@@ -28,6 +28,8 @@
 //               tau.  The mask is a cursor into the row's sorted CSR column list with a four-deep
 //               look-ahead queue in registers.
 //   warp 12     MMA issuer (one lane) + TMEM owner; accumulators double-buffered (2 x 256 cols).
+// Row strides 160..512 (WIDE) do not fit the parked user tile: there a stage carries the users'
+// chunk next to the items' (3 stages x 64 KB), streamed and split again for every item tile.
 // A small second kernel merges the per-split candidate lists and writes (index, score, count).
 #include <cub/block/block_radix_sort.cuh>
 
@@ -50,6 +52,8 @@ constexpr int STAGES = 3;
 constexpr int kMaxKc = 4;    // ld <= 128
 constexpr int kTileBytes = TM * 128;         // 16 KB: 128 rows x 32 tf32
 constexpr int kStageBytes = 2 * kTileBytes;  // hi | lo
+constexpr int kStageBytesWide = 2 * kStageBytes;  // users hi | lo, items hi | lo
+constexpr int kMaxLdWide = 512;
 constexpr int kProdWarps = 4, kProdGroup = 4;  // one group: every stage
 constexpr int kEpiWarps = 8;                   // two per TMEM lane quadrant, 64 columns of a tile each
 constexpr int kMmaWarp = kProdWarps + kEpiWarps;
@@ -168,18 +172,27 @@ __device__ __forceinline__ float4 tf32_hi(float4 u) {
 __device__ __forceinline__ float4 sub4(float4 a, float4 b) {
   return make_float4(a.x - b.x, a.y - b.y, a.z - b.z, a.w - b.w);
 }
+__device__ __forceinline__ void sts128(uint32_t addr, float4 v) {
+  asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
+               : "memory");
+}
 
 // ALLOW: the allow-list cursor is compiled in (a separate instantiation: without it the kernel
 // keeps the register budget it was tuned to)
-template <int M, bool ALLOW>
+// WIDE: row strides above 128 (up to 512).  The user tile (128 KB of hi | lo per 128 features) no
+// longer fits beside the ring, so it is streamed instead of parked: a stage is the same 32-feature
+// chunk of the 128 users and of the 128 items, [A hi | A lo | B hi | B lo] (64 KB), and the
+// producers load and split both.  MMA, epilogue, mask and allow-list code are shared.
+template <int M, bool ALLOW, bool WIDE>
 __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(ScoreTcArgs a) {
   constexpr int CAP = 32 * M;
+  constexpr int kStage = WIDE ? kStageBytesWide : kStageBytes;
   extern __shared__ unsigned char smem_raw[];
   // dynamic shared memory is only guaranteed 16-byte aligned: round up to the swizzle atom
   unsigned char *base = reinterpret_cast<unsigned char *>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  unsigned char *As = base;                          // [kMaxKc][hi 16 KB | lo 16 KB]
-  unsigned char *Bs = base + kMaxKc * kStageBytes;   // [STAGES][hi | lo]
-  uint64_t *bars = reinterpret_cast<uint64_t *>(Bs + STAGES * kStageBytes);
+  unsigned char *As = base;                                       // [kMaxKc][hi 16 KB | lo 16 KB]
+  unsigned char *Bs = base + (WIDE ? 0 : kMaxKc * kStageBytes);   // [STAGES][hi | lo] (WIDE: [A | B])
+  uint64_t *bars = reinterpret_cast<uint64_t *>(Bs + STAGES * kStage);
   uint64_t *full = bars;                      // [STAGES] producers -> MMA
   uint64_t *empty = bars + STAGES;            // [STAGES] MMA (commit) -> producers
   uint64_t *accfull = bars + 2 * STAGES;      // [2] MMA (commit) -> epilogue
@@ -208,7 +221,7 @@ __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(ScoreTcArgs a) {
   if (warp == kMmaWarp) tmem_alloc(tmem_slot, kTmemCols);
 
   // ---- prologue: the user tile, split and swizzled, stays in shared memory ----
-  {
+  if constexpr (!WIDE) {
     const int f4_per_row = ld / 4;
     for (int f = tid; f < TM * f4_per_row; f += kThreads) {
       const int r = f / f4_per_row, c = f % f4_per_row;
@@ -226,7 +239,85 @@ __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(ScoreTcArgs a) {
   fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  if (warp < kProdWarps) {
+  if (WIDE && warp < kProdWarps) {
+    // ============================ PRODUCERS (WIDE) =============================
+    // Same lane layout as below; each stage is two loads of eight 16-byte chunks per lane, the
+    // users' chunk kc and then the items' chunk kc.  The users' loads come from L2 after the first
+    // item tile.  `vu` always holds a user chunk and `vi` an item chunk, so the next load is in
+    // flight while the current chunk is converted, as in the parked-user loop.
+    const int pw = warp;
+    const int rsub = lane >> 3, c16 = lane & 7;
+    const unsigned total = (unsigned)n_tiles * (unsigned)n_kc;
+    // the lane's rows 32 pw + 4 i + rsub have swizzle phase rsub (i even) or rsub + 4 (i odd): two
+    // offsets and an immediate of (i >> 1) * 1024 instead of eight registers, which spilled here
+    const uint32_t off_even = sw128_offset(32 * pw + rsub, c16), off_odd = sw128_offset(32 * pw + 4 + rsub, c16);
+    const size_t row_step = (size_t)4 * ld;
+    const int64_t u0 = row0 + 32 * pw + rsub;  // this lane's first user row
+    const float *usrc = a.users + u0 * ld + c16 * 4;
+    int ukc = 0;
+    auto load_users = [&](float4(&v)[8]) {
+      if (u0 + 28 < a.n_rows) {
+#pragma unroll
+        for (int i = 0; i < 8; i++) v[i] = __ldg(reinterpret_cast<const float4 *>(usrc + i * row_step + ukc * KC));
+      } else {
+#pragma unroll
+        for (int i = 0; i < 8; i++)
+          v[i] = u0 + 4 * i < a.n_rows ? __ldg(reinterpret_cast<const float4 *>(usrc + i * row_step + ukc * KC))
+                                       : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+      if (++ukc == n_kc) ukc = 0;
+    };
+    int lt = 0, lkc = 0;
+    const float *lsrc = a.items + ((size_t)tile_begin * TN + 32 * pw + rsub) * ld + c16 * 4;
+    auto load_items = [&](float4(&v)[8]) {
+      const int64_t j0 = (int64_t)(tile_begin + lt) * TN + 32 * pw + rsub;
+      if (j0 + 28 < a.n_items) {
+#pragma unroll
+        for (int i = 0; i < 8; i++) v[i] = __ldg(reinterpret_cast<const float4 *>(lsrc + i * row_step));
+      } else {
+#pragma unroll
+        for (int i = 0; i < 8; i++)
+          v[i] = j0 + 4 * i < a.n_items ? __ldg(reinterpret_cast<const float4 *>(lsrc + i * row_step))
+                                        : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+      lsrc += KC;
+      if (++lkc == n_kc) {
+        lkc = 0;
+        lt++;
+        lsrc += (size_t)TN * ld - (size_t)n_kc * KC;
+      }
+    };
+    int s = 0;
+    uint32_t ph = 1;
+    // 32-bit shared-window addresses: generic 64-bit ones cost the registers this loop lacks
+    const uint32_t ring = smem_u32(Bs);
+    auto split_store = [&](const float4(&v)[8], uint32_t hi) {
+#pragma unroll
+      for (int i = 0; i < 8; i++) {
+        const float4 h = tf32_hi(v[i]), l = sub4(v[i], h);
+        const uint32_t dst = hi + ((i & 1) ? off_odd : off_even) + (i >> 1) * 1024;
+        sts128(dst, h);
+        sts128(dst + kTileBytes, l);
+      }
+    };
+    float4 vu[8], vi[8];
+    if (total > 0) load_users(vu);
+    for (unsigned it = 0; it < total; it++) {
+      load_items(vi);
+      mbar_wait(&empty[s], ph);
+      const uint32_t st = ring + s * kStage;
+      split_store(vu, st);
+      if (it + 1 < total) load_users(vu);
+      split_store(vi, st + kStageBytes);
+      fence_proxy_async_smem();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&full[s]);
+      if (++s == STAGES) {
+        s = 0;
+        ph ^= 1;
+      }
+    }
+  } else if (warp < kProdWarps) {
     // ================================ PRODUCERS ================================
     // One group serves every stage, so its loop is kept lean (r02o: 348 instructions per stage
     // and warp made the producers the bottleneck of the eight-warp epilogue): the lane's eight
@@ -303,8 +394,9 @@ __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(ScoreTcArgs a) {
         mbar_wait(&full[s], (it / STAGES) & 1);
         fence_after();
         if (lane == 0) {
-          const uint32_t a_hi = smem_u32(As + kc * kStageBytes), a_lo = a_hi + kTileBytes;
-          const uint32_t b = smem_u32(Bs + s * kStageBytes);
+          const uint32_t a_hi = WIDE ? smem_u32(Bs + s * kStage) : smem_u32(As + kc * kStageBytes);
+          const uint32_t a_lo = a_hi + kTileBytes;
+          const uint32_t b = WIDE ? a_hi + kStageBytes : smem_u32(Bs + s * kStage);
 #pragma unroll
           for (int kk = 0; kk < KC / 8; kk++) {
             const uint64_t db = desc_kmajor_sw128(b + kk * 32);
@@ -596,28 +688,40 @@ __global__ void csr_sorted_kernel(const int64_t *__restrict__ indptr, const int3
   if (bad) atomicExch(unsorted, 1);
 }
 
-template <int M, bool ALLOW>
+template <int M, bool ALLOW, bool WIDE>
 void launch_fused_as(const ScoreTcArgs &a, int user_tiles, cudaStream_t s) {
-  const size_t smem = (size_t)(kMaxKc + STAGES) * kStageBytes + 1024 + 16 * 8;
+  const size_t smem = (WIDE ? (size_t)STAGES * kStageBytesWide : (size_t)(kMaxKc + STAGES) * kStageBytes) +
+                      1024 + 16 * 8;
   static PerDeviceOnce configured;
   configured.run([&] {
-    CUDA_CHECK(cudaFuncSetAttribute(score_tc_kernel<M, ALLOW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    CUDA_CHECK(cudaFuncSetAttribute(score_tc_kernel<M, ALLOW, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)smem));
   });
   dim3 grid((unsigned)user_tiles, (unsigned)a.n_splits);
-  score_tc_kernel<M, ALLOW><<<grid, kThreads, smem, s>>>(a);
+  score_tc_kernel<M, ALLOW, WIDE><<<grid, kThreads, smem, s>>>(a);
   count_launch();
   CUDA_CHECK(cudaGetLastError());
 }
-template <int M>
+template <int M, bool WIDE>
 void launch_fused(const ScoreTcArgs &a, int user_tiles, cudaStream_t s) {
-  if (a.a_n_lists > 0) launch_fused_as<M, true>(a, user_tiles, s);
-  else launch_fused_as<M, false>(a, user_tiles, s);
+  if (a.a_n_lists > 0) launch_fused_as<M, true, WIDE>(a, user_tiles, s);
+  else launch_fused_as<M, false, WIDE>(a, user_tiles, s);
+}
+template <bool WIDE>
+void launch_fused_cap(const ScoreTcArgs &a, int user_tiles, int cap, cudaStream_t s) {
+  switch (cap) {
+    case 64: launch_fused<2, WIDE>(a, user_tiles, s); break;
+    case 128: launch_fused<4, WIDE>(a, user_tiles, s); break;
+    default: launch_fused<8, WIDE>(a, user_tiles, s); break;
+  }
 }
 
 }  // namespace
 
 bool score_tc_supported(int ld, int64_t k) { return ld % 32 == 0 && ld >= 32 && ld <= 128 && k >= 1 && k <= 128; }
+bool score_topk_tc_supported(int ld, int64_t k) {
+  return ld % 32 == 0 && ld >= 32 && ld <= kMaxLdWide && k >= 1 && k <= 128;
+}
 // candidate keys per row, split and column half: k + one 16-column chunk + room between two
 // compactions (128 keys for k = 10 measured slower than 64: r02n 8.97 against r02l 8.43 ms)
 int score_tc_capacity(int64_t k) { return k <= 16 ? 64 : (k <= 48 ? 128 : 256); }
@@ -662,7 +766,7 @@ void launch_score_topk_tc(const float *user_rows, int64_t n_rows, const float *i
                           const int32_t *a_indices, int64_t a_row0, const uint32_t *a_bitmap,
                           const int64_t *m_rowmap) {
   if (n_rows == 0) return;
-  if (!score_tc_supported(ld, k)) throw NotImplemented("tensor-core top-k: ld must be 32..128 and k <= 128");
+  if (!score_topk_tc_supported(ld, k)) throw NotImplemented("tensor-core top-k: ld must be 32..512 and k <= 128");
   if (n_items >= (1ll << 31) - 256) throw InvalidArgument("too many items");
   ScoreTcArgs a{};
   a.users = user_rows;
@@ -687,11 +791,8 @@ void launch_score_topk_tc(const float *user_rows, int64_t n_rows, const float *i
   a.cand = static_cast<unsigned long long *>(scratch);
   const int user_tiles = (int)ceil_div(n_rows, TM);
   const int cap = score_tc_capacity(k);
-  switch (cap) {
-    case 64: launch_fused<2>(a, user_tiles, s); break;
-    case 128: launch_fused<4>(a, user_tiles, s); break;
-    default: launch_fused<8>(a, user_tiles, s); break;
-  }
+  if (ld > kMaxKc * KC) launch_fused_cap<true>(a, user_tiles, cap, s);
+  else launch_fused_cap<false>(a, user_tiles, cap, s);
   const unsigned grid = (unsigned)std::min<int64_t>(n_rows, (int64_t)kNumSMsB200 * 8);
   merge_topk_kernel<<<grid, kMgThreads, 0, s>>>(a.cand, n_rows, 2 * a.n_splits, cap, k, out_idx, out_score,
                                                  out_count);
@@ -715,7 +816,7 @@ void launch_scores_tc(const float *user_rows, int64_t n_rows, const float *item,
   a.tiles_per_split = (int)ceil_div(ceil_div(n_items, TN), a.n_splits);
   a.out_scores = out;
   a.out_ld = out_ld;
-  launch_fused<2>(a, (int)ceil_div(n_rows, TM), s);
+  launch_fused<2, false>(a, (int)ceil_div(n_rows, TM), s);
 }
 
 }  // namespace ials
