@@ -372,6 +372,7 @@ IALS_API int64_t ials_kernel_launch_count(void);
  *   for side in (user, item):
  *     ials_trainer_gram_partial(1 - side) -> all-reduce(sum) the K*K buffer
  *     ials_trainer_solve_shard(side)       (writes local + peer replicas)
+ * (the feature-aware epoch adds a refit per side, see below).
  * ials_trainer_step / half_step / compute_loss refuse a sharded trainer. */
 IALS_API int ials_trainer_create_sharded(const ials_model_config *config, int64_t n_users,
                                 int64_t n_items, int64_t user_begin, int64_t user_end,
@@ -389,8 +390,58 @@ IALS_API int ials_trainer_shard_range(ials_trainer *t, int side, int64_t *begin,
 IALS_API int ials_trainer_gram_partial(ials_trainer *t, int factor_side, float **d_out, int64_t *count);
 /* Solve this rank's rows of `side` using the (already all-reduced) Gram buffer
  * of the other side; writes the rows into the local replica and, if peer
- * replicas were registered, into every peer's replica as well. */
+ * replicas were registered, into every peer's replica as well.  A side that uses
+ * its features (set with ials_trainer_set_shard_features, past the warm-up) is
+ * solved towards the prior features x weight of the shard's rows, as
+ * ials_trainer_step does (IALSTrainer.hpp:762-787), and its weight refit becomes due.
+ * The item side (side 1) ends the epoch: it advances the epoch counter that the
+ * warm-up is measured in (:788). */
 IALS_API int ials_trainer_solve_shard(ials_trainer *t, int side, const ials_solver_config *solver);
+
+/* ---- feature-aware iALS on a row-sharded trainer ----
+ * The feature-aware epoch of IALSTrainer::step (:758-789) across ranks.  Per side:
+ *   ials_trainer_gram_partial(1 - side) -> all-reduce
+ *   ials_trainer_solve_shard(side)             (prior F_own W when the side uses features)
+ *   ials_trainer_feature_partials(side) -> all-reduce each buffer with a non-zero count
+ *   ials_trainer_feature_refit(side)           (every rank solves the same summed system)
+ * The weights stay identical on every rank; ials_trainer_get_feature_weight /
+ * _set_feature_weight read and write this rank's copy. */
+/* IALSTrainer(config, X, user_feature, item_feature) for this rank's rows of `side`
+ * (initialize_feature_aware :1001-1014): n_rows = the shard's rows, dense or CSR, the arguments
+ * and errors of ials_trainer_set_features.  *has_empty_row (may be NULL) reports whether one of
+ * the shard's rows of X (side 0) / X^T (side 1) is empty: the guard of step_with_prior
+ * (:639-652) needs the OR over all ranks, see ials_trainer_check_shard_step. */
+IALS_API int ials_trainer_set_shard_features(ials_trainer *t, int side, int64_t n_rows, int64_t n_cols,
+                                             const float *dense, const int64_t *indptr, const int32_t *indices,
+                                             const float *data, float lambda_feature,
+                                             int64_t feature_warmup_epochs, int *has_empty_row);
+/* The rejections of a feature-aware epoch (:759-761 "Feature-aware iALS does not support IALSPP.",
+ * the weight shape of :1016-1042, the empty-row guard of :639-652 with the given OR over all
+ * ranks), from state that is the same on every rank: a caller that runs it before the epoch's
+ * first collective sees every rank fail alike, before any factor or weight changes. */
+IALS_API int ials_trainer_check_shard_step(ials_trainer *t, const ials_solver_config *solver,
+                                           int user_has_empty_row, int item_has_empty_row);
+/* The rank's partial sums of the weight refit W = (F^T D F + lambda I)^-1 F^T D X
+ * (initialize_feature_weight_cache :1083-1132, solve_feature_weight :1134-1180) over its own rows,
+ * D = diag(compute_reg) of those rows: F^T D F in a trainer-owned device buffer of n_w * n_w floats
+ * (only before the first refit: the factor is cached, like cache_ready; count 0 afterwards) and
+ * F^T D X in one of n_w * ld floats.  Both counts are 0 when the side's last solve used no prior.
+ * The caller all-reduces (sum) each buffer in place. */
+IALS_API int ials_trainer_feature_partials(ials_trainer *t, int side, float **d_gram, int64_t *gram_count,
+                                           float **d_rhs, int64_t *rhs_count);
+/* After that all-reduce: factors F^T D F + lambda I (first time only), solves for W and stores it
+ * as the side's weight.  No-op when ials_trainer_feature_partials returned zero counts.
+ * "Feature ridge Cholesky decomposition failed." / "Feature ridge solve failed." surface at the
+ * next ials_trainer_sync. */
+IALS_API int ials_trainer_feature_refit(ials_trainer *t, int side);
+/* This rank's share of IALSTrainer::compute_loss (:836-940), halved, in float64: the data term and
+ * the regulariser (|x - prior|^2 for a side with features) of its own user rows and the
+ * regulariser of its own item rows; with include_global != 0 also sum(P_user .* P_item) / alpha0
+ * from the full replicas and lambda |W|^2 of each side with features.  The sum over ranks, with
+ * include_global on exactly one of them, is the loss.  Reads the full replicas: every rank's
+ * solves must have completed (ials_trainer_sync + a barrier). */
+IALS_API int ials_trainer_compute_loss_shard(ials_trainer *t, const ials_solver_config *solver, int include_global,
+                                             double *out);
 /* CUDA IPC plumbing for peer replicas: 64-byte handle of this trainer's factor
  * matrix; registration of the peers' handles (world entries, own rank skipped). */
 IALS_API int ials_trainer_ipc_handle(ials_trainer *t, int side, unsigned char handle_out[64]);

@@ -94,6 +94,11 @@ def _load() -> ctypes.CDLL:
         "ials_trainer_shard_range": (c_int, [H, c_int, POINTER(c_int64), POINTER(c_int64)]),
         "ials_trainer_gram_partial": (c_int, [H, c_int, POINTER(c_void_p), POINTER(c_int64)]),
         "ials_trainer_solve_shard": (c_int, [H, c_int, SC]),
+        "ials_trainer_set_shard_features": (c_int, [H, c_int, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_int64, POINTER(c_int)]),
+        "ials_trainer_check_shard_step": (c_int, [H, SC, c_int, c_int]),
+        "ials_trainer_feature_partials": (c_int, [H, c_int, POINTER(c_void_p), POINTER(c_int64), POINTER(c_void_p), POINTER(c_int64)]),
+        "ials_trainer_feature_refit": (c_int, [H, c_int]),
+        "ials_trainer_compute_loss_shard": (c_int, [H, SC, c_int, POINTER(ctypes.c_double)]),
         "ials_trainer_ipc_handle": (c_int, [H, c_int, POINTER(c_ubyte)]),
         "ials_trainer_ipc_open_peers": (c_int, [H, c_int, c_void_p, c_int, c_int]),
     }

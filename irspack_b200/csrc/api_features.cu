@@ -35,6 +35,39 @@ void upload_features(ials_trainer::FeatureSide &owner, int64_t n_rows, int64_t n
   F.data = owner.csr.data.get();
 }
 
+// initialize_feature_aware (:1001-1014) for the rows the trainer holds of the side's interaction
+// matrix (all of them, or a rank's shard); records whether one of those rows is empty
+void init_features(ials_trainer *t, int side, int64_t n_rows, int64_t n_cols, const float *dense,
+                   const int64_t *indptr, const int32_t *indices, const float *data, float lambda_feature,
+                   int64_t feature_warmup_epochs) {
+  if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix");
+  const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
+  if (n_rows != csr.n_rows) throw InvalidArgument("Feature matrix row count mismatch.");
+  if (n_cols > 0 && !(lambda_feature > 0.f))
+    throw InvalidArgument("Feature weight regularization must be positive.");
+  DeviceGuard g(t->device);
+  ials_trainer::FeatureSide &f = t->feat[side];
+  f = ials_trainer::FeatureSide{};
+  upload_features(f, n_rows, n_cols, dense, indptr, indices, data);
+  f.given = f.weight_set = true;
+  f.n_w = n_cols;
+  f.lambda = lambda_feature;
+  CUDA_CHECK(cudaMemset(f.weight.alloc(std::max<int64_t>(n_cols * t->ld, 1)), 0,
+                        sizeof(float) * std::max<int64_t>(n_cols * t->ld, 1)));  // setZero, :1012
+  {  // does the side's interaction matrix have an empty row? (step_with_prior's guard)
+    std::vector<int64_t> ip((size_t)csr.n_rows + 1);
+    CUDA_CHECK(cudaMemcpy(ip.data(), csr.indptr.get(), sizeof(int64_t) * (csr.n_rows + 1), cudaMemcpyDeviceToHost));
+    f.has_empty_row = false;
+    for (int64_t r = 0; r < csr.n_rows; r++)
+      if (ip[r] == ip[r + 1]) {
+        f.has_empty_row = true;
+        break;
+      }
+  }
+  t->feature_aware = true;
+  t->feature_warmup = feature_warmup_epochs;
+}
+
 const char *side_name(int side) { return side == 0 ? "user" : "item"; }
 const char *side_Name(int side) { return side == 0 ? "User" : "Item"; }
 
@@ -78,10 +111,11 @@ void check_feature_weight_shapes(const ials_trainer *t, bool any_epoch) {
   }
 }
 
-// stored_user_feature_prior / stored_item_feature_prior (:1044-1050) into feat[side].prior
+// stored_user_feature_prior / stored_item_feature_prior (:1044-1050) into feat[side].prior: one row
+// per feature row (every row of the side, or a rank's own rows)
 const float *stored_prior(ials_trainer *t, int side) {
   ials_trainer::FeatureSide &f = t->feat[side];
-  const int64_t n = t->n_rows(side);
+  const int64_t n = f.F.n_rows;
   launch_feature_prior(f.F, f.weight.get(), t->ld, f.prior.ensure(std::max<int64_t>(n * t->ld, 1)), t->stream);
   return f.prior.get();
 }
@@ -127,33 +161,20 @@ int ials_trainer_set_features(ials_trainer *t, int side, int64_t n_rows, int64_t
     require_side(side);
     require(n_rows >= 0 && n_cols >= 0 && feature_warmup_epochs >= 0, "negative shape");
     if (t->sharded) throw NotImplemented("feature-aware iALS on a row-sharded trainer is not implemented");
-    if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix");
-    // initialize_feature_aware (:1001-1014)
-    if (n_rows != t->n_rows(side)) throw InvalidArgument("Feature matrix row count mismatch.");
-    if (n_cols > 0 && !(lambda_feature > 0.f))
-      throw InvalidArgument("Feature weight regularization must be positive.");
-    DeviceGuard g(t->device);
-    ials_trainer::FeatureSide &f = t->feat[side];
-    f = ials_trainer::FeatureSide{};
-    upload_features(f, n_rows, n_cols, dense, indptr, indices, data);
-    f.given = f.weight_set = true;
-    f.n_w = n_cols;
-    f.lambda = lambda_feature;
-    CUDA_CHECK(cudaMemset(f.weight.alloc(std::max<int64_t>(n_cols * t->ld, 1)), 0,
-                          sizeof(float) * std::max<int64_t>(n_cols * t->ld, 1)));  // setZero, :1012
-    {  // does the side's interaction matrix have an empty row? (step_with_prior's guard)
-      const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
-      std::vector<int64_t> ip((size_t)csr.n_rows + 1);
-      CUDA_CHECK(cudaMemcpy(ip.data(), csr.indptr.get(), sizeof(int64_t) * (csr.n_rows + 1), cudaMemcpyDeviceToHost));
-      f.has_empty_row = false;
-      for (int64_t r = 0; r < csr.n_rows; r++)
-        if (ip[r] == ip[r + 1]) {
-          f.has_empty_row = true;
-          break;
-        }
-    }
-    t->feature_aware = true;
-    t->feature_warmup = feature_warmup_epochs;
+    init_features(t, side, n_rows, n_cols, dense, indptr, indices, data, lambda_feature, feature_warmup_epochs);
+  });
+}
+
+int ials_trainer_set_shard_features(ials_trainer *t, int side, int64_t n_rows, int64_t n_cols, const float *dense,
+                                    const int64_t *indptr, const int32_t *indices, const float *data,
+                                    float lambda_feature, int64_t feature_warmup_epochs, int *has_empty_row) {
+  return guarded([&] {
+    require(t != nullptr, "trainer is null");
+    require_side(side);
+    require(n_rows >= 0 && n_cols >= 0 && feature_warmup_epochs >= 0, "negative shape");
+    require(t->sharded, "not a row-sharded trainer: use ials_trainer_set_features");
+    init_features(t, side, n_rows, n_cols, dense, indptr, indices, data, lambda_feature, feature_warmup_epochs);
+    if (has_empty_row) *has_empty_row = t->feat[side].has_empty_row ? 1 : 0;
   });
 }
 

@@ -58,13 +58,117 @@ int ials_trainer_solve_shard(ials_trainer *t, int side, const ials_solver_config
     require_side(side);
     check_solver(solver);
     if (!t->has_X) throw std::runtime_error("no interaction matrix");
+    check_feature_solver(t, solver);
+    check_feature_weight_shapes(t, false);
     DeviceGuard g(t->device);
     const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
     SolveArgs a = make_args(t, side, t->factor[side].get(), csr, solver);
     a.n_peers = t->n_peers[side];
     for (int p = 0; p < a.n_peers; p++) a.peers[p] = t->peers[side][p];
+    ials_trainer::FeatureSide &f = t->feat[side];
+    f.refit_pending = side_uses_features(t, side);  // IALSTrainer.hpp:762, 777
+    if (f.refit_pending) {
+      check_prior_defined(t, side, f.has_empty_row);
+      // the kernels read the prior of factor row gu at prior[gu * ld]; the buffer holds the shard's rows
+      a.prior = stored_prior(t, side) - csr.row_base * t->ld;
+    }
     if (side == 0) consume_flagged_upload(t, solver, a, csr.row_base);
     run_solver(t, a, csr, solver, t->stream);
+    if (side == 1) t->epoch++;  // the item half ends the epoch (:788)
+  });
+}
+
+int ials_trainer_check_shard_step(ials_trainer *t, const ials_solver_config *solver, int user_has_empty_row,
+                                  int item_has_empty_row) {
+  return guarded([&] {
+    require(t != nullptr, "trainer is null");
+    check_solver(solver);
+    check_feature_solver(t, solver);
+    check_feature_weight_shapes(t, false);
+    const bool empty[2] = {user_has_empty_row != 0, item_has_empty_row != 0};
+    for (int side = 0; side < 2; side++)
+      if (side_uses_features(t, side)) check_prior_defined(t, side, empty[side]);
+  });
+}
+
+int ials_trainer_feature_partials(ials_trainer *t, int side, float **d_gram, int64_t *gram_count, float **d_rhs,
+                                  int64_t *rhs_count) {
+  return guarded([&] {
+    require(t != nullptr && d_gram != nullptr && gram_count != nullptr && d_rhs != nullptr && rhs_count != nullptr,
+            "null argument");
+    require_side(side);
+    require(t->sharded, "not a row-sharded trainer");
+    *d_gram = *d_rhs = nullptr;
+    *gram_count = *rhs_count = 0;
+    ials_trainer::FeatureSide &f = t->feat[side];
+    if (!f.refit_pending) return;
+    DeviceGuard g(t->device);
+    const DeviceCsr &csr = side == 0 ? t->X : t->Xt;
+    if (!f.cache_ready) {  // initialize_feature_weight_cache (:1083-1132), over the shard's rows
+      f.rw.ensure(std::max<int64_t>(csr.n_rows, 1));
+      f.llt.ensure(f.n_w * f.n_w);
+      launch_feature_row_weights(csr.indptr.get(), csr.n_rows, t->n_rows(1 - side), t->cfg.alpha0, t->cfg.reg,
+                                 t->cfg.nu, f.rw.get(), t->stream);
+      launch_feature_gram(f.F, f.rw.get(), f.llt.get(), t->stream);
+      *d_gram = f.llt.get();
+      *gram_count = f.n_w * f.n_w;
+    }
+    // solve_feature_weight's right-hand side (:1134-1160) over the shard's freshly solved rows
+    f.rhs.ensure(f.n_w * t->ld);
+    launch_feature_rhs(f.F, f.rw.get(), t->factor[side].get() + csr.row_base * t->ld, t->ld, f.rhs.get(),
+                       t->stream);
+    *d_rhs = f.rhs.get();
+    *rhs_count = f.n_w * t->ld;
+  });
+}
+
+int ials_trainer_feature_refit(ials_trainer *t, int side) {
+  return guarded([&] {
+    require(t != nullptr, "trainer is null");
+    require_side(side);
+    require(t->sharded, "not a row-sharded trainer");
+    ials_trainer::FeatureSide &f = t->feat[side];
+    if (!f.refit_pending) return;
+    f.refit_pending = false;
+    DeviceGuard g(t->device);
+    if (!f.cache_ready) {
+      launch_feature_llt(f.llt.get(), f.n_w, f.lambda, t->err_flags.get() + kErrFeatureLlt, t->stream);
+      f.cache_ready = true;
+    }
+    launch_feature_solve(f.llt.get(), f.n_w, f.rhs.get(), t->ld, t->err_flags.get() + kErrFeatureSolve, t->stream);
+    CUDA_CHECK(cudaMemcpyAsync(f.weight.get(), f.rhs.get(), sizeof(float) * f.n_w * t->ld, cudaMemcpyDeviceToDevice,
+                               t->stream));
+  });
+}
+
+int ials_trainer_compute_loss_shard(ials_trainer *t, const ials_solver_config *solver, int include_global,
+                                    double *out) {
+  return guarded([&] {
+    require(t != nullptr && out != nullptr, "null argument");
+    require(solver != nullptr && solver->n_threads > 0, "n_threads must be strictly positive.");
+    require(t->sharded, "not a row-sharded trainer: use ials_trainer_compute_loss");
+    check_feature_weight_shapes(t, true);
+    DeviceGuard g(t->device);
+    const float *P[2] = {nullptr, nullptr};
+    if (include_global) {  // sum(P_user .* P_item) / alpha0 from the full replicas
+      gram_side(t, 0);
+      gram_side(t, 1);
+      P[0] = t->P[0].get();
+      P[1] = t->P[1].get();
+    }
+    const float bias = t->cfg.loss_type == IALS_LOSS_IALSPP ? 0.f : t->cfg.alpha0;
+    const float *prior[2] = {nullptr, nullptr};
+    for (int side = 0; side < 2; side++)
+      if (t->feature_aware && t->feat[side].n_w > 0) prior[side] = stored_prior(t, side);
+    launch_loss_shard(t->factor[0].get(), t->factor[1].get(), t->U, t->I, t->ld, t->X, t->Xt, P[0], P[1],
+                      t->cfg.alpha0, t->cfg.reg, t->cfg.nu, bias, prior[0], prior[1], t->d_loss.get(), t->stream);
+    for (int side = 0; side < 2; side++)
+      if (include_global && prior[side])
+        launch_loss_add_sumsq(t->feat[side].weight.get(), t->feat[side].n_w * t->ld, t->feat[side].lambda,
+                              t->d_loss.get(), t->stream);
+    launch_loss_halve(t->d_loss.get(), t->stream);
+    CUDA_CHECK(cudaMemcpyAsync(out, t->d_loss.get(), sizeof(double), cudaMemcpyDeviceToHost, t->stream));
+    CUDA_CHECK(cudaStreamSynchronize(t->stream));
   });
 }
 

@@ -315,6 +315,12 @@ void launch_loss(const float *user, const float *item, int64_t U, int64_t I, int
                  float alpha0, float reg, float nu, float bias, const float *prior_u,
                  const float *prior_i, double *d_out, cudaStream_t s);
 void launch_loss_add_sumsq(const float *v, int64_t n, float scale, double *d_out, cudaStream_t s);
+// One rank's share of the sum of a row-sharded trainer: the rows X.row_base + [0, X.n_rows) of `user`
+// and Xt.row_base + [0, Xt.n_rows) of `item` (full replicas); prior_u / prior_i hold those rows only;
+// the Gram term is added when Pu != nullptr.  Zeroes *d_out first and leaves the sum un-halved.
+void launch_loss_shard(const float *user, const float *item, int64_t U, int64_t I, int ld, const DeviceCsr &X,
+                       const DeviceCsr &Xt, const float *Pu, const float *Pi, float alpha0, float reg, float nu,
+                       float bias, const float *prior_u, const float *prior_i, double *d_out, cudaStream_t s);
 void launch_loss_halve(double *d_out, cudaStream_t s);
 
 // ---- feature-aware iALS (feature.cu; IALSTrainer.hpp:696-702, 1066-1209) ----
@@ -339,6 +345,12 @@ void launch_feature_gram_llt(const FeatureDev &F, const float *rw, float lambda,
 // *fail is raised when the solution is not finite
 void launch_feature_ridge_solve(const FeatureDev &F, const float *rw, const float *X, int ld,
                                 const float *L, float *R, int *fail, cudaStream_t s);
+// The two halves of each, for the row-sharded trainer, which all-reduces the F^T products in between:
+// G = F^T diag(rw) F / R = F^T diag(rw) X over F's rows, and the steps that follow on the summed G / R
+void launch_feature_gram(const FeatureDev &F, const float *rw, float *G, cudaStream_t s);
+void launch_feature_llt(float *G, int64_t n, float lambda, int *fail, cudaStream_t s);
+void launch_feature_rhs(const FeatureDev &F, const float *rw, const float *X, int ld, float *R, cudaStream_t s);
+void launch_feature_solve(const float *L, int64_t n, float *R, int ld, int *fail, cudaStream_t s);
 
 // ranking metrics of recommendation lists (metrics.cu); acc = {hit, recall, ndcg, map, precision} sums
 void launch_metrics_rows(const int32_t *rec, const int32_t *cnt, int64_t rows, int k, const int64_t *gt_indptr,

@@ -184,8 +184,7 @@ void launch_feature_row_weights(const int64_t *indptr, int64_t n_rows, int64_t n
   CUDA_CHECK(cudaGetLastError());
 }
 
-void launch_feature_gram_llt(const FeatureDev &F, const float *rw, float lambda, float *G, int *fail,
-                             cudaStream_t s) {
+void launch_feature_gram(const FeatureDev &F, const float *rw, float *G, cudaStream_t s) {
   const int64_t n = F.n_cols;
   if (n <= 0) return;
   CUDA_CHECK(cudaMemsetAsync(G, 0, sizeof(float) * n * n, s));
@@ -193,6 +192,11 @@ void launch_feature_gram_llt(const FeatureDev &F, const float *rw, float lambda,
     feature_gram_kernel<<<warp_grid(F.n_rows), kFThreads, 0, s>>>(F, rw, G);
     count_launch();
   }
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void launch_feature_llt(float *G, int64_t n, float lambda, int *fail, cudaStream_t s) {
+  if (n <= 0) return;
   feature_add_diag_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, s>>>(G, n, lambda);
   count_launch();
   feature_llt_kernel<<<1, 1024, 0, s>>>(G, (int)n, fail);
@@ -200,8 +204,13 @@ void launch_feature_gram_llt(const FeatureDev &F, const float *rw, float lambda,
   CUDA_CHECK(cudaGetLastError());
 }
 
-void launch_feature_ridge_solve(const FeatureDev &F, const float *rw, const float *X, int ld,
-                                const float *L, float *R, int *fail, cudaStream_t s) {
+void launch_feature_gram_llt(const FeatureDev &F, const float *rw, float lambda, float *G, int *fail,
+                             cudaStream_t s) {
+  launch_feature_gram(F, rw, G, s);
+  launch_feature_llt(G, F.n_cols, lambda, fail, s);
+}
+
+void launch_feature_rhs(const FeatureDev &F, const float *rw, const float *X, int ld, float *R, cudaStream_t s) {
   const int64_t n = F.n_cols;
   if (n <= 0) return;
   CUDA_CHECK(cudaMemsetAsync(R, 0, sizeof(float) * n * ld, s));
@@ -209,9 +218,20 @@ void launch_feature_ridge_solve(const FeatureDev &F, const float *rw, const floa
     feature_rhs_kernel<<<warp_grid(F.n_rows), kFThreads, 0, s>>>(F, rw, X, ld, R);
     count_launch();
   }
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void launch_feature_solve(const float *L, int64_t n, float *R, int ld, int *fail, cudaStream_t s) {
+  if (n <= 0) return;
   feature_solve_kernel<<<(unsigned)ceil_div(ld, 64), 64, 0, s>>>(L, (int)n, R, ld, fail);
   count_launch();
   CUDA_CHECK(cudaGetLastError());
+}
+
+void launch_feature_ridge_solve(const FeatureDev &F, const float *rw, const float *X, int ld,
+                                const float *L, float *R, int *fail, cudaStream_t s) {
+  launch_feature_rhs(F, rw, X, ld, R, s);
+  launch_feature_solve(L, F.n_cols, R, ld, fail, s);
 }
 
 }  // namespace ials

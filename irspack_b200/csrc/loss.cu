@@ -101,6 +101,30 @@ void launch_loss(const float *user, const float *item, int64_t U, int64_t I, int
   CUDA_CHECK(cudaGetLastError());
 }
 
+void launch_loss_shard(const float *user, const float *item, int64_t U, int64_t I, int ld, const DeviceCsr &X,
+                       const DeviceCsr &Xt, const float *Pu, const float *Pi, float alpha0, float reg, float nu,
+                       float bias, const float *prior_u, const float *prior_i, double *d_out, cudaStream_t s) {
+  CUDA_CHECK(cudaMemsetAsync(d_out, 0, sizeof(double), s));
+  if (Pu != nullptr && alpha0 != 0.f) {
+    loss_gram_kernel<<<32, 256, 0, s>>>(Pu, Pi, ld * ld, alpha0, d_out);
+    count_launch();
+  }
+  const int T = 256;
+  if (X.n_rows > 0) {
+    loss_rows_kernel<<<(unsigned)std::min<int64_t>(ceil_div(X.n_rows * kWarp, T), kNumSMsB200 * 16), T, 0, s>>>(
+        user + X.row_base * ld, item, X.n_rows, I, ld, X.indptr.get(), X.indices.get(), X.data.get(), alpha0, reg,
+        nu, bias, 1, prior_u, d_out);
+    count_launch();
+  }
+  if (Xt.n_rows > 0) {
+    loss_rows_kernel<<<(unsigned)std::min<int64_t>(ceil_div(Xt.n_rows * kWarp, T), kNumSMsB200 * 16), T, 0, s>>>(
+        item + Xt.row_base * ld, user, Xt.n_rows, U, ld, Xt.indptr.get(), Xt.indices.get(), Xt.data.get(), alpha0,
+        reg, nu, bias, 0, prior_i, d_out);
+    count_launch();
+  }
+  CUDA_CHECK(cudaGetLastError());
+}
+
 // *d_out += scale * sum v^2   (lambda |W|^2 of the feature weights, :929, :939)
 void launch_loss_add_sumsq(const float *v, int64_t n, float scale, double *d_out, cudaStream_t s) {
   if (n <= 0) return;

@@ -69,11 +69,14 @@ struct ials_trainer {
     ials::DeviceCsr csr;
     int64_t n_w = 0;                   // rows of the weight (= feature columns)
     ials::DeviceBuffer<float> weight;  // [n_w x ld]
-    ials::DeviceBuffer<float> prior;   // [n_rows x ld]
+    ials::DeviceBuffer<float> prior;   // [F.n_rows x ld] (a row-sharded trainer: its own rows only)
     ials::DeviceBuffer<float> rw;      // [n_rows]   compute_reg of every row (FeatureWeightCache::row_weights)
     ials::DeviceBuffer<float> llt;     // [n_w x n_w] Cholesky factor of F^T D F + lambda I (FeatureWeightCache::llt)
     ials::DeviceBuffer<float> rhs;     // [n_w x ld]
     bool cache_ready = false;
+    // row-sharded trainer: the last ials_trainer_solve_shard of this side used the prior, so its
+    // weight refit (ials_trainer_feature_partials / _feature_refit) is due
+    bool refit_pending = false;
     float lambda = 0.f;
   } feat[2];
   bool feature_aware = false;

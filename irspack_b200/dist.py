@@ -264,17 +264,26 @@ class ShardedIALSTrainer:
     rank's items x all users (CSR) -- two scipy matrices, or two device CSR triples
     ``(indptr, indices, data)`` of torch tensors on this rank's GPU
     (``exchange_transposed_shards_device``).  ``user`` / ``item`` return the local full
-    replicas, identical on every rank after ``sync()``."""
+    replicas, identical on every rank after ``sync()``.
+
+    ``user_feature`` / ``item_feature`` (both or neither): this rank's rows of the feature
+    matrices, dense or scipy sparse -- the feature-aware model of
+    ``IALSTrainer(config, X, user_feature, item_feature)`` with the config's
+    ``lambda_*_feature`` and ``feature_warmup_epochs``.  Each epoch then refits the feature
+    weights from sums over all ranks; every rank holds the same weights."""
 
     def __init__(self, model_config: Any, X_user_rows: sps.csr_matrix, user_begin: int,
                  n_users: int, Xt_item_rows: sps.csr_matrix, item_begin: int, n_items: int,
-                 init_on_device: bool = False) -> None:
+                 init_on_device: bool = False, user_feature: Any = None, item_feature: Any = None) -> None:
         import torch
         import torch.distributed as dist
 
         from . import _ials_core as core
         from ._lib import check, lib
 
+        if (user_feature is None) != (item_feature is None):
+            raise TypeError("the feature-aware trainer takes both user_feature and item_feature; pass a "
+                            "matrix with 0 columns for a side without features")
         self._core, self._lib, self._check = core, lib, check
         self.rank = dist.get_rank() if dist.is_initialized() else 0
         self.world = dist.get_world_size() if dist.is_initialized() else 1
@@ -327,14 +336,56 @@ class ShardedIALSTrainer:
         self._handle = h
         check(lib.ials_trainer_set_stream(h, ctypes.c_void_p(stream)))
         self._torch = torch
-        self._gram_views: dict = {}
+        self._buffer_views: dict = {}
+        # per side: does some rank's shard hold an empty row (the guard of step_with_prior needs the
+        # OR over all ranks, so that every rank rejects an epoch alike)
+        self._empty_row = (0, 0)
+        if user_feature is not None:
+            self._set_features(model_config, (user_feature, item_feature))
         if self.world > 1:
             self._open_peers()
 
+    def _set_features(self, model_config: Any, features: Tuple[Any, Any]) -> None:
+        lams = (model_config.lambda_user_feature, model_config.lambda_item_feature)
+        empty = [0, 0]
+        err: Optional[BaseException] = None
+        try:
+            for side, F in enumerate(features):
+                rows, cols, dense, ip, ix, dt = self._core._feature_arrays(F)
+                flag = ctypes.c_int(0)
+                p = self._core._ptr
+                self._check(self._lib.ials_trainer_set_shard_features(
+                    self._handle, side, rows, cols, p(dense), p(ip), p(ix), p(dt), ctypes.c_float(lams[side]),
+                    int(model_config.feature_warmup_epochs), ctypes.byref(flag)))
+                empty[side] = flag.value
+        except (RuntimeError, ValueError, TypeError) as e:  # a shard of the wrong size may be one rank's
+            err = e
+        failed, *self._empty_row = self._max_over_ranks([1 if err is not None else 0] + empty)
+        self._raise_agreed(err, failed)
+
+    def _max_over_ranks(self, values: List[int]) -> List[int]:
+        import torch.distributed as dist
+
+        if self.world == 1:
+            return list(values)
+        dev = f"cuda:{self._device}" if dist.get_backend() == "nccl" else "cpu"
+        t = self._torch.tensor(values, dtype=self._torch.int64, device=dev)
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        return [int(v) for v in t.tolist()]
+
+    @staticmethod
+    def _raise_agreed(err: Optional[BaseException], failed: int) -> None:
+        """Raise this rank's exception, or report a peer's failure, on every rank alike."""
+        if err is not None:
+            raise err
+        if failed:
+            raise RuntimeError("a peer rank failed (see that rank's exception)")
+
     @classmethod
     def from_global(cls, model_config: Any, X: sps.csr_matrix, rank: Optional[int] = None,
-                    world: Optional[int] = None, **kw: Any) -> "ShardedIALSTrainer":
-        """Shard a matrix every rank holds in full (tests, small problems)."""
+                    world: Optional[int] = None, user_feature: Any = None, item_feature: Any = None,
+                    **kw: Any) -> "ShardedIALSTrainer":
+        """Shard a matrix (and the feature matrices) every rank holds in full (tests, small problems)."""
         import torch.distributed as dist
 
         rank = dist.get_rank() if rank is None else rank
@@ -343,8 +394,16 @@ class ShardedIALSTrainer:
         Xt = sps.csr_matrix(X.T)
         ub = balanced_bounds(np.diff(X.indptr) + 1, world)
         ib = balanced_bounds(np.diff(Xt.indptr) + 1, world)
+
+        def rows(F: Any, b: int, e: int) -> Any:
+            if F is None:
+                return None
+            return (sps.csr_matrix(F) if sps.issparse(F) else np.asarray(F))[b:e]
+
         return cls(model_config, X[ub[rank]:ub[rank + 1]], ub[rank], X.shape[0],
-                   Xt[ib[rank]:ib[rank + 1]], ib[rank], X.shape[1], **kw)
+                   Xt[ib[rank]:ib[rank + 1]], ib[rank], X.shape[1],
+                   user_feature=rows(user_feature, ub[rank], ub[rank + 1]),
+                   item_feature=rows(item_feature, ib[rank], ib[rank + 1]), **kw)
 
     def __del__(self) -> None:
         h = getattr(self, "_handle", None)
@@ -370,15 +429,37 @@ class ShardedIALSTrainer:
         stream = self._core._stream_of(self._device)  # the trainer's own device, not torch's current one
         self._check(self._lib.ials_trainer_set_stream(self._handle, ctypes.c_void_p(stream)))
 
+    def _buffer_view(self, ptr: ctypes.c_void_p, count: ctypes.c_int64) -> Any:
+        """Zero-copy flat torch view of a trainer-owned float buffer (cached per buffer)."""
+        key = (int(ptr.value), int(count.value))
+        if key not in self._buffer_views:
+            arr = self._core._DeviceArray(key[0], (key[1],), (4,))
+            self._buffer_views[key] = self._torch.as_tensor(arr, device=f"cuda:{self._device}")
+        return self._buffer_views[key]
+
     def _gram_partial(self, factor_side: int) -> Any:
         ptr, cnt = ctypes.c_void_p(0), ctypes.c_int64(0)
         self._check(self._lib.ials_trainer_gram_partial(self._handle, factor_side, ctypes.byref(ptr),
                                                         ctypes.byref(cnt)))
-        key = (factor_side, int(ptr.value))
-        if key not in self._gram_views:
-            arr = self._core._DeviceArray(int(ptr.value), (int(cnt.value),), (4,))
-            self._gram_views[key] = self._torch.as_tensor(arr, device=f"cuda:{self._device}")
-        return self._gram_views[key]
+        return self._buffer_view(ptr, cnt)
+
+    def _refit(self, side: int) -> None:
+        """The feature-weight refit of ``side`` after its solve (IALSTrainer.hpp:777-778): this rank's
+        F^T D F (first refit only) and F^T D X, all-reduced, then the same ridge solve on every rank.
+        Nothing (and no collective, on any rank) when the solve used no prior."""
+        bufs = [(ctypes.c_void_p(0), ctypes.c_int64(0)) for _ in range(2)]
+        self._check(self._lib.ials_trainer_feature_partials(
+            self._handle, side, ctypes.byref(bufs[0][0]), ctypes.byref(bufs[0][1]), ctypes.byref(bufs[1][0]),
+            ctypes.byref(bufs[1][1])))
+        for ptr, cnt in bufs:
+            if cnt.value:
+                self._all_reduce(self._buffer_view(ptr, cnt))
+        self._check(self._lib.ials_trainer_feature_refit(self._handle, side))
+
+    def _check_step(self, sc: Any) -> None:
+        """The rejections of a feature-aware epoch, before its first collective and before any factor
+        changes; decided from state every rank shares, so every rank raises alike."""
+        self._check(self._lib.ials_trainer_check_shard_step(self._handle, ctypes.byref(sc), *self._empty_row))
 
     def _all_reduce(self, view: Any) -> None:
         import torch.distributed as dist
@@ -393,10 +474,12 @@ class ShardedIALSTrainer:
             view.copy_(h)
 
     def step_async(self, solver_config: Any, events: Optional[list] = None) -> None:
-        """One epoch (IALSTrainer::step, IALSTrainer.hpp:784-788) across all ranks.  With
+        """One epoch (IALSTrainer::step, IALSTrainer.hpp:758-789) across all ranks.  With
         ``events`` (a list) seven CUDA events are appended: start, then after the partial Gram,
-        the Gram all-reduce and the row solve of each side (``phase_ms`` turns them into ms)."""
+        the Gram all-reduce and the row solve (with the feature-weight refit) of each side
+        (``phase_ms`` turns them into ms)."""
         sc = self._core.IALSTrainer._solver(solver_config)
+        self._check_step(sc)
         self._use_current_stream()
 
         def mark() -> None:
@@ -412,6 +495,7 @@ class ShardedIALSTrainer:
             self._all_reduce(view)
             mark()
             self._check(self._lib.ials_trainer_solve_shard(self._handle, side, ctypes.byref(sc)))
+            self._refit(side)
             mark()
 
     PHASES = ("gram_item_partial", "gram_item_allreduce", "solve_users",
@@ -455,6 +539,53 @@ class ShardedIALSTrainer:
     def step(self, solver_config: Any) -> None:
         self.step_async(solver_config)
         self.sync()
+
+    def compute_loss(self, solver_config: Any) -> float:
+        """IALSTrainer::compute_loss (IALSTrainer.hpp:836-940) of the sharded model, the same float
+        on every rank: every rank sums the terms of its own rows, rank 0 adds the Gram and the
+        feature-weight terms, and the float64 partials are all-reduced.  Call it after ``step`` /
+        ``sync`` (it reads the full replicas)."""
+        import torch.distributed as dist
+
+        sc = self._core.IALSTrainer._solver(solver_config)
+        self._use_current_stream()
+        out = ctypes.c_double(0.0)
+        self._check(self._lib.ials_trainer_compute_loss_shard(self._handle, ctypes.byref(sc),
+                                                              int(self.rank == 0), ctypes.byref(out)))
+        total = out.value
+        if self.world > 1:
+            dev = f"cuda:{self._device}" if dist.get_backend() == "nccl" else "cpu"
+            t = self._torch.tensor([total], dtype=self._torch.float64, device=dev)
+            dist.all_reduce(t)
+            total = float(t.item())
+        return float(np.float32(total))  # the reference returns a float (IALSTrainer.hpp:836)
+
+    def _get_feature_weight(self, side: int) -> np.ndarray:
+        n = ctypes.c_int64(0)
+        self._check(self._lib.ials_trainer_feature_weight_rows(self._handle, side, ctypes.byref(n)))
+        out = np.zeros((int(n.value), self.K), dtype=np.float32)
+        if n.value:
+            self._use_current_stream()
+            self._check(self._lib.ials_trainer_get_feature_weight(self._handle, side, self._core._ptr(out)))
+        return out
+
+    def _set_feature_weight(self, side: int, value: np.ndarray) -> None:
+        """Collective: every rank calls it; rank 0's matrix becomes every rank's weight."""
+        import torch.distributed as dist
+
+        if self.world > 1:
+            box = [np.ascontiguousarray(value, dtype=np.float32)]
+            dist.broadcast_object_list(box, src=0)
+            value = box[0]
+        value = np.ascontiguousarray(value, dtype=np.float32)
+        if value.ndim != 2 or (value.shape[0] and value.shape[1] != self.K):
+            raise ValueError(f"expected an (n, {self.K}) matrix, got {value.shape}")
+        self._use_current_stream()
+        self._check(self._lib.ials_trainer_set_feature_weight(self._handle, side, int(value.shape[0]),
+                                                              self._core._ptr(value)))
+
+    user_feature_weight = property(lambda s: s._get_feature_weight(0), lambda s, v: s._set_feature_weight(0, v))
+    item_feature_weight = property(lambda s: s._get_feature_weight(1), lambda s, v: s._set_feature_weight(1, v))
 
     def _get(self, side: int) -> np.ndarray:
         n = self.n_users if side == 0 else self.n_items
@@ -519,6 +650,7 @@ class ShardedIALSTrainer:
         ``user_rows`` / ``item_rows``: pinned float32 torch tensors of shape (shard rows, K)."""
         torch = self._torch
         sc = self._core.IALSTrainer._solver(solver_config)
+        self._check_step(sc)  # before the uploads: a rejected call leaves the factors as they were
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = torch.cuda.Stream(device=self._device)
             self._views = [self._factors_view(0), self._factors_view(1)]
@@ -543,6 +675,7 @@ class ShardedIALSTrainer:
                 with torch.cuda.stream(self._copy_stream):
                     self._copy_stream.wait_event(done)
                     user_rows.copy_(self._views[0][b:e, : self.K], non_blocking=True)
+            self._refit(side)
         b, e = self.item_range
         item_rows.copy_(self._views[1][b:e, : self.K], non_blocking=True)
         self._copy_stream.synchronize()
