@@ -298,6 +298,39 @@ IALS_API int ials_metrics_accumulate(const int32_t *rec, const int32_t *count, i
                                      int recall_with_cutoff, const double *discount, int device,
                                      void *cuda_stream, double *acc, int64_t *valid_user, int64_t *item_cnt);
 
+/* ---- evaluation passes that keep the lists on the device ----
+ * An evaluation set holds, on the trainer's device, everything an Evaluator pass needs besides the
+ * model: the ground-truth rows of users [row_begin, row_begin + n_rows) (CSR from 0, rows sorted
+ * ascending; host arrays, or device arrays with gt_on_device != 0, which are copied), the mask (both
+ * mask pointers NULL: the trainer's training rows, as the Evaluator's "train"; else a host CSR of
+ * n_rows rows without stored zeros), the allow-lists of ials_trainer_recommend_allowed (allow_n_lists
+ * 0, 1 or n_rows; rows relative to row_begin; they need the fused kernel: every cutoff <= 128, else
+ * IALS_ERR_NOT_IMPLEMENTED), the cutoffs (each in [1, n_items], <= 1024), recall_with_cutoff, and
+ * per cutoff the accumulators of Metrics::update (cpp_source/evaluator.cpp:127-166): five float64 sums,
+ * valid_user / total_user and the item-count histogram.  Uploaded once. */
+typedef struct ials_eval_set ials_eval_set;
+IALS_API int ials_eval_set_create(ials_trainer *t, int64_t row_begin, int64_t n_rows, const int64_t *gt_indptr,
+                                  const int32_t *gt_indices, int gt_on_device, const int64_t *mask_indptr,
+                                  const int32_t *mask_indices, int64_t allow_n_lists, const int64_t *allow_indptr,
+                                  const int32_t *allow_indices, const int64_t *cutoffs, int64_t n_cutoffs,
+                                  int recall_with_cutoff, ials_eval_set **out);
+IALS_API void ials_eval_set_destroy(ials_eval_set *e);
+/* Zeroes the accumulators on `cuda_stream`. */
+IALS_API int ials_eval_set_reset(ials_eval_set *e, void *cuda_stream);
+/* Device pointers of the accumulators, for an all-reduce in place: sums[n_cutoffs][5] (float64 hit,
+ * recall, ndcg, map, precision), counts[2][n_cutoffs] (int64 valid_user, then total_user) and
+ * hist[n_cutoffs][n_items] (int64). */
+IALS_API int ials_eval_set_buffers(ials_eval_set *e, double **sums, int64_t **counts, int64_t **hist,
+                                   int64_t *n_cutoffs, int64_t *n_items);
+/* out[n_cutoffs][3] = {appeared_item, entropy, gini_index} of each histogram, as Metrics::as_dict
+ * (:87-123) computes them, on the device without sorting; synchronous. */
+IALS_API int ials_eval_set_diversity(ials_eval_set *e, void *cuda_stream, double *out);
+/* One evaluation pass over users [user_begin, user_end) (inside the set's rows and, with the training
+ * mask, inside the rank's shard): the lists of ials_trainer_recommend[_allowed] with k = max(cutoffs),
+ * in chunks, each followed by the metrics kernel, on the trainer's stream; ADDS to the accumulators.
+ * The sums are deterministic: the same pass gives the same bits.  Returns when the pass is done. */
+IALS_API int ials_trainer_evaluate(ials_trainer *t, ials_eval_set *e, int64_t user_begin, int64_t user_end);
+
 /* retrieve_recommend_from_score<float>                 cpp_source/util.hpp:426-504
  * (bound as irspack.utils._util_cpp.retrieve_recommend_from_score_f32,
  * cpp_source/util.cpp; caller: utils/id_mapping.py:29-46, 297-324).

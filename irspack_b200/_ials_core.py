@@ -259,9 +259,9 @@ def _stream_of(device: int) -> int:
 class _DeviceArray:
     """Minimal ``__cuda_array_interface__`` carrier for zero-copy torch views."""
 
-    def __init__(self, ptr: int, shape: Tuple[int, ...], strides: Tuple[int, ...]) -> None:
+    def __init__(self, ptr: int, shape: Tuple[int, ...], strides: Tuple[int, ...], typestr: str = "<f4") -> None:
         self.__cuda_array_interface__ = {
-            "shape": shape, "typestr": "<f4", "data": (ptr, False), "version": 3,
+            "shape": shape, "typestr": typestr, "data": (ptr, False), "version": 3,
             "strides": strides,
         }
 

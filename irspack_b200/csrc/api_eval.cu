@@ -1,0 +1,243 @@
+// Evaluation passes behind the C ABI: an evaluation set (ground truth, optional mask and allow-lists,
+// cutoffs and per-cutoff accumulators, uploaded once) and one call that produces the lists of a range of
+// users and accumulates their metrics without the lists leaving the device.  A row-sharded trainer runs
+// it on its own users; the caller all-reduces the accumulators and reduces the merged histograms.
+#include <algorithm>
+#include <cmath>
+#include <vector>
+
+#include "trainer.cuh"
+
+using namespace ials;
+
+struct ials_eval_set {
+  int device = 0;
+  int64_t row_begin = 0, n_rows = 0, n_items = 0;
+  DeviceBuffer<int64_t> gt_indptr;  // [n_rows + 1], from 0
+  DeviceBuffer<int32_t> gt_indices;
+  int mask_mode = 0;                // 0: the trainer's training rows, 2: the mask below
+  DeviceBuffer<int64_t> m_indptr;
+  DeviceBuffer<int32_t> m_indices;
+  bool mask_sorted = true;
+  ListJob allow;                    // allow_n_lists / a_* of the lists (rows relative to row_begin)
+  DeviceBuffer<int64_t> a_indptr;
+  DeviceBuffer<int32_t> a_indices;
+  std::vector<uint32_t> a_words;
+  int n_cut = 0;
+  int64_t kmax = 0;
+  int recall_with_cutoff = 0;
+  DeviceBuffer<int32_t> cutoffs;           // [n_cut]
+  DeviceBuffer<double> discount, cum;      // [kmax]
+  DeviceBuffer<double> sums;               // [n_cut][5] hit, recall, ndcg, map, precision
+  DeviceBuffer<unsigned long long> counts; // valid_user[n_cut] | total_user[n_cut]
+  DeviceBuffer<unsigned long long> hist;   // [n_cut][n_items]
+  DeviceBuffer<double> partial;            // metrics kernel scratch
+  DeviceBuffer<unsigned char> div_ws;
+  DeviceBuffer<double> div_out;            // [3]
+};
+
+namespace {
+
+void zero_accumulators(ials_eval_set *e, cudaStream_t s) {
+  CUDA_CHECK(cudaMemsetAsync(e->sums.get(), 0, sizeof(double) * 5 * e->n_cut, s));
+  CUDA_CHECK(cudaMemsetAsync(e->counts.get(), 0, sizeof(unsigned long long) * 2 * e->n_cut, s));
+  CUDA_CHECK(cudaMemsetAsync(e->hist.get(), 0, sizeof(unsigned long long) * e->n_cut * e->n_items, s));
+}
+
+}  // namespace
+
+extern "C" {
+
+int ials_eval_set_create(ials_trainer *t, int64_t row_begin, int64_t n_rows, const int64_t *gt_indptr,
+                         const int32_t *gt_indices, int gt_on_device, const int64_t *mask_indptr,
+                         const int32_t *mask_indices, int64_t allow_n_lists, const int64_t *allow_indptr,
+                         const int32_t *allow_indices, const int64_t *cutoffs, int64_t n_cutoffs,
+                         int recall_with_cutoff, ials_eval_set **out) {
+  return guarded([&] {
+    require(t != nullptr && out != nullptr, "null pointer");
+    *out = nullptr;
+    require(row_begin >= 0 && n_rows >= 0 && row_begin + n_rows <= t->U, "bad user block");
+    require(n_cutoffs >= 1 && cutoffs != nullptr, "at least one cutoff");
+    int64_t kmax = 0;
+    for (int64_t c = 0; c < n_cutoffs; c++) {
+      require(cutoffs[c] >= 1 && cutoffs[c] <= t->I, "cutoff must be in [1, n_items]");  // evaluator.cpp:265-266
+      require(cutoffs[c] <= 1024, "k > 1024 is not supported");
+      kmax = std::max(kmax, cutoffs[c]);
+    }
+    require(gt_indptr != nullptr, "ground-truth indptr is null");
+    require(allow_n_lists == 0 || allow_n_lists == 1 || allow_n_lists == n_rows,
+            "allow-lists: one shared list or one per row");
+    const bool custom_mask = mask_indptr != nullptr;
+    if (!custom_mask) {
+      if (!t->has_X) throw std::runtime_error("no training matrix to mask with");
+      require(n_rows == 0 || (row_begin >= t->X.row_base && row_begin + n_rows <= t->X.row_base + t->X.n_rows),
+              "mask='train' on a sharded trainer needs a user block inside the rank's shard");
+    }
+    DeviceGuard g(t->device);
+    cudaStream_t s = t->stream;
+    auto e = std::make_unique<ials_eval_set>();
+    StreamSyncOnExit sync{s};  // the host staging below outlives the asynchronous copies
+    e->device = t->device;
+    e->row_begin = row_begin;
+    e->n_rows = n_rows;
+    e->n_items = t->I;
+    e->n_cut = (int)n_cutoffs;
+    e->kmax = kmax;
+    e->recall_with_cutoff = recall_with_cutoff ? 1 : 0;
+    // ground truth: rows sorted ascending (a binary search per recommended item)
+    int64_t gnnz = 0;
+    e->gt_indptr.alloc(n_rows + 1);
+    if (gt_on_device) {
+      int64_t ends[2] = {0, 0};
+      CUDA_CHECK(cudaMemcpyAsync(&ends[0], gt_indptr, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+      CUDA_CHECK(cudaMemcpyAsync(&ends[1], gt_indptr + n_rows, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+      CUDA_CHECK(cudaStreamSynchronize(s));
+      require(ends[0] == 0 && ends[1] >= 0, "ground-truth indptr must start at 0");
+      gnnz = ends[1];
+      require(gnnz == 0 || gt_indices != nullptr, "ground-truth indices are null");
+      CUDA_CHECK(cudaMemcpyAsync(e->gt_indptr.get(), gt_indptr, sizeof(int64_t) * (n_rows + 1),
+                                 cudaMemcpyDeviceToDevice, s));
+      e->gt_indices.alloc(std::max<int64_t>(gnnz, 1));
+      if (gnnz)
+        CUDA_CHECK(cudaMemcpyAsync(e->gt_indices.get(), gt_indices, sizeof(int32_t) * gnnz,
+                                   cudaMemcpyDeviceToDevice, s));
+    } else {
+      require(gt_indptr[0] == 0, "ground-truth indptr must start at 0");
+      gnnz = gt_indptr[n_rows];
+      require(gnnz == 0 || gt_indices != nullptr, "ground-truth indices are null");
+      for (int64_t r = 0; r < n_rows; r++) {
+        require(gt_indptr[r + 1] >= gt_indptr[r], "ground-truth indptr must be non-decreasing");
+        for (int64_t j = gt_indptr[r] + 1; j < gt_indptr[r + 1]; j++)
+          require(gt_indices[j - 1] <= gt_indices[j], "ground-truth rows must be sorted");
+      }
+      CUDA_CHECK(cudaMemcpyAsync(e->gt_indptr.get(), gt_indptr, sizeof(int64_t) * (n_rows + 1),
+                                 cudaMemcpyHostToDevice, s));
+      e->gt_indices.alloc(std::max<int64_t>(gnnz, 1));
+      if (gnnz)
+        CUDA_CHECK(cudaMemcpyAsync(e->gt_indices.get(), gt_indices, sizeof(int32_t) * gnnz,
+                                   cudaMemcpyHostToDevice, s));
+    }
+    if (custom_mask) {  // stored zeros already removed, as scipy's .nonzero() does
+      e->mask_mode = 2;
+      stage_mask(n_rows, t->I, mask_indptr, mask_indices, e->m_indptr, e->m_indices, s);
+      e->mask_sorted = mask_rows_sorted(n_rows, mask_indptr, mask_indices);
+    } else {
+      if (t->X.sorted_state < 0)
+        t->X.sorted_state = csr_rows_strictly_sorted(t->X.indptr.get(), t->X.indices.get(), t->X.n_rows, s) ? 1 : 0;
+      e->mask_sorted = t->X.sorted_state == 1;
+    }
+    if (allow_n_lists > 0) {
+      if (!(score_topk_tc_supported(t->ld, kmax) && e->mask_sorted))
+        throw NotImplemented("allow-lists need the fused tensor-core kernel (cutoff <= 128, sorted mask rows)");
+      stage_allow_lists(t->I, allow_n_lists, allow_indptr, allow_indices, e->a_words, e->a_indptr, e->a_indices,
+                        s, e->allow);
+    }
+    // prepare_dcg_discount (evaluator.cpp:42-48) and its prefix sums, the Evaluator's table
+    std::vector<double> disc((size_t)kmax), cum((size_t)kmax);
+    std::vector<int32_t> cut32((size_t)n_cutoffs);
+    double run = 0;
+    for (int64_t j = 0; j < kmax; j++) {
+      disc[j] = 1.0 / std::log2(2.0 + (double)j);
+      cum[j] = (run += disc[j]);
+    }
+    for (int64_t c = 0; c < n_cutoffs; c++) cut32[c] = (int32_t)cutoffs[c];
+    CUDA_CHECK(cudaMemcpyAsync(e->discount.alloc(kmax), disc.data(), sizeof(double) * kmax, cudaMemcpyHostToDevice, s));
+    CUDA_CHECK(cudaMemcpyAsync(e->cum.alloc(kmax), cum.data(), sizeof(double) * kmax, cudaMemcpyHostToDevice, s));
+    CUDA_CHECK(cudaMemcpyAsync(e->cutoffs.alloc(n_cutoffs), cut32.data(), sizeof(int32_t) * n_cutoffs,
+                               cudaMemcpyHostToDevice, s));
+    e->sums.alloc(5 * n_cutoffs);
+    e->counts.alloc(2 * n_cutoffs);
+    e->hist.alloc(n_cutoffs * t->I);
+    e->partial.alloc(5 * metrics_partials(kListSlabRows) * std::min<int64_t>(n_cutoffs, kMaxMetricsCutoffs));
+    e->div_out.alloc(3);
+    zero_accumulators(e.get(), s);
+    *out = e.release();
+  });
+}
+
+void ials_eval_set_destroy(ials_eval_set *e) {
+  if (e == nullptr) return;
+  int prev = -1;
+  cudaGetDevice(&prev);
+  cudaSetDevice(e->device);
+  delete e;
+  if (prev >= 0) cudaSetDevice(prev);
+}
+
+int ials_eval_set_reset(ials_eval_set *e, void *cuda_stream) {
+  return guarded([&] {
+    require(e != nullptr, "evaluation set is null");
+    DeviceGuard g(e->device);
+    zero_accumulators(e, (cudaStream_t)cuda_stream);
+  });
+}
+
+int ials_eval_set_buffers(ials_eval_set *e, double **sums, int64_t **counts, int64_t **hist, int64_t *n_cutoffs,
+                          int64_t *n_items) {
+  return guarded([&] {
+    require(e && sums && counts && hist && n_cutoffs && n_items, "null pointer");
+    *sums = e->sums.get();
+    *counts = reinterpret_cast<int64_t *>(e->counts.get());
+    *hist = reinterpret_cast<int64_t *>(e->hist.get());
+    *n_cutoffs = e->n_cut;
+    *n_items = e->n_items;
+  });
+}
+
+int ials_eval_set_diversity(ials_eval_set *e, void *cuda_stream, double *out) {
+  return guarded([&] {
+    require(e != nullptr && out != nullptr, "null pointer");
+    DeviceGuard g(e->device);
+    cudaStream_t s = (cudaStream_t)cuda_stream;
+    StreamSyncOnExit sync{s};
+    for (int c = 0; c < e->n_cut; c++) {
+      diversity_of_histogram(e->hist.get() + (int64_t)c * e->n_items, e->n_items, e->div_ws, e->div_out.get(), s);
+      CUDA_CHECK(cudaMemcpyAsync(out + 3 * c, e->div_out.get(), sizeof(double) * 3, cudaMemcpyDeviceToHost, s));
+      CUDA_CHECK(cudaStreamSynchronize(s));
+    }
+  });
+}
+
+int ials_trainer_evaluate(ials_trainer *t, ials_eval_set *e, int64_t user_begin, int64_t user_end) {
+  return guarded([&] {
+    require(t != nullptr && e != nullptr, "null pointer");
+    require(e->device == t->device && e->n_items == t->I, "the evaluation set belongs to another model");
+    require(user_begin >= e->row_begin && user_begin <= user_end && user_end <= e->row_begin + e->n_rows,
+            "users outside the evaluation set's rows");
+    const int64_t rows = user_end - user_begin;
+    if (rows == 0) return;
+    if (e->mask_mode == 0)
+      require(user_begin >= t->X.row_base && user_end <= t->X.row_base + t->X.n_rows,
+              "mask='train' on a sharded trainer needs a user block inside the rank's shard");
+    DeviceGuard g(t->device);
+    StreamSyncOnExit sync{t->stream};
+    const int64_t k = e->kmax, chunk = std::min(rows, kListSlabRows);
+    ListJob job = e->allow;
+    job.k = k;
+    job.mask_mode = e->mask_mode;
+    job.m_indptr = e->m_indptr.get();
+    job.m_indices = e->m_indices.get();
+    job.mask_sorted = e->mask_sorted;
+    job.idx = t->rec_idx.ensure(chunk * k);
+    job.score = t->rec_score.ensure(chunk * k);
+    job.count = t->rec_count.ensure(chunk);
+    for (int64_t b = 0; b < rows; b += chunk) {
+      const int64_t m = std::min(chunk, rows - b), r0 = user_begin + b - e->row_begin;  // set row of the chunk
+      job.user_rows = t->factor[0].get() + (user_begin + b) * t->ld;
+      job.rows = m;
+      job.x_row0 = user_begin + b - t->X.row_base;
+      job.m_row0 = r0;
+      job.a_row0 = r0;
+      produce_lists(t, job);
+      for (int c0 = 0; c0 < e->n_cut; c0 += kMaxMetricsCutoffs) {
+        const int nc = std::min(kMaxMetricsCutoffs, e->n_cut - c0);
+        launch_metrics_rows(job.idx, job.count, m, (int)k, e->gt_indptr.get() + r0, e->gt_indices.get(),
+                            e->discount.get(), e->cum.get(), e->cutoffs.get() + c0, nc, e->recall_with_cutoff,
+                            e->n_items, e->partial.get(), e->sums.get() + 5 * c0, e->counts.get() + c0,
+                            e->counts.get() + e->n_cut + c0, e->hist.get() + (int64_t)c0 * e->n_items, t->stream);
+      }
+    }
+  });
+}
+
+}  // extern "C"

@@ -18,8 +18,19 @@ void check_mask_pointers(int64_t rows, const int64_t *indptr, const int32_t *ind
           "mask indptr / indices must both be given");
 }
 
-// Validates a host mask CSR of `rows` rows over n_cols items and copies it into d_indptr / d_indices
-// (grown as needed) on stream s.
+// Copies the top-k lists of `rows` rows back to the host (out_score optional) and waits for them.
+void download_lists(const int32_t *d_idx, const float *d_sc, const int32_t *d_cnt, int64_t rows, int64_t k,
+                    int32_t *out_idx, float *out_score, int32_t *out_count, cudaStream_t s) {
+  CUDA_CHECK(cudaMemcpyAsync(out_idx, d_idx, sizeof(int32_t) * rows * k, cudaMemcpyDeviceToHost, s));
+  if (out_score) CUDA_CHECK(cudaMemcpyAsync(out_score, d_sc, sizeof(float) * rows * k, cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaMemcpyAsync(out_count, d_cnt, sizeof(int32_t) * rows, cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+}
+
+}  // namespace
+
+namespace ials {
+
 void stage_mask(int64_t rows, int64_t n_cols, const int64_t *indptr, const int32_t *indices,
                 DeviceBuffer<int64_t> &d_indptr, DeviceBuffer<int32_t> &d_indices, cudaStream_t s) {
   require(indptr != nullptr && indptr[0] == 0, "mask indptr must start at 0");
@@ -33,16 +44,87 @@ void stage_mask(int64_t rows, int64_t n_cols, const int64_t *indptr, const int32
     CUDA_CHECK(cudaMemcpyAsync(d_indices.get(), indices, sizeof(int32_t) * nnz, cudaMemcpyHostToDevice, s));
 }
 
-// Copies the top-k lists of `rows` rows back to the host (out_score optional) and waits for them.
-void download_lists(const int32_t *d_idx, const float *d_sc, const int32_t *d_cnt, int64_t rows, int64_t k,
-                    int32_t *out_idx, float *out_score, int32_t *out_count, cudaStream_t s) {
-  CUDA_CHECK(cudaMemcpyAsync(out_idx, d_idx, sizeof(int32_t) * rows * k, cudaMemcpyDeviceToHost, s));
-  if (out_score) CUDA_CHECK(cudaMemcpyAsync(out_score, d_sc, sizeof(float) * rows * k, cudaMemcpyDeviceToHost, s));
-  CUDA_CHECK(cudaMemcpyAsync(out_count, d_cnt, sizeof(int32_t) * rows, cudaMemcpyDeviceToHost, s));
-  CUDA_CHECK(cudaStreamSynchronize(s));
+bool mask_rows_sorted(int64_t rows, const int64_t *indptr, const int32_t *indices) {
+  for (int64_t r = 0; r < rows; r++)
+    for (int64_t j = indptr[r] + 1; j < indptr[r + 1]; j++)
+      if (indices[j - 1] >= indices[j]) return false;
+  return true;
 }
 
-}  // namespace
+void stage_allow_lists(int64_t n_items, int64_t n_lists, const int64_t *indptr, const int32_t *indices,
+                       std::vector<uint32_t> &words, DeviceBuffer<int64_t> &d_indptr,
+                       DeviceBuffer<int32_t> &d_indices, cudaStream_t s, ListJob &job) {
+  require(indptr != nullptr && indptr[0] == 0, "allow indptr must start at 0");
+  const int64_t annz = indptr[n_lists];
+  require(annz == 0 || indices != nullptr, "allow indices are null");
+  for (int64_t r = 0; r < n_lists; r++)
+    for (int64_t j = indptr[r]; j < indptr[r + 1]; j++) {
+      require(indices[j] >= 0 && indices[j] < n_items, "allowed item out of range");
+      require(j == indptr[r] || indices[j - 1] < indices[j], "allow-lists must be strictly ascending");
+    }
+  job.allow_n_lists = n_lists;
+  if (n_lists == 1) {  // a shared list goes to the kernel as a bitmap of the catalogue
+    words.assign((size_t)((n_items + 31) / 32), 0u);  // outlives the asynchronous copy
+    for (int64_t j = 0; j < annz; j++) words[indices[j] >> 5] |= 1u << (indices[j] & 31);
+    uint32_t *bitmap = reinterpret_cast<uint32_t *>(d_indices.ensure(words.size()));
+    CUDA_CHECK(cudaMemcpyAsync(bitmap, words.data(), sizeof(uint32_t) * words.size(), cudaMemcpyHostToDevice, s));
+    job.a_bitmap = bitmap;
+  } else {
+    int64_t *ip = d_indptr.ensure(n_lists + 1);
+    int32_t *ix = d_indices.ensure(std::max<int64_t>(annz, 1));
+    CUDA_CHECK(cudaMemcpyAsync(ip, indptr, sizeof(int64_t) * (n_lists + 1), cudaMemcpyHostToDevice, s));
+    if (annz) CUDA_CHECK(cudaMemcpyAsync(ix, indices, sizeof(int32_t) * annz, cudaMemcpyHostToDevice, s));
+    job.a_indptr = ip;
+    job.a_indices = ix;
+  }
+}
+
+void produce_lists(ials_trainer *t, const ListJob &j) {
+  const bool fused = score_topk_tc_supported(t->ld, j.k) && j.mask_sorted;
+  if (j.rowmap != nullptr && j.mask_mode == 0 && !fused)
+    throw NotImplemented("mask='train' for users picked by index needs the fused tensor-core kernel");
+  if (j.allow_n_lists > 0 && !fused)
+    throw NotImplemented("allow-lists need the fused tensor-core kernel (cutoff <= 128, sorted mask rows)");
+  const int64_t rows = j.rows, k = j.k;
+  if (fused) {
+    // scores + mask + top-k in one tcgen05 kernel; only candidate keys touch HBM
+    for (int64_t b = 0; b < rows; b += kListSlabRows) {
+      const int64_t m = std::min(kListSlabRows, rows - b);
+      void *scratch = ensure_score_buf(t, score_tc_scratch_bytes(m, t->I, k));
+      const int64_t *mip = nullptr;
+      const int32_t *mix = nullptr;
+      const float *mdt = nullptr;
+      int64_t mrow0 = 0;
+      const int64_t *mrowmap = nullptr;
+      if (j.mask_mode == 0) {
+        mip = t->X.indptr.get(); mix = t->X.indices.get(); mdt = t->X.data.get();
+        mrow0 = j.x_row0 + b;
+        if (j.rowmap) { mrowmap = j.rowmap + b; mrow0 = -t->X.row_base; }
+      } else if (j.mask_mode == 2) {
+        mip = j.m_indptr; mix = j.m_indices; mrow0 = j.m_row0 + b;
+      }
+      launch_score_topk_tc(j.user_rows + b * t->ld, m, t->factor[1].get(), t->I, t->ld, mip,
+                           mix, mdt, mrow0, (int)k, scratch, j.idx + b * k, j.score + b * k,
+                           j.count + b, t->stream, (int)std::min<int64_t>(j.allow_n_lists, 2), j.a_indptr,
+                           j.a_indices, j.a_row0 + b, j.a_bitmap, mrowmap);
+    }
+    return;
+  }
+  const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 29) / (4 * t->I)));
+  float *buf = ensure_score_buf(t, sizeof(float) * slab * t->I);
+  for (int64_t b = 0; b < rows; b += slab) {
+    const int64_t m = std::min(slab, rows - b);
+    launch_scores(j.user_rows + b * t->ld, m, t->factor[1].get(), t->I, t->ld, buf, t->I, t->stream);
+    if (j.mask_mode == 0)
+      launch_mask_rows(buf, t->I, t->X.indptr.get(), t->X.indices.get(), t->X.data.get(), j.x_row0 + b, m, 0,
+                       t->stream);
+    else if (j.mask_mode == 2)
+      launch_mask_rows(buf, t->I, j.m_indptr, j.m_indices, nullptr, j.m_row0 + b, m, 0, t->stream);
+    launch_topk_rows(buf, t->I, m, t->I, (int)k, j.idx + b * k, j.score + b * k, j.count + b, t->stream);
+  }
+}
+
+}  // namespace ials
 
 extern "C" {
 
@@ -119,109 +201,47 @@ static int recommend_impl(ials_trainer *t, const int64_t *user_idx, const float 
     }
     if (mask_mode == 2) {
       stage_mask(rows, t->I, mask_indptr, mask_indices, t->rec_mindptr, t->rec_mindices, t->stream);
-      for (int64_t r = 0; r < rows && mask_sorted; r++)
-        for (int64_t j = mask_indptr[r] + 1; j < mask_indptr[r + 1]; j++)
-          if (mask_indices[j - 1] >= mask_indices[j]) {
-            mask_sorted = false;
-            break;
-          }
+      mask_sorted = mask_rows_sorted(rows, mask_indptr, mask_indices);
       d_mindptr = t->rec_mindptr.get();
       d_mindices = t->rec_mindices.get();
     }
     int32_t *d_idx = t->rec_idx.ensure(rows * k);
     float *d_sc = t->rec_score.ensure(rows * k);
     int32_t *d_cnt = t->rec_count.ensure(rows);
-    // allow-lists (recommendable items): strictly ascending int32 lists, one shared or one per row
-    int64_t *d_aindptr = nullptr;
-    int32_t *d_aindices = nullptr;
-    uint32_t *d_abitmap = nullptr;
+    ListJob job;
+    job.user_rows = t->factor[0].get() + begin * t->ld;
+    job.rows = rows;
+    job.k = k;
+    job.mask_mode = mask_mode;
+    job.x_row0 = begin - t->X.row_base;
+    job.m_indptr = d_mindptr;
+    job.m_indices = d_mindices;
+    job.mask_sorted = mask_sorted;
+    job.idx = d_idx;
+    job.score = d_sc;
+    job.count = d_cnt;
     if (allow_n_lists > 0) {
       require(allow_n_lists == 1 || allow_n_lists == rows, "allow-lists: one shared list or one per row");
-      require(allow_indptr != nullptr && allow_indptr[0] == 0, "allow indptr must start at 0");
-      const int64_t annz = allow_indptr[allow_n_lists];
-      require(annz == 0 || allow_indices != nullptr, "allow indices are null");
-      for (int64_t r = 0; r < allow_n_lists; r++)
-        for (int64_t j = allow_indptr[r]; j < allow_indptr[r + 1]; j++) {
-          require(allow_indices[j] >= 0 && allow_indices[j] < t->I, "allowed item out of range");
-          require(j == allow_indptr[r] || allow_indices[j - 1] < allow_indices[j],
-                  "allow-lists must be strictly ascending");
-        }
-      if (allow_n_lists == 1) {  // a shared list goes to the kernel as a bitmap of the catalogue
-        std::vector<uint32_t> &words = t->rec_abitmap_host;  // outlives the asynchronous copy
-        words.assign((size_t)((t->I + 31) / 32), 0u);
-        for (int64_t j = 0; j < annz; j++) words[allow_indices[j] >> 5] |= 1u << (allow_indices[j] & 31);
-        d_abitmap = reinterpret_cast<uint32_t *>(t->rec_aindices.ensure(words.size()));
-        CUDA_CHECK(cudaMemcpyAsync(d_abitmap, words.data(), sizeof(uint32_t) * words.size(),
-                                   cudaMemcpyHostToDevice, t->stream));
-      } else {
-        d_aindptr = t->rec_aindptr.ensure(allow_n_lists + 1);
-        d_aindices = t->rec_aindices.ensure(std::max<int64_t>(annz, 1));
-        CUDA_CHECK(cudaMemcpyAsync(d_aindptr, allow_indptr, sizeof(int64_t) * (allow_n_lists + 1),
-                                   cudaMemcpyHostToDevice, t->stream));
-        if (annz)
-          CUDA_CHECK(cudaMemcpyAsync(d_aindices, allow_indices, sizeof(int32_t) * annz, cudaMemcpyHostToDevice,
-                                     t->stream));
-      }
+      stage_allow_lists(t->I, allow_n_lists, allow_indptr, allow_indices, t->rec_abitmap_host, t->rec_aindptr,
+                        t->rec_aindices, t->stream, job);
     }
-    const bool fused = score_topk_tc_supported(t->ld, k) && mask_sorted;
     // users picked by index: their factor rows are gathered into a dense block first
-    const float *user_rows = t->factor[0].get() + begin * t->ld;
-    int64_t *d_uidx = nullptr;
     if (user_idx != nullptr) {
-      d_uidx = t->rec_uidx.ensure(rows);
+      int64_t *d_uidx = t->rec_uidx.ensure(rows);
       float *gathered = t->rec_users.ensure(rows * t->ld);
       CUDA_CHECK(cudaMemcpyAsync(d_uidx, user_idx, sizeof(int64_t) * rows, cudaMemcpyHostToDevice, t->stream));
       launch_gather_rows(t->factor[0].get(), t->ld, d_uidx, rows, gathered, t->stream);
-      user_rows = gathered;
-      if (mask_mode == 0 && !fused)
-        throw NotImplemented("mask='train' for users picked by index needs the fused tensor-core kernel");
+      job.user_rows = gathered;
+      job.rowmap = d_uidx;
     }
     if (user_emb != nullptr) {  // host embeddings [rows x K] -> padded device rows [rows x ld]
       float *staged = t->rec_emb.ensure(rows * t->K);
       float *padded = t->rec_users.ensure(rows * t->ld);
       CUDA_CHECK(cudaMemcpyAsync(staged, user_emb, sizeof(float) * rows * t->K, cudaMemcpyHostToDevice, t->stream));
       launch_pad_copy(staged, rows, (int)t->K, padded, t->ld, t->stream);
-      user_rows = padded;
+      job.user_rows = padded;
     }
-    if (allow_n_lists > 0 && !fused)
-      throw NotImplemented("allow-lists need the fused tensor-core kernel (cutoff <= 128, sorted mask rows)");
-    if (fused) {
-      // scores + mask + top-k in one tcgen05 kernel; only candidate keys touch HBM
-      const int64_t slab_rows = std::max<int64_t>(128, ((1ll << 29) / (8 * 256)) / 128 * 128);
-      for (int64_t b = 0; b < rows; b += slab_rows) {
-        const int64_t m = std::min(slab_rows, rows - b);
-        void *scratch = ensure_score_buf(t, score_tc_scratch_bytes(m, t->I, k));
-        const int64_t *mip = nullptr;
-        const int32_t *mix = nullptr;
-        const float *mdt = nullptr;
-        int64_t mrow0 = 0;
-        const int64_t *mrowmap = nullptr;
-        if (mask_mode == 0) {
-          mip = t->X.indptr.get(); mix = t->X.indices.get(); mdt = t->X.data.get();
-          mrow0 = begin + b - t->X.row_base;
-          if (d_uidx) { mrowmap = d_uidx + b; mrow0 = -t->X.row_base; }
-        } else if (mask_mode == 2) {
-          mip = d_mindptr; mix = d_mindices; mrow0 = b;
-        }
-        launch_score_topk_tc(user_rows + b * t->ld, m, t->factor[1].get(), t->I, t->ld, mip,
-                             mix, mdt, mrow0, (int)k, scratch, d_idx + b * k, d_sc + b * k,
-                             d_cnt + b, t->stream, (int)std::min<int64_t>(allow_n_lists, 2), d_aindptr,
-                             d_aindices, b, d_abitmap, mrowmap);
-      }
-    }
-    const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 29) / (4 * t->I)));
-    float *buf = fused ? nullptr : ensure_score_buf(t, sizeof(float) * slab * t->I);
-    for (int64_t b = 0; b < rows && !fused; b += slab) {
-      const int64_t m = std::min(slab, rows - b);
-      launch_scores(user_rows + b * t->ld, m, t->factor[1].get(), t->I, t->ld, buf, t->I, t->stream);
-      if (mask_mode == 0)
-        launch_mask_rows(buf, t->I, t->X.indptr.get(), t->X.indices.get(), t->X.data.get(),
-                         begin + b - t->X.row_base, m, 0, t->stream);
-      else if (mask_mode == 2)
-        launch_mask_rows(buf, t->I, d_mindptr, d_mindices, nullptr, b, m, 0, t->stream);
-      launch_topk_rows(buf, t->I, m, t->I, (int)k, d_idx + b * k, d_sc + b * k, d_cnt + b,
-                       t->stream);
-    }
+    produce_lists(t, job);
     download_lists(d_idx, d_sc, d_cnt, rows, k, out_idx, out_score, out_count, t->stream);
   });
 }
@@ -286,13 +306,17 @@ int ials_metrics_accumulate(const int32_t *rec, const int32_t *count, int64_t ro
     std::vector<double> cum((size_t)k);
     double run = 0;
     for (int64_t j = 0; j < k; j++) cum[j] = (run += discount[j]);
-    // one allocation: rec | count | gt indptr | gt indices | discount | cum | acc[5] | valid | item_cnt
+    // one allocation: rec | count | gt indptr | gt indices | discount | cum | cutoff | partials |
+    // acc[5] | valid | total | item_cnt
+    const int32_t cutoff = (int32_t)k;
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
     const size_t o_rec = take(sizeof(int32_t) * rows * k), o_cnt = take(sizeof(int32_t) * rows),
                  o_ip = take(sizeof(int64_t) * (rows + 1)), o_ix = take(sizeof(int32_t) * std::max<int64_t>(gnnz, 1)),
-                 o_d = take(sizeof(double) * k), o_c = take(sizeof(double) * k), o_acc = take(sizeof(double) * 5),
-                 o_v = take(sizeof(unsigned long long)), o_ic = take(sizeof(unsigned long long) * n_items);
+                 o_d = take(sizeof(double) * k), o_c = take(sizeof(double) * k), o_k = take(sizeof(int32_t)),
+                 o_p = take(sizeof(double) * 5 * metrics_partials(rows)), o_acc = take(sizeof(double) * 5),
+                 o_v = take(sizeof(unsigned long long)), o_t = take(sizeof(unsigned long long)),
+                 o_ic = take(sizeof(unsigned long long) * n_items);
     DeviceBuffer<char> buf;
     StreamSyncOnExit sync{s};
     char *d = buf.alloc(off);
@@ -302,12 +326,14 @@ int ials_metrics_accumulate(const int32_t *rec, const int32_t *count, int64_t ro
     if (gnnz) CUDA_CHECK(cudaMemcpyAsync(d + o_ix, gt_indices, sizeof(int32_t) * gnnz, cudaMemcpyHostToDevice, s));
     CUDA_CHECK(cudaMemcpyAsync(d + o_d, discount, sizeof(double) * k, cudaMemcpyHostToDevice, s));
     CUDA_CHECK(cudaMemcpyAsync(d + o_c, cum.data(), sizeof(double) * k, cudaMemcpyHostToDevice, s));
+    CUDA_CHECK(cudaMemcpyAsync(d + o_k, &cutoff, sizeof(int32_t), cudaMemcpyHostToDevice, s));
     CUDA_CHECK(cudaMemsetAsync(d + o_acc, 0, off - o_acc, s));
     launch_metrics_rows(reinterpret_cast<int32_t *>(d + o_rec), reinterpret_cast<int32_t *>(d + o_cnt), rows, (int)k,
                         reinterpret_cast<int64_t *>(d + o_ip), reinterpret_cast<int32_t *>(d + o_ix),
                         reinterpret_cast<double *>(d + o_d), reinterpret_cast<double *>(d + o_c),
-                        recall_with_cutoff, reinterpret_cast<double *>(d + o_acc),
-                        reinterpret_cast<unsigned long long *>(d + o_v),
+                        reinterpret_cast<int32_t *>(d + o_k), 1, recall_with_cutoff, n_items,
+                        reinterpret_cast<double *>(d + o_p), reinterpret_cast<double *>(d + o_acc),
+                        reinterpret_cast<unsigned long long *>(d + o_v), reinterpret_cast<unsigned long long *>(d + o_t),
                         reinterpret_cast<unsigned long long *>(d + o_ic), s);
     double h_acc[5];
     unsigned long long h_valid = 0;

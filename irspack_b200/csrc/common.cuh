@@ -352,11 +352,23 @@ void launch_feature_llt(float *G, int64_t n, float lambda, int *fail, cudaStream
 void launch_feature_rhs(const FeatureDev &F, const float *rw, const float *X, int ld, float *R, cudaStream_t s);
 void launch_feature_solve(const float *L, int64_t n, float *R, int ld, int *fail, cudaStream_t s);
 
-// ranking metrics of recommendation lists (metrics.cu); acc = {hit, recall, ndcg, map, precision} sums
+// ranking metrics of recommendation lists (metrics.cu).  rec [rows x k] holds lists of length k; each of
+// the n_cut (<= kMaxMetricsCutoffs) device cutoffs (<= k) reads their prefix.  Per cutoff c:
+// acc[c][5] += {hit, recall, ndcg, map, precision} sums, valid_user[c] / total_user[c] counts,
+// item_cnt[c][n_items] += its histogram.  partial: metrics_partials(rows) x n_cut x 5 doubles of scratch.
+// Deterministic: the float64 sums are added in a fixed order.
+constexpr int kMaxMetricsCutoffs = 32;
+int64_t metrics_partials(int64_t rows);
 void launch_metrics_rows(const int32_t *rec, const int32_t *cnt, int64_t rows, int k, const int64_t *gt_indptr,
                          const int32_t *gt_indices, const double *discount, const double *cum_discount,
-                         int recall_with_cutoff, double *acc, unsigned long long *valid_user,
-                         unsigned long long *item_cnt, cudaStream_t s);
+                         const int32_t *cutoffs, int n_cut, int recall_with_cutoff, int64_t n_items,
+                         double *partial, double *acc, unsigned long long *valid_user,
+                         unsigned long long *total_user, unsigned long long *item_cnt, cudaStream_t s);
+// d_out[3] = {appeared_item, entropy, gini_index} of an item-count histogram (Metrics::as_dict without its
+// sort); ws: grow-only workspace.  Synchronises the stream once (the count-of-counts table is sized by the
+// largest count).
+void diversity_of_histogram(const unsigned long long *hist, int64_t n_items, DeviceBuffer<unsigned char> &ws,
+                            double *d_out, cudaStream_t s);
 void launch_gather_rows(const float *src, int ld, const int64_t *rows, int64_t n_rows, float *dst,
                         cudaStream_t s);
 void launch_pad_copy(const float *src, int64_t n_rows, int K, float *dst, int ld, cudaStream_t s);

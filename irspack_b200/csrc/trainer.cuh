@@ -181,6 +181,41 @@ void run_solver(ials_trainer *t, const SolveArgs &a, const DeviceCsr &csr,
 void ensure_copy_stream(ials_trainer *t);
 void enqueue_flagged_user_upload(ials_trainer *t, int64_t row_begin, int64_t n_rows, const float *rows_host);
 void consume_flagged_upload(ials_trainer *t, const ials_solver_config *sc, SolveArgs &a, int64_t row_begin);
+// api_recommend.cu: top-k lists of `rows` user rows, everything already on the device.  The fused
+// tensor-core kernel where it applies (score_topk_tc_supported, sorted mask rows), else scores + mask +
+// SIMT top-k; allow-lists and users picked by index with mask_mode 0 need the fused route
+// (NotImplemented otherwise).  Enqueued on t->stream.
+constexpr int64_t kListSlabRows = 262144;  // rows per fused launch: bounds its scratch (score_buf)
+struct ListJob {
+  const float *user_rows = nullptr;  // [rows x ld]
+  int64_t rows = 0, k = 0;
+  int mask_mode = 1;                 // 0: rows of X, 1: none, 2: the CSR below
+  int64_t x_row0 = 0;                // mode 0: row of X (local to the shard) that masks block row 0
+  const int64_t *rowmap = nullptr;   // mode 0, users picked by index: block row r is user rowmap[r]
+  const int64_t *m_indptr = nullptr; // mode 2: block row r is masked by CSR row m_row0 + r
+  const int32_t *m_indices = nullptr;
+  int64_t m_row0 = 0;
+  bool mask_sorted = true;           // column ids strictly ascending in every mask row
+  int64_t allow_n_lists = 0;         // 0, 1 (a_bitmap) or per row (CSR row a_row0 + r)
+  const int64_t *a_indptr = nullptr;
+  const int32_t *a_indices = nullptr;
+  const uint32_t *a_bitmap = nullptr;
+  int64_t a_row0 = 0;
+  int32_t *idx = nullptr;            // [rows x k] out
+  float *score = nullptr;            // [rows x k] out
+  int32_t *count = nullptr;          // [rows] out
+};
+void produce_lists(ials_trainer *t, const ListJob &j);
+// Validates a host mask CSR of `rows` rows over n_cols items and copies it into d_indptr / d_indices
+// (grown as needed) on stream s
+void stage_mask(int64_t rows, int64_t n_cols, const int64_t *indptr, const int32_t *indices,
+                DeviceBuffer<int64_t> &d_indptr, DeviceBuffer<int32_t> &d_indices, cudaStream_t s);
+bool mask_rows_sorted(int64_t rows, const int64_t *indptr, const int32_t *indices);
+// Validates host allow-lists (strictly ascending int32 ids in [0, n_items)) and uploads them on stream s
+// into job.allow_n_lists / a_bitmap (one shared list, staged in `words`) or a_indptr / a_indices
+void stage_allow_lists(int64_t n_items, int64_t n_lists, const int64_t *indptr, const int32_t *indices,
+                       std::vector<uint32_t> &words, DeviceBuffer<int64_t> &d_indptr,
+                       DeviceBuffer<int32_t> &d_indices, cudaStream_t s, ListJob &job);
 // api_features.cu
 void check_prior_defined(const ials_trainer *t, int side, bool has_empty_row);
 bool side_uses_features(const ials_trainer *t, int side);

@@ -340,6 +340,7 @@ class ShardedIALSTrainer:
         # per side: does some rank's shard hold an empty row (the guard of step_with_prior needs the
         # OR over all ranks, so that every rank rejects an epoch alike)
         self._empty_row = (0, 0)
+        self._feature_aware = user_feature is not None
         if user_feature is not None:
             self._set_features(model_config, (user_feature, item_feature))
         if self.world > 1:
@@ -460,6 +461,19 @@ class ShardedIALSTrainer:
         """The rejections of a feature-aware epoch, before its first collective and before any factor
         changes; decided from state every rank shares, so every rank raises alike."""
         self._check(self._lib.ials_trainer_check_shard_step(self._handle, ctypes.byref(sc), *self._empty_row))
+
+    def _all_reduce_max(self, host: Any) -> None:
+        """Element-wise MAX over ranks of a host tensor, in place."""
+        import torch.distributed as dist
+
+        if self.world == 1:
+            return
+        if dist.get_backend() == "nccl":
+            dev = host.to(f"cuda:{self._device}")
+            dist.all_reduce(dev, op=dist.ReduceOp.MAX)
+            host.copy_(dev.cpu())
+        else:
+            dist.all_reduce(host, op=dist.ReduceOp.MAX)
 
     def _all_reduce(self, view: Any) -> None:
         import torch.distributed as dist
@@ -696,6 +710,60 @@ class ShardedIALSTrainer:
                                                      p(None), p(None), p(idx), p(None), p(cnt)))
         return idx, cnt
 
+    # -- validation-based early stopping (BaseRecommenderWithEarlyStopping, base_earlystop.py:106-149) --
+    def save_state(self, state: Optional[dict] = None) -> dict:
+        """This rank's own rows of both factor matrices (into pinned host buffers: ``state`` from an
+        earlier call is reused) and, for the feature-aware model, the feature weights."""
+        if state is None:
+            state = {side: self._torch.empty((e - b, self.K), dtype=self._torch.float32, pin_memory=True)
+                     for side, (b, e) in enumerate((self.user_range, self.item_range))}
+        for side in (0, 1):
+            self.get_shard_rows(side, state[side].numpy())
+        if self._feature_aware:
+            state["weights"] = (self.user_feature_weight, self.item_feature_weight)
+        return state
+
+    def load_state(self, state: dict) -> None:
+        """Collective: every rank uploads its saved rows and copies them into the peers' replicas, the
+        weights are set on every rank, and ``sync`` leaves every replica on every rank identical."""
+        for side in (0, 1):
+            self.set_shard_rows(side, state[side].numpy(), push_to_peers=True)
+        if "weights" in state:
+            self.user_feature_weight, self.item_feature_weight = state["weights"]
+        self.sync()
+
+    def learn_with_optimizer(self, solver_config: Any, evaluator: Any = None, max_epoch: int = 128,
+                             validate_epoch: int = 5, score_degradation_max: int = 5) -> int:
+        """Collective epoch loop with validation-based early stopping (``IALSRecommender.
+        learn_with_optimizer``, base_earlystop.py:106-149).  ``evaluator``: a ``ShardedEvaluator`` of
+        this trainer; its score is the same on every rank, so is every decision.  Returns the number
+        of epochs of the model left in the trainer: the best validated one (``max_epoch`` without an
+        evaluator)."""
+        best_score = -float("inf")
+        best_epoch = 0
+        n_score_degradation = 0
+        state = None
+        for epoch in range(max_epoch):
+            self.step(solver_config)
+            if (epoch + 1) % validate_epoch or evaluator is None:
+                continue
+            target_score = evaluator.get_target_score(self)
+            if target_score > best_score:
+                best_score = target_score
+                state = self.save_state(state)
+                best_epoch = epoch + 1
+                n_score_degradation = 0
+            else:
+                n_score_degradation += 1
+                if n_score_degradation >= score_degradation_max:
+                    break
+        if evaluator is None:
+            return max_epoch
+        if state is None:
+            raise RuntimeError("'load_state' called before achieving any results.")
+        self.load_state(state)
+        return best_epoch
+
     def set_profiling(self, enabled: bool) -> None:
         self._check(self._lib.ials_trainer_set_profiling(self._handle, int(bool(enabled))))
 
@@ -706,6 +774,204 @@ class ShardedIALSTrainer:
         keys = ("rows", "nnz", "heavy_rows", "heavy_nnz", "jobs", "max_degree", "has_negative",
                 "reserved")
         return dict(zip(keys, (int(v) for v in out)))
+
+
+class ShardedEvaluator:
+    """The ``Evaluator`` of a row-sharded model, one per rank.
+
+    ``ground_truth`` holds THIS rank's user rows only (``trainer.user_range``), shape
+    ``(user_end - user_begin, n_items)``: a scipy matrix, or a device CSR triple ``(indptr, indices,
+    data)`` of torch tensors on the trainer's GPU (only the indices are read, stored zeros included, as
+    the ``Evaluator`` reads them).  ``per_user_recommendable_items`` and ``masked_interactions`` hold
+    the same rows; the other arguments are the ``Evaluator``'s.  ``from_global`` slices matrices every
+    rank holds in full.
+
+    ``get_score`` / ``get_scores`` / ``get_target_score`` are collective and return, on every rank,
+    what ``Evaluator`` returns for the gathered model.  Each rank scores and judges its own users on the
+    device (``ials_trainer_evaluate``: the fused lists of ``max(cutoffs)``, then the metrics of every
+    cutoff, no list leaves the device), the per-cutoff sums, counts and item histograms are
+    all-reduced, and the diversity metrics are reduced from the merged histograms on the device.
+    ``catalog_coverage`` divides by the number of recommendable items over ALL ranks' lists."""
+
+    def __init__(self, trainer: "ShardedIALSTrainer", ground_truth: Any, cutoff: int = 10,
+                 target_metric: str = "ndcg", recommendable_items: Optional[List[int]] = None,
+                 per_user_recommendable_items: Any = None, masked_interactions: Any = None,
+                 recall_with_cutoff: bool = False) -> None:
+        import torch
+
+        from .evaluation import Evaluator
+
+        self._trainer = trainer
+        self._sets: dict = {}
+        self._gt_device = None
+        self._lists = recommendable_items is not None or per_user_recommendable_items is not None
+        self.last_timings: dict = {}
+        ub, ue = trainer.user_range
+        err: Optional[BaseException] = None
+        try:
+            gt = ground_truth
+            if isinstance(gt, (tuple, list)):  # device CSR: rows sorted here, on the device
+                ip = gt[0].to(torch.int64)
+                ix = gt[1].to(torch.int64)
+                n_rows = ip.numel() - 1
+                if ip.device != torch.device(f"cuda:{trainer._device}") or ix.device != ip.device:
+                    raise ValueError(f"device CSR arrays must live on cuda:{trainer._device}")
+                rows = torch.repeat_interleave(torch.arange(n_rows, device=ip.device), ip[1:] - ip[:-1])
+                keys = torch.sort(rows * trainer.n_items + ix).values
+                self._gt_device = ((ip - ip[0]).contiguous(),
+                                   (keys - rows * trainer.n_items).to(torch.int32).contiguous())
+                gt = sps.csr_matrix((n_rows, trainer.n_items))
+            if gt.shape[1] != trainer.n_items:
+                raise ValueError("The model and evaluator assume different n_items.")
+            if gt.shape[0] != ue - ub:
+                raise ValueError(f"ground_truth must hold this rank's {ue - ub} user rows "
+                                 f"[{ub}, {ue}), got {gt.shape[0]}.")
+            self._ev = Evaluator(gt, offset=ub, cutoff=cutoff, target_metric=target_metric,
+                                 recommendable_items=recommendable_items,
+                                 per_user_recommendable_items=per_user_recommendable_items,
+                                 masked_interactions=masked_interactions, recall_with_cutoff=recall_with_cutoff)
+        except (ValueError, TypeError, KeyError, RuntimeError) as e:
+            err = e
+        failed, = trainer._max_over_ranks([1 if err is not None else 0])
+        trainer._raise_agreed(err, failed)
+        if recommendable_items is None and per_user_recommendable_items is not None:
+            # the union of every rank's lists: one OR of the catalogue bitmaps
+            seen = torch.zeros(trainer.n_items, dtype=torch.int32)
+            seen[torch.from_numpy(self._ev._allow_sorted_flat.astype(np.int64))] = 1
+            trainer._all_reduce_max(seen)
+            self._ev.n_recommendable_items = int(seen.sum())
+
+    @classmethod
+    def from_global(cls, trainer: "ShardedIALSTrainer", ground_truth: Any,
+                    per_user_recommendable_items: Any = None, masked_interactions: Any = None,
+                    **kw: Any) -> "ShardedEvaluator":
+        """Slice matrices (and per-user lists) that every rank holds in full by ``trainer.user_range``."""
+        ub, ue = trainer.user_range
+
+        def rows(m: Any) -> Any:
+            if m is None:
+                return None
+            return sps.csr_matrix(m)[ub:ue] if sps.issparse(m) else m[ub:ue]
+
+        return cls(trainer, rows(sps.csr_matrix(ground_truth)), per_user_recommendable_items=rows(
+            per_user_recommendable_items), masked_interactions=rows(masked_interactions), **kw)
+
+    def __del__(self) -> None:
+        from ._lib import lib
+
+        for h in getattr(self, "_sets", {}).values():
+            lib.ials_eval_set_destroy(h)
+        self._sets = {}
+
+    @property
+    def cutoff(self) -> int:
+        return self._ev.cutoff
+
+    @property
+    def target_metric_name(self) -> str:
+        return self._ev.target_metric_name
+
+    def get_target_score(self, trainer: "ShardedIALSTrainer") -> float:
+        return self.get_score(trainer)[self._ev.target_metric.name]
+
+    def get_score(self, trainer: "ShardedIALSTrainer") -> dict:
+        return self._get_scores_as_list(trainer, [self._ev.cutoff])[0]
+
+    def get_scores(self, trainer: "ShardedIALSTrainer", cutoffs: List[int]) -> dict:
+        return self._ev._flatten(cutoffs, self._get_scores_as_list(trainer, cutoffs))
+
+    def _set_for(self, trainer: "ShardedIALSTrainer", cutoffs: Tuple[int, ...]) -> ctypes.c_void_p:
+        from . import _ials_core as core
+        from .evaluation import _mask_csr
+        from ._lib import check, lib
+
+        h = self._sets.get(cutoffs)
+        if h is not None:
+            return h
+        ev, p = self._ev, core._ptr
+        ub, ue = trainer.user_range
+        if self._gt_device is not None:
+            gi, gx = self._gt_device
+            g_ptrs, on_device = (ctypes.c_void_p(gi.data_ptr()), ctypes.c_void_p(gx.data_ptr())), 1
+        else:
+            gi = np.ascontiguousarray(ev.ground_truth.indptr, dtype=np.int64)
+            gx = np.ascontiguousarray(ev.ground_truth.indices, dtype=np.int32)
+            g_ptrs, on_device = (p(gi), p(gx)), 0
+        mi = mx = None
+        if ev.masked_interactions is not None:
+            mi, mx = _mask_csr(ev.masked_interactions)
+        n_lists, ai, ax = ev._allowed_for(0, ue - ub, canonical=True) or (0, None, None)
+        cut = np.ascontiguousarray(cutoffs, dtype=np.int64)
+        h = ctypes.c_void_p(0)
+        trainer._use_current_stream()
+        check(lib.ials_eval_set_create(trainer._handle, ub, ue - ub, g_ptrs[0], g_ptrs[1], on_device, p(mi),
+                                       p(mx), int(n_lists), p(ai), p(ax), p(cut), len(cutoffs),
+                                       int(bool(ev.recall_with_cutoff)), ctypes.byref(h)))
+        self._sets[cutoffs] = h
+        return h
+
+    def _views(self, h: ctypes.c_void_p) -> Tuple[Any, Any, Any]:
+        """Zero-copy torch views of the set's sums (float64), counts and histograms (int64)."""
+        from . import _ials_core as core
+        from ._lib import check, lib
+
+        ptrs = [ctypes.c_void_p(0) for _ in range(3)]
+        n_cut, n_items = ctypes.c_int64(0), ctypes.c_int64(0)
+        check(lib.ials_eval_set_buffers(h, *(ctypes.byref(x) for x in ptrs), ctypes.byref(n_cut),
+                                        ctypes.byref(n_items)))
+        dev = f"cuda:{self._trainer._device}"
+        out = []
+        for ptr, n, typ in zip(ptrs, (5 * n_cut.value, 2 * n_cut.value, n_cut.value * n_items.value),
+                               ("<f8", "<i8", "<i8")):
+            out.append(self._trainer._torch.as_tensor(core._DeviceArray(int(ptr.value), (n,), (8,), typ),
+                                                      device=dev))
+        return out[0], out[1], out[2]
+
+    def _get_scores_as_list(self, trainer: "ShardedIALSTrainer", cutoffs: List[int]) -> List[dict]:
+        from .evaluation import Metrics
+        from ._lib import check, lib
+
+        ev = self._ev
+        cutoffs = [int(c) for c in cutoffs]
+        ev._check_cutoffs(cutoffs)  # the same cutoffs and n_items on every rank: every rank raises alike
+        if self._lists and max(cutoffs) > 128:
+            raise NotImplementedError("allow-lists need the fused tensor-core kernel (cutoff <= 128)")
+        torch = trainer._torch
+        timings = {}
+        err: Optional[BaseException] = None
+        t0 = time.perf_counter()
+        try:
+            if trainer is not self._trainer:
+                raise ValueError("the ShardedEvaluator was built for another trainer")
+            h = self._set_for(trainer, tuple(cutoffs))
+            stream = trainer._core._stream_of(trainer._device)
+            check(lib.ials_eval_set_reset(h, ctypes.c_void_p(stream)))
+            trainer._use_current_stream()
+            ub, ue = trainer.user_range
+            check(lib.ials_trainer_evaluate(trainer._handle, h, ub, ue))
+        except (ValueError, RuntimeError, NotImplementedError) as e:
+            err = e
+        failed, = trainer._max_over_ranks([1 if err is not None else 0])
+        trainer._raise_agreed(err, failed)
+        t1 = time.perf_counter()
+        sums, counts, hist = self._views(h)
+        for view in (sums, counts, hist):
+            trainer._all_reduce(view)
+        torch.cuda.current_stream(trainer._device).synchronize()
+        t2 = time.perf_counter()
+        div = np.empty((len(cutoffs), 3), dtype=np.float64)
+        check(lib.ials_eval_set_diversity(h, ctypes.c_void_p(stream), div.ctypes.data_as(ctypes.c_void_p)))
+        t3 = time.perf_counter()
+        s_host, c_host = sums.cpu().numpy().reshape(-1, 5), counts.cpu().numpy()
+        self.last_timings = {"evaluate_s": t1 - t0, "allreduce_s": t2 - t1, "diversity_s": t3 - t2}
+        out = []
+        n_cut = len(cutoffs)
+        for c in range(n_cut):
+            m = Metrics(ev.n_items)
+            m.hit, m.recall, m.ndcg, m.map, m.precision = (float(v) for v in s_host[c])
+            m.valid_user, m.total_user = int(c_host[c]), int(c_host[n_cut + c])
+            out.append(ev._metrics_as_dict(m, tuple(float(v) for v in div[c])))
+        return out
 
 
 # ----------------------------------------------------------------------------

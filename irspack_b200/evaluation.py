@@ -132,6 +132,25 @@ class Metrics:
         self.map += float((ap / n_gt).sum())
         self.item_cnt += np.bincount(rec[in_list], minlength=self.n_item)
 
+    @staticmethod
+    def diversity(item_cnt: np.ndarray) -> Tuple[float, float, float]:
+        """(appeared_item, entropy, gini_index) of an item-count histogram (evaluator.cpp:87-123)."""
+        cnt = np.sort(item_cnt)
+        total_item = float(cnt.sum())
+        nz = cnt > 0
+        appeared = float(nz.sum())
+        entropy = 0.0
+        gini = 0.0
+        n = cnt.shape[0]
+        if appeared:
+            p = cnt[nz] / total_item
+            entropy = float((-np.log(p) * p).sum())
+            idx = np.flatnonzero(nz).astype(np.float64)
+            gini = float(((2 * idx - n + 1) * cnt[nz]).sum())
+        if total_item > 0:
+            gini /= n * total_item
+        return appeared, entropy, gini
+
     def _update_block_device(self, rec: np.ndarray, n_rec: np.ndarray, gt: sps.csr_matrix,
                              recall_with_cutoff: bool) -> None:
         rows, cutoff = rec.shape
@@ -159,21 +178,13 @@ class Metrics:
         self.map += float(acc[3])
         self.precision += float(acc[4])
 
-    def as_dict(self) -> Dict[str, float]:  # evaluator.cpp:87-123
-        cnt = np.sort(self.item_cnt)
-        total_item = float(cnt.sum())
-        nz = cnt > 0
-        appeared = float(nz.sum())
-        entropy = 0.0
-        gini = 0.0
-        n = cnt.shape[0]
-        if appeared:
-            p = cnt[nz] / total_item
-            entropy = float((-np.log(p) * p).sum())
-            idx = np.flatnonzero(nz).astype(np.float64)
-            gini = float(((2 * idx - n + 1) * cnt[nz]).sum())
-        if total_item > 0:
-            gini /= n * total_item
+    def as_dict(self, diversity: Optional[Tuple[float, float, float]] = None) -> Dict[str, float]:
+        """evaluator.cpp:87-123.  ``diversity``: (appeared_item, entropy, gini_index) when they were
+        reduced elsewhere (``ShardedEvaluator``: on the device, from the histogram merged over ranks);
+        None reduces ``item_cnt`` here."""
+        if diversity is None:
+            diversity = self.diversity(self.item_cnt)
+        appeared, entropy, gini = diversity
         den = self.valid_user if self.valid_user > 0 else 1
         return {
             "total_user": float(self.total_user), "valid_user": float(self.valid_user),
@@ -439,8 +450,9 @@ class Evaluator:
                 result[f"{name}@{cutoff}"] = score[name]
         return result
 
-    def _metrics_as_dict(self, metrics: Metrics) -> Dict[str, float]:  # evaluator.py:326-334
-        result = metrics.as_dict()
+    def _metrics_as_dict(self, metrics: Metrics, diversity: Optional[Tuple[float, float, float]] = None
+                         ) -> Dict[str, float]:  # evaluator.py:326-334
+        result = metrics.as_dict(diversity)
         result["catalog_coverage"] = (
             result["appeared_item"] / self.n_recommendable_items
             if self.n_recommendable_items else float("nan"))
