@@ -15,6 +15,7 @@ from __future__ import annotations
 import ctypes
 import enum
 import os
+import types
 from typing import Any, Optional, Tuple
 
 import numpy as np
@@ -256,14 +257,26 @@ def _stream_of(device: int) -> int:
     return 0
 
 
-class _DeviceArray:
-    """Minimal ``__cuda_array_interface__`` carrier for zero-copy torch views."""
+def _device_view(ptr: int, shape: Tuple[int, ...], strides: Tuple[int, ...], device: int,
+                 typestr: str = "<f4") -> Any:
+    """Zero-copy torch view of library-owned memory on ``cuda:device`` (``strides`` in bytes)."""
+    import torch
 
-    def __init__(self, ptr: int, shape: Tuple[int, ...], strides: Tuple[int, ...], typestr: str = "<f4") -> None:
-        self.__cuda_array_interface__ = {
-            "shape": shape, "typestr": typestr, "data": (ptr, False), "version": 3,
-            "strides": strides,
-        }
+    carrier = types.SimpleNamespace(__cuda_array_interface__={
+        "shape": shape, "typestr": typestr, "data": (ptr, False), "version": 3, "strides": strides})
+    return torch.as_tensor(carrier, device=f"cuda:{device}")
+
+
+def _factors_device(handle: ctypes.c_void_p, side: int, device: int) -> Any:
+    """Zero-copy view ([n, K], row stride ld) of a trainer's factor matrix (or replica) of ``side``."""
+    import torch
+
+    p, n, K, ld = ctypes.c_void_p(0), ctypes.c_int64(0), ctypes.c_int64(0), ctypes.c_int64(0)
+    check(lib.ials_trainer_factors_device(handle, side, ctypes.byref(p), ctypes.byref(n), ctypes.byref(K),
+                                          ctypes.byref(ld)))
+    if n.value == 0:
+        return torch.empty((0, K.value), dtype=torch.float32, device=f"cuda:{device}")
+    return _device_view(int(p.value), (int(n.value), int(ld.value)), (int(ld.value) * 4, 4), device)[:, : K.value]
 
 
 class IALSTrainer:
@@ -650,12 +663,4 @@ class IALSTrainer:
 
     def factors_device(self, side: int):
         """Zero-copy ``torch`` view ([n, K], row stride ld) of a factor matrix."""
-        import torch
-
-        p, n, K, ld = ctypes.c_void_p(0), ctypes.c_int64(0), ctypes.c_int64(0), ctypes.c_int64(0)
-        check(lib.ials_trainer_factors_device(self._handle, side, ctypes.byref(p), ctypes.byref(n),
-                                              ctypes.byref(K), ctypes.byref(ld)))
-        if n.value == 0:
-            return torch.empty((0, K.value), dtype=torch.float32, device=f"cuda:{self._device}")
-        arr = _DeviceArray(int(p.value), (int(n.value), int(ld.value)), (int(ld.value) * 4, 4))
-        return torch.as_tensor(arr, device=f"cuda:{self._device}")[:, : K.value]
+        return _factors_device(self._handle, side, self._device)

@@ -23,11 +23,12 @@ for the world_size-2 CPU tests.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 import json
 import os
 import time
-from typing import Any, List, Optional, Sequence, Tuple
+from typing import Any, Callable, Iterator, List, Optional, Sequence, Tuple
 
 import numpy as np
 import scipy.sparse as sps
@@ -53,49 +54,44 @@ def balanced_bounds(weights: np.ndarray, world: int) -> np.ndarray:
     return np.maximum.accumulate(np.minimum(bounds, n))
 
 
-def transposed_pieces(X_local: sps.csr_matrix, user_offset: int, item_bounds: Sequence[int]
-                      ) -> List[Tuple[np.ndarray, np.ndarray, np.ndarray]]:
-    """Cut this rank's user block (rows = its users, columns = all items) into the
-    pieces of X^T each rank needs: for destination d, items
-    ``[item_bounds[d], item_bounds[d+1])`` as (per-item counts int64, global user
-    ids int32 ascending within an item, values float32)."""
-    Xc = sps.csc_matrix(X_local)
-    Xc.sort_indices()
-    indptr = Xc.indptr.astype(np.int64)
-    out = []
-    for d in range(len(item_bounds) - 1):
-        b, e = int(item_bounds[d]), int(item_bounds[d + 1])
-        s, t = indptr[b], indptr[e]
-        counts = np.diff(indptr[b:e + 1]).astype(np.int64)
-        users = (Xc.indices[s:t].astype(np.int64) + user_offset).astype(np.int32)
-        out.append((counts, users, Xc.data[s:t].astype(np.float32)))
-    return out
+def _all_reduce(t: Any, device: Any, op: str = "sum") -> Any:
+    """In-place all-reduce (``op`` "sum" or "max") of the tensor ``t`` over the ranks; nothing at world 1.
+    NCCL reduces on the CUDA ``device`` (an ordinal or a torch.device) and gloo on the host: a tensor
+    that lives elsewhere is staged there and copied back.  Returns ``t``."""
+    import torch.distributed as dist
+
+    if not dist.is_initialized() or dist.get_world_size() == 1:
+        return t
+    work = t.cuda(device) if dist.get_backend() == "nccl" else t.cpu()
+    dist.all_reduce(work, op=dist.ReduceOp.MAX if op == "max" else dist.ReduceOp.SUM)
+    if work is not t:
+        t.copy_(work)
+    return t
 
 
-def assemble_transposed_shard(pieces: Sequence[Tuple[np.ndarray, np.ndarray, np.ndarray]],
-                              n_users_global: int) -> sps.csr_matrix:
-    """Merge the pieces received from ranks 0..world-1 (ascending user blocks) into
-    this rank's rows of X^T (CSR: items x all users, user ids ascending)."""
-    n_items = pieces[0][0].shape[0]
-    counts = np.stack([p[0] for p in pieces])            # [world, n_items]
-    total = counts.sum(axis=0)
-    indptr = np.zeros(n_items + 1, dtype=np.int64)
-    np.cumsum(total, out=indptr[1:])
-    nnz = int(indptr[-1])
-    indices = np.empty(nnz, dtype=np.int32)
-    data = np.empty(nnz, dtype=np.float32)
-    before = np.cumsum(counts, axis=0) - counts          # entries of earlier sources per item
-    for s, (cnt, users, vals) in enumerate(pieces):
-        if users.size == 0:
-            continue
-        start = indptr[:-1] + before[s]                  # destination of each item's run
-        src_start = np.concatenate([[0], np.cumsum(cnt)[:-1]])
-        pos = np.repeat(start - src_start, cnt) + np.arange(users.size, dtype=np.int64)
-        indices[pos] = users
-        data[pos] = vals
-    M = sps.csr_matrix((data, indices, indptr), shape=(n_items, n_users_global))
-    M.has_sorted_indices = True
-    return M
+@contextlib.contextmanager
+def _agreement(device: Any, values: Optional[List[int]] = None) -> Iterator[None]:
+    """``with _agreement(device):`` around the rank-local part of a collective call makes every rank
+    raise or none: the rank that raised gets its own exception, the others a ``RuntimeError`` naming
+    a peer's failure, after one all-reduce(max) of the failure flag.  The integers of ``values``
+    ride on the same all-reduce: on exit the list holds their maximum over the ranks.
+
+    It agrees on the exceptions that argument checks and ``_lib.check`` raise; any other exception
+    skips the agreement and leaves this rank's peers waiting in their next collective."""
+    import torch
+
+    values = [] if values is None else values
+    err: Optional[BaseException] = None
+    try:
+        yield
+    except (ValueError, TypeError, KeyError, RuntimeError) as e:  # NotImplementedError is a RuntimeError
+        err = e
+    flags = _all_reduce(torch.tensor([int(err is not None)] + values, dtype=torch.int64), device, "max").tolist()
+    if err is not None:
+        raise err
+    if flags[0]:
+        raise RuntimeError("a peer rank failed (see that rank's exception)")
+    values[:] = flags[1:]
 
 
 def _p2p_exchange(send: List[Any], rank: int, world: int, device: Any) -> List[Any]:
@@ -125,39 +121,10 @@ def _p2p_exchange(send: List[Any], rank: int, world: int, device: Any) -> List[A
     return recv
 
 
-def exchange_transposed_shards(X_local: sps.csr_matrix, user_offset: int, n_users_global: int,
-                               item_bounds: Sequence[int], device: Any = "cpu") -> sps.csr_matrix:
-    """Collective: every rank contributes its user block and receives its rows of
-    X^T (items ``[item_bounds[rank], item_bounds[rank+1])`` x all users)."""
-    import torch
-    import torch.distributed as dist
-
-    rank, world = dist.get_rank(), dist.get_world_size()
-    pieces = transposed_pieces(X_local, user_offset, item_bounds)
-    got = []
-    for field, dtype in ((0, torch.int64), (1, torch.int32), (2, torch.float32)):
-        send = [torch.from_numpy(np.ascontiguousarray(p[field])).to(device=device, dtype=dtype)
-                for p in pieces]
-        got.append([t.cpu().numpy() for t in _p2p_exchange(send, rank, world, device)])
-    merged = [(got[0][s], got[1][s], got[2][s]) for s in range(world)]
-    return assemble_transposed_shard(merged, n_users_global)
-
-
-def global_item_bounds(X_local: sps.csr_matrix, device: Any = "cpu") -> np.ndarray:
-    """nnz-balanced item ranges from the global item degrees (all-reduce of bincounts)."""
-    import torch
-    import torch.distributed as dist
-
-    cnt = torch.from_numpy(np.bincount(X_local.indices, minlength=X_local.shape[1]).astype(np.int64))
-    cnt = cnt.to(device)
-    dist.all_reduce(cnt)
-    return balanced_bounds(cnt.cpu().numpy() + 1, dist.get_world_size())
-
-
 # ----------------------------------------------------------------------------
-# device-resident shard construction (1 B-interaction matrices: BASELINE configs[3], [4]).
-# Same results as the scipy functions above, on torch tensors of any device: nothing of the
-# matrix touches the host, so a 125 M-interaction shard per rank is built in seconds.
+# shard construction on torch tensors of any device (1 B-interaction matrices: BASELINE
+# configs[3], [4]): on the GPU nothing of the matrix touches the host, so a 125 M-interaction
+# shard per rank is built in seconds.
 # ----------------------------------------------------------------------------
 
 
@@ -199,25 +166,23 @@ def synth_user_block_device(n_users_block: int, n_items: int, nnz_block: int, se
     return indptr, indices, torch.ones(nnz_block, dtype=torch.float32, device=device)
 
 
-def global_item_bounds_device(indices: Any, n_items: int) -> np.ndarray:
-    """``global_item_bounds`` for a device-resident block (all-reduce of the item degrees)."""
+def global_item_bounds(indices: Any, n_items: int) -> np.ndarray:
+    """nnz-balanced item ranges from the global item degrees: ``indices`` are this rank's column
+    indices, their bincounts are all-reduced."""
     import torch
     import torch.distributed as dist
 
-    cnt = torch.bincount(indices.to(torch.int64), minlength=n_items)
-    if dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(cnt)
+    cnt = _all_reduce(torch.bincount(indices.to(torch.int64), minlength=n_items), indices.device)
     world = dist.get_world_size() if dist.is_initialized() else 1
     return balanced_bounds(cnt.cpu().numpy() + 1, world)
 
 
-def exchange_transposed_shards_device(indptr: Any, indices: Any, data: Any, user_offset: int,
-                                      n_users_global: int, item_bounds: Sequence[int]
-                                      ) -> Tuple[Any, Any, Any]:
-    """``exchange_transposed_shards`` on device tensors: every rank contributes its user block
-    (CSR, local rows) and receives its rows of X^T -- items
-    ``[item_bounds[rank], item_bounds[rank + 1])`` x all users -- as a device CSR
-    ``(indptr int64, indices int32 = global user ids ascending, data float32)``.
+def exchange_transposed_shards(indptr: Any, indices: Any, data: Any, user_offset: int, n_users_global: int,
+                               item_bounds: Sequence[int]) -> Tuple[Any, Any, Any]:
+    """Collective: every rank contributes its user block (CSR of torch tensors, local rows) and
+    receives its rows of X^T -- items ``[item_bounds[rank], item_bounds[rank + 1])`` x all users --
+    as a CSR on the same device ``(indptr int64, indices int32 = global user ids ascending, data
+    float32)``.
 
     One key per interaction, ``item * n_users_global + user``: sorting the keys IS the
     transposition; destinations are contiguous key ranges."""
@@ -257,13 +222,30 @@ def exchange_transposed_shards_device(indptr: Any, indices: Any, data: Any, user
 # ----------------------------------------------------------------------------
 
 
+def _device_csr(triple: Any, device: int) -> Tuple[Any, Any, Any]:
+    """A device CSR ``(indptr, indices, data)`` of torch tensors as contiguous int64, int32 and
+    float32 tensors, rejected unless it lives on ``cuda:device`` and its lengths fit together."""
+    import torch
+
+    ip, ix, dt = triple
+    ip = ip.to(dtype=torch.int64).contiguous()
+    ix = ix.to(dtype=torch.int32).contiguous()
+    dt = dt.to(dtype=torch.float32).contiguous()
+    for t in (ip, ix, dt):
+        if not t.is_cuda or t.device.index != device:
+            raise ValueError(f"device CSR arrays must live on cuda:{device}")
+    if ix.numel() != dt.numel() or ip.numel() < 1:
+        raise ValueError("malformed device CSR")
+    return ip, ix, dt
+
+
 class ShardedIALSTrainer:
     """One rank of the row-sharded trainer (``ials_trainer_create_sharded``).
 
     ``X_user_rows``: this rank's users x all items (CSR); ``Xt_item_rows``: this
     rank's items x all users (CSR) -- two scipy matrices, or two device CSR triples
     ``(indptr, indices, data)`` of torch tensors on this rank's GPU
-    (``exchange_transposed_shards_device``).  ``user`` / ``item`` return the local full
+    (``exchange_transposed_shards``).  ``user`` / ``item`` return the local full
     replicas, identical on every rank after ``sync()``.
 
     ``user_feature`` / ``item_feature`` (both or neither): this rank's rows of the feature
@@ -292,28 +274,11 @@ class ShardedIALSTrainer:
         on_device = isinstance(X_user_rows, (tuple, list))
         if on_device != isinstance(Xt_item_rows, (tuple, list)):
             raise ValueError("both shards must be scipy matrices or both device CSR triples")
-        if on_device:
-            # (indptr int64, indices int32, data float32) torch tensors on this rank's GPU
-            # (exchange_transposed_shards_device); the library copies them (device to device)
-            keep = []
-            ptrs = []
-            rows = []
-            for triple in (X_user_rows, Xt_item_rows):
-                ip, ix, dt = triple
-                ip = ip.to(dtype=torch.int64).contiguous()
-                ix = ix.to(dtype=torch.int32).contiguous()
-                dt = dt.to(dtype=torch.float32).contiguous()
-                for t in (ip, ix, dt):
-                    if not t.is_cuda or t.device.index != self._device:
-                        raise ValueError(f"device CSR arrays must live on cuda:{self._device}")
-                if ix.numel() != dt.numel() or ip.numel() < 1:
-                    raise ValueError("malformed device CSR")
-                keep.append((ip, ix, dt))
-                ptrs.append(tuple(ctypes.c_void_p(t.data_ptr()) for t in (ip, ix, dt)))
-                rows.append(ip.numel() - 1)
+        if on_device:  # the library copies them (device to device)
+            keep = [_device_csr(X_user_rows, self._device), _device_csr(Xt_item_rows, self._device)]
+            ua, ia = (tuple(ctypes.c_void_p(t.data_ptr()) for t in triple) for triple in keep)
             torch.cuda.current_stream(self._device).synchronize()  # the copies below are synchronous
-            ua, ia = ptrs
-            n_u_rows, n_i_rows = rows
+            n_u_rows, n_i_rows = (triple[0].numel() - 1 for triple in keep)
             self.nnz_local = int(keep[0][1].numel())
         else:
             Xu = core._canonical_csr(X_user_rows)
@@ -349,8 +314,7 @@ class ShardedIALSTrainer:
     def _set_features(self, model_config: Any, features: Tuple[Any, Any]) -> None:
         lams = (model_config.lambda_user_feature, model_config.lambda_item_feature)
         empty = [0, 0]
-        err: Optional[BaseException] = None
-        try:
+        with _agreement(self._device, empty):  # a shard of the wrong size may be one rank's
             for side, F in enumerate(features):
                 rows, cols, dense, ip, ix, dt = self._core._feature_arrays(F)
                 flag = ctypes.c_int(0)
@@ -359,28 +323,7 @@ class ShardedIALSTrainer:
                     self._handle, side, rows, cols, p(dense), p(ip), p(ix), p(dt), ctypes.c_float(lams[side]),
                     int(model_config.feature_warmup_epochs), ctypes.byref(flag)))
                 empty[side] = flag.value
-        except (RuntimeError, ValueError, TypeError) as e:  # a shard of the wrong size may be one rank's
-            err = e
-        failed, *self._empty_row = self._max_over_ranks([1 if err is not None else 0] + empty)
-        self._raise_agreed(err, failed)
-
-    def _max_over_ranks(self, values: List[int]) -> List[int]:
-        import torch.distributed as dist
-
-        if self.world == 1:
-            return list(values)
-        dev = f"cuda:{self._device}" if dist.get_backend() == "nccl" else "cpu"
-        t = self._torch.tensor(values, dtype=self._torch.int64, device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return [int(v) for v in t.tolist()]
-
-    @staticmethod
-    def _raise_agreed(err: Optional[BaseException], failed: int) -> None:
-        """Raise this rank's exception, or report a peer's failure, on every rank alike."""
-        if err is not None:
-            raise err
-        if failed:
-            raise RuntimeError("a peer rank failed (see that rank's exception)")
+        self._empty_row = tuple(empty)
 
     @classmethod
     def from_global(cls, model_config: Any, X: sps.csr_matrix, rank: Optional[int] = None,
@@ -434,8 +377,7 @@ class ShardedIALSTrainer:
         """Zero-copy flat torch view of a trainer-owned float buffer (cached per buffer)."""
         key = (int(ptr.value), int(count.value))
         if key not in self._buffer_views:
-            arr = self._core._DeviceArray(key[0], (key[1],), (4,))
-            self._buffer_views[key] = self._torch.as_tensor(arr, device=f"cuda:{self._device}")
+            self._buffer_views[key] = self._core._device_view(key[0], (key[1],), (4,), self._device)
         return self._buffer_views[key]
 
     def _gram_partial(self, factor_side: int) -> Any:
@@ -454,7 +396,7 @@ class ShardedIALSTrainer:
             ctypes.byref(bufs[1][1])))
         for ptr, cnt in bufs:
             if cnt.value:
-                self._all_reduce(self._buffer_view(ptr, cnt))
+                _all_reduce(self._buffer_view(ptr, cnt), self._device)
         self._check(self._lib.ials_trainer_feature_refit(self._handle, side))
 
     def _check_step(self, sc: Any) -> None:
@@ -462,55 +404,41 @@ class ShardedIALSTrainer:
         changes; decided from state every rank shares, so every rank raises alike."""
         self._check(self._lib.ials_trainer_check_shard_step(self._handle, ctypes.byref(sc), *self._empty_row))
 
-    def _all_reduce_max(self, host: Any) -> None:
-        """Element-wise MAX over ranks of a host tensor, in place."""
-        import torch.distributed as dist
-
-        if self.world == 1:
-            return
-        if dist.get_backend() == "nccl":
-            dev = host.to(f"cuda:{self._device}")
-            dist.all_reduce(dev, op=dist.ReduceOp.MAX)
-            host.copy_(dev.cpu())
-        else:
-            dist.all_reduce(host, op=dist.ReduceOp.MAX)
-
-    def _all_reduce(self, view: Any) -> None:
-        import torch.distributed as dist
-
-        if self.world == 1:
-            return
-        if dist.get_backend() == "nccl":
-            dist.all_reduce(view)
-        else:  # gloo control plane (several ranks on one GPU in the tests): stage through the host
-            h = view.cpu()
-            dist.all_reduce(h)
-            view.copy_(h)
-
-    def step_async(self, solver_config: Any, events: Optional[list] = None) -> None:
-        """One epoch (IALSTrainer::step, IALSTrainer.hpp:758-789) across all ranks.  With
-        ``events`` (a list) seven CUDA events are appended: start, then after the partial Gram,
-        the Gram all-reduce and the row solve (with the feature-weight refit) of each side
-        (``phase_ms`` turns them into ms)."""
+    def half_step(self, side: int, solver_config: Any, after: Optional[Callable[[str], None]] = None) -> None:
+        """Half an epoch (``side`` 0: users, 1: items) across all ranks, asynchronous: the partial Gram
+        of this rank's rows of the other side, its all-reduce, the solve of this rank's rows of ``side``
+        (stored into every replica) and the feature-weight refit.  ``after(stage)`` runs on the host
+        after each of them: "gram", "all_reduce", "solve", "refit".  A feature-aware half-step the
+        trainer cannot run is rejected on every rank before its first collective."""
         sc = self._core.IALSTrainer._solver(solver_config)
         self._check_step(sc)
         self._use_current_stream()
+        after = after or (lambda stage: None)
+        view = self._gram_partial(1 - side)
+        after("gram")
+        _all_reduce(view, self._device)
+        after("all_reduce")
+        self._check(self._lib.ials_trainer_solve_shard(self._handle, side, ctypes.byref(sc)))
+        after("solve")
+        self._refit(side)
+        after("refit")
 
-        def mark() -> None:
-            if events is not None:
+    def step_async(self, solver_config: Any, events: Optional[list] = None) -> None:
+        """One epoch (IALSTrainer::step, IALSTrainer.hpp:758-789) across all ranks: the user, then
+        the item ``half_step``.  With ``events`` (a list) seven CUDA events are appended: start, then
+        after the partial Gram, the Gram all-reduce and the row solve (with the feature-weight refit)
+        of each side (``phase_ms`` turns them into ms)."""
+        self._check_step(self._core.IALSTrainer._solver(solver_config))  # a rejected epoch records no event
+
+        def mark(stage: str) -> None:
+            if events is not None and stage != "solve":
                 e = self._torch.cuda.Event(enable_timing=True)
                 e.record(self._torch.cuda.current_stream(self._device))
                 events.append(e)
 
-        mark()
+        mark("start")
         for side in (0, 1):
-            view = self._gram_partial(1 - side)
-            mark()
-            self._all_reduce(view)
-            mark()
-            self._check(self._lib.ials_trainer_solve_shard(self._handle, side, ctypes.byref(sc)))
-            self._refit(side)
-            mark()
+            self.half_step(side, solver_config, mark)
 
     PHASES = ("gram_item_partial", "gram_item_allreduce", "solve_users",
               "gram_user_partial", "gram_user_allreduce", "solve_items")
@@ -531,24 +459,12 @@ class ShardedIALSTrainer:
         stores into the local replicas complete (barrier)."""
         import torch.distributed as dist
 
-        if self.world == 1:
-            self._check(self._lib.ials_trainer_sync(self._handle))
-            return
         # a solver failure on ONE rank (singular CG system, failed Cholesky) must not leave the
         # others blocked in the barrier: agree on the status first, then raise everywhere
-        err: Optional[BaseException] = None
-        try:
+        with _agreement(self._device):
             self._check(self._lib.ials_trainer_sync(self._handle))
-        except (RuntimeError, ValueError) as e:  # the exception types `check` maps status codes to
-            err = e
-        flag = self._torch.tensor([1 if err is not None else 0], dtype=self._torch.int32,
-                                  device=f"cuda:{self._device}" if dist.get_backend() == "nccl" else "cpu")
-        dist.all_reduce(flag, op=dist.ReduceOp.MAX)
-        dist.barrier()
-        if err is not None:
-            raise err
-        if int(flag.item()):
-            raise RuntimeError("a peer rank's row solver failed (see that rank's exception)")
+        if self.world > 1:
+            dist.barrier()
 
     def step(self, solver_config: Any) -> None:
         self.step_async(solver_config)
@@ -559,19 +475,12 @@ class ShardedIALSTrainer:
         on every rank: every rank sums the terms of its own rows, rank 0 adds the Gram and the
         feature-weight terms, and the float64 partials are all-reduced.  Call it after ``step`` /
         ``sync`` (it reads the full replicas)."""
-        import torch.distributed as dist
-
         sc = self._core.IALSTrainer._solver(solver_config)
         self._use_current_stream()
         out = ctypes.c_double(0.0)
         self._check(self._lib.ials_trainer_compute_loss_shard(self._handle, ctypes.byref(sc),
                                                               int(self.rank == 0), ctypes.byref(out)))
-        total = out.value
-        if self.world > 1:
-            dev = f"cuda:{self._device}" if dist.get_backend() == "nccl" else "cpu"
-            t = self._torch.tensor([total], dtype=self._torch.float64, device=dev)
-            dist.all_reduce(t)
-            total = float(t.item())
+        total = _all_reduce(self._torch.tensor([out.value], dtype=self._torch.float64), self._device).item()
         return float(np.float32(total))  # the reference returns a float (IALSTrainer.hpp:836)
 
     def _get_feature_weight(self, side: int) -> np.ndarray:
@@ -602,10 +511,8 @@ class ShardedIALSTrainer:
     item_feature_weight = property(lambda s: s._get_feature_weight(1), lambda s, v: s._set_feature_weight(1, v))
 
     def _get(self, side: int) -> np.ndarray:
-        n = self.n_users if side == 0 else self.n_items
-        out = np.empty((n, self.K), dtype=np.float32)
-        self._use_current_stream()
-        self._check(self._lib.ials_trainer_get_factors(self._handle, side, self._core._ptr(out)))
+        out = np.empty((self.n_users if side == 0 else self.n_items, self.K), dtype=np.float32)
+        self.get_factors_into(side, out)
         return out
 
     def _set(self, side: int, value: np.ndarray) -> None:
@@ -620,6 +527,10 @@ class ShardedIALSTrainer:
     item = property(lambda s: s._get(1), lambda s, v: s._set(1, v))
 
     def get_factors_into(self, side: int, out: np.ndarray) -> None:
+        """Device -> host copy of this rank's replica into a caller-owned (e.g. pinned) C-contiguous buffer."""
+        n = self.n_users if side == 0 else self.n_items
+        if out.dtype != np.float32 or out.shape != (n, self.K) or not out.flags.c_contiguous:
+            raise ValueError("output buffer must be C-contiguous float32 of the factor shape")
         self._use_current_stream()
         self._check(self._lib.ials_trainer_get_factors(self._handle, side, self._core._ptr(out)))
 
@@ -648,13 +559,9 @@ class ShardedIALSTrainer:
         self._check(self._lib.ials_trainer_get_factor_rows(self._handle, side, b, e - b,
                                                            self._core._ptr(out)))
 
-    def _factors_view(self, side: int) -> Any:
-        """Zero-copy torch view ([n, ld]) of this rank's replica of a factor matrix."""
-        p, n, K, ld = ctypes.c_void_p(0), ctypes.c_int64(0), ctypes.c_int64(0), ctypes.c_int64(0)
-        self._check(self._lib.ials_trainer_factors_device(self._handle, side, ctypes.byref(p), ctypes.byref(n),
-                                                          ctypes.byref(K), ctypes.byref(ld)))
-        arr = self._core._DeviceArray(int(p.value), (int(n.value), int(ld.value)), (int(ld.value) * 4, 4))
-        return self._torch.as_tensor(arr, device=f"cuda:{self._device}")
+    def factors_device(self, side: int) -> Any:
+        """Zero-copy ``torch`` view ([n, K], row stride ld) of this rank's replica of a factor matrix."""
+        return self._core._factors_device(self._handle, side, self._device)
 
     def step_io(self, solver_config: Any, user_rows: Any, item_rows: Any) -> None:
         """One epoch on HOST-resident shards, in place (the row-sharded twin of
@@ -663,11 +570,11 @@ class ShardedIALSTrainer:
         fresh rows come back -- the user rows on a second stream while the item half-epoch runs.
         ``user_rows`` / ``item_rows``: pinned float32 torch tensors of shape (shard rows, K)."""
         torch = self._torch
-        sc = self._core.IALSTrainer._solver(solver_config)
-        self._check_step(sc)  # before the uploads: a rejected call leaves the factors as they were
+        # before the uploads: a rejected call leaves the factors as they were
+        self._check_step(self._core.IALSTrainer._solver(solver_config))
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = torch.cuda.Stream(device=self._device)
-            self._views = [self._factors_view(0), self._factors_view(1)]
+            self._views = [self.factors_device(0), self.factors_device(1)]
         self.set_shard_rows(1, item_rows.numpy())  # item first: the user half-epoch starts with Gram(item)
         # the user rows are only the warm starts of this rank's solves: the peers' copies of them are
         # first read in the item half-epoch, after the solve kernels have stored the new values there;
@@ -679,19 +586,19 @@ class ShardedIALSTrainer:
         self._use_current_stream()
         self._check(self._lib.ials_trainer_set_user_rows_flagged(self._handle, ub, ue - ub, self._core._ptr(un)))
         main = torch.cuda.current_stream(self._device)
-        for side in (0, 1):
-            self._all_reduce(self._gram_partial(1 - side))
-            self._check(self._lib.ials_trainer_solve_shard(self._handle, side, ctypes.byref(sc)))
-            if side == 0:  # the rank's new user rows are final: they travel back during the item half
+
+        def copy_user_rows_back(stage: str) -> None:
+            if stage == "solve":  # the rank's new user rows are final: they travel back during the item half
                 done = torch.cuda.Event()
                 done.record(main)
-                b, e = self.user_range
                 with torch.cuda.stream(self._copy_stream):
                     self._copy_stream.wait_event(done)
-                    user_rows.copy_(self._views[0][b:e, : self.K], non_blocking=True)
-            self._refit(side)
+                    user_rows.copy_(self._views[0][ub:ue], non_blocking=True)
+
+        self.half_step(0, solver_config, copy_user_rows_back)
+        self.half_step(1, solver_config)
         b, e = self.item_range
-        item_rows.copy_(self._views[1][b:e, : self.K], non_blocking=True)
+        item_rows.copy_(self._views[1][b:e], non_blocking=True)
         self._copy_stream.synchronize()
         self.sync()
 
@@ -807,15 +714,11 @@ class ShardedEvaluator:
         self._lists = recommendable_items is not None or per_user_recommendable_items is not None
         self.last_timings: dict = {}
         ub, ue = trainer.user_range
-        err: Optional[BaseException] = None
-        try:
+        with _agreement(trainer._device):
             gt = ground_truth
             if isinstance(gt, (tuple, list)):  # device CSR: rows sorted here, on the device
-                ip = gt[0].to(torch.int64)
-                ix = gt[1].to(torch.int64)
+                ip, ix, _ = _device_csr(gt, trainer._device)
                 n_rows = ip.numel() - 1
-                if ip.device != torch.device(f"cuda:{trainer._device}") or ix.device != ip.device:
-                    raise ValueError(f"device CSR arrays must live on cuda:{trainer._device}")
                 rows = torch.repeat_interleave(torch.arange(n_rows, device=ip.device), ip[1:] - ip[:-1])
                 keys = torch.sort(rows * trainer.n_items + ix).values
                 self._gt_device = ((ip - ip[0]).contiguous(),
@@ -830,15 +733,11 @@ class ShardedEvaluator:
                                  recommendable_items=recommendable_items,
                                  per_user_recommendable_items=per_user_recommendable_items,
                                  masked_interactions=masked_interactions, recall_with_cutoff=recall_with_cutoff)
-        except (ValueError, TypeError, KeyError, RuntimeError) as e:
-            err = e
-        failed, = trainer._max_over_ranks([1 if err is not None else 0])
-        trainer._raise_agreed(err, failed)
         if recommendable_items is None and per_user_recommendable_items is not None:
             # the union of every rank's lists: one OR of the catalogue bitmaps
             seen = torch.zeros(trainer.n_items, dtype=torch.int32)
             seen[torch.from_numpy(self._ev._allow_sorted_flat.astype(np.int64))] = 1
-            trainer._all_reduce_max(seen)
+            _all_reduce(seen, trainer._device, "max")
             self._ev.n_recommendable_items = int(seen.sum())
 
     @classmethod
@@ -919,13 +818,9 @@ class ShardedEvaluator:
         n_cut, n_items = ctypes.c_int64(0), ctypes.c_int64(0)
         check(lib.ials_eval_set_buffers(h, *(ctypes.byref(x) for x in ptrs), ctypes.byref(n_cut),
                                         ctypes.byref(n_items)))
-        dev = f"cuda:{self._trainer._device}"
-        out = []
-        for ptr, n, typ in zip(ptrs, (5 * n_cut.value, 2 * n_cut.value, n_cut.value * n_items.value),
-                               ("<f8", "<i8", "<i8")):
-            out.append(self._trainer._torch.as_tensor(core._DeviceArray(int(ptr.value), (n,), (8,), typ),
-                                                      device=dev))
-        return out[0], out[1], out[2]
+        sizes = (5 * n_cut.value, 2 * n_cut.value, n_cut.value * n_items.value)
+        return tuple(core._device_view(int(ptr.value), (n,), (8,), self._trainer._device, typ)
+                     for ptr, n, typ in zip(ptrs, sizes, ("<f8", "<i8", "<i8")))
 
     def _get_scores_as_list(self, trainer: "ShardedIALSTrainer", cutoffs: List[int]) -> List[dict]:
         from .evaluation import Metrics
@@ -937,10 +832,8 @@ class ShardedEvaluator:
         if self._lists and max(cutoffs) > 128:
             raise NotImplementedError("allow-lists need the fused tensor-core kernel (cutoff <= 128)")
         torch = trainer._torch
-        timings = {}
-        err: Optional[BaseException] = None
         t0 = time.perf_counter()
-        try:
+        with _agreement(trainer._device):
             if trainer is not self._trainer:
                 raise ValueError("the ShardedEvaluator was built for another trainer")
             h = self._set_for(trainer, tuple(cutoffs))
@@ -949,14 +842,10 @@ class ShardedEvaluator:
             trainer._use_current_stream()
             ub, ue = trainer.user_range
             check(lib.ials_trainer_evaluate(trainer._handle, h, ub, ue))
-        except (ValueError, RuntimeError, NotImplementedError) as e:
-            err = e
-        failed, = trainer._max_over_ranks([1 if err is not None else 0])
-        trainer._raise_agreed(err, failed)
         t1 = time.perf_counter()
         sums, counts, hist = self._views(h)
         for view in (sums, counts, hist):
-            trainer._all_reduce(view)
+            _all_reduce(view, trainer._device)
         torch.cuda.current_stream(trainer._device).synchronize()
         t2 = time.perf_counter()
         div = np.empty((len(cutoffs), 3), dtype=np.float64)
@@ -1020,18 +909,10 @@ def run_c4(hyper: dict, steps: int, warmup: int, scale: float = 1.0, e2e_steps: 
             dist.barrier()
 
     def max_over_ranks(x: float) -> float:
-        if not multi:
-            return x
-        t = torch.tensor([x], device=dev, dtype=torch.float64)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item())
+        return float(_all_reduce(torch.tensor([x], dtype=torch.float64), dev, "max").item())
 
     def sum_over_ranks(x: int) -> int:
-        if not multi:
-            return x
-        t = torch.tensor([x], device=dev, dtype=torch.int64)
-        dist.all_reduce(t)
-        return int(t.item())
+        return int(_all_reduce(torch.tensor([x], dtype=torch.int64), dev).item())
 
     # user blocks of equal row count and equal nnz (the generator draws exactly nnz/world pairs
     # per block): nnz-balanced by construction; items are cut by their global degrees
@@ -1040,8 +921,8 @@ def run_c4(hyper: dict, steps: int, warmup: int, scale: float = 1.0, e2e_steps: 
     n_rows, n_nnz = int(ub[rank + 1] - ub[rank]), int(nb[rank + 1] - nb[rank])
     t0 = time.perf_counter()
     ip, ix, dt = synth_user_block_device(n_rows, I, n_nnz, seed=1004 + rank, device=dev, item_seed=1004)
-    item_bounds = global_item_bounds_device(ix, I)
-    t_ip, t_ix, t_dt = exchange_transposed_shards_device(ip, ix, dt, int(ub[rank]), U, item_bounds)
+    item_bounds = global_item_bounds(ix, I)
+    t_ip, t_ix, t_dt = exchange_transposed_shards(ip, ix, dt, int(ub[rank]), U, item_bounds)
     torch.cuda.synchronize()
     t_build = time.perf_counter() - t0
     cfg = (core.IALSModelConfigBuilder().set_K(K).set_alpha0(hyper["alpha0"]).set_reg(hyper["reg"])
@@ -1154,24 +1035,20 @@ def run_c4(hyper: dict, steps: int, warmup: int, scale: float = 1.0, e2e_steps: 
     # imports it).  Collective: every rank passes the same ``parity_check is not None``. ----
     parity = None
     if parity_check is not None and parity_sample > 0:
-        import ctypes as _ct
-
         b0 = int(ub[rank])
-        views = [tr._factors_view(0), tr._factors_view(1)]
+        views = [tr.factors_device(0), tr.factors_device(1)]
         before = items_host = gidx = None
         if parity_rows is not None:
             gidx = torch.tensor([b0 + r for r in parity_rows[0]], device=dev)
-            before = views[0][gidx, :K].cpu().numpy()
-            items_host = views[1][:, :K].cpu().numpy()
-        tr._use_current_stream()
-        tr._all_reduce(tr._gram_partial(1))
-        tr._check(tr._lib.ials_trainer_solve_shard(tr._handle, 0, _ct.byref(core.IALSTrainer._solver(sc))))
+            before = views[0][gidx].cpu().numpy()
+            items_host = views[1].cpu().numpy()
+        tr.half_step(0, sc)
         tr.sync()
         if parity_rows is not None:
-            after = views[0][gidx, :K].cpu().numpy()
+            after = views[0][gidx].cpu().numpy()
             parity = parity_check(before=before, after=after, other=items_host, rows=parity_rows[1], solver=solver,
                                   hyper=hyper)
-    stats = [tr.plan_stats(0), tr.plan_stats(1)] if hasattr(tr, "plan_stats") else None
+    stats = [tr.plan_stats(0), tr.plan_stats(1)]
     del tr
     torch.cuda.empty_cache()
     if rank != 0:

@@ -1,35 +1,26 @@
 """Row-sharded multi-GPU path (irspack_b200/dist.py).
 
-CPU (``-m "not gpu"``): the host logic -- nnz-balanced partitioning and the
-collective that builds every rank's rows of X^T -- on world_size-2 ``gloo``.
+CPU (``-m "not gpu"``): the host logic -- nnz-balanced partitioning, the
+collective that builds every rank's rows of X^T and the agreement of ranks on a
+failure -- on world_size-2 and -3 ``gloo``.
 GPU (``-m gpu``): two ranks on ONE device (gloo control plane, CUDA-IPC peer
 replicas exactly as on two devices) must reproduce the single-process trainer.
+The workers run under a bounded join: a rank left blocked in a collective fails the test.
 """
 import os
-import socket
 import sys
 
 import numpy as np
 import pytest
 import scipy.sparse as sps
 
+from test_dist_features import _n_devices, _spawn
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _free_port() -> int:
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
-
-
-def _spawn(fn, world, *args):
-    import torch.multiprocessing as mp
-
-    port = _free_port()
-    mp.spawn(fn, args=(world, port) + args, nprocs=world, join=True)
-
-
 def _init(rank, world, port):
+    """gloo without selecting a CUDA device: the CPU workers must run on a machine without one."""
     import torch.distributed as dist
 
     if ROOT not in sys.path:
@@ -74,52 +65,6 @@ def test_balanced_bounds():
     assert np.all(np.abs(np.diff(big) - 125) <= 1)
 
 
-def test_transposed_pieces_roundtrip_single_process():
-    d = _dist_module()
-    X = _matrix()
-    U, I = X.shape
-    world = 3
-    ub = d.balanced_bounds(np.diff(X.indptr) + 1, world)
-    ib = d.balanced_bounds(np.bincount(X.indices, minlength=I) + 1, world)
-    pieces = [d.transposed_pieces(X[ub[r]:ub[r + 1]], int(ub[r]), ib) for r in range(world)]
-    Xt = sps.csr_matrix(X.T)
-    Xt.sort_indices()
-    for dst in range(world):
-        got = d.assemble_transposed_shard([pieces[src][dst] for src in range(world)], U)
-        want = Xt[ib[dst]:ib[dst + 1]]
-        assert (got != want).nnz == 0
-        assert np.array_equal(got.indptr, want.indptr) and np.array_equal(got.indices, want.indices)
-
-
-def _worker_exchange(rank, world, port):
-    _init(rank, world, port)
-    import torch.distributed as dist
-
-    d = _dist_module()
-    X = _matrix()
-    U, I = X.shape
-    ub = d.balanced_bounds(np.diff(X.indptr) + 1, world)
-    mine = X[ub[rank]:ub[rank + 1]]
-    ib = d.global_item_bounds(mine)
-    want_ib = d.balanced_bounds(np.bincount(X.indices, minlength=I) + 1, world)
-    assert np.array_equal(ib, want_ib)
-    got = d.exchange_transposed_shards(mine, int(ub[rank]), U, ib)
-    want = sps.csr_matrix(X.T)[ib[rank]:ib[rank + 1]]
-    want.sort_indices()
-    assert got.shape == want.shape and (got != want).nnz == 0
-    assert np.array_equal(got.indices, want.indices)
-    dist.barrier()
-    dist.destroy_process_group()
-
-
-def test_exchange_transposed_shards_gloo_world2():
-    _spawn(_worker_exchange, 2)
-
-
-def test_exchange_transposed_shards_gloo_world3():
-    _spawn(_worker_exchange, 3)
-
-
 def _csr_to_torch(X):
     import torch
 
@@ -127,8 +72,8 @@ def _csr_to_torch(X):
             torch.from_numpy(X.data.astype(np.float32)))
 
 
-def _worker_exchange_device(rank, world, port):
-    """The torch (device-resident) twin of the scipy collective, run on CPU tensors."""
+def _worker_exchange(rank, world, port):
+    """The collective on CPU tensors: every rank's rows of X^T equal scipy's."""
     _init(rank, world, port)
     import torch.distributed as dist
 
@@ -138,9 +83,9 @@ def _worker_exchange_device(rank, world, port):
     ub = d.balanced_bounds(np.diff(X.indptr) + 1, world)
     mine = X[ub[rank]:ub[rank + 1]]
     ip, ix, dt = _csr_to_torch(mine)
-    ib = d.global_item_bounds_device(ix, I)
+    ib = d.global_item_bounds(ix, I)
     assert np.array_equal(ib, d.balanced_bounds(np.bincount(X.indices, minlength=I) + 1, world))
-    t_ip, t_ix, t_dt = d.exchange_transposed_shards_device(ip, ix, dt, int(ub[rank]), U, ib)
+    t_ip, t_ix, t_dt = d.exchange_transposed_shards(ip, ix, dt, int(ub[rank]), U, ib)
     want = sps.csr_matrix(X.T)[ib[rank]:ib[rank + 1]]
     want.sort_indices()
     assert np.array_equal(t_ip.numpy(), want.indptr)
@@ -150,23 +95,54 @@ def _worker_exchange_device(rank, world, port):
     dist.destroy_process_group()
 
 
-def test_exchange_transposed_shards_device_gloo_world2():
-    _spawn(_worker_exchange_device, 2)
+def test_exchange_transposed_shards_torch_gloo_world2():
+    _spawn(_worker_exchange, 2)
 
 
-def test_exchange_transposed_shards_device_gloo_world3():
-    _spawn(_worker_exchange_device, 3)
+def test_exchange_transposed_shards_torch_gloo_world3():
+    _spawn(_worker_exchange, 3)
 
 
-def test_exchange_transposed_shards_device_single_process():
+def test_exchange_transposed_shards_torch_single_process():
     d = _dist_module()
     X = _matrix(seed=8, U=120, I=90, nnz=2500)
     ip, ix, dt = _csr_to_torch(X)
-    t_ip, t_ix, t_dt = d.exchange_transposed_shards_device(ip, ix, dt, 0, X.shape[0], [0, X.shape[1]])
+    t_ip, t_ix, t_dt = d.exchange_transposed_shards(ip, ix, dt, 0, X.shape[0], [0, X.shape[1]])
     want = sps.csr_matrix(X.T)
     want.sort_indices()
     assert np.array_equal(t_ip.numpy(), want.indptr) and np.array_equal(t_ix.numpy(), want.indices)
     assert np.array_equal(t_dt.numpy(), want.data)
+
+
+def _worker_agreement(rank, world, port):
+    _init(rank, world, port)
+    import torch.distributed as dist
+
+    d = _dist_module()
+    # one rank raises: it gets its own exception, every other rank a RuntimeError naming a peer
+    for i, kind in enumerate((ValueError, TypeError, KeyError, RuntimeError, NotImplementedError)):
+        culprit = i % world
+        mine = kind(f"rank {rank} failed")
+        with pytest.raises(Exception) as got:
+            with d._agreement(None):
+                if rank == culprit:
+                    raise mine
+        if rank == culprit:
+            assert got.value is mine
+        else:
+            assert type(got.value) is RuntimeError and "peer rank failed" in str(got.value)
+    # no rank raises: the piggybacked integers come back as their maximum over the ranks
+    values = [rank, 10 * (world - 1 - rank), -rank]
+    with d._agreement(None, values):
+        pass
+    assert values == [world - 1, 10 * (world - 1), 0]
+    dist.barrier()
+    dist.destroy_process_group()
+
+
+@pytest.mark.parametrize("world", [2, 3])
+def test_agreement_raises_on_every_rank_gloo(world):
+    _spawn(_worker_agreement, world)
 
 
 def test_synth_user_block_device_is_a_well_formed_power_law_block():
@@ -243,6 +219,24 @@ def test_two_ranks_one_device_match_single_process(tmp_path, solver):
     # epochs of unconverged CG amplify that rounding (TOL_STEP of test_gpu_parity.py is 2e-4)
     for a, b in ((r["user"], r["ref_user"]), (r["item"], r["ref_item"])):
         assert np.abs(a - b).max() <= 1e-4 * np.abs(b).max()
+
+
+@pytest.mark.gpu
+def test_get_factors_into_rejects_a_buffer_of_the_wrong_layout():
+    from irspack_b200 import _ials_core as core
+    from irspack_b200.dist import ShardedIALSTrainer
+
+    K = 32
+    X = _matrix()
+    tr = ShardedIALSTrainer.from_global(core.IALSModelConfigBuilder().set_K(K).build(), X, rank=0, world=1)
+    for side, n in ((0, X.shape[0]), (1, X.shape[1])):
+        for bad in (np.empty((n - 1, K), np.float32), np.empty((n, K + 1), np.float32),
+                    np.empty((n, K), np.float64), np.empty((K, n), np.float32).T):
+            with pytest.raises(ValueError):
+                tr.get_factors_into(side, bad)
+        out = np.empty((n, K), np.float32)
+        tr.get_factors_into(side, out)
+        assert np.array_equal(out, tr.user if side == 0 else tr.item)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -323,15 +317,6 @@ def _worker_multi_device(rank, world, port, out_path):
     dist.barrier()
     del tr
     dist.destroy_process_group()
-
-
-def _n_devices() -> int:
-    try:
-        import torch
-
-        return torch.cuda.device_count()
-    except Exception:
-        return 0
 
 
 @pytest.mark.gpu

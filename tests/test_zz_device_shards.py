@@ -12,8 +12,8 @@ def test_sharded_trainer_from_device_csr_matches_host_csr():
     import torch
 
     from irspack_b200 import _ials_core as core
-    from irspack_b200.dist import (ShardedIALSTrainer, exchange_transposed_shards_device,
-                                   global_item_bounds_device, synth_user_block_device)
+    from irspack_b200.dist import (ShardedIALSTrainer, exchange_transposed_shards,
+                                   global_item_bounds, synth_user_block_device)
     from irspack_b200.synth import init_factors
 
     dev = torch.device("cuda:0")
@@ -21,9 +21,9 @@ def test_sharded_trainer_from_device_csr_matches_host_csr():
     U, I, nnz, K = 3000, 900, 60000, 128
     ip, ix, dt = synth_user_block_device(U, I, nnz, seed=3, device=dev, item_seed=1)
     assert ip.is_cuda and int(ip[-1]) == nnz
-    bounds = global_item_bounds_device(ix, I)
+    bounds = global_item_bounds(ix, I)
     assert list(bounds) == [0, I]
-    t_ip, t_ix, t_dt = exchange_transposed_shards_device(ip, ix, dt, 0, U, bounds)
+    t_ip, t_ix, t_dt = exchange_transposed_shards(ip, ix, dt, 0, U, bounds)
     X = sps.csr_matrix((dt.cpu().numpy(), ix.cpu().numpy(), ip.cpu().numpy()), shape=(U, I))
     Xt = sps.csr_matrix(X.T)
     Xt.sort_indices()

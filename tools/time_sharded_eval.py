@@ -68,8 +68,8 @@ def main() -> None:
 
     from bench import HYPER
     from irspack_b200 import _ials_core as core
-    from irspack_b200.dist import (ShardedEvaluator, ShardedIALSTrainer, c4_shape, exchange_transposed_shards_device,
-                                   global_item_bounds_device, synth_user_block_device)
+    from irspack_b200.dist import (ShardedEvaluator, ShardedIALSTrainer, c4_shape, exchange_transposed_shards,
+                                   global_item_bounds, synth_user_block_device)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -101,8 +101,8 @@ def main() -> None:
     nb = np.linspace(0, nnz, world + 1).astype(np.int64)
     n_rows, n_nnz = int(ub[rank + 1] - ub[rank]), int(nb[rank + 1] - nb[rank])
     ip, ix, dt = synth_user_block_device(n_rows, I, n_nnz, seed=1004 + rank, device=dev, item_seed=1004)
-    bounds = global_item_bounds_device(ix, I)
-    t_csr = exchange_transposed_shards_device(ip, ix, dt, int(ub[rank]), U, bounds)
+    bounds = global_item_bounds(ix, I)
+    t_csr = exchange_transposed_shards(ip, ix, dt, int(ub[rank]), U, bounds)
     cfg = (core.IALSModelConfigBuilder().set_K(K).set_alpha0(HYPER["alpha0"]).set_reg(HYPER["reg"])
            .set_nu(HYPER["nu"]).build())
     tr = ShardedIALSTrainer(cfg, (ip, ix, dt), int(ub[rank]), U, t_csr, int(bounds[rank]), I, init_on_device=True)
