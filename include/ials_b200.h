@@ -330,6 +330,29 @@ IALS_API int ials_eval_set_diversity(ials_eval_set *e, void *cuda_stream, double
  * in chunks, each followed by the metrics kernel, on the trainer's stream; ADDS to the accumulators.
  * The sums are deterministic: the same pass gives the same bits.  Returns when the pass is done. */
 IALS_API int ials_trainer_evaluate(ials_trainer *t, ials_eval_set *e, int64_t user_begin, int64_t user_end);
+/* A cold evaluation set (EvaluatorWithColdUser, evaluation/evaluator.py:470-657): n_rows users that are
+ * not rows of the model.  Their input rows (CSR [n_rows x n_cols], n_cols == n_items, else "Shape mismatch:
+ * ..." as Solver::X_to_vector :126-131) are what the fold-in solves, as given: stored zeros count in nnz and
+ * add bias * y.  The mask (both mask pointers NULL) is the input's non-zeros, as scipy's .nonzero() gives
+ * them (evaluator.py:432); a host CSR of n_rows rows without stored zeros replaces it (masked_interactions,
+ * evaluator.py:574-577).  Ground truth, allow-lists (rows relative to the set), cutoffs and accumulators as
+ * in ials_eval_set_create.  The input and ground-truth arrays are host arrays, or device arrays with
+ * on_device != 0; the input is validated and planned once, in chunks of the pass. */
+IALS_API int ials_eval_set_create_cold(ials_trainer *t, int64_t n_rows, int64_t n_cols, const int64_t *in_indptr,
+                                       const int32_t *in_indices, const float *in_data, const int64_t *gt_indptr,
+                                       const int32_t *gt_indices, int on_device, const int64_t *mask_indptr,
+                                       const int32_t *mask_indices, int64_t allow_n_lists, const int64_t *allow_indptr,
+                                       const int32_t *allow_indices, const int64_t *cutoffs, int64_t n_cutoffs,
+                                       int recall_with_cutoff, ials_eval_set **out);
+/* One pass over the cold set's rows [row_begin, row_end), on the trainer's stream with one synchronisation
+ * at the end: P = alpha0 item^T item of the full item factors once, then per chunk the fold-in of
+ * ials_trainer_transform (side 0, from zero, every solver route of `solver`) into a device slab, the lists
+ * of ials_trainer_evaluate on that slab and the metrics of every cutoff; ADDS to the accumulators.  No
+ * training state changes.  Solver failures raise with the reference's messages (IALSTrainer.hpp:252-253,
+ * 318, 322).  A row-sharded trainer runs it on its own share of the cold users; its item factors are a
+ * full replica, so the pass needs no collective. */
+IALS_API int ials_trainer_evaluate_cold(ials_trainer *t, ials_eval_set *e, const ials_solver_config *solver,
+                                        int64_t row_begin, int64_t row_end);
 
 /* retrieve_recommend_from_score<float>                 cpp_source/util.hpp:426-504
  * (bound as irspack.utils._util_cpp.retrieve_recommend_from_score_f32,

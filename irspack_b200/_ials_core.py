@@ -267,6 +267,20 @@ def _device_view(ptr: int, shape: Tuple[int, ...], strides: Tuple[int, ...], dev
     return torch.as_tensor(carrier, device=f"cuda:{device}")
 
 
+def _transform(handle: ctypes.c_void_p, K: int, device: int, side: int, interaction: Any,
+               sc: SolverConfigStruct) -> np.ndarray:
+    """``ials_trainer_transform`` of a trainer (or a row-sharded trainer's replicas) on its device's
+    current stream: the fold-in of a host CSR, returned as host rows [n_new, K]."""
+    X = _canonical_csr(interaction)
+    indptr, indices, data = _csr_arrays(X)
+    n_new = X.shape[0] if side == 0 else X.shape[1]
+    out = np.empty((n_new, K), dtype=np.float32)
+    check(lib.ials_trainer_set_stream(handle, ctypes.c_void_p(_stream_of(device))))
+    check(lib.ials_trainer_transform(handle, side, X.shape[0], X.shape[1], _ptr(indptr), _ptr(indices),
+                                     _ptr(data), ctypes.byref(sc), _ptr(out)))
+    return out
+
+
 def _factors_device(handle: ctypes.c_void_p, side: int, device: int) -> Any:
     """Zero-copy view ([n, K], row stride ld) of a trainer's factor matrix (or replica) of ``side``."""
     import torch
@@ -370,15 +384,7 @@ class IALSTrainer:
         return out
 
     def _transform(self, side: int, interaction: Any, solver_config: IALSSolverConfig) -> np.ndarray:
-        sc = self._solver(solver_config)
-        X = _canonical_csr(interaction)
-        indptr, indices, data = _csr_arrays(X)
-        n_new = X.shape[0] if side == 0 else X.shape[1]
-        out = np.empty((n_new, self.K), dtype=np.float32)
-        self._use_current_stream()
-        check(lib.ials_trainer_transform(self._handle, side, X.shape[0], X.shape[1], _ptr(indptr),
-                                         _ptr(indices), _ptr(data), ctypes.byref(sc), _ptr(out)))
-        return out
+        return _transform(self._handle, self.K, self._device, side, interaction, self._solver(solver_config))
 
     def transform_user(self, interaction: Any, solver_config: IALSSolverConfig) -> np.ndarray:
         return self._transform(0, interaction, solver_config)  # wrapper.cpp:140-141

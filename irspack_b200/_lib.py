@@ -88,6 +88,8 @@ def _load() -> ctypes.CDLL:
         "ials_eval_set_buffers": (c_int, [H, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int64), POINTER(c_int64)]),
         "ials_eval_set_diversity": (c_int, [H, c_void_p, c_void_p]),
         "ials_trainer_evaluate": (c_int, [H, H, c_int64, c_int64]),
+        "ials_eval_set_create_cold": (c_int, [H, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int, POINTER(H)]),
+        "ials_trainer_evaluate_cold": (c_int, [H, H, SC, c_int64, c_int64]),
         "ials_topk_scores": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
         "ials_retrieve_recommend": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
         "ials_weighted_gram": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_float, c_int, c_void_p, c_void_p]),

@@ -271,12 +271,7 @@ void epoch_side(ials_trainer *t, int side, const ials_solver_config *sc, SolveAr
 }
 
 void half_step(ials_trainer *t, int side, const ials_solver_config *sc) {
-  struct NoProfiling {  // phase marks are per epoch (ials_trainer_step*) only
-    ials_trainer *t;
-    bool saved;
-    explicit NoProfiling(ials_trainer *t_) : t(t_), saved(t_->profiling) { t->profiling = false; }
-    ~NoProfiling() { t->profiling = saved; }
-  } guard(t);
+  NoProfiling guard(t);
   if (t->sharded) throw std::runtime_error("sharded trainer: drive the epoch with gram_partial / solve_shard");
   if (!t->has_X) throw std::runtime_error("this trainer was restored without its interaction matrix; it cannot train");
   check_feature_solver(t, sc);

@@ -151,6 +151,14 @@ inline void rows_to_host(float *dst, int64_t K, const float *src, int64_t ld, in
                                cudaMemcpyDeviceToHost, s));
 }
 
+// Phase marks are per epoch (ials_trainer_step*) only: a scope that solves outside an epoch turns them off
+struct NoProfiling {
+  ials_trainer *t;
+  bool saved;
+  explicit NoProfiling(ials_trainer *t_) : t(t_), saved(t_->profiling) { t->profiling = false; }
+  ~NoProfiling() { t->profiling = saved; }
+};
+
 // A trainer under construction: a failed create* releases it through ials_trainer_destroy
 using TrainerPtr = std::unique_ptr<ials_trainer, void (*)(ials_trainer *)>;
 

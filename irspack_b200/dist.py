@@ -617,6 +617,18 @@ class ShardedIALSTrainer:
                                                      p(None), p(None), p(idx), p(None), p(cnt)))
         return idx, cnt
 
+    def transform_user(self, X: Any, solver_config: Any) -> np.ndarray:
+        """Fold-in of new users' rows ``X`` (n x n_items) against this rank's full item replica
+        (``IALSTrainer.transform_user``, IALSTrainer.hpp:791-796): rank-local, no collective."""
+        return self._core._transform(self._handle, self.K, self._device, 0, X,
+                                     self._core.IALSTrainer._solver(solver_config))
+
+    def transform_item(self, X: Any, solver_config: Any) -> np.ndarray:
+        """Fold-in of new items' columns ``X`` (n_users x n) against this rank's full user replica
+        (``IALSTrainer.transform_item``, IALSTrainer.hpp:797-802): rank-local, no collective."""
+        return self._core._transform(self._handle, self.K, self._device, 1, X,
+                                     self._core.IALSTrainer._solver(solver_config))
+
     # -- validation-based early stopping (BaseRecommenderWithEarlyStopping, base_earlystop.py:106-149) --
     def save_state(self, state: Optional[dict] = None) -> dict:
         """This rank's own rows of both factor matrices (into pinned host buffers: ``state`` from an
@@ -642,8 +654,8 @@ class ShardedIALSTrainer:
     def learn_with_optimizer(self, solver_config: Any, evaluator: Any = None, max_epoch: int = 128,
                              validate_epoch: int = 5, score_degradation_max: int = 5) -> int:
         """Collective epoch loop with validation-based early stopping (``IALSRecommender.
-        learn_with_optimizer``, base_earlystop.py:106-149).  ``evaluator``: a ``ShardedEvaluator`` of
-        this trainer; its score is the same on every rank, so is every decision.  Returns the number
+        learn_with_optimizer``, base_earlystop.py:106-149).  ``evaluator``: a ``ShardedEvaluator`` or
+        ``ShardedEvaluatorWithColdUser`` of this trainer; its score is the same on every rank, so is every decision.  Returns the number
         of epochs of the model left in the trainer: the best validated one (``max_epoch`` without an
         evaluator)."""
         best_score = -float("inf")
@@ -683,77 +695,30 @@ class ShardedIALSTrainer:
         return dict(zip(keys, (int(v) for v in out)))
 
 
-class ShardedEvaluator:
-    """The ``Evaluator`` of a row-sharded model, one per rank.
+class _ShardedEvaluation:
+    """What ``ShardedEvaluator`` and ``ShardedEvaluatorWithColdUser`` share: the evaluation sets (one per
+    tuple of cutoffs, built by the subclass's ``_create_set``), the pass (the subclass's ``_run``), the
+    all-reduce of the sums, counts and item histograms over the ranks, the diversity reduction of the
+    merged histograms on the device, and the dict of the wrapped single-process evaluator ``_ev``, whose
+    ``catalog_coverage`` divides by the recommendable items of ALL ranks' lists."""
 
-    ``ground_truth`` holds THIS rank's user rows only (``trainer.user_range``), shape
-    ``(user_end - user_begin, n_items)``: a scipy matrix, or a device CSR triple ``(indptr, indices,
-    data)`` of torch tensors on the trainer's GPU (only the indices are read, stored zeros included, as
-    the ``Evaluator`` reads them).  ``per_user_recommendable_items`` and ``masked_interactions`` hold
-    the same rows; the other arguments are the ``Evaluator``'s.  ``from_global`` slices matrices every
-    rank holds in full.
+    _ev: Any
 
-    ``get_score`` / ``get_scores`` / ``get_target_score`` are collective and return, on every rank,
-    what ``Evaluator`` returns for the gathered model.  Each rank scores and judges its own users on the
-    device (``ials_trainer_evaluate``: the fused lists of ``max(cutoffs)``, then the metrics of every
-    cutoff, no list leaves the device), the per-cutoff sums, counts and item histograms are
-    all-reduced, and the diversity metrics are reduced from the merged histograms on the device.
-    ``catalog_coverage`` divides by the number of recommendable items over ALL ranks' lists."""
-
-    def __init__(self, trainer: "ShardedIALSTrainer", ground_truth: Any, cutoff: int = 10,
-                 target_metric: str = "ndcg", recommendable_items: Optional[List[int]] = None,
-                 per_user_recommendable_items: Any = None, masked_interactions: Any = None,
-                 recall_with_cutoff: bool = False) -> None:
+    def _setup(self, trainer: "ShardedIALSTrainer", recommendable_items: Optional[List[int]],
+               per_user_recommendable_items: Any) -> None:
+        """Collective, after ``_ev`` is built on every rank."""
         import torch
-
-        from .evaluation import Evaluator
 
         self._trainer = trainer
         self._sets: dict = {}
-        self._gt_device = None
         self._lists = recommendable_items is not None or per_user_recommendable_items is not None
         self.last_timings: dict = {}
-        ub, ue = trainer.user_range
-        with _agreement(trainer._device):
-            gt = ground_truth
-            if isinstance(gt, (tuple, list)):  # device CSR: rows sorted here, on the device
-                ip, ix, _ = _device_csr(gt, trainer._device)
-                n_rows = ip.numel() - 1
-                rows = torch.repeat_interleave(torch.arange(n_rows, device=ip.device), ip[1:] - ip[:-1])
-                keys = torch.sort(rows * trainer.n_items + ix).values
-                self._gt_device = ((ip - ip[0]).contiguous(),
-                                   (keys - rows * trainer.n_items).to(torch.int32).contiguous())
-                gt = sps.csr_matrix((n_rows, trainer.n_items))
-            if gt.shape[1] != trainer.n_items:
-                raise ValueError("The model and evaluator assume different n_items.")
-            if gt.shape[0] != ue - ub:
-                raise ValueError(f"ground_truth must hold this rank's {ue - ub} user rows "
-                                 f"[{ub}, {ue}), got {gt.shape[0]}.")
-            self._ev = Evaluator(gt, offset=ub, cutoff=cutoff, target_metric=target_metric,
-                                 recommendable_items=recommendable_items,
-                                 per_user_recommendable_items=per_user_recommendable_items,
-                                 masked_interactions=masked_interactions, recall_with_cutoff=recall_with_cutoff)
         if recommendable_items is None and per_user_recommendable_items is not None:
             # the union of every rank's lists: one OR of the catalogue bitmaps
             seen = torch.zeros(trainer.n_items, dtype=torch.int32)
             seen[torch.from_numpy(self._ev._allow_sorted_flat.astype(np.int64))] = 1
             _all_reduce(seen, trainer._device, "max")
             self._ev.n_recommendable_items = int(seen.sum())
-
-    @classmethod
-    def from_global(cls, trainer: "ShardedIALSTrainer", ground_truth: Any,
-                    per_user_recommendable_items: Any = None, masked_interactions: Any = None,
-                    **kw: Any) -> "ShardedEvaluator":
-        """Slice matrices (and per-user lists) that every rank holds in full by ``trainer.user_range``."""
-        ub, ue = trainer.user_range
-
-        def rows(m: Any) -> Any:
-            if m is None:
-                return None
-            return sps.csr_matrix(m)[ub:ue] if sps.issparse(m) else m[ub:ue]
-
-        return cls(trainer, rows(sps.csr_matrix(ground_truth)), per_user_recommendable_items=rows(
-            per_user_recommendable_items), masked_interactions=rows(masked_interactions), **kw)
 
     def __del__(self) -> None:
         from ._lib import lib
@@ -782,32 +747,29 @@ class ShardedEvaluator:
     def _set_for(self, trainer: "ShardedIALSTrainer", cutoffs: Tuple[int, ...]) -> ctypes.c_void_p:
         from . import _ials_core as core
         from .evaluation import _mask_csr
-        from ._lib import check, lib
 
         h = self._sets.get(cutoffs)
         if h is not None:
             return h
-        ev, p = self._ev, core._ptr
-        ub, ue = trainer.user_range
-        if self._gt_device is not None:
-            gi, gx = self._gt_device
-            g_ptrs, on_device = (ctypes.c_void_p(gi.data_ptr()), ctypes.c_void_p(gx.data_ptr())), 1
-        else:
-            gi = np.ascontiguousarray(ev.ground_truth.indptr, dtype=np.int64)
-            gx = np.ascontiguousarray(ev.ground_truth.indices, dtype=np.int32)
-            g_ptrs, on_device = (p(gi), p(gx)), 0
-        mi = mx = None
-        if ev.masked_interactions is not None:
-            mi, mx = _mask_csr(ev.masked_interactions)
-        n_lists, ai, ax = ev._allowed_for(0, ue - ub, canonical=True) or (0, None, None)
+        ev = self._ev
+        mask = (None, None) if ev.masked_interactions is None else _mask_csr(ev.masked_interactions)
+        allow = ev._allowed_for(0, ev.n_users, canonical=True) or (0, None, None)
         cut = np.ascontiguousarray(cutoffs, dtype=np.int64)
-        h = ctypes.c_void_p(0)
+        p = core._ptr
+        common = (p(mask[0]), p(mask[1]), int(allow[0]), p(allow[1]), p(allow[2]), p(cut), len(cutoffs),
+                  int(bool(ev.recall_with_cutoff)))
         trainer._use_current_stream()
-        check(lib.ials_eval_set_create(trainer._handle, ub, ue - ub, g_ptrs[0], g_ptrs[1], on_device, p(mi),
-                                       p(mx), int(n_lists), p(ai), p(ax), p(cut), len(cutoffs),
-                                       int(bool(ev.recall_with_cutoff)), ctypes.byref(h)))
-        self._sets[cutoffs] = h
-        return h
+        self._sets[cutoffs] = self._create_set(trainer, common)
+        return self._sets[cutoffs]
+
+    def _create_set(self, trainer: "ShardedIALSTrainer", common: tuple) -> ctypes.c_void_p:
+        """The set of this rank's rows; ``common``: mask, allow-list, cutoff and recall arguments of
+        ``ials_eval_set_create``."""
+        raise NotImplementedError
+
+    def _run(self, trainer: "ShardedIALSTrainer", h: ctypes.c_void_p) -> None:
+        """The pass over this rank's rows, adding to the set's accumulators."""
+        raise NotImplementedError
 
     def _views(self, h: ctypes.c_void_p) -> Tuple[Any, Any, Any]:
         """Zero-copy torch views of the set's sums (float64), counts and histograms (int64)."""
@@ -835,13 +797,12 @@ class ShardedEvaluator:
         t0 = time.perf_counter()
         with _agreement(trainer._device):
             if trainer is not self._trainer:
-                raise ValueError("the ShardedEvaluator was built for another trainer")
+                raise ValueError(f"the {type(self).__name__} was built for another trainer")
             h = self._set_for(trainer, tuple(cutoffs))
             stream = trainer._core._stream_of(trainer._device)
             check(lib.ials_eval_set_reset(h, ctypes.c_void_p(stream)))
             trainer._use_current_stream()
-            ub, ue = trainer.user_range
-            check(lib.ials_trainer_evaluate(trainer._handle, h, ub, ue))
+            self._run(trainer, h)
         t1 = time.perf_counter()
         sums, counts, hist = self._views(h)
         for view in (sums, counts, hist):
@@ -861,6 +822,176 @@ class ShardedEvaluator:
             m.valid_user, m.total_user = int(c_host[c]), int(c_host[n_cut + c])
             out.append(ev._metrics_as_dict(m, tuple(float(v) for v in div[c])))
         return out
+
+
+class ShardedEvaluator(_ShardedEvaluation):
+    """The ``Evaluator`` of a row-sharded model, one per rank.
+
+    ``ground_truth`` holds THIS rank's user rows only (``trainer.user_range``), shape
+    ``(user_end - user_begin, n_items)``: a scipy matrix, or a device CSR triple ``(indptr, indices,
+    data)`` of torch tensors on the trainer's GPU (only the indices are read, stored zeros included, as
+    the ``Evaluator`` reads them).  ``per_user_recommendable_items`` and ``masked_interactions`` hold
+    the same rows; the other arguments are the ``Evaluator``'s.  ``from_global`` slices matrices every
+    rank holds in full.
+
+    ``get_score`` / ``get_scores`` / ``get_target_score`` are collective and return, on every rank,
+    what ``Evaluator`` returns for the gathered model.  Each rank scores and judges its own users on the
+    device (``ials_trainer_evaluate``: the fused lists of ``max(cutoffs)``, then the metrics of every
+    cutoff, no list leaves the device), the per-cutoff sums, counts and item histograms are
+    all-reduced, and the diversity metrics are reduced from the merged histograms on the device.
+    ``catalog_coverage`` divides by the number of recommendable items over ALL ranks' lists."""
+
+    def __init__(self, trainer: "ShardedIALSTrainer", ground_truth: Any, cutoff: int = 10,
+                 target_metric: str = "ndcg", recommendable_items: Optional[List[int]] = None,
+                 per_user_recommendable_items: Any = None, masked_interactions: Any = None,
+                 recall_with_cutoff: bool = False) -> None:
+        import torch
+
+        from .evaluation import Evaluator
+
+        self._gt_device = None
+        ub, ue = trainer.user_range
+        with _agreement(trainer._device):
+            gt = ground_truth
+            if isinstance(gt, (tuple, list)):  # device CSR: rows sorted here, on the device
+                ip, ix, _ = _device_csr(gt, trainer._device)
+                n_rows = ip.numel() - 1
+                rows = torch.repeat_interleave(torch.arange(n_rows, device=ip.device), ip[1:] - ip[:-1])
+                keys = torch.sort(rows * trainer.n_items + ix).values
+                self._gt_device = ((ip - ip[0]).contiguous(),
+                                   (keys - rows * trainer.n_items).to(torch.int32).contiguous())
+                gt = sps.csr_matrix((n_rows, trainer.n_items))
+            if gt.shape[1] != trainer.n_items:
+                raise ValueError("The model and evaluator assume different n_items.")
+            if gt.shape[0] != ue - ub:
+                raise ValueError(f"ground_truth must hold this rank's {ue - ub} user rows "
+                                 f"[{ub}, {ue}), got {gt.shape[0]}.")
+            self._ev = Evaluator(gt, offset=ub, cutoff=cutoff, target_metric=target_metric,
+                                 recommendable_items=recommendable_items,
+                                 per_user_recommendable_items=per_user_recommendable_items,
+                                 masked_interactions=masked_interactions, recall_with_cutoff=recall_with_cutoff)
+        self._setup(trainer, recommendable_items, per_user_recommendable_items)
+
+    @classmethod
+    def from_global(cls, trainer: "ShardedIALSTrainer", ground_truth: Any,
+                    per_user_recommendable_items: Any = None, masked_interactions: Any = None,
+                    **kw: Any) -> "ShardedEvaluator":
+        """Slice matrices (and per-user lists) that every rank holds in full by ``trainer.user_range``."""
+        ub, ue = trainer.user_range
+
+        def rows(m: Any) -> Any:
+            if m is None:
+                return None
+            return sps.csr_matrix(m)[ub:ue] if sps.issparse(m) else m[ub:ue]
+
+        return cls(trainer, rows(sps.csr_matrix(ground_truth)), per_user_recommendable_items=rows(
+            per_user_recommendable_items), masked_interactions=rows(masked_interactions), **kw)
+
+    def _create_set(self, trainer: "ShardedIALSTrainer", common: tuple) -> ctypes.c_void_p:
+        from . import _ials_core as core
+        from ._lib import check, lib
+
+        ub, ue = trainer.user_range
+        if self._gt_device is not None:
+            gi, gx = self._gt_device
+            g_ptrs, on_device = (ctypes.c_void_p(gi.data_ptr()), ctypes.c_void_p(gx.data_ptr())), 1
+        else:
+            gi = np.ascontiguousarray(self._ev.ground_truth.indptr, dtype=np.int64)
+            gx = np.ascontiguousarray(self._ev.ground_truth.indices, dtype=np.int32)
+            g_ptrs, on_device = (core._ptr(gi), core._ptr(gx)), 0
+        h = ctypes.c_void_p(0)
+        check(lib.ials_eval_set_create(trainer._handle, ub, ue - ub, g_ptrs[0], g_ptrs[1], on_device, *common,
+                                       ctypes.byref(h)))
+        return h
+
+    def _run(self, trainer: "ShardedIALSTrainer", h: ctypes.c_void_p) -> None:
+        from ._lib import check, lib
+
+        ub, ue = trainer.user_range
+        check(lib.ials_trainer_evaluate(trainer._handle, h, ub, ue))
+
+
+class ShardedEvaluatorWithColdUser(_ShardedEvaluation):
+    """The ``EvaluatorWithColdUser`` of a row-sharded model (evaluator.py:470-657), one per rank:
+    cold users, who are not rows of the model, are folded in from ``input_interaction`` and judged
+    against ``ground_truth``.
+
+    ``input_interaction`` and ``ground_truth`` hold THIS rank's share of the cold users (any number of
+    rows, zero included), ``n_items`` columns each; ``per_user_recommendable_items`` and
+    ``masked_interactions`` hold the same rows; the other arguments are the ``EvaluatorWithColdUser``'s.
+    The input is folded in as given (confidence scaling is the recommender's job, as for the trainer's
+    own matrix) with ``solver_config``, the prediction-time solver (``ials.IALSTrainer``: 5 CG steps,
+    7 iALS++ iterations); the mask is its non-zeros unless ``masked_interactions`` replaces it.
+    ``from_global`` splits matrices every rank holds in full.
+
+    ``get_score`` / ``get_scores`` / ``get_target_score`` are collective and return, on every rank,
+    what ``EvaluatorWithColdUser`` returns on the gathered input for the gathered model.  Every rank
+    holds the full item factors, so it folds in, ranks and judges its own cold users alone
+    (``ials_trainer_evaluate_cold``: nothing leaves the device between the upload of the input and the
+    metric sums); the merge is ``ShardedEvaluator``'s."""
+
+    def __init__(self, trainer: "ShardedIALSTrainer", input_interaction: Any, ground_truth: Any,
+                 solver_config: Any, cutoff: int = 10, target_metric: str = "ndcg",
+                 recommendable_items: Optional[List[int]] = None, per_user_recommendable_items: Any = None,
+                 masked_interactions: Any = None, recall_with_cutoff: bool = False) -> None:
+        from .evaluation import EvaluatorWithColdUser
+
+        core = trainer._core
+        with _agreement(trainer._device):
+            self._sc = core.IALSTrainer._solver(solver_config)
+            if input_interaction.shape[1] != trainer.n_items:  # evaluator.py:585-589
+                raise ValueError("The model and input_interaction assume different numbers of "
+                                 "training items.")
+            if ground_truth.shape[1] != trainer.n_items:
+                raise ValueError("The model and evaluator assume different n_items.")
+            self._ev = EvaluatorWithColdUser(input_interaction, ground_truth, cutoff=cutoff,
+                                             target_metric=target_metric, recommendable_items=recommendable_items,
+                                             per_user_recommendable_items=per_user_recommendable_items,
+                                             masked_interactions=masked_interactions,
+                                             recall_with_cutoff=recall_with_cutoff)
+            self._input = core._csr_arrays(core._canonical_csr(input_interaction))
+        self._setup(trainer, recommendable_items, per_user_recommendable_items)
+
+    @classmethod
+    def from_global(cls, trainer: "ShardedIALSTrainer", input_interaction: Any, ground_truth: Any,
+                    solver_config: Any, per_user_recommendable_items: Any = None,
+                    masked_interactions: Any = None, **kw: Any) -> "ShardedEvaluatorWithColdUser":
+        """Split matrices (and per-user lists) of all cold users, which every rank holds in full, into
+        contiguous shares of balanced input nnz (``balanced_bounds``)."""
+        import torch.distributed as dist
+
+        rank = dist.get_rank() if dist.is_initialized() else 0
+        world = dist.get_world_size() if dist.is_initialized() else 1
+        X = sps.csr_matrix(input_interaction)
+        b = balanced_bounds(np.diff(X.indptr) + 1, world)
+        lo, hi = int(b[rank]), int(b[rank + 1])
+
+        def rows(m: Any) -> Any:
+            if m is None:
+                return None
+            return sps.csr_matrix(m)[lo:hi] if sps.issparse(m) else m[lo:hi]
+
+        return cls(trainer, X[lo:hi], rows(sps.csr_matrix(ground_truth)), solver_config,
+                   per_user_recommendable_items=rows(per_user_recommendable_items),
+                   masked_interactions=rows(masked_interactions), **kw)
+
+    def _create_set(self, trainer: "ShardedIALSTrainer", common: tuple) -> ctypes.c_void_p:
+        from . import _ials_core as core
+        from ._lib import check, lib
+
+        p = core._ptr
+        ip, ix, dt = self._input
+        gi = np.ascontiguousarray(self._ev.ground_truth.indptr, dtype=np.int64)
+        gx = np.ascontiguousarray(self._ev.ground_truth.indices, dtype=np.int32)
+        h = ctypes.c_void_p(0)
+        check(lib.ials_eval_set_create_cold(trainer._handle, self._ev.n_users, trainer.n_items, p(ip), p(ix),
+                                            p(dt), p(gi), p(gx), 0, *common, ctypes.byref(h)))
+        return h
+
+    def _run(self, trainer: "ShardedIALSTrainer", h: ctypes.c_void_p) -> None:
+        from ._lib import check, lib
+
+        check(lib.ials_trainer_evaluate_cold(trainer._handle, h, ctypes.byref(self._sc), 0, self._ev.n_users))
 
 
 # ----------------------------------------------------------------------------
