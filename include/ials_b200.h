@@ -61,6 +61,9 @@ extern "C" {
 
 #define IALS_SIDE_USER 0
 #define IALS_SIDE_ITEM 1
+/* ials_trainer_similar */
+#define IALS_SIMILARITY_DOT 0
+#define IALS_SIMILARITY_COSINE 1
 
 /* struct IALSModelConfig                            IALSLearningConfig.hpp:15-31 */
 typedef struct ials_model_config {
@@ -278,6 +281,22 @@ IALS_API int ials_trainer_recommend_embeddings(ials_trainer *t, const float *use
                                                const int32_t *mask_indices, int64_t allow_n_lists,
                                                const int64_t *allow_indptr, const int32_t *allow_indices,
                                                int32_t *out_idx, float *out_score, int32_t *out_count);
+/* Nearest neighbours within one side (new: the reference has no such query): for each query row of
+ * `side` (0: similar users, 1: similar items), the best `k` rows of the same side, ordered by
+ * (-score, index) as the lists above.  Queries: query_idx[0 .. end) (host, any order, repeats allowed;
+ * begin must be 0) or, with query_idx null, the rows [begin, end) of the side.  metric
+ * IALS_SIMILARITY_COSINE: q.y / (|q| |y|), 0 when either row is zero (the side is copied at unit norm on
+ * every call); IALS_SIMILARITY_DOT: q.y.  exclude_self hides the query row itself; forbid_indptr /
+ * forbid_indices (optional host CSR, one row per query, any order) hide more rows; allow-lists as in
+ * ials_trainer_recommend_allowed, over the side's rows.  1 <= k <= min(1024, rows of the side); k <= 128
+ * runs the fused tensor-core kernel, larger k dense scores + SIMT top-k (allow-lists: k <= 128 only,
+ * IALS_ERR_NOT_IMPLEMENTED otherwise).  Lists shorter than k are padded with -1 (out_count: their
+ * lengths); out_score (optional) holds the scores.  No trainer state changes. */
+IALS_API int ials_trainer_similar(ials_trainer *t, int side, const int64_t *query_idx, int64_t begin, int64_t end,
+                                  int64_t k, int metric, int exclude_self, const int64_t *forbid_indptr,
+                                  const int32_t *forbid_indices, int64_t allow_n_lists, const int64_t *allow_indptr,
+                                  const int32_t *allow_indices, int32_t *out_idx, float *out_score,
+                                  int32_t *out_count);
 
 /* Mask + top-`k` for a block of precomputed float32 scores (any recommender;
  * replaces EvaluatorCore::get_metrics_local's selection, evaluator.cpp:324-355,

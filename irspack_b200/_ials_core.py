@@ -281,6 +281,62 @@ def _transform(handle: ctypes.c_void_p, K: int, device: int, side: int, interact
     return out
 
 
+_SIMILARITY_METRICS = {"dot": 0, "cosine": 1}  # IALS_SIMILARITY_DOT / IALS_SIMILARITY_COSINE
+
+
+def _allowed_arrays(allowed: Any) -> Tuple[int, Optional[np.ndarray], Optional[np.ndarray]]:
+    """``(n_lists, indptr, indices)`` allow-lists as the C ABI takes them (``None``: no list)."""
+    if allowed is None:
+        return 0, None, None
+    n_lists, a_indptr, a_indices = allowed
+    ai = np.ascontiguousarray(a_indptr, dtype=np.int64)
+    ax = np.ascontiguousarray(a_indices, dtype=np.int32)
+    if ai.shape != (int(n_lists) + 1,) or (ai.size and int(ai[-1]) != ax.size):
+        raise ValueError("allowed = (n_lists, indptr[n_lists + 1], indices[indptr[-1]])")
+    return int(n_lists), ai, ax
+
+
+def _similar(handle: ctypes.c_void_p, device: int, n_side: int, side: int, indices: Any, cutoff: int,
+             metric: str, exclude_self: bool, forbidden: Any, allowed: Any, return_scores: bool):
+    """``ials_trainer_similar`` of a trainer (or a row-sharded trainer's replicas) on its device's current
+    stream.  ``indices``: None (every row of the side), a ``range`` of step 1, or row indices."""
+    if side not in (0, 1):
+        raise ValueError("side must be 0 or 1")
+    if metric not in _SIMILARITY_METRICS:
+        raise ValueError("metric must be 'cosine' or 'dot'")
+    cutoff = int(cutoff)
+    if not 1 <= cutoff <= n_side:
+        raise ValueError("cutoff must be in [1, rows of the side]")
+    q = None
+    if indices is None:
+        begin, end = 0, n_side
+    elif isinstance(indices, range):
+        if indices.step != 1 or not 0 <= indices.start <= indices.stop <= n_side:
+            raise ValueError("bad query block")
+        begin, end = indices.start, indices.stop
+    else:
+        q = np.ascontiguousarray(indices, dtype=np.int64).reshape(-1)
+        begin, end = 0, q.size
+    rows = end - begin
+    fi = fx = None
+    if forbidden is not None:
+        f = sps.csr_matrix(forbidden, copy=True)
+        if f.shape != (rows, n_side):
+            raise ValueError("forbidden has the wrong shape")
+        f.eliminate_zeros()  # a stored zero forbids nothing, as in the recommend masks
+        fi = np.ascontiguousarray(f.indptr, dtype=np.int64)
+        fx = np.ascontiguousarray(f.indices, dtype=np.int32)
+    n_lists, ai, ax = _allowed_arrays(allowed)
+    idx = np.empty((rows, cutoff), dtype=np.int32)
+    cnt = np.empty((rows,), dtype=np.int32)
+    sc = np.empty((rows, cutoff), dtype=np.float32) if return_scores else None
+    check(lib.ials_trainer_set_stream(handle, ctypes.c_void_p(_stream_of(device))))
+    check(lib.ials_trainer_similar(handle, side, _ptr(q), begin, end, cutoff, _SIMILARITY_METRICS[metric],
+                                   int(bool(exclude_self)), _ptr(fi), _ptr(fx), n_lists, _ptr(ai), _ptr(ax),
+                                   _ptr(idx), _ptr(sc), _ptr(cnt)))
+    return (idx, cnt, sc) if return_scores else (idx, cnt)
+
+
 def _factors_device(handle: ctypes.c_void_p, side: int, device: int) -> Any:
     """Zero-copy view ([n, K], row stride ld) of a trainer's factor matrix (or replica) of ``side``."""
     import torch
@@ -614,13 +670,7 @@ class IALSTrainer:
             mi = np.ascontiguousarray(m.indptr, dtype=np.int64)
             mx = np.ascontiguousarray(m.indices, dtype=np.int32)
             mode = 2
-        n_lists, ai, ax = 0, None, None
-        if allowed is not None:
-            n_lists, a_indptr, a_indices = allowed
-            ai = np.ascontiguousarray(a_indptr, dtype=np.int64)
-            ax = np.ascontiguousarray(a_indices, dtype=np.int32)
-            if ai.shape != (int(n_lists) + 1,) or (ai.size and int(ai[-1]) != ax.size):
-                raise ValueError("allowed = (n_lists, indptr[n_lists + 1], indices[indptr[-1]])")
+        n_lists, ai, ax = _allowed_arrays(allowed)
         self._use_current_stream()
         if users is not None and users.dtype == np.float32:
             check(lib.ials_trainer_recommend_embeddings(
@@ -638,6 +688,21 @@ class IALSTrainer:
                 self._handle, begin, end, int(cutoff), mode, _ptr(mi), _ptr(mx),
                 int(n_lists), _ptr(ai), _ptr(ax), _ptr(idx), _ptr(sc), _ptr(cnt)))
         return (idx, cnt, sc) if return_scores else (idx, cnt)
+
+    def similar(self, side: int, indices: Any = None, cutoff: int = 10, metric: str = "cosine",
+                exclude_self: bool = True, forbidden: Any = None, allowed: Any = None,
+                return_scores: bool = True):
+        """Nearest neighbours within one side (0: similar users, 1: similar items): for each query row,
+        the best ``cutoff`` rows of the same side by ``metric`` ("cosine": q.y / (|q| |y|), 0 when
+        either row is zero; "dot": q.y), ordered by (-score, index).
+
+        ``indices``: None (every row of the side), a ``range`` of step 1, or row indices (any order,
+        repeats allowed).  ``exclude_self`` hides each query row itself; ``forbidden``: None or a
+        sparse matrix with one row per query whose non-zeros are hidden as well; ``allowed`` as in
+        ``recommend`` (allow-lists need ``cutoff <= 128``).  Returns (indices int32 [n, cutoff]
+        padded with -1, counts int32 [n] [, scores float32 [n, cutoff]]).  No trainer state changes."""
+        return _similar(self._handle, self._device, self.n_users if side == 0 else self.n_items, side, indices,
+                        cutoff, metric, exclude_self, forbidden, allowed, return_scores)
 
     def get_factors_into(self, side: int, out: np.ndarray) -> None:
         """Device -> host copy into a caller-owned (e.g. pinned) C-contiguous buffer."""

@@ -142,6 +142,8 @@ void stage_lists_and_accumulators(ials_trainer *t, ials_eval_set *e, int64_t all
 // The list job of a pass: top-kmax with the set's mask and allow-lists into the trainer's list buffers
 ListJob list_job(ials_trainer *t, const ials_eval_set *e, int64_t chunk) {
   ListJob job = e->allow;
+  job.catalog = t->factor[1].get();
+  job.n_catalog = t->I;
   job.k = e->kmax;
   job.mask_mode = e->mask_mode;
   job.m_indptr = e->m_indptr.get();

@@ -80,17 +80,18 @@ void stage_allow_lists(int64_t n_items, int64_t n_lists, const int64_t *indptr, 
 }
 
 void produce_lists(ials_trainer *t, const ListJob &j) {
+  require(j.catalog != nullptr || j.n_catalog == 0, "list job without a catalogue");
   const bool fused = score_topk_tc_supported(t->ld, j.k) && j.mask_sorted;
   if (j.rowmap != nullptr && j.mask_mode == 0 && !fused)
     throw NotImplemented("mask='train' for users picked by index needs the fused tensor-core kernel");
   if (j.allow_n_lists > 0 && !fused)
     throw NotImplemented("allow-lists need the fused tensor-core kernel (cutoff <= 128, sorted mask rows)");
-  const int64_t rows = j.rows, k = j.k;
+  const int64_t rows = j.rows, k = j.k, n = j.n_catalog;
   if (fused) {
     // scores + mask + top-k in one tcgen05 kernel; only candidate keys touch HBM
     for (int64_t b = 0; b < rows; b += kListSlabRows) {
       const int64_t m = std::min(kListSlabRows, rows - b);
-      void *scratch = ensure_score_buf(t, score_tc_scratch_bytes(m, t->I, k));
+      void *scratch = ensure_score_buf(t, score_tc_scratch_bytes(m, n, k));
       const int64_t *mip = nullptr;
       const int32_t *mix = nullptr;
       const float *mdt = nullptr;
@@ -103,24 +104,24 @@ void produce_lists(ials_trainer *t, const ListJob &j) {
       } else if (j.mask_mode == 2) {
         mip = j.m_indptr; mix = j.m_indices; mrow0 = j.m_row0 + b;
       }
-      launch_score_topk_tc(j.user_rows + b * t->ld, m, t->factor[1].get(), t->I, t->ld, mip,
+      launch_score_topk_tc(j.user_rows + b * t->ld, m, j.catalog, n, t->ld, mip,
                            mix, mdt, mrow0, (int)k, scratch, j.idx + b * k, j.score + b * k,
                            j.count + b, t->stream, (int)std::min<int64_t>(j.allow_n_lists, 2), j.a_indptr,
                            j.a_indices, j.a_row0 + b, j.a_bitmap, mrowmap);
     }
     return;
   }
-  const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 29) / (4 * t->I)));
-  float *buf = ensure_score_buf(t, sizeof(float) * slab * t->I);
+  const int64_t slab = std::max<int64_t>(1, std::min<int64_t>(rows, (1ll << 29) / (4 * n)));
+  float *buf = ensure_score_buf(t, sizeof(float) * slab * n);
   for (int64_t b = 0; b < rows; b += slab) {
     const int64_t m = std::min(slab, rows - b);
-    launch_scores(j.user_rows + b * t->ld, m, t->factor[1].get(), t->I, t->ld, buf, t->I, t->stream);
+    launch_scores(j.user_rows + b * t->ld, m, j.catalog, n, t->ld, buf, n, t->stream);
     if (j.mask_mode == 0)
-      launch_mask_rows(buf, t->I, t->X.indptr.get(), t->X.indices.get(), t->X.data.get(), j.x_row0 + b, m, 0,
+      launch_mask_rows(buf, n, t->X.indptr.get(), t->X.indices.get(), t->X.data.get(), j.x_row0 + b, m, 0,
                        t->stream);
     else if (j.mask_mode == 2)
-      launch_mask_rows(buf, t->I, j.m_indptr, j.m_indices, nullptr, j.m_row0 + b, m, 0, t->stream);
-    launch_topk_rows(buf, t->I, m, t->I, (int)k, j.idx + b * k, j.score + b * k, j.count + b, t->stream);
+      launch_mask_rows(buf, n, j.m_indptr, j.m_indices, nullptr, j.m_row0 + b, m, 0, t->stream);
+    launch_topk_rows(buf, n, m, n, (int)k, j.idx + b * k, j.score + b * k, j.count + b, t->stream);
   }
 }
 
@@ -210,6 +211,8 @@ static int recommend_impl(ials_trainer *t, const int64_t *user_idx, const float 
     int32_t *d_cnt = t->rec_count.ensure(rows);
     ListJob job;
     job.user_rows = t->factor[0].get() + begin * t->ld;
+    job.catalog = t->factor[1].get();
+    job.n_catalog = t->I;
     job.rows = rows;
     job.k = k;
     job.mask_mode = mask_mode;
@@ -281,6 +284,114 @@ int ials_trainer_recommend_embeddings(ials_trainer *t, const float *user_embeddi
   return recommend_impl(t, nullptr, user_embeddings ? user_embeddings : &none, 0, n_rows, k, mask_mode,
                         mask_indptr, mask_indices, allow_n_lists, allow_indptr, allow_indices, out_idx, out_score,
                         out_count);
+}
+
+int ials_trainer_similar(ials_trainer *t, int side, const int64_t *query_idx, int64_t begin, int64_t end,
+                         int64_t k, int metric, int exclude_self, const int64_t *forbid_indptr,
+                         const int32_t *forbid_indices, int64_t allow_n_lists, const int64_t *allow_indptr,
+                         const int32_t *allow_indices, int32_t *out_idx, float *out_score, int32_t *out_count) {
+  return guarded([&] {
+    require(t != nullptr, "trainer is null");
+    require_side(side);
+    const int64_t n = t->n_rows(side);
+    require(end >= begin && begin >= 0 && (query_idx != nullptr ? begin == 0 : end <= n), "bad query block");
+    require(metric == IALS_SIMILARITY_DOT || metric == IALS_SIMILARITY_COSINE, "metric must be 'cosine' or 'dot'");
+    require(k >= 1 && k <= n, "cutoff must be in [1, rows of the side]");
+    require(k <= 1024, "k > 1024 is not supported");
+    const int64_t rows = end - begin;
+    if (rows == 0) return;
+    require(out_idx != nullptr && out_count != nullptr, "output pointer is null");
+    if (query_idx != nullptr)
+      for (int64_t r = 0; r < rows; r++) require(query_idx[r] >= 0 && query_idx[r] < n, "query index out of range");
+    const bool forbid = forbid_indptr != nullptr;
+    if (forbid) {
+      require(forbid_indptr[0] == 0, "forbidden indptr must start at 0");
+      for (int64_t r = 0; r < rows; r++)
+        require(forbid_indptr[r + 1] >= forbid_indptr[r], "forbidden indptr must be non-decreasing");
+    }
+    check_mask_pointers(rows, forbid_indptr, forbid_indices);
+    if (allow_n_lists > 0)
+      require(allow_n_lists == 1 || allow_n_lists == rows, "allow-lists: one shared list or one per query");
+    DeviceGuard g(t->device);
+    // the mask: row r hides the query itself and its forbidden rows, strictly ascending (the fused
+    // kernel's cursor).  A range of queries without forbidden lists reads row begin + r of a CSR built
+    // on the device; otherwise the rows are merged here, one per query.
+    std::vector<int64_t> m_indptr;
+    std::vector<int32_t> m_indices;
+    StreamSyncOnExit sync{t->stream};  // the staging buffers stay with the trainer
+    ListJob job;
+    job.mask_mode = 1;
+    int64_t m_base = 0;
+    if (forbid || (exclude_self && query_idx != nullptr)) {
+      m_indptr.assign((size_t)rows + 1, 0);
+      m_indices.reserve((size_t)((forbid ? forbid_indptr[rows] : 0) + (exclude_self ? rows : 0)));
+      for (int64_t r = 0; r < rows; r++) {
+        const size_t first = m_indices.size();
+        if (forbid)
+          for (int64_t j = forbid_indptr[r]; j < forbid_indptr[r + 1]; j++) {
+            require(forbid_indices[j] >= 0 && forbid_indices[j] < n, "forbidden index out of range");
+            m_indices.push_back(forbid_indices[j]);
+          }
+        if (exclude_self) m_indices.push_back((int32_t)(query_idx != nullptr ? query_idx[r] : begin + r));
+        std::sort(m_indices.begin() + first, m_indices.end());
+        m_indices.erase(std::unique(m_indices.begin() + first, m_indices.end()), m_indices.end());
+        m_indptr[r + 1] = (int64_t)m_indices.size();
+      }
+      stage_mask(rows, n, m_indptr.data(), m_indices.data(), t->rec_mindptr, t->rec_mindices, t->stream);
+      job.mask_mode = 2;
+      job.m_indptr = t->rec_mindptr.get();
+      job.m_indices = t->rec_mindices.get();
+    } else if (exclude_self) {
+      int64_t *ip = t->sim_self_indptr.ensure(n + 1);
+      int32_t *ix = t->sim_self_indices.ensure(n);
+      launch_self_mask(ip, ix, n, t->stream);
+      job.mask_mode = 2;
+      job.m_indptr = ip;
+      job.m_indices = ix;
+      m_base = begin;
+    }
+    if (allow_n_lists > 0)
+      stage_allow_lists(n, allow_n_lists, allow_indptr, allow_indices, t->rec_abitmap_host, t->rec_aindptr,
+                        t->rec_aindices, t->stream, job);
+    // cosine: the same product on a copy of the side scaled to unit norm, queries included
+    const float *Y = t->factor[side].get();
+    if (metric == IALS_SIMILARITY_COSINE) {
+      float *unit = t->sim_norm.ensure(n * t->ld);
+      launch_normalize_rows(Y, n, t->ld, unit, t->stream);
+      Y = unit;
+    }
+    job.catalog = Y;
+    job.n_catalog = n;
+    const float *queries = Y + begin * t->ld;
+    if (query_idx != nullptr) {
+      int64_t *d_q = t->rec_uidx.ensure(rows);
+      float *gathered = t->rec_users.ensure(rows * t->ld);
+      CUDA_CHECK(cudaMemcpyAsync(d_q, query_idx, sizeof(int64_t) * rows, cudaMemcpyHostToDevice, t->stream));
+      launch_gather_rows(Y, t->ld, d_q, rows, gathered, t->stream);
+      queries = gathered;
+    }
+    // slabs of queries: the list buffers stay bounded and each slab's lists go to the host behind it
+    const int64_t slab = std::min(rows, kListSlabRows);
+    job.k = k;
+    job.idx = t->rec_idx.ensure(slab * k);
+    job.score = t->rec_score.ensure(slab * k);
+    job.count = t->rec_count.ensure(slab);
+    for (int64_t b = 0; b < rows; b += slab) {
+      const int64_t m = std::min(slab, rows - b);
+      job.user_rows = queries + b * t->ld;
+      job.rows = m;
+      job.m_row0 = m_base + b;
+      job.a_row0 = b;
+      produce_lists(t, job);
+      CUDA_CHECK(cudaMemcpyAsync(out_idx + b * k, job.idx, sizeof(int32_t) * m * k, cudaMemcpyDeviceToHost,
+                                 t->stream));
+      if (out_score)
+        CUDA_CHECK(cudaMemcpyAsync(out_score + b * k, job.score, sizeof(float) * m * k, cudaMemcpyDeviceToHost,
+                                   t->stream));
+      CUDA_CHECK(cudaMemcpyAsync(out_count + b, job.count, sizeof(int32_t) * m, cudaMemcpyDeviceToHost, t->stream));
+    }
+    CUDA_CHECK(cudaStreamSynchronize(t->stream));
+  });
 }
 
 int ials_metrics_accumulate(const int32_t *rec, const int32_t *count, int64_t rows, int64_t k,

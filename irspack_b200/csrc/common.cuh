@@ -372,6 +372,10 @@ void diversity_of_histogram(const unsigned long long *hist, int64_t n_items, Dev
 void launch_gather_rows(const float *src, int ld, const int64_t *rows, int64_t n_rows, float *dst,
                         cudaStream_t s);
 void launch_pad_copy(const float *src, int64_t n_rows, int K, float *dst, int ld, cudaStream_t s);
+// dst[r] = src[r] / |src[r]|, rows of norm 0 left at 0 (rows of ld floats, ld % 4 == 0)
+void launch_normalize_rows(const float *src, int64_t n_rows, int ld, float *dst, cudaStream_t s);
+// indptr[0 .. n] = 0 .. n, indices[0 .. n) = 0 .. n - 1: the mask CSR whose row i hides column i
+void launch_self_mask(int64_t *indptr, int32_t *indices, int64_t n, cudaStream_t s);
 void launch_unpad_copy(const float *src, int64_t n_rows, int K, int ld, float *dst, cudaStream_t s);
 void launch_init_normal(float *dst, int64_t n_rows, int K, int ld, float stdev, uint64_t seed,
                         cudaStream_t s);

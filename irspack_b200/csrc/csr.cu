@@ -85,6 +85,35 @@ __global__ void gather_rows_kernel(const float *__restrict__ src, int ld, const 
   reinterpret_cast<float4 *>(dst + r * ld)[c] = reinterpret_cast<const float4 *>(src + rows[r] * ld)[c];
 }
 
+// dst[r] = src[r] / |src[r]| (rows of `ld` floats, ld % 4 == 0; a row of norm 0 stays 0): one warp per
+// row, the sum of squares in float64 so that neither tiny nor huge rows lose their direction
+__global__ void normalize_rows_kernel(const float *__restrict__ src, int64_t n_rows, int ld, float *__restrict__ dst) {
+  const int64_t r = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / kWarp;
+  const int lane = threadIdx.x % kWarp;
+  if (r >= n_rows) return;
+  const float4 *row = reinterpret_cast<const float4 *>(src + r * ld);
+  double ss = 0.0;
+  for (int c = lane; c < (ld >> 2); c += kWarp) {
+    const float4 v = row[c];
+    ss += (double)v.x * v.x + (double)v.y * v.y + (double)v.z * v.z + (double)v.w * v.w;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+  const double inv = ss > 0.0 ? 1.0 / sqrt(ss) : 0.0;
+  float4 *out = reinterpret_cast<float4 *>(dst + r * ld);
+  for (int c = lane; c < (ld >> 2); c += kWarp) {
+    const float4 v = row[c];
+    out[c] = make_float4((float)(v.x * inv), (float)(v.y * inv), (float)(v.z * inv), (float)(v.w * inv));
+  }
+}
+
+// The CSR whose row i lists column i alone: indptr[i] = i (i <= n), indices[i] = i (i < n)
+__global__ void self_mask_kernel(int64_t *__restrict__ indptr, int32_t *__restrict__ indices, int64_t n) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i <= n) indptr[i] = i;
+  if (i < n) indices[i] = (int32_t)i;
+}
+
 __global__ void unpad_copy_kernel(const float *__restrict__ src, int64_t n_rows, int K, int ld,
                                   float *__restrict__ dst) {
   int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -272,6 +301,17 @@ void launch_unpad_copy(const float *src, int64_t n_rows, int K, int ld, float *d
   int64_t total = n_rows * K;
   if (total == 0) return;
   unpad_copy_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(src, n_rows, K, ld, dst); count_launch();
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void launch_normalize_rows(const float *src, int64_t n_rows, int ld, float *dst, cudaStream_t s) {
+  if (n_rows == 0) return;
+  normalize_rows_kernel<<<(unsigned)ceil_div(n_rows * kWarp, 256), 256, 0, s>>>(src, n_rows, ld, dst); count_launch();
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void launch_self_mask(int64_t *indptr, int32_t *indices, int64_t n, cudaStream_t s) {
+  self_mask_kernel<<<(unsigned)ceil_div(n + 1, 256), 256, 0, s>>>(indptr, indices, n); count_launch();
   CUDA_CHECK(cudaGetLastError());
 }
 

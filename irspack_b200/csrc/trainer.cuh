@@ -33,6 +33,11 @@ struct ials_trainer {
   ials::DeviceBuffer<int64_t> rec_mindptr, rec_aindptr, rec_uidx;
   ials::DeviceBuffer<float> rec_score, rec_users, rec_emb;
   std::vector<uint32_t> rec_abitmap_host;  // shared allow-list as a bitmap, staged for the upload
+  // ials_trainer_similar (grow-only): the side's rows scaled to unit norm, and the mask CSR whose row i
+  // hides row i (the query itself, for a range of queries without forbidden lists)
+  ials::DeviceBuffer<float> sim_norm;
+  ials::DeviceBuffer<int64_t> sim_self_indptr;
+  ials::DeviceBuffer<int32_t> sim_self_indices;
   // shard (multi-GPU): rows owned (solved) by this rank, per side; X / Xt then hold only
   // those rows (DeviceCsr::row_base = shard begin) while both factor matrices are full replicas
   bool sharded = false;
@@ -189,13 +194,17 @@ void run_solver(ials_trainer *t, const SolveArgs &a, const DeviceCsr &csr,
 void ensure_copy_stream(ials_trainer *t);
 void enqueue_flagged_user_upload(ials_trainer *t, int64_t row_begin, int64_t n_rows, const float *rows_host);
 void consume_flagged_upload(ials_trainer *t, const ials_solver_config *sc, SolveArgs &a, int64_t row_begin);
-// api_recommend.cu: top-k lists of `rows` user rows, everything already on the device.  The fused
+// api_recommend.cu: top-k lists of `rows` query rows against a catalogue, everything already on the
+// device (the recommend entry points and the evaluation sets: user rows against the item factors;
+// ials_trainer_similar: rows of one side against that side).  The fused
 // tensor-core kernel where it applies (score_topk_tc_supported, sorted mask rows), else scores + mask +
 // SIMT top-k; allow-lists and users picked by index with mask_mode 0 need the fused route
 // (NotImplemented otherwise).  Enqueued on t->stream.
 constexpr int64_t kListSlabRows = 262144;  // rows per fused launch: bounds its scratch (score_buf)
 struct ListJob {
-  const float *user_rows = nullptr;  // [rows x ld]
+  const float *user_rows = nullptr;  // [rows x ld] queries
+  const float *catalog = nullptr;    // [n_catalog x ld] rows ranked for each query
+  int64_t n_catalog = 0;
   int64_t rows = 0, k = 0;
   int mask_mode = 1;                 // 0: rows of X, 1: none, 2: the CSR below
   int64_t x_row0 = 0;                // mode 0: row of X (local to the shard) that masks block row 0

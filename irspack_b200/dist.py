@@ -617,6 +617,14 @@ class ShardedIALSTrainer:
                                                      p(None), p(None), p(idx), p(None), p(cnt)))
         return idx, cnt
 
+    def similar(self, side: int, indices: Any = None, cutoff: int = 10, metric: str = "cosine",
+                exclude_self: bool = True, forbidden: Any = None, allowed: Any = None,
+                return_scores: bool = True):
+        """``IALSTrainer.similar`` on this rank's full replicas: rank-local, no collective; any rank
+        answers any query (after ``sync()`` every rank gives the same lists)."""
+        return self._core._similar(self._handle, self._device, self.n_users if side == 0 else self.n_items, side,
+                                   indices, cutoff, metric, exclude_self, forbidden, allowed, return_scores)
+
     def transform_user(self, X: Any, solver_config: Any) -> np.ndarray:
         """Fold-in of new users' rows ``X`` (n x n_items) against this rank's full item replica
         (``IALSTrainer.transform_user``, IALSTrainer.hpp:791-796): rank-local, no collective."""

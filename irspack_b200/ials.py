@@ -377,6 +377,33 @@ class IALSRecommender:
         return self.trainer_as_ials.core_trainer.recommend_users(
             u, cutoff, mask=mask, return_scores=return_scores, allowed=allowed)
 
+    def _similar(self, side: int, indices: Any, cutoff: int, **kw: Any):
+        n = self.n_users if side == 0 else self.n_items
+        if indices is not None:  # negative and boolean indices as get_score takes them
+            indices = np.asarray(indices)
+            if indices.dtype == bool:
+                indices = np.flatnonzero(indices)
+            indices = indices.astype(np.int64).reshape(-1)
+            indices = np.where(indices < 0, indices + n, indices)
+        return self.trainer_as_ials.core_trainer.similar(side, indices, cutoff, **kw)
+
+    def get_similar_items(self, item_indices: Any, cutoff: int = 10, metric: str = "cosine",
+                          exclude_self: bool = True, forbidden: Any = None, allowed: Any = None,
+                          return_scores: bool = True):
+        """B200 extension: the ``cutoff`` items most similar to each of ``item_indices`` (None: every
+        item) in the item factor space, on the device (``IALSTrainer.similar``, side 1):
+        (indices, counts, scores)."""
+        return self._similar(1, item_indices, cutoff, metric=metric, exclude_self=exclude_self,
+                             forbidden=forbidden, allowed=allowed, return_scores=return_scores)
+
+    def get_similar_users(self, user_indices: Any, cutoff: int = 10, metric: str = "cosine",
+                          exclude_self: bool = True, forbidden: Any = None, allowed: Any = None,
+                          return_scores: bool = True):
+        """B200 extension: the ``cutoff`` users most similar to each of ``user_indices`` (None: every
+        user) in the user factor space (``IALSTrainer.similar``, side 0): (indices, counts, scores)."""
+        return self._similar(0, user_indices, cutoff, metric=metric, exclude_self=exclude_self,
+                             forbidden=forbidden, allowed=allowed, return_scores=return_scores)
+
     def recommend_cold_block(self, X: Any, cutoff: int, mask: Any = "input", allowed: Any = None,
                              return_scores: bool = False):
         """B200 extension, the cold-user twin of ``recommend_block``: fold the rows of ``X``

@@ -160,20 +160,65 @@ class ItemIDMapper(Generic[ItemIdType]):
         mask: Any = None
         if forbidden_item_ids is not None:
             mask = (sps.csr_matrix(seen()) != 0).astype(np.float32) + self._index_lists_csr(rows, forbidden_item_ids)
-        allowed = None
-        if per_user_allowed_item_ids is not None:
-            a = self._index_lists_csr(rows, per_user_allowed_item_ids)
-            a.sort_indices()
-            allowed = (rows, a.indptr.astype(np.int64), a.indices.astype(np.int32))
-        elif allowed_item_ids is not None:
-            a = np.unique(np.asarray(self._item_id_list_to_index_list(allowed_item_ids), dtype=np.int32))
-            allowed = (1, np.array([0, a.size], dtype=np.int64), a)
+        allowed = self._allow_lists(rows, allowed_item_ids, per_user_allowed_item_ids)
         try:
             idx, cnt, sc = call(k, mask, allowed)
         except NotImplementedError:
             return None
-        ids = self.item_ids
-        return [[(ids[i], float(v)) for i, v in zip(idx[r, :cnt[r]], sc[r, :cnt[r]])] for r in range(rows)]
+        return self._id_lists(self.item_ids, idx, cnt, sc)
+
+    def _allow_lists(self, rows: int, allowed_item_ids: Optional[List[ItemIdType]],
+                     per_row_allowed_item_ids: Optional[List[List[ItemIdType]]]) -> Any:
+        """``(n_lists, indptr, indices)`` allow-lists of the fused kernel (None: every item)."""
+        if per_row_allowed_item_ids is not None:
+            a = self._index_lists_csr(rows, per_row_allowed_item_ids)
+            a.sort_indices()
+            return (rows, a.indptr.astype(np.int64), a.indices.astype(np.int32))
+        if allowed_item_ids is not None:
+            a = np.unique(np.asarray(self._item_id_list_to_index_list(allowed_item_ids), dtype=np.int32))
+            return (1, np.array([0, a.size], dtype=np.int64), a)
+        return None
+
+    @staticmethod
+    def _id_lists(ids: List[Any], idx: np.ndarray, cnt: np.ndarray, sc: np.ndarray) -> List[List[Tuple[Any, float]]]:
+        return [[(ids[i], float(v)) for i, v in zip(idx[r, :cnt[r]], sc[r, :cnt[r]])] for r in range(len(cnt))]
+
+    @staticmethod
+    def _query_indices(id_to_index: Dict[Any, int], ids: Iterable[Any], what: str) -> np.ndarray:
+        out = []
+        for i in ids:
+            if i not in id_to_index:
+                raise RuntimeError(f"{what} with {what.lower()}_id {i} not found.")
+            out.append(id_to_index[i])
+        return np.asarray(out, dtype=np.int64)
+
+    def similar_items(self, recommender: Any, item_ids: List[ItemIdType], cutoff: int = 20,
+                      allowed_item_ids: Optional[List[ItemIdType]] = None,
+                      per_item_allowed_item_ids: Optional[List[List[ItemIdType]]] = None,
+                      forbidden_item_ids: Optional[List[List[ItemIdType]]] = None
+                      ) -> List[List[Tuple[ItemIdType, float]]]:
+        """B200 extension: for each of ``item_ids``, the ``cutoff`` most similar other items (cosine
+        similarity of the item factors) as [(item id, score)], best first; ties in ascending index
+        order.  ``allowed_item_ids`` (shared) / ``per_item_allowed_item_ids`` restrict the candidates,
+        ``forbidden_item_ids`` (one list per queried item) hides items; unknown ids in those lists are
+        ignored, an unknown queried id raises ``RuntimeError``.  The recommender must provide
+        ``get_similar_items`` (an ``IALSRecommender``): there is no host path."""
+        self._check_recommender_n_items(recommender)
+        if not hasattr(recommender, "get_similar_items"):
+            raise NotImplementedError("similar_items needs a recommender with get_similar_items")
+        q = self._query_indices(self.item_id_to_index, item_ids, "Item")
+        rows = q.size
+        if forbidden_item_ids is not None:
+            assert len(forbidden_item_ids) == rows
+        if per_item_allowed_item_ids is not None:
+            assert len(per_item_allowed_item_ids) == rows
+        if rows == 0:
+            return []
+        forbidden = None if forbidden_item_ids is None else self._index_lists_csr(rows, forbidden_item_ids)
+        idx, cnt, sc = recommender.get_similar_items(
+            q, min(int(cutoff), len(self.item_ids)), forbidden=forbidden,
+            allowed=self._allow_lists(rows, allowed_item_ids, per_item_allowed_item_ids), return_scores=True)
+        return self._id_lists(self.item_ids, idx, cnt, sc)
 
     def recommend_for_new_user(self, recommender: Any, user_profile: Profile, cutoff: int = 20,
                                allowed_item_ids: Optional[List[ItemIdType]] = None,
@@ -309,3 +354,17 @@ class IDMapper(Generic[UserIdType, ItemIdType], ItemIDMapper[ItemIdType]):
         score = recommender.get_score_remove_seen(u)
         return self.score_to_recommended_items_batch(
             score, cutoff, allowed_item_ids, per_user_allowed_item_ids, forbidden_item_ids, n_threads)
+
+    def similar_users(self, recommender: Any, user_ids: List[UserIdType], cutoff: int = 20
+                      ) -> List[List[Tuple[UserIdType, float]]]:
+        """B200 extension, the user twin of ``similar_items``: for each of ``user_ids``, the ``cutoff``
+        most similar other users (cosine similarity of the user factors) as [(user id, score)].  The
+        recommender must provide ``get_similar_users``."""
+        self._check_recommender_n_users(recommender)
+        if not hasattr(recommender, "get_similar_users"):
+            raise NotImplementedError("similar_users needs a recommender with get_similar_users")
+        q = self._query_indices(self.user_id_to_index, user_ids, "User")
+        if q.size == 0:
+            return []
+        idx, cnt, sc = recommender.get_similar_users(q, min(int(cutoff), len(self.user_ids)), return_scores=True)
+        return self._id_lists(self.user_ids, idx, cnt, sc)
