@@ -297,6 +297,33 @@ IALS_API int ials_trainer_similar(ials_trainer *t, int side, const int64_t *quer
                                   const int32_t *forbid_indices, int64_t allow_n_lists, const int64_t *allow_indptr,
                                   const int32_t *allow_indices, int32_t *out_idx, float *out_score,
                                   int32_t *out_count);
+/* Candidate ranking (new: the reference ranks allowed items by computing every item's score first):
+ * for each query row, the best `k` items of its own candidate list by the score q . item, ordered by
+ * (-score, index) as the lists above.  The cost follows the number of (row, candidate) pairs, not the
+ * catalogue: the candidates' item rows are gathered and dotted in FP32, and each list is selected on
+ * its own.  Queries: user_idx[0 .. end) (host, any order, repeats allowed; begin must be 0), or
+ * user_emb[end * K] (host embeddings, e.g. fold-in results; begin must be 0), or, with both null, the
+ * users [begin, end); both non-null is an error.  mask_mode as in ials_trainer_recommend_users (0: each
+ * user's training row, not with embeddings and, on a row-sharded trainer, only for the rank's own users;
+ * 1: none; 2: one host CSR row per query).  Candidates: a CSR of int32 item ids, one list shared by
+ * every row (cand_n_lists = 1) or one per row (cand_n_lists = end - begin), each list strictly ascending
+ * in [0, n_items).  1 <= k <= min(1024, n_items).  Masked candidates are dropped; lists shorter than k
+ * are padded with -1 (scores -inf), out_count holds their lengths, out_score may be NULL.  Rows run in
+ * slabs whose lists are copied to the host one after the other.  Every invalid argument is
+ * IALS_ERR_INVALID_ARGUMENT.  No trainer state changes. */
+IALS_API int ials_trainer_rank_candidates(ials_trainer *t, const int64_t *user_idx, const float *user_emb,
+                                          int64_t begin, int64_t end, int64_t k, int mask_mode,
+                                          const int64_t *mask_indptr, const int32_t *mask_indices,
+                                          int64_t cand_n_lists, const int64_t *cand_indptr,
+                                          const int32_t *cand_indices, int32_t *out_idx, float *out_score,
+                                          int32_t *out_count);
+/* The scores alone ("predict" of the factor model, or iALS scores as features of another ranker):
+ * out_scores[j] = q_r . item[cand_indices[j]] in FP32 for every entry j of row r of the CSR
+ * cand_indptr[end - begin + 1] / cand_indices (any order, repeats allowed, ids in [0, n_items)), in
+ * input order.  Queries as in ials_trainer_rank_candidates.  No mask, no selection. */
+IALS_API int ials_trainer_candidate_scores(ials_trainer *t, const int64_t *user_idx, const float *user_emb,
+                                           int64_t begin, int64_t end, const int64_t *cand_indptr,
+                                           const int32_t *cand_indices, float *out_scores);
 
 /* Mask + top-`k` for a block of precomputed float32 scores (any recommender;
  * replaces EvaluatorCore::get_metrics_local's selection, evaluator.cpp:324-355,

@@ -337,6 +337,128 @@ def _similar(handle: ctypes.c_void_p, device: int, n_side: int, side: int, indic
     return (idx, cnt, sc) if return_scores else (idx, cnt)
 
 
+def _mask_arrays(mask: Any, rows: int, n_items: int) -> Tuple[int, Optional[np.ndarray], Optional[np.ndarray]]:
+    """``(mask_mode, indptr, indices)`` of a list request's mask: "train" (0), None (1) or a sparse matrix
+    with one row per query (2; stored zeros dropped, as scipy's ``.nonzero()`` drops them, evaluator.py:432)."""
+    if isinstance(mask, str):
+        if mask != "train":
+            raise ValueError("mask must be 'train', None or a sparse matrix")
+        return 0, None, None
+    if mask is None:
+        return 1, None, None
+    m = sps.csr_matrix(mask)
+    if m.shape != (rows, n_items):
+        raise ValueError("mask has the wrong shape")
+    m = sps.csr_matrix(m, copy=True)
+    m.eliminate_zeros()
+    m.sort_indices()
+    return 2, np.ascontiguousarray(m.indptr, dtype=np.int64), np.ascontiguousarray(m.indices, dtype=np.int32)
+
+
+def _candidate_lists(candidates: Any, rows: int, n_items: int,
+                     rank: bool = True) -> Tuple[int, np.ndarray, np.ndarray]:
+    """``(n_lists, indptr, indices)`` of candidate items given as ``(n_lists, indptr, indices)`` (the
+    format of ``allowed``) or as a sequence of index lists: one list shared by every query row or one
+    per row.  Ids must lie in ``[0, n_items)``.  ``rank``: each list is sorted and its repeats dropped
+    (the strictly ascending lists the ranking takes); otherwise the lists are kept as given."""
+    if isinstance(candidates, tuple) and len(candidates) == 3 and np.isscalar(candidates[0]):
+        n_lists = int(candidates[0])
+        ip = np.ascontiguousarray(candidates[1], dtype=np.int64).reshape(-1)
+        ix = np.asarray(candidates[2]).reshape(-1)
+        if (ip.shape != (n_lists + 1,) or ip[0] != 0 or np.any(np.diff(ip) < 0) or int(ip[-1]) != ix.size):
+            raise ValueError("candidates = (n_lists, indptr[n_lists + 1], indices[indptr[-1]])")
+    else:
+        lists = [np.asarray(x).reshape(-1) for x in candidates]
+        n_lists = len(lists)
+        ip = np.zeros(n_lists + 1, dtype=np.int64)
+        np.cumsum([x.size for x in lists], out=ip[1:])
+        ix = np.concatenate([x for x in lists if x.size]) if ip[-1] else np.empty(0, dtype=np.int64)
+    if n_lists != rows and n_lists != 1:
+        raise ValueError("candidates: one shared list or one list per row")
+    if ix.size and not np.issubdtype(ix.dtype, np.integer):
+        raise ValueError("candidate item ids must be integers")
+    # int32 lists to be ranked are range-checked by their first and last ids once sorted (one id per
+    # list instead of every id); anything else before the cast, which could wrap
+    full_check = ix.dtype != np.int32 or not rank
+    if full_check and ix.size and (ix.min() < 0 or ix.max() >= n_items):
+        raise ValueError("candidate item out of range")
+    ix = np.ascontiguousarray(ix, dtype=np.int32)
+    if rank and ix.size > 1:
+        ascending = ix[1:] > ix[:-1]
+        starts = ip[1:-1]
+        ascending[starts[(starts > 0) & (starts < ix.size)] - 1] = True  # a list's first id follows another list
+        if not ascending.all():
+            row = np.repeat(np.arange(n_lists, dtype=np.int64), np.diff(ip))
+            order = np.lexsort((ix, row))
+            ix, row = ix[order], row[order]
+            keep = np.ones(ix.size, dtype=bool)
+            keep[1:] = (ix[1:] != ix[:-1]) | (row[1:] != row[:-1])
+            ix, row = np.ascontiguousarray(ix[keep]), row[keep]
+            ip = np.zeros(n_lists + 1, dtype=np.int64)
+            np.cumsum(np.bincount(row, minlength=n_lists), out=ip[1:])
+    if not full_check and ix.size:
+        filled = ip[1:] > ip[:-1]
+        if ix[ip[:-1][filled]].min() < 0 or ix[ip[1:][filled] - 1].max() >= n_items:
+            raise ValueError("candidate item out of range")
+    return n_lists, ip, ix
+
+
+def _query_block(users: Any, n_users: int) -> Tuple[Optional[np.ndarray], int, int]:
+    """``(user_idx, begin, end)`` of users given as a ``range`` of step 1 or as indices."""
+    if isinstance(users, range):
+        if users.step != 1 or not 0 <= users.start <= users.stop <= n_users:
+            raise ValueError("bad user block")
+        return None, users.start, users.stop
+    u = np.ascontiguousarray(users, dtype=np.int64).reshape(-1)
+    return u, 0, u.size
+
+
+def _rank_candidates(handle: ctypes.c_void_p, device: int, n_users: int, n_items: int, K: int, users: Any,
+                     embeddings: Any, candidates: Any, cutoff: int, mask: Any, return_scores: bool):
+    """``ials_trainer_rank_candidates`` of a trainer (or a row-sharded trainer's replicas) on its device's
+    current stream.  Queries: ``users`` (a step-1 ``range`` or indices) or, when it is None, the host rows
+    ``embeddings`` [n, K]."""
+    cutoff = int(cutoff)
+    if not 1 <= cutoff <= min(1024, n_items):
+        raise ValueError("cutoff must be in [1, min(1024, n_items)]")
+    emb = None
+    if users is None:
+        emb = np.ascontiguousarray(embeddings, dtype=np.float32)
+        if emb.ndim != 2 or emb.shape[1] != K:
+            raise ValueError("embedding must be (n, n_components)")
+        if isinstance(mask, str):
+            raise ValueError("embeddings have no training rows: mask must be None or a sparse matrix")
+        q, begin, end = None, 0, emb.shape[0]
+    else:
+        q, begin, end = _query_block(users, n_users)
+    rows = end - begin
+    mode, mi, mx = _mask_arrays(mask, rows, n_items)
+    n_lists, ci, cx = _candidate_lists(candidates, rows, n_items)
+    idx = np.empty((rows, cutoff), dtype=np.int32)
+    cnt = np.empty((rows,), dtype=np.int32)
+    sc = np.empty((rows, cutoff), dtype=np.float32) if return_scores else None
+    check(lib.ials_trainer_set_stream(handle, ctypes.c_void_p(_stream_of(device))))
+    check(lib.ials_trainer_rank_candidates(handle, _ptr(q), _ptr(emb), begin, end, cutoff, mode, _ptr(mi), _ptr(mx),
+                                           n_lists, _ptr(ci), _ptr(cx), _ptr(idx), _ptr(sc), _ptr(cnt)))
+    return (idx, cnt, sc) if return_scores else (idx, cnt)
+
+
+def _candidate_scores(handle: ctypes.c_void_p, device: int, n_users: int, n_items: int, users: Any,
+                      candidates: Any) -> np.ndarray:
+    """``ials_trainer_candidate_scores``: the scores of every (row, candidate) pair, float32 in the order
+    of the candidate lists (a shared list counts once per row)."""
+    q, begin, end = _query_block(users, n_users)
+    rows = end - begin
+    n_lists, ci, cx = _candidate_lists(candidates, rows, n_items, rank=False)
+    if n_lists != rows:  # one shared list: repeated for every row
+        ci = np.arange(rows + 1, dtype=np.int64) * cx.size
+        cx = np.tile(cx, rows)
+    out = np.empty(cx.size, dtype=np.float32)
+    check(lib.ials_trainer_set_stream(handle, ctypes.c_void_p(_stream_of(device))))
+    check(lib.ials_trainer_candidate_scores(handle, _ptr(q), None, begin, end, _ptr(ci), _ptr(cx), _ptr(out)))
+    return out
+
+
 def _factors_device(handle: ctypes.c_void_p, side: int, device: int) -> Any:
     """Zero-copy view ([n, K], row stride ld) of a trainer's factor matrix (or replica) of ``side``."""
     import torch
@@ -653,23 +775,7 @@ class IALSTrainer:
         idx = np.empty((rows, cutoff), dtype=np.int32)
         cnt = np.empty((rows,), dtype=np.int32)
         sc = np.empty((rows, cutoff), dtype=np.float32) if return_scores else None
-        mi = mx = None
-        if isinstance(mask, str):
-            if mask != "train":
-                raise ValueError("mask must be 'train', None or a sparse matrix")
-            mode = 0
-        elif mask is None:
-            mode = 1
-        else:
-            m = sps.csr_matrix(mask)
-            if m.shape != (rows, self.n_items):
-                raise ValueError("mask has the wrong shape")
-            m = sps.csr_matrix(m, copy=True)
-            m.eliminate_zeros()  # scipy's .nonzero() drops stored zeros (evaluator.py:432)
-            m.sort_indices()
-            mi = np.ascontiguousarray(m.indptr, dtype=np.int64)
-            mx = np.ascontiguousarray(m.indices, dtype=np.int32)
-            mode = 2
+        mode, mi, mx = _mask_arrays(mask, rows, self.n_items)
         n_lists, ai, ax = _allowed_arrays(allowed)
         self._use_current_stream()
         if users is not None and users.dtype == np.float32:
@@ -703,6 +809,33 @@ class IALSTrainer:
         padded with -1, counts int32 [n] [, scores float32 [n, cutoff]]).  No trainer state changes."""
         return _similar(self._handle, self._device, self.n_users if side == 0 else self.n_items, side, indices,
                         cutoff, metric, exclude_self, forbidden, allowed, return_scores)
+
+    def rank_candidates(self, user_indices: Any, candidates: Any, cutoff: int, mask: Any = "train",
+                        return_scores: bool = True):
+        """Ranks each user's own candidate items: the best ``cutoff`` of them by score, ordered by
+        (-score, index), at a cost that follows the number of (user, candidate) pairs, not the catalogue.
+
+        ``user_indices``: a ``range`` of step 1 or user indices (any order, repeats allowed).
+        ``candidates``: ``(n_lists, indptr, indices)`` as ``allowed`` takes it, or a sequence of index
+        lists; one list shared by every user or one per user.  Lists are sorted and their repeats dropped
+        here.  ``mask``: "train" (each user's training row), None, or a sparse matrix with one row per
+        user; masked candidates are dropped.  ``1 <= cutoff <= min(1024, n_items)``.  Returns (indices
+        int32 [n, cutoff] padded with -1, counts int32 [n] [, scores float32 [n, cutoff]]).  No trainer
+        state changes."""
+        return _rank_candidates(self._handle, self._device, self.n_users, self.n_items, self.K, user_indices,
+                                None, candidates, cutoff, mask, return_scores)
+
+    def rank_candidates_embeddings(self, user_embedding: Any, candidates: Any, cutoff: int, mask: Any = None,
+                                   return_scores: bool = True):
+        """``rank_candidates`` for embeddings that are not rows of the model (fold-in results).
+        ``mask``: None or one sparse row per embedding."""
+        return _rank_candidates(self._handle, self._device, self.n_users, self.n_items, self.K, None,
+                                user_embedding, candidates, cutoff, mask, return_scores)
+
+    def candidate_scores(self, user_indices: Any, candidates: Any) -> np.ndarray:
+        """The score of every (user, candidate) pair, float32, in the order of the candidate lists
+        (any order, repeats allowed; a shared list counts once per user)."""
+        return _candidate_scores(self._handle, self._device, self.n_users, self.n_items, user_indices, candidates)
 
     def get_factors_into(self, side: int, out: np.ndarray) -> None:
         """Device -> host copy into a caller-owned (e.g. pinned) C-contiguous buffer."""

@@ -127,6 +127,135 @@ void produce_lists(ials_trainer *t, const ListJob &j) {
 
 }  // namespace ials
 
+namespace {
+
+// The query rows and the mask of a list request, staged on the device into job.user_rows, rowmap,
+// mask_mode, x_row0, m_indptr / m_indices and mask_sorted.  user_idx != nullptr: the rows are users
+// user_idx[0 .. rows), gathered on the device; user_emb != nullptr: the rows are the host embeddings
+// user_emb[rows x K] (fold-in results); otherwise users [begin, begin + rows).  Call under the trainer's
+// device, with its stream synchronised on exit (the staging buffers stay with the trainer).
+void stage_queries(ials_trainer *t, const int64_t *user_idx, const float *user_emb, int64_t begin,
+                          int64_t rows, int mask_mode, const int64_t *mask_indptr, const int32_t *mask_indices,
+                          ListJob &job) {
+  if (mask_mode == 0 && !t->has_X) throw std::runtime_error("no training matrix to mask with");
+  if (mask_mode == 0 && user_idx == nullptr && user_emb == nullptr)  // a sharded trainer only holds its own users' rows of X
+    require(begin >= t->X.row_base && begin + rows <= t->X.row_base + t->X.n_rows,
+            "mask='train' on a sharded trainer needs a user block inside the rank's shard");
+  if (user_idx != nullptr)
+    for (int64_t r = 0; r < rows; r++) {
+      require(user_idx[r] >= 0 && user_idx[r] < t->U, "user index out of range");
+      if (mask_mode == 0)
+        require(user_idx[r] >= t->X.row_base && user_idx[r] < t->X.row_base + t->X.n_rows,
+                "mask='train' on a sharded trainer needs users inside the rank's shard");
+    }
+  // the fused tensor-core kernel walks each mask row with a cursor: column ids must ascend
+  job.mask_sorted = true;
+  if (mask_mode == 0) {
+    if (t->X.sorted_state < 0)
+      t->X.sorted_state =
+          csr_rows_strictly_sorted(t->X.indptr.get(), t->X.indices.get(), t->X.n_rows, t->stream) ? 1 : 0;
+    job.mask_sorted = t->X.sorted_state == 1;
+  }
+  if (mask_mode == 2) {
+    stage_mask(rows, t->I, mask_indptr, mask_indices, t->rec_mindptr, t->rec_mindices, t->stream);
+    job.mask_sorted = mask_rows_sorted(rows, mask_indptr, mask_indices);
+    job.m_indptr = t->rec_mindptr.get();
+    job.m_indices = t->rec_mindices.get();
+  }
+  job.mask_mode = mask_mode;
+  job.x_row0 = begin - t->X.row_base;
+  job.user_rows = t->factor[0].get() + begin * t->ld;
+  // users picked by index: their factor rows are gathered into a dense block first
+  if (user_idx != nullptr) {
+    int64_t *d_uidx = t->rec_uidx.ensure(rows);
+    float *gathered = t->rec_users.ensure(rows * t->ld);
+    CUDA_CHECK(cudaMemcpyAsync(d_uidx, user_idx, sizeof(int64_t) * rows, cudaMemcpyHostToDevice, t->stream));
+    launch_gather_rows(t->factor[0].get(), t->ld, d_uidx, rows, gathered, t->stream);
+    job.user_rows = gathered;
+    job.rowmap = d_uidx;
+  }
+  if (user_emb != nullptr) {  // host embeddings [rows x K] -> padded device rows [rows x ld]
+    float *staged = t->rec_emb.ensure(rows * t->K);
+    float *padded = t->rec_users.ensure(rows * t->ld);
+    CUDA_CHECK(cudaMemcpyAsync(staged, user_emb, sizeof(float) * rows * t->K, cudaMemcpyHostToDevice, t->stream));
+    launch_pad_copy(staged, rows, (int)t->K, padded, t->ld, t->stream);
+    job.user_rows = padded;
+  }
+}
+
+// Validates host candidate lists: indptr from 0 and non-decreasing, item ids in [0, n_items), and
+// strictly ascending inside each list when `strict` (lists that are ranked; scored pairs may repeat)
+void check_candidates(int64_t n_items, int64_t n_lists, const int64_t *indptr, const int32_t *indices,
+                             bool strict) {
+  require(indptr != nullptr && indptr[0] == 0, "candidate indptr must start at 0");
+  for (int64_t r = 0; r < n_lists; r++) require(indptr[r + 1] >= indptr[r], "candidate indptr must be non-decreasing");
+  require(indptr[n_lists] == 0 || indices != nullptr, "candidate indices are null");
+  for (int64_t r = 0; r < n_lists; r++)
+    for (int64_t j = indptr[r]; j < indptr[r + 1]; j++) {
+      require(indices[j] >= 0 && indices[j] < n_items, "candidate item out of range");
+      require(!strict || j == indptr[r] || indices[j - 1] < indices[j], "candidate lists must be strictly ascending");
+    }
+}
+
+// Uploads validated candidate lists into the trainer's grow-only list buffers; shared: list 0 serves
+// every row
+CandSegments stage_candidates(ials_trainer *t, int64_t n_lists, const int64_t *indptr,
+                                     const int32_t *indices, bool shared) {
+  const int64_t nnz = indptr[n_lists];
+  int64_t *ip = t->rec_aindptr.ensure(n_lists + 1);
+  int32_t *ix = t->rec_aindices.ensure(std::max<int64_t>(nnz, 1));
+  CUDA_CHECK(cudaMemcpyAsync(ip, indptr, sizeof(int64_t) * (n_lists + 1), cudaMemcpyHostToDevice, t->stream));
+  if (nnz) CUDA_CHECK(cudaMemcpyAsync(ix, indices, sizeof(int32_t) * nnz, cudaMemcpyHostToDevice, t->stream));
+  return CandSegments{ip, ix, 0, 0, shared ? nnz : -1};
+}
+
+// Rows [b, b + m) of a call whose (row, candidate) pairs share one pass of the score scratch: at most
+// kListSlabRows rows and, unless one row alone has more, kCandSlabPairs pairs.  tasks[r] (rows + 1
+// entries): the first score task of row r, one per kCandChunk of its candidates (launch_cand_scores).
+struct CandSlab {
+  int64_t b, m, pairs, max_len;
+};
+constexpr int64_t kCandSlabPairs = 1ll << 26;  // 256 MB of FP32 scores
+std::vector<CandSlab> plan_candidate_slabs(int64_t rows, const int64_t *indptr, bool shared,
+                                           std::vector<int64_t> &tasks) {
+  std::vector<CandSlab> slabs;
+  tasks.assign((size_t)rows + 1, 0);
+  for (int64_t r = 0; r < rows; r++) {
+    const int64_t len = shared ? indptr[1] : indptr[r + 1] - indptr[r];
+    tasks[r + 1] = tasks[r] + ceil_div(len, kCandChunk);
+    if (slabs.empty() || slabs.back().m == kListSlabRows || slabs.back().pairs + len > kCandSlabPairs)
+      slabs.push_back(CandSlab{r, 0, 0, 0});
+    CandSlab &c = slabs.back();
+    c.m++;
+    c.pairs += len;
+    c.max_len = std::max(c.max_len, len);
+  }
+  return slabs;
+}
+
+const int64_t *stage_candidate_tasks(ials_trainer *t, const std::vector<int64_t> &tasks) {
+  int64_t *d = t->cand_tasks.ensure(tasks.size());
+  CUDA_CHECK(cudaMemcpyAsync(d, tasks.data(), sizeof(int64_t) * tasks.size(), cudaMemcpyHostToDevice, t->stream));
+  return d;
+}
+
+int64_t max_slab_pairs(const std::vector<CandSlab> &slabs) {
+  int64_t n = 1;
+  for (const CandSlab &c : slabs) n = std::max(n, c.pairs);
+  return n;
+}
+
+// Checks common to the candidate entry points: the query form (user_idx / user_emb / [begin, end))
+void check_query_form(const ials_trainer *t, const int64_t *user_idx, const float *user_emb, int64_t begin,
+                             int64_t end) {
+  require(t != nullptr, "trainer is null");
+  require(user_idx == nullptr || user_emb == nullptr, "give users by index or embeddings, not both");
+  require(end >= begin && begin >= 0 && (user_idx != nullptr || user_emb != nullptr ? begin == 0 : end <= t->U),
+          "bad user block");
+}
+
+}  // namespace
+
 extern "C" {
 
 int ials_trainer_user_scores(ials_trainer *t, int64_t begin, int64_t end,
@@ -177,49 +306,17 @@ static int recommend_impl(ials_trainer *t, const int64_t *user_idx, const float 
     const int64_t rows = end - begin;
     if (rows == 0) return;
     require(out_idx != nullptr && out_count != nullptr, "output pointer is null");
-    if (mask_mode == 0 && !t->has_X) throw std::runtime_error("no training matrix to mask with");
-    if (mask_mode == 0 && user_idx == nullptr && user_emb == nullptr)  // a sharded trainer only holds its own users' rows of X
-      require(begin >= t->X.row_base && end <= t->X.row_base + t->X.n_rows,
-              "mask='train' on a sharded trainer needs a user block inside the rank's shard");
-    if (user_idx != nullptr)
-      for (int64_t r = 0; r < rows; r++) {
-        require(user_idx[r] >= 0 && user_idx[r] < t->U, "user index out of range");
-        if (mask_mode == 0)
-          require(user_idx[r] >= t->X.row_base && user_idx[r] < t->X.row_base + t->X.n_rows,
-                  "mask='train' on a sharded trainer needs users inside the rank's shard");
-      }
     DeviceGuard g(t->device);
     StreamSyncOnExit sync{t->stream};  // the staging buffers stay with the trainer
-    const int64_t *d_mindptr = nullptr;
-    const int32_t *d_mindices = nullptr;
-    // the fused tensor-core kernel walks each mask row with a cursor: column ids must ascend
-    bool mask_sorted = true;
-    if (mask_mode == 0) {
-      if (t->X.sorted_state < 0)
-        t->X.sorted_state =
-            csr_rows_strictly_sorted(t->X.indptr.get(), t->X.indices.get(), t->X.n_rows, t->stream) ? 1 : 0;
-      mask_sorted = t->X.sorted_state == 1;
-    }
-    if (mask_mode == 2) {
-      stage_mask(rows, t->I, mask_indptr, mask_indices, t->rec_mindptr, t->rec_mindices, t->stream);
-      mask_sorted = mask_rows_sorted(rows, mask_indptr, mask_indices);
-      d_mindptr = t->rec_mindptr.get();
-      d_mindices = t->rec_mindices.get();
-    }
+    ListJob job;
+    stage_queries(t, user_idx, user_emb, begin, rows, mask_mode, mask_indptr, mask_indices, job);
     int32_t *d_idx = t->rec_idx.ensure(rows * k);
     float *d_sc = t->rec_score.ensure(rows * k);
     int32_t *d_cnt = t->rec_count.ensure(rows);
-    ListJob job;
-    job.user_rows = t->factor[0].get() + begin * t->ld;
     job.catalog = t->factor[1].get();
     job.n_catalog = t->I;
     job.rows = rows;
     job.k = k;
-    job.mask_mode = mask_mode;
-    job.x_row0 = begin - t->X.row_base;
-    job.m_indptr = d_mindptr;
-    job.m_indices = d_mindices;
-    job.mask_sorted = mask_sorted;
     job.idx = d_idx;
     job.score = d_sc;
     job.count = d_cnt;
@@ -227,22 +324,6 @@ static int recommend_impl(ials_trainer *t, const int64_t *user_idx, const float 
       require(allow_n_lists == 1 || allow_n_lists == rows, "allow-lists: one shared list or one per row");
       stage_allow_lists(t->I, allow_n_lists, allow_indptr, allow_indices, t->rec_abitmap_host, t->rec_aindptr,
                         t->rec_aindices, t->stream, job);
-    }
-    // users picked by index: their factor rows are gathered into a dense block first
-    if (user_idx != nullptr) {
-      int64_t *d_uidx = t->rec_uidx.ensure(rows);
-      float *gathered = t->rec_users.ensure(rows * t->ld);
-      CUDA_CHECK(cudaMemcpyAsync(d_uidx, user_idx, sizeof(int64_t) * rows, cudaMemcpyHostToDevice, t->stream));
-      launch_gather_rows(t->factor[0].get(), t->ld, d_uidx, rows, gathered, t->stream);
-      job.user_rows = gathered;
-      job.rowmap = d_uidx;
-    }
-    if (user_emb != nullptr) {  // host embeddings [rows x K] -> padded device rows [rows x ld]
-      float *staged = t->rec_emb.ensure(rows * t->K);
-      float *padded = t->rec_users.ensure(rows * t->ld);
-      CUDA_CHECK(cudaMemcpyAsync(staged, user_emb, sizeof(float) * rows * t->K, cudaMemcpyHostToDevice, t->stream));
-      launch_pad_copy(staged, rows, (int)t->K, padded, t->ld, t->stream);
-      job.user_rows = padded;
     }
     produce_lists(t, job);
     download_lists(d_idx, d_sc, d_cnt, rows, k, out_idx, out_score, out_count, t->stream);
@@ -389,6 +470,99 @@ int ials_trainer_similar(ials_trainer *t, int side, const int64_t *query_idx, in
         CUDA_CHECK(cudaMemcpyAsync(out_score + b * k, job.score, sizeof(float) * m * k, cudaMemcpyDeviceToHost,
                                    t->stream));
       CUDA_CHECK(cudaMemcpyAsync(out_count + b, job.count, sizeof(int32_t) * m, cudaMemcpyDeviceToHost, t->stream));
+    }
+    CUDA_CHECK(cudaStreamSynchronize(t->stream));
+  });
+}
+
+int ials_trainer_rank_candidates(ials_trainer *t, const int64_t *user_idx, const float *user_emb, int64_t begin,
+                                 int64_t end, int64_t k, int mask_mode, const int64_t *mask_indptr,
+                                 const int32_t *mask_indices, int64_t cand_n_lists, const int64_t *cand_indptr,
+                                 const int32_t *cand_indices, int32_t *out_idx, float *out_score,
+                                 int32_t *out_count) {
+  return guarded([&] {
+    check_query_form(t, user_idx, user_emb, begin, end);
+    require(user_emb == nullptr || mask_mode != 0, "embeddings have no training rows: give the mask explicitly");
+    require(k >= 1 && k <= t->I, "cutoff must be in [1, n_items]");
+    require(k <= 1024, "k > 1024 is not supported");
+    require(mask_mode >= 0 && mask_mode <= 2, "mask_mode must be 0, 1 or 2");
+    const int64_t rows = end - begin;
+    require(cand_n_lists == 1 || cand_n_lists == rows, "candidates: one shared list or one per row");
+    check_candidates(t->I, cand_n_lists, cand_indptr, cand_indices, true);
+    if (rows == 0) return;
+    require(out_idx != nullptr && out_count != nullptr, "output pointer is null");
+    DeviceGuard g(t->device);
+    StreamSyncOnExit sync{t->stream};  // the staging buffers stay with the trainer
+    ListJob job;
+    stage_queries(t, user_idx, user_emb, begin, rows, mask_mode, mask_indptr, mask_indices, job);
+    const bool shared = cand_n_lists == 1;
+    const CandSegments lists = stage_candidates(t, cand_n_lists, cand_indptr, cand_indices, shared);
+    CandMask mask;
+    mask.sorted = job.mask_sorted;
+    if (mask_mode == 0) {
+      mask.indptr = t->X.indptr.get();
+      mask.indices = t->X.indices.get();
+      mask.data = t->X.data.get();
+    } else if (mask_mode == 2) {
+      mask.indptr = job.m_indptr;
+      mask.indices = job.m_indices;
+    }
+    std::vector<int64_t> tasks;
+    const std::vector<CandSlab> slabs = plan_candidate_slabs(rows, cand_indptr, shared, tasks);
+    const int64_t *d_tasks = stage_candidate_tasks(t, tasks);
+    float *scratch = ensure_score_buf(t, sizeof(float) * max_slab_pairs(slabs));
+    const int64_t slab_rows = std::min(rows, kListSlabRows);
+    int32_t *d_idx = t->rec_idx.ensure(slab_rows * k);
+    float *d_sc = t->rec_score.ensure(slab_rows * k);
+    int32_t *d_cnt = t->rec_count.ensure(slab_rows);
+    for (const CandSlab &c : slabs) {
+      CandSegments seg = lists;
+      if (!shared) { seg.row0 = c.b; seg.base = cand_indptr[c.b]; }
+      CandMask m = mask;
+      if (mask_mode == 0 && job.rowmap != nullptr) { m.rowmap = job.rowmap + c.b; m.row0 = -t->X.row_base; }
+      else if (mask_mode == 0) m.row0 = job.x_row0 + c.b;
+      else if (mask_mode == 2) m.row0 = c.b;
+      launch_cand_scores(job.user_rows + c.b * t->ld, c.m, t->ld, t->factor[1].get(), seg, d_tasks + c.b,
+                         tasks[c.b + c.m] - tasks[c.b], m, scratch, t->stream);
+      launch_topk_segments(scratch, seg, c.m, c.max_len, (int)k, d_idx, d_sc, d_cnt, t->stream);
+      CUDA_CHECK(cudaMemcpyAsync(out_idx + c.b * k, d_idx, sizeof(int32_t) * c.m * k, cudaMemcpyDeviceToHost,
+                                 t->stream));
+      if (out_score)
+        CUDA_CHECK(cudaMemcpyAsync(out_score + c.b * k, d_sc, sizeof(float) * c.m * k, cudaMemcpyDeviceToHost,
+                                   t->stream));
+      CUDA_CHECK(cudaMemcpyAsync(out_count + c.b, d_cnt, sizeof(int32_t) * c.m, cudaMemcpyDeviceToHost, t->stream));
+    }
+    CUDA_CHECK(cudaStreamSynchronize(t->stream));
+  });
+}
+
+int ials_trainer_candidate_scores(ials_trainer *t, const int64_t *user_idx, const float *user_emb, int64_t begin,
+                                  int64_t end, const int64_t *cand_indptr, const int32_t *cand_indices,
+                                  float *out_scores) {
+  return guarded([&] {
+    check_query_form(t, user_idx, user_emb, begin, end);
+    const int64_t rows = end - begin;
+    check_candidates(t->I, rows, cand_indptr, cand_indices, false);
+    if (rows == 0 || cand_indptr[rows] == 0) return;
+    require(out_scores != nullptr, "output pointer is null");
+    DeviceGuard g(t->device);
+    StreamSyncOnExit sync{t->stream};  // the staging buffers stay with the trainer
+    ListJob job;
+    stage_queries(t, user_idx, user_emb, begin, rows, 1, nullptr, nullptr, job);
+    const CandSegments lists = stage_candidates(t, rows, cand_indptr, cand_indices, false);
+    std::vector<int64_t> tasks;
+    const std::vector<CandSlab> slabs = plan_candidate_slabs(rows, cand_indptr, false, tasks);
+    const int64_t *d_tasks = stage_candidate_tasks(t, tasks);
+    float *scratch = ensure_score_buf(t, sizeof(float) * max_slab_pairs(slabs));
+    for (const CandSlab &c : slabs) {
+      CandSegments seg = lists;
+      seg.row0 = c.b;
+      seg.base = cand_indptr[c.b];
+      launch_cand_scores(job.user_rows + c.b * t->ld, c.m, t->ld, t->factor[1].get(), seg, d_tasks + c.b,
+                         tasks[c.b + c.m] - tasks[c.b], CandMask{}, scratch, t->stream);
+      if (c.pairs)
+        CUDA_CHECK(cudaMemcpyAsync(out_scores + seg.base, scratch, sizeof(float) * c.pairs, cudaMemcpyDeviceToHost,
+                                   t->stream));
     }
     CUDA_CHECK(cudaStreamSynchronize(t->stream));
   });

@@ -129,6 +129,20 @@ inline void count_launch(int n = 1) { __atomic_fetch_add(&g_kernel_launches, (in
 __host__ __device__ inline int64_t round_up(int64_t x, int64_t m) { return (x + m - 1) / m * m; }
 __host__ __device__ inline int64_t ceil_div(int64_t x, int64_t m) { return (x + m - 1) / m; }
 
+// Top-k sort key: (order-preserving bits of -score) << 32 | column id, so that ascending keys order
+// by (-score, id) -- the reference's lexicographic pair comparison (evaluator.cpp:324-355)
+__device__ __forceinline__ unsigned long long make_key(float s, uint32_t j) {
+  s += 0.0f;  // -0.0 -> +0.0 so that equal scores compare equal, as floats do
+  const uint32_t b = __float_as_uint(s);
+  const uint32_t asc = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+  return ((unsigned long long)(~asc) << 32) | j;
+}
+__device__ __forceinline__ float key_score(unsigned long long key) {
+  const uint32_t asc = ~(uint32_t)(key >> 32);
+  const uint32_t b = (asc & 0x80000000u) ? (asc & 0x7fffffffu) : ~asc;
+  return __uint_as_float(b);
+}
+
 // Rows of a CSR whose neighbour lists are cut into jobs of <= job_len entries for the tensor-core
 // Gram: the first n_heavy entries of the CSR's `order` (jobs of the h-th: [heavy_first_job[h],
 // heavy_first_job[h + 1]))
@@ -287,6 +301,42 @@ void launch_allow_rows(const float *src, float *dst, int64_t ld, const int64_t *
                        int64_t n_items, cudaStream_t s);
 void launch_topk_rows(const float *scores, int64_t out_ld, int64_t n_rows, int64_t n_items, int k,
                       int32_t *out_idx, float *out_score, int32_t *out_count, cudaStream_t s);
+
+// candidates.cu: caller-given candidate lists, one CSR row of item ids per query row.  Row r of a
+// slab reads list row0 + r (or list 0 for every row when shared_len >= 0) and keeps its scores in a
+// scratch laid out in the same order, from position out(r).
+struct CandSegments {
+  const int64_t *indptr;
+  const int32_t *indices;
+  int64_t row0;        // list of slab row 0 (per-row lists)
+  int64_t base;        // indptr[row0]: scratch position of slab row 0 (per-row lists)
+  int64_t shared_len;  // >= 0: one list of this length shared by every row; -1: one list per row
+  __device__ int64_t begin(int64_t r) const { return shared_len >= 0 ? 0 : indptr[row0 + r]; }
+  __device__ int64_t end(int64_t r) const { return shared_len >= 0 ? shared_len : indptr[row0 + r + 1]; }
+  __device__ int64_t out(int64_t r) const { return shared_len >= 0 ? r * shared_len : indptr[row0 + r] - base; }
+};
+// The items hidden from each query row (indptr == nullptr: none): CSR row row0 + r, or rowmap[r] + row0
+// for users picked by index.  Entries whose data is 0 hide nothing (data may be null).  sorted: column
+// ids strictly ascending in every row (binary search; otherwise the row is scanned).
+struct CandMask {
+  const int64_t *indptr = nullptr;
+  const int32_t *indices = nullptr;
+  const float *data = nullptr;
+  int64_t row0 = 0;
+  const int64_t *rowmap = nullptr;
+  bool sorted = true;
+};
+// scores[out(r) + j] = queries[r] . item[list_r[j]] in FP32, -inf where the mask hides the item.  The work
+// is cut into tasks of kCandChunk candidates of one row: row r owns tasks [tasks[r], tasks[r + 1]) (device,
+// n_rows + 1 entries, ceil(length / kCandChunk) per row; tasks[0] need not be 0), n_tasks in all.
+constexpr int kCandChunk = 256;
+void launch_cand_scores(const float *queries, int64_t n_rows, int ld, const float *item, const CandSegments &seg,
+                        const int64_t *tasks, int64_t n_tasks, const CandMask &mask, float *scores, cudaStream_t s);
+// top-k of each row's segment of `scores` (candidates.cu), ordered by (-score, item id), -inf dropped.
+// max_len, the longest list of the slab, picks the selection: a warp per row up to 256 candidates, a CTA
+// per row above
+void launch_topk_segments(const float *scores, const CandSegments &seg, int64_t n_rows, int64_t max_len, int k,
+                          int32_t *out_idx, float *out_score, int32_t *out_count, cudaStream_t s);
 
 // score_tc.cu: scores + seen mask + top-k fused on tcgen05 (ld a multiple of 32 in [32, 512],
 // k <= 128; mask rows strictly ascending).  The dense score block (launch_scores_tc) takes

@@ -9,9 +9,7 @@
 // CTA-per-row threshold-filter top-k that orders 64-bit keys
 // (order-preserving bits of -score) << 32 | index, i.e. exactly the reference's
 // lexicographic pair comparison.
-#include <cub/block/block_radix_sort.cuh>
-
-#include "common.cuh"
+#include "topk.cuh"
 
 namespace ials {
 namespace {
@@ -118,86 +116,24 @@ __global__ void allow_rows_kernel(const float *__restrict__ src, float *__restri
   }
 }
 
-constexpr int kTkThreads = 256;
-constexpr int kTkItems = 8;
-constexpr int kTkCap = kTkThreads * kTkItems;  // 2048 candidate keys
-constexpr int kTkChunk = 1024;                 // columns scanned between capacity checks
-
-__device__ __forceinline__ unsigned long long make_key(float s, uint32_t j) {
-  s += 0.0f;  // -0.0 -> +0.0 so that equal scores compare equal, as floats do
-  uint32_t b = __float_as_uint(s);
-  uint32_t asc = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-  return ((unsigned long long)(~asc) << 32) | j;
-}
-__device__ __forceinline__ float key_score(unsigned long long key) {
-  uint32_t asc = ~(uint32_t)(key >> 32);
-  uint32_t b = (asc & 0x80000000u) ? (asc & 0x7fffffffu) : ~asc;
-  return __uint_as_float(b);
-}
+// dense score rows: row r is scores[r * out_ld, + n_items), the column id is the position
+struct DenseRows {
+  const float *scores;
+  int64_t out_ld, n_items;
+  struct Row {
+    const float *s;
+    int64_t n;
+    __device__ float score(int64_t j) const { return s[j]; }
+    __device__ uint32_t id(int64_t j) const { return (uint32_t)j; }
+  };
+  __device__ Row row(int64_t r) const { return {scores + r * out_ld, n_items}; }
+};
 
 __global__ void __launch_bounds__(kTkThreads)
 topk_rows_kernel(const float *__restrict__ scores, int64_t out_ld, int64_t n_rows, int64_t n_items,
                  int k, int32_t *__restrict__ out_idx, float *__restrict__ out_score,
                  int32_t *__restrict__ out_count) {
-  using Sort = cub::BlockRadixSort<unsigned long long, kTkThreads, kTkItems>;
-  __shared__ typename Sort::TempStorage sort_tmp;
-  __shared__ unsigned long long buf[kTkCap];
-  __shared__ int cnt;
-  __shared__ unsigned long long tau;
-  const int tid = threadIdx.x;
-
-  auto compact = [&]() {  // sort the candidates, keep the best k, tighten the threshold
-    unsigned long long keys[kTkItems];
-    const int n = cnt;
-#pragma unroll
-    for (int i = 0; i < kTkItems; i++) {
-      const int p = tid * kTkItems + i;
-      keys[i] = p < n ? buf[p] : ~0ull;
-    }
-    __syncthreads();
-    Sort(sort_tmp).Sort(keys);
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < kTkItems; i++) buf[tid * kTkItems + i] = keys[i];
-    __syncthreads();
-    if (tid == 0) {
-      if (n >= k) { cnt = k; tau = buf[k - 1]; }
-    }
-    __syncthreads();
-  };
-
-  for (int64_t row = blockIdx.x; row < n_rows; row += gridDim.x) {
-    __syncthreads();
-    if (tid == 0) { cnt = 0; tau = ~0ull; }
-    __syncthreads();
-    const float *srow = scores + row * out_ld;
-    for (int64_t base = 0; base < n_items; base += kTkChunk) {
-      const unsigned long long t = tau;
-#pragma unroll
-      for (int q = 0; q < kTkChunk / kTkThreads; q++) {
-        const int64_t j = base + tid + q * kTkThreads;
-        if (j < n_items) {
-          const float sc = srow[j];
-          if (sc != -INFINITY) {
-            const unsigned long long key = make_key(sc, (uint32_t)j);
-            if (key < t) buf[atomicAdd(&cnt, 1)] = key;
-          }
-        }
-      }
-      __syncthreads();
-      const int settled = cnt;
-      __syncthreads();  // every thread has read cnt before the next chunk's atomicAdd moves it
-      if (settled > kTkCap - kTkChunk) compact();  // uniform
-    }
-    compact();
-    const int n_out = min(cnt, k);
-    for (int i = tid; i < k; i += kTkThreads) {
-      const bool ok = i < n_out;
-      out_idx[row * k + i] = ok ? (int32_t)(buf[i] & 0xffffffffu) : -1;
-      if (out_score) out_score[row * k + i] = ok ? key_score(buf[i]) : -INFINITY;
-    }
-    if (tid == 0) out_count[row] = n_out;
-  }
+  topk_rows_body(DenseRows{scores, out_ld, n_items}, n_rows, k, out_idx, out_score, out_count);
 }
 
 }  // namespace

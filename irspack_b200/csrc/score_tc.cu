@@ -92,17 +92,6 @@ struct ScoreTcArgs {
   int64_t out_ld;
 };
 
-__device__ __forceinline__ unsigned long long make_key(float s, uint32_t j) {
-  s += 0.0f;  // -0.0 -> +0.0 so that equal scores compare equal, as floats do
-  const uint32_t b = __float_as_uint(s);
-  const uint32_t asc = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-  return ((unsigned long long)(~asc) << 32) | j;
-}
-__device__ __forceinline__ float key_score(unsigned long long key) {
-  const uint32_t asc = ~(uint32_t)(key >> 32);
-  const uint32_t b = (asc & 0x80000000u) ? (asc & 0x7fffffffu) : ~asc;
-  return __uint_as_float(b);
-}
 __device__ __forceinline__ unsigned long long shfl_xor_u64(unsigned long long v, int m) {
   return __shfl_xor_sync(0xffffffffu, v, m);
 }

@@ -38,6 +38,8 @@ struct ials_trainer {
   ials::DeviceBuffer<float> sim_norm;
   ials::DeviceBuffer<int64_t> sim_self_indptr;
   ials::DeviceBuffer<int32_t> sim_self_indices;
+  // candidate ranking (grow-only): the first score task of each query row (launch_cand_scores)
+  ials::DeviceBuffer<int64_t> cand_tasks;
   // shard (multi-GPU): rows owned (solved) by this rank, per side; X / Xt then hold only
   // those rows (DeviceCsr::row_base = shard begin) while both factor matrices are full replicas
   bool sharded = false;

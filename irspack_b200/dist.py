@@ -625,6 +625,14 @@ class ShardedIALSTrainer:
         return self._core._similar(self._handle, self._device, self.n_users if side == 0 else self.n_items, side,
                                    indices, cutoff, metric, exclude_self, forbidden, allowed, return_scores)
 
+    def rank_candidates(self, user_indices: Any, candidates: Any, cutoff: int, mask: Any = "train",
+                        return_scores: bool = True):
+        """``IALSTrainer.rank_candidates`` on this rank's full item replica: rank-local, no collective.
+        ``mask="train"`` needs users of this rank's shard (the rank holds only their training rows);
+        other users take an explicit mask or none."""
+        return self._core._rank_candidates(self._handle, self._device, self.n_users, self.n_items, self.K,
+                                           user_indices, None, candidates, cutoff, mask, return_scores)
+
     def transform_user(self, X: Any, solver_config: Any) -> np.ndarray:
         """Fold-in of new users' rows ``X`` (n x n_items) against this rank's full item replica
         (``IALSTrainer.transform_user``, IALSTrainer.hpp:791-796): rank-local, no collective."""

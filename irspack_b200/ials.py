@@ -404,6 +404,47 @@ class IALSRecommender:
         return self._similar(0, user_indices, cutoff, metric=metric, exclude_self=exclude_self,
                              forbidden=forbidden, allowed=allowed, return_scores=return_scores)
 
+    def _user_index_array(self, user_indices: Any) -> np.ndarray:
+        """Negative and boolean user indices as ``get_score`` takes them."""
+        u = np.asarray(user_indices)
+        if u.dtype == bool:
+            u = np.flatnonzero(u)
+        u = u.astype(np.int64).reshape(-1)
+        return np.where(u < 0, u + self.n_users, u)
+
+    def rank_candidates(self, user_indices: Any, candidates: Any, cutoff: int = 10, mask: Any = "train",
+                        return_scores: bool = True):
+        """B200 extension: the best ``cutoff`` of each user's own candidate items, on the device at a cost
+        that follows the number of (user, candidate) pairs (``IALSTrainer.rank_candidates``).
+        ``candidates``: ``(n_lists, indptr, indices)`` or a sequence of index lists, one shared list or
+        one per user.  Returns (indices, counts[, scores])."""
+        return self.trainer_as_ials.core_trainer.rank_candidates(
+            self._user_index_array(user_indices), candidates, cutoff, mask=mask, return_scores=return_scores)
+
+    def rank_candidates_cold_user(self, X: Any, candidates: Any, cutoff: int = 10, mask: Any = "input",
+                                  return_scores: bool = True):
+        """B200 extension, the cold-user twin of ``rank_candidates``: fold the rows of ``X`` in
+        (``compute_user_embedding``), then rank each row's candidates.  ``mask``: "input" (the entries of
+        ``X`` itself), None, or a sparse matrix with one row per row of ``X``."""
+        if isinstance(mask, str) and mask != "input":
+            raise ValueError("mask must be 'input', None or a sparse matrix")
+        X = sps.csr_matrix(X)
+        core = self.trainer_as_ials.core_trainer
+        emb = (self.compute_user_embedding(X) if X.shape[0] else np.empty((0, core.K), dtype=np.float32))
+        return core.rank_candidates_embeddings(emb, candidates, cutoff, mask=X if isinstance(mask, str) else mask,
+                                               return_scores=return_scores)
+
+    def get_score_pairs(self, user_indices: Any, item_indices: Any) -> np.ndarray:
+        """B200 extension: ``score[u, i]`` for each pair (``user_indices[j]``, ``item_indices[j]``),
+        float32[n], computed on the device for those pairs only."""
+        u = self._user_index_array(user_indices)
+        i = np.asarray(item_indices, dtype=np.int64).reshape(-1)
+        if u.shape != i.shape:
+            raise ValueError("user_indices and item_indices must have the same length")
+        i = np.where(i < 0, i + self.n_items, i)
+        n = u.size
+        return self.trainer_as_ials.core_trainer.candidate_scores(u, (n, np.arange(n + 1, dtype=np.int64), i))
+
     def recommend_cold_block(self, X: Any, cutoff: int, mask: Any = "input", allowed: Any = None,
                              return_scores: bool = False):
         """B200 extension, the cold-user twin of ``recommend_block``: fold the rows of ``X``

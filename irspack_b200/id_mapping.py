@@ -220,6 +220,28 @@ class ItemIDMapper(Generic[ItemIdType]):
             allowed=self._allow_lists(rows, allowed_item_ids, per_item_allowed_item_ids), return_scores=True)
         return self._id_lists(self.item_ids, idx, cnt, sc)
 
+    def _candidate_cutoff(self, cutoff: int, lists: Sequence[Sequence[int]]) -> int:
+        """The cutoff a ranking call needs: no list returns more items than it holds."""
+        return min(int(cutoff), len(self.item_ids), max([len(x) for x in lists] + [1]))
+
+    def rank_items_for_new_user(self, recommender: Any, user_profile: Profile,
+                                candidate_item_ids: List[ItemIdType], cutoff: int = 20,
+                                remove_seen: bool = True) -> List[Tuple[ItemIdType, float]]:
+        """B200 extension: order the items ``candidate_item_ids`` for a user who is not in the model
+        (folded in from ``user_profile``) as [(item id, score)], best first, at most ``cutoff``; ties in
+        ascending index order.  Unknown and repeated candidate ids are ignored; with ``remove_seen`` the
+        profile's items are dropped.  The recommender must provide ``rank_candidates_cold_user`` (an
+        ``IALSRecommender``): there is no host path."""
+        self._check_recommender_n_items(recommender)
+        if not hasattr(recommender, "rank_candidates_cold_user"):
+            raise NotImplementedError("rank_items_for_new_user needs a recommender with rank_candidates_cold_user")
+        X = self.list_of_user_profile_to_matrix([user_profile])
+        lists = [self._item_id_list_to_index_list(candidate_item_ids)]
+        idx, cnt, sc = recommender.rank_candidates_cold_user(
+            X, lists, self._candidate_cutoff(cutoff, lists), mask="input" if remove_seen else None,
+            return_scores=True)
+        return self._id_lists(self.item_ids, idx, cnt, sc)[0]
+
     def recommend_for_new_user(self, recommender: Any, user_profile: Profile, cutoff: int = 20,
                                allowed_item_ids: Optional[List[ItemIdType]] = None,
                                forbidden_item_ids: Optional[List[ItemIdType]] = None
@@ -354,6 +376,28 @@ class IDMapper(Generic[UserIdType, ItemIdType], ItemIDMapper[ItemIdType]):
         score = recommender.get_score_remove_seen(u)
         return self.score_to_recommended_items_batch(
             score, cutoff, allowed_item_ids, per_user_allowed_item_ids, forbidden_item_ids, n_threads)
+
+    def rank_items_for_known_users(self, recommender: Any, user_ids: List[UserIdType],
+                                   candidate_item_ids: List[List[ItemIdType]], cutoff: int = 20,
+                                   remove_seen: bool = True) -> List[List[Tuple[ItemIdType, float]]]:
+        """B200 extension: for each of ``user_ids``, order that user's list in ``candidate_item_ids`` as
+        [(item id, score)], best first, at most ``cutoff``; ties in ascending index order.  Unknown and
+        repeated candidate ids are ignored, an unknown user id raises ``RuntimeError``; with
+        ``remove_seen`` the users' training items are dropped.  The recommender must provide
+        ``rank_candidates`` (an ``IALSRecommender``): there is no host path."""
+        self._check_recommender_n_users(recommender)
+        self._check_recommender_n_items(recommender)
+        if not hasattr(recommender, "rank_candidates"):
+            raise NotImplementedError("rank_items_for_known_users needs a recommender with rank_candidates")
+        u = self._query_indices(self.user_id_to_index, user_ids, "User")
+        if len(candidate_item_ids) != u.size:
+            raise ValueError("candidate_item_ids must hold one list per user")
+        if u.size == 0:
+            return []
+        lists = [self._item_id_list_to_index_list(x) for x in candidate_item_ids]
+        idx, cnt, sc = recommender.rank_candidates(u, lists, self._candidate_cutoff(cutoff, lists),
+                                                   mask="train" if remove_seen else None, return_scores=True)
+        return self._id_lists(self.item_ids, idx, cnt, sc)
 
     def similar_users(self, recommender: Any, user_ids: List[UserIdType], cutoff: int = 20
                       ) -> List[List[Tuple[UserIdType, float]]]:
