@@ -324,6 +324,30 @@ IALS_API int ials_trainer_rank_candidates(ials_trainer *t, const int64_t *user_i
 IALS_API int ials_trainer_candidate_scores(ials_trainer *t, const int64_t *user_idx, const float *user_emb,
                                            int64_t begin, int64_t end, const int64_t *cand_indptr,
                                            const int32_t *cand_indices, float *out_scores);
+/* Explanations (new; Hu, Koren and Volinsky, ICDM 2008, section 5, and `implicit`'s ALS.explain): why a
+ * row of `side` (0: users) scores a target row t of the other side.  With Y the other side's factors,
+ * P = alpha0 Y^T Y (recomputed from Y on every call, into the side's P), the row's history (j, c_j),
+ * reg_u = reg (alpha0 n_other + nnz_u)^nu, bias = alpha0 (ORIGINAL) or 0 (IALSPP) and prior_u the stored
+ * feature prior F W (rows by index past the warm-up epochs only):
+ *   A_u = P + sum_j c_j y_j y_j^T + reg_u I,  x_u = A_u^-1 (sum_j (bias + c_j) y_j + reg_u prior_u),
+ *   w_t = A_u^-1 y_t,  score = y_t . x_u = sum_j (bias + c_j) w_t . y_j + reg_u w_t . prior_u.
+ * Per (query row, target) pair: out_score = y_t . x_u, out_prior (optional) = reg_u w_t . prior_u, and
+ * the best n_top history entries by contribution (bias + c_j) w_t . y_j, ordered by (-contribution,
+ * column id), as column ids (out_idx [pairs x n_top], padded with -1) and contributions (out_contrib,
+ * optional, padded with -inf), out_count = min(n_top, history length).  Every stored entry counts (stored
+ * zeros, repeated columns).  A row with an empty history and no prior gives 0, 0 and count 0.
+ * Queries: query_idx[0 .. end) (host, any order, repeats allowed, begin = 0), or a host CSR of `end` cold
+ * rows hist_indptr / hist_indices / hist_data over the other side's ids (begin = 0, no prior), or, with
+ * all of them null, the rows [begin, end).  On a row-sharded trainer rows by index must be the rank's own.
+ * Targets: a host CSR of one list per query row (any order, repeats allowed, ids in [0, n_other)); the
+ * pairs come out in its order.  1 <= n_top <= 1024.  A failed factorisation raises "Cholesky decomposition
+ * failed." (IALS_ERR_RUNTIME); K > 256 is IALS_ERR_NOT_IMPLEMENTED; every invalid argument is
+ * IALS_ERR_INVALID_ARGUMENT.  The factors do not change. */
+IALS_API int ials_trainer_explain(ials_trainer *t, int side, const int64_t *query_idx, int64_t begin, int64_t end,
+                                  const int64_t *hist_indptr, const int32_t *hist_indices, const float *hist_data,
+                                  const int64_t *target_indptr, const int32_t *target_indices, int64_t n_top,
+                                  float *out_score, float *out_prior, int32_t *out_idx, float *out_contrib,
+                                  int32_t *out_count);
 
 /* Mask + top-`k` for a block of precomputed float32 scores (any recommender;
  * replaces EvaluatorCore::get_metrics_local's selection, evaluator.cpp:324-355,

@@ -16,7 +16,7 @@ import ctypes
 import enum
 import os
 import types
-from typing import Any, Optional, Tuple
+from typing import Any, NamedTuple, Optional, Tuple
 
 import numpy as np
 import scipy.sparse as sps
@@ -459,6 +459,80 @@ def _candidate_scores(handle: ctypes.c_void_p, device: int, n_users: int, n_item
     return out
 
 
+class Explanation(NamedTuple):
+    """Explanations of (query row, target) pairs, pairs in target-list order: the pairs of query row r
+    are ``indptr[r]:indptr[r + 1]``.  Per pair: ``score`` = y_t . x_u, ``prior`` = reg_u w_t . prior_u
+    (0 without a feature prior), the best history entries as column ids ``indices`` [pairs, n_top]
+    (padded with -1) and their ``contributions`` (bias + c_j) w_t . y_j (padded with -inf), ordered by
+    (-contribution, column id), and ``counts`` = min(n_top, history length).  With every entry listed,
+    the contributions plus the prior add up to the score."""
+    indptr: np.ndarray
+    score: np.ndarray
+    prior: np.ndarray
+    indices: np.ndarray
+    contributions: np.ndarray
+    counts: np.ndarray
+
+
+def _target_lists(targets: Any, rows: int, n_other: int) -> Tuple[np.ndarray, np.ndarray]:
+    """``(indptr, indices)`` of one target list per query row, given as a tuple of two arrays
+    ``(indptr, indices)`` or as a sequence of index lists (any order, repeats allowed)."""
+    if isinstance(targets, tuple) and len(targets) == 2 and all(isinstance(x, np.ndarray) for x in targets):
+        ip = np.ascontiguousarray(targets[0], dtype=np.int64).reshape(-1)
+        ix = np.asarray(targets[1]).reshape(-1)
+        if ip.shape != (rows + 1,) or ip[0] != 0 or np.any(np.diff(ip) < 0) or int(ip[-1]) != ix.size:
+            raise ValueError("targets = (indptr[rows + 1], indices[indptr[-1]])")
+    else:
+        lists = [np.asarray(x).reshape(-1) for x in targets]
+        if len(lists) != rows:
+            raise ValueError("targets: one list per query row")
+        ip = np.zeros(rows + 1, dtype=np.int64)
+        np.cumsum([x.size for x in lists], out=ip[1:])
+        ix = np.concatenate([x for x in lists if x.size]) if ip[-1] else np.empty(0, dtype=np.int64)
+    if ix.size and not np.issubdtype(ix.dtype, np.integer):
+        raise ValueError("target ids must be integers")
+    if ix.size and (ix.min() < 0 or ix.max() >= n_other):
+        raise ValueError("target id out of range")
+    return ip, np.ascontiguousarray(ix, dtype=np.int32)
+
+
+def _explain(handle: ctypes.c_void_p, device: int, n_rows: Tuple[int, int], side: int, indices: Any, X: Any,
+             targets: Any, n_top: int) -> Explanation:
+    """``ials_trainer_explain`` of a trainer (or a row-sharded trainer's replicas) on its device's current
+    stream.  Queries: ``indices`` (a step-1 ``range`` or row indices of ``side``) or, when ``X`` is given,
+    its rows as cold histories over the other side (every stored entry counts, as given)."""
+    if side not in (0, 1):
+        raise ValueError("side must be 0 or 1")
+    n_side, n_other = n_rows[side], n_rows[1 - side]
+    n_top = int(n_top)
+    if not 1 <= n_top <= 1024:
+        raise ValueError("n_top must be in [1, 1024]")
+    hi = hx = hd = None
+    if X is None:
+        q, begin, end = _query_block(indices, n_side)
+    else:
+        if not sps.issparse(X):
+            raise TypeError("X must be a scipy sparse matrix")
+        Xc = sps.csr_matrix(X)
+        if Xc.shape[1] != n_other:
+            raise ValueError("X must have one column per row of the other side")
+        hi, hx, hd = _csr_arrays(Xc)
+        q, begin, end = None, 0, Xc.shape[0]
+    rows = end - begin
+    ip, ix = _target_lists(targets, rows, n_other)
+    pairs = ix.size
+    score = np.empty(pairs, dtype=np.float32)
+    prior = np.empty(pairs, dtype=np.float32)
+    idx = np.empty((pairs, n_top), dtype=np.int32)
+    contrib = np.empty((pairs, n_top), dtype=np.float32)
+    cnt = np.empty(pairs, dtype=np.int32)
+    check(lib.ials_trainer_set_stream(handle, ctypes.c_void_p(_stream_of(device))))
+    check(lib.ials_trainer_explain(handle, side, _ptr(q), begin, end, _ptr(hi), _ptr(hx), _ptr(hd), _ptr(ip),
+                                   _ptr(ix), n_top, _ptr(score), _ptr(prior), _ptr(idx), _ptr(contrib),
+                                   _ptr(cnt)))
+    return Explanation(ip, score, prior, idx, contrib, cnt)
+
+
 def _factors_device(handle: ctypes.c_void_p, side: int, device: int) -> Any:
     """Zero-copy view ([n, K], row stride ld) of a trainer's factor matrix (or replica) of ``side``."""
     import torch
@@ -836,6 +910,24 @@ class IALSTrainer:
         """The score of every (user, candidate) pair, float32, in the order of the candidate lists
         (any order, repeats allowed; a shared list counts once per user)."""
         return _candidate_scores(self._handle, self._device, self.n_users, self.n_items, user_indices, candidates)
+
+    def explain(self, side: int, indices: Any, targets: Any, n_top: int = 10) -> Explanation:
+        """Why rows of ``side`` (0: users) score their targets (rows of the other side): each score split
+        into the contributions of the row's training history, exactly (Hu, Koren and Volinsky, ICDM 2008,
+        section 5; ``implicit``'s ``ALS.explain``), solved on the device against the current factors.
+
+        ``indices``: a ``range`` of step 1 or row indices (any order, repeats allowed).  ``targets``: one
+        list of target ids per query row, as a sequence of lists or ``(indptr, indices)`` arrays.
+        ``1 <= n_top <= 1024`` history entries are kept per pair.  Past the feature warm-up the stored
+        feature prior enters as ``prior``.  The factors do not change."""
+        return _explain(self._handle, self._device, (self.n_users, self.n_items), side, indices, None, targets,
+                        n_top)
+
+    def explain_history(self, side: int, X: Any, targets: Any, n_top: int = 10) -> Explanation:
+        """``explain`` for rows that are not in the model: the rows of the sparse matrix ``X`` (one column
+        per row of the other side) are the histories, every stored entry counting as given (zeros and
+        repeated columns included), without a feature prior."""
+        return _explain(self._handle, self._device, (self.n_users, self.n_items), side, None, X, targets, n_top)
 
     def get_factors_into(self, side: int, out: np.ndarray) -> None:
         """Device -> host copy into a caller-owned (e.g. pinned) C-contiguous buffer."""

@@ -84,6 +84,7 @@ def _load() -> ctypes.CDLL:
         "ials_trainer_similar": (c_int, [H, c_int, c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
         "ials_trainer_rank_candidates": (c_int, [H, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
         "ials_trainer_candidate_scores": (c_int, [H, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
+        "ials_trainer_explain": (c_int, [H, c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
         "ials_metrics_accumulate": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
         "ials_eval_set_create": (c_int, [H, c_int64, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int, POINTER(H)]),
         "ials_eval_set_destroy": (None, [H]),

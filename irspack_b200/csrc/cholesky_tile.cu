@@ -34,6 +34,13 @@
 // right-hand side is  P[d0:d0+S, :] x + reg x_S + sum (c (pred - 1) - bias) y_S,  the solution is
 // SUBTRACTED from x_S and from the cached predictions of the row's entries (:499-508).
 // ialspp_predict_kernel is Solver::_prediction (:387-424).
+//
+// The EXPLAIN instantiation splits scores into the contributions of the row's history (Hu, Koren and
+// Volinsky, ICDM 2008, section 5): it forms and factors A_u exactly as MODE 0, keeps the factor in
+// shared memory and, for each target t of the row, solves A_u w_t = y_t (one warp per target, the
+// lane-register layout of the backward substitution below, up to kStage targets at a time in V).
+// The history rows are then read once per group of targets:  score(u, t) = y_t . x_u
+// = sum_j (bias + c_j) w_t . y_j + reg_u w_t . prior_u.
 #include "common.cuh"
 
 namespace ials {
@@ -75,12 +82,13 @@ __host__ __device__ inline size_t tile_smem_floats(int kd) {
   return packed + (size_t)kStage * pad8(kd) + 8 * (size_t)pad8(kd) + 64 + 3 * (size_t)kd + 2 * kStage;
 }
 
-// MODE 0: Solver::step_cholesky; 1 (SUB): the iALS++ block.  (256-column factors take the
-// tensor-core Gram + cholesky_ll.cu instead; this kernel stays their fallback for rows with negative
-// stored values and for IALS_CHOL=simt.)
+// MODE 0: Solver::step_cholesky; 1 (SUB): the iALS++ block; 2 (EXPLAIN): explanations, see the
+// header.  (256-column factors take the tensor-core Gram + cholesky_ll.cu instead; this kernel stays
+// their fallback for rows with negative stored values and for IALS_CHOL=simt.)
 template <int MODE>
 __global__ void __launch_bounds__(kMaxThreads, 1) cholesky_tile_kernel(SolveArgs a, SubspaceArgs sub) {
   constexpr bool SUB = MODE == 1;
+  constexpr bool EXPLAIN = MODE == 2;
   extern __shared__ __align__(16) float smem[];
   const int ld = a.ld;
   const int K = SUB ? sub.S : a.K;   // order of the system
@@ -133,6 +141,13 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cholesky_tile_kernel(SolveArgs
     const int64_t nnz = e - s;
     const float reg_u = a.reg * powf(a.alpha0 * (float)a.n_other + (float)nnz, a.nu);  // :309-310
     const float *xrow = a.target + gu * ld;
+    if (EXPLAIN && nnz == 0 && a.prior == nullptr) {  // x = 0 (cg_warp_kernel's), nothing to solve
+      for (int64_t p = sub.pair_ptr[slot] + tid; p < sub.pair_ptr[slot + 1]; p += n_threads) {
+        sub.score[p] = 0.f;
+        if (sub.prior) sub.prior[p] = 0.f;
+      }
+      continue;
+    }
 
     // acc <- P tile, b <- 0                                        (:296-299)
     float2 acc[8][4];
@@ -376,13 +391,13 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cholesky_tile_kernel(SolveArgs
       if (tid == 0) atomicExch(&a.err_flags[kErrCholSolve], 1);
       continue;
     }
-    if (!SUB) {
+    if (MODE == 0) {
       for (int k = tid; k < ld; k += n_threads) {
         const float v = k < K ? sm.x[k] : 0.f;
         a.target[gu * ld + k] = v;
         for (int pi = 0; pi < a.n_peers; pi++) a.peers[pi][gu * ld + k] = v;
       }
-    } else {  // x_S -= delta, pred -= delta . y_S  (:499-508)
+    } else if (SUB) {  // x_S -= delta, pred -= delta . y_S  (:499-508)
       for (int k = tid; k < K; k += n_threads) {
         const float v = xrow[d0 + k] - sm.x[k];
         a.target[gu * ld + d0 + k] = v;
@@ -395,6 +410,100 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cholesky_tile_kernel(SolveArgs
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
         if (lane == 0) sub.pred[j] -= part;
+      }
+    } else {  // EXPLAIN
+      constexpr int NX = 8;
+      const unsigned full = 0xffffffffu;
+      const float *prior_u = a.prior ? a.prior + gu * ld : nullptr;
+      const int64_t p0 = sub.pair_ptr[slot], p1 = sub.pair_ptr[slot + 1];
+      for (int64_t g0 = p0; g0 < p1; g0 += kStage) {
+        const int m = (int)min((int64_t)kStage, p1 - g0);
+        __syncthreads();  // V is free: the rank updates (or the previous group) are done with it
+        // w_t = A^-1 y_t by warp, t < m:  U^T D^-1 z = y  (z_c -= a_ic z_i / a_ii, the forward
+        // substitution of the factorisation), then U w = z as the backward substitution above
+        for (int t = warp; t < m; t += n_warps) {
+          const float *y = a.other + (int64_t)sub.targets[g0 + t] * ld;
+          float zr[NX];  // z, then w from the back: w_c for c > i, z_c for c <= i at pivot i
+#pragma unroll
+          for (int j = 0; j < NX; j++) {
+            const int c = lane + 32 * j;
+            zr[j] = c < K ? y[c] : 0.f;
+          }
+#pragma unroll
+          for (int jb = 0; jb < NX; jb++) {
+            for (int il = 0; il < kWarp && 32 * jb + il < K; il++) {
+              const int i = 32 * jb + il;
+              const float zi = __shfl_sync(full, zr[jb], il) * sm.dinv[i];
+              const float *Ui = sm.U + packed_row(i, kd) - i;
+#pragma unroll
+              for (int j = jb; j < NX; j++) {
+                const int c = lane + 32 * j;
+                if (c > i && c < K) zr[j] = fmaf(-Ui[c], zi, zr[j]);
+              }
+            }
+          }
+#pragma unroll
+          for (int jb = NX - 1; jb >= 0; jb--) {
+            for (int il = min(kWarp, K - 32 * jb) - 1; il >= 0; il--) {
+              const int i = 32 * jb + il;
+              const float *Ui = sm.U + packed_row(i, kd) - i;
+              float part = 0.f;
+#pragma unroll
+              for (int j = jb; j < NX; j++) {
+                const int c = lane + 32 * j;
+                if (c > i && c < K) part = fmaf(Ui[c], zr[j], part);
+              }
+#pragma unroll
+              for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(full, part, o);
+              const float wi = (__shfl_sync(full, zr[jb], il) - part) * sm.dinv[i];
+              zr[jb] = lane == il ? wi : zr[jb];
+            }
+          }
+#pragma unroll
+          for (int j = 0; j < NX; j++) {  // V[c][t] (kStage x kd floats of the kStage x kp)
+            const int c = lane + 32 * j;
+            if (c < kd) sm.V[c * kStage + t] = zr[j];
+          }
+        }
+        __syncthreads();
+        // one warp per history entry j, lane t forms w_t . y_j: y_j is read once per group of targets
+        // (the same address in every lane), the columns of V without bank conflicts
+        for (int64_t j = s + warp; j < e; j += n_warps) {
+          const int32_t col = a.indices[j];
+          const float4 *y = reinterpret_cast<const float4 *>(a.other + (int64_t)col * ld);
+          const float *v = sm.V + lane;
+          float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f;
+          for (int c = 0; c < kd; c += 4, v += 4 * kStage) {  // w_t is 0 in the columns [K, kd)
+            const float4 yc = __ldg(y + c / 4);
+            d0 = fmaf(yc.x, v[0], d0);
+            d1 = fmaf(yc.y, v[kStage], d1);
+            d2 = fmaf(yc.z, v[2 * kStage], d2);
+            d3 = fmaf(yc.w, v[3 * kStage], d3);
+          }
+          if (lane < m) {
+            const int64_t o = sub.contrib_ptr[g0 + lane] + (j - s);
+            sub.contrib[o] = (a.bias + a.data[j]) * ((d0 + d1) + (d2 + d3));
+            sub.contrib_idx[o] = col;
+          }
+        }
+        // score_t = y_t . x (computed apart from the contributions), prior_t = reg_u w_t . prior_u
+        for (int t = warp; t < m; t += n_warps) {
+          const float *y = a.other + (int64_t)sub.targets[g0 + t] * ld;
+          float sc = 0.f, pr = 0.f;
+          for (int c = lane; c < K; c += kWarp) {
+            sc = fmaf(y[c], sm.x[c], sc);
+            if (prior_u) pr = fmaf(sm.V[c * kStage + t], prior_u[c], pr);
+          }
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) {
+            sc += __shfl_xor_sync(full, sc, o);
+            pr += __shfl_xor_sync(full, pr, o);
+          }
+          if (lane == 0) {
+            sub.score[g0 + t] = sc;
+            if (sub.prior) sub.prior[g0 + t] = prior_u ? reg_u * pr : 0.f;
+          }
+        }
       }
     }
   }
@@ -482,6 +591,12 @@ void launch_ialspp_predict(const SolveArgs &a, float *pred, cudaStream_t s) {
 }
 
 bool ialspp_block_supported(int S) { return S >= 1 && tile_kd_supported((S + 7) & ~7); }
+
+void launch_explain_tile(const SolveArgs &a, const SubspaceArgs &ex, cudaStream_t s) {
+  if (a.n_sched <= 0) return;
+  if (!cholesky_tile_supported(a)) throw NotImplemented("explanations: n_components > 256 not supported");
+  launch_tile<2>(a, ex, tile_system_kd(a, -1), s);
+}
 
 void launch_ialspp_block(const SolveArgs &a, float *pred, int d0, int S, cudaStream_t s) {
   if (a.n_sched <= 0) return;

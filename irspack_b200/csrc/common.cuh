@@ -222,6 +222,17 @@ __device__ __forceinline__ void wait_row_ready(const SolveArgs &a, int64_t gu) {
 struct SubspaceArgs {
   float *pred;
   int d0, S;
+  // Explanations (cholesky_tile.cu, EXPLAIN instantiation; null in the others, whose parameter
+  // offsets stay where they were because these follow): the scheduled slot s explains the pairs
+  // [pair_ptr[s], pair_ptr[s + 1]) of its row, pair p against the row `targets[p]` of `other`;
+  // score[p] = y_t . x_u, prior[p] = reg_u w_t . prior_u (optional), and the contribution
+  // (bias + c_j) w_t . y_j of the row's j-th history entry goes to contrib[contrib_ptr[p] + j]
+  // with its column id in contrib_idx, where w_t = A_u^-1 y_t.  Pair indices are slab-local.
+  const int64_t *pair_ptr;
+  const int32_t *targets;
+  const int64_t *contrib_ptr;
+  float *score, *prior, *contrib;
+  int32_t *contrib_idx;
 };
 
 // Arguments of the tensor-core weighted Gram (wgram.cu).  Job j accumulates the entries
@@ -289,6 +300,10 @@ void launch_solve_cholesky_tile(const SolveArgs &a, cudaStream_t s);  // registe
 void launch_ialspp_predict(const SolveArgs &a, float *pred, cudaStream_t s);
 bool ialspp_block_supported(int S);
 void launch_ialspp_block(const SolveArgs &a, float *pred, int d0, int S, cudaStream_t s);
+// Explanations of scheduled rows (cholesky_tile.cu): `a` as for launch_solve_cholesky_tile (P, the
+// history CSR, order = the rows to explain, prior), nothing written to a.target; `ex` as in SubspaceArgs.
+// A row without history and without a prior is not solved: its scores and priors are 0.
+void launch_explain_tile(const SolveArgs &a, const SubspaceArgs &ex, cudaStream_t s);
 
 void launch_scores(const float *user_rows, int64_t n_rows, const float *item, int64_t n_items,
                    int ld, float *out, int64_t out_ld, cudaStream_t s);

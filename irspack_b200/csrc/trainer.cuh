@@ -40,6 +40,13 @@ struct ials_trainer {
   ials::DeviceBuffer<int32_t> sim_self_indices;
   // candidate ranking (grow-only): the first score task of each query row (launch_cand_scores)
   ials::DeviceBuffer<int64_t> cand_tasks;
+  // explanations (grow-only): the schedule, slot -> pair and pair -> contribution offsets, targets, cold
+  // rows, and per slab the pair scores / priors and the contribution scratch; host copies of the indptr
+  // of X and Xt, made on first use (the training matrices never change)
+  ials::DeviceBuffer<int64_t> expl_offsets, expl_hist_indptr;
+  ials::DeviceBuffer<int32_t> expl_rows, expl_targets, expl_hist_indices, expl_contrib_idx;
+  ials::DeviceBuffer<float> expl_hist_data, expl_pair_out, expl_contrib;
+  std::vector<int64_t> indptr_host[2];
   // shard (multi-GPU): rows owned (solved) by this rank, per side; X / Xt then hold only
   // those rows (DeviceCsr::row_base = shard begin) while both factor matrices are full replicas
   bool sharded = false;

@@ -633,6 +633,17 @@ class ShardedIALSTrainer:
         return self._core._rank_candidates(self._handle, self._device, self.n_users, self.n_items, self.K,
                                            user_indices, None, candidates, cutoff, mask, return_scores)
 
+    def explain(self, side: int, indices: Any, targets: Any, n_top: int = 10) -> Any:
+        """``IALSTrainer.explain`` on this rank's replicas: rank-local, no collective.  Rows by index must
+        be this rank's own rows of ``side`` (the rank holds only their histories)."""
+        return self._core._explain(self._handle, self._device, (self.n_users, self.n_items), side, indices, None,
+                                   targets, n_top)
+
+    def explain_history(self, side: int, X: Any, targets: Any, n_top: int = 10) -> Any:
+        """``IALSTrainer.explain_history`` on this rank's replicas (any cold rows): rank-local."""
+        return self._core._explain(self._handle, self._device, (self.n_users, self.n_items), side, None, X,
+                                   targets, n_top)
+
     def transform_user(self, X: Any, solver_config: Any) -> np.ndarray:
         """Fold-in of new users' rows ``X`` (n x n_items) against this rank's full item replica
         (``IALSTrainer.transform_user``, IALSTrainer.hpp:791-796): rank-local, no collective."""

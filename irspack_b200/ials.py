@@ -445,6 +445,19 @@ class IALSRecommender:
         n = u.size
         return self.trainer_as_ials.core_trainer.candidate_scores(u, (n, np.arange(n + 1, dtype=np.int64), i))
 
+    def explain(self, user_indices: Any, item_lists: Any, n_top: int = 10) -> Any:
+        """B200 extension: why each user scores the items of their list, as the contributions of the
+        user's training items to each score (``IALSTrainer.explain``; indices as ``get_score`` takes
+        them).  ``item_lists``: one list of item indices per user.  Returns an ``Explanation``."""
+        return self.trainer_as_ials.core_trainer.explain(0, self._user_index_array(user_indices), item_lists,
+                                                         n_top)
+
+    def explain_cold_user(self, X: Any, item_lists: Any, n_top: int = 10) -> Any:
+        """B200 extension, the cold-user twin of ``explain``: the rows of ``X`` are histories of users
+        who are not in the model, scaled as ``compute_user_embedding`` scales them."""
+        X = self._scale_X(sps.csr_matrix(X).astype(np.float32), self.confidence_scaling, self.epsilon)
+        return self.trainer_as_ials.core_trainer.explain_history(0, X, item_lists, n_top)
+
     def recommend_cold_block(self, X: Any, cutoff: int, mask: Any = "input", allowed: Any = None,
                              return_scores: bool = False):
         """B200 extension, the cold-user twin of ``recommend_block``: fold the rows of ``X``

@@ -242,6 +242,32 @@ class ItemIDMapper(Generic[ItemIdType]):
             return_scores=True)
         return self._id_lists(self.item_ids, idx, cnt, sc)[0]
 
+    def _explanations(self, e: Any, rows: int, lists: Sequence[Sequence[int]]
+                      ) -> List[List[Tuple[ItemIdType, float, List[Tuple[ItemIdType, float]]]]]:
+        """Per query row, per target: (item id, score, [(history item id, contribution), ...])."""
+        ids = self.item_ids
+        out = []
+        for r in range(rows):
+            row = []
+            for p in range(int(e.indptr[r]), int(e.indptr[r + 1])):
+                because = [(ids[int(e.indices[p, k])], float(e.contributions[p, k])) for k in range(int(e.counts[p]))]
+                row.append((ids[lists[r][p - int(e.indptr[r])]], float(e.score[p]), because))
+            out.append(row)
+        return out
+
+    def explain_for_new_user(self, recommender: Any, user_profile: Profile, item_ids: List[ItemIdType],
+                             n_top: int = 10) -> List[Tuple[ItemIdType, float, List[Tuple[ItemIdType, float]]]]:
+        """B200 extension: why a user who is not in the model (``user_profile``) scores each of
+        ``item_ids``: [(item id, score, [(history item id, contribution), ...])], the ``n_top`` largest
+        contributions first.  Unknown item and profile ids are ignored.  The recommender must provide
+        ``explain_cold_user`` (an ``IALSRecommender``): there is no host path."""
+        self._check_recommender_n_items(recommender)
+        if not hasattr(recommender, "explain_cold_user"):
+            raise NotImplementedError("explain_for_new_user needs a recommender with explain_cold_user")
+        X = self.list_of_user_profile_to_matrix([user_profile])
+        lists = [self._item_id_list_to_index_list(item_ids)]
+        return self._explanations(recommender.explain_cold_user(X, lists, n_top=n_top), 1, lists)[0]
+
     def recommend_for_new_user(self, recommender: Any, user_profile: Profile, cutoff: int = 20,
                                allowed_item_ids: Optional[List[ItemIdType]] = None,
                                forbidden_item_ids: Optional[List[ItemIdType]] = None
@@ -398,6 +424,26 @@ class IDMapper(Generic[UserIdType, ItemIdType], ItemIDMapper[ItemIdType]):
         idx, cnt, sc = recommender.rank_candidates(u, lists, self._candidate_cutoff(cutoff, lists),
                                                    mask="train" if remove_seen else None, return_scores=True)
         return self._id_lists(self.item_ids, idx, cnt, sc)
+
+    def explain_for_known_users(self, recommender: Any, user_ids: List[UserIdType],
+                                item_ids_per_user: List[List[ItemIdType]], n_top: int = 10
+                                ) -> List[List[Tuple[ItemIdType, float, List[Tuple[ItemIdType, float]]]]]:
+        """B200 extension: for each of ``user_ids``, why that user scores each item of their list in
+        ``item_ids_per_user``: [(item id, score, [(history item id, contribution), ...])], the ``n_top``
+        largest contributions of the user's training items first.  Unknown item ids are ignored, an
+        unknown user id raises ``RuntimeError``.  The recommender must provide ``explain`` (an
+        ``IALSRecommender``): there is no host path."""
+        self._check_recommender_n_users(recommender)
+        self._check_recommender_n_items(recommender)
+        if not hasattr(recommender, "explain"):
+            raise NotImplementedError("explain_for_known_users needs a recommender with explain")
+        u = self._query_indices(self.user_id_to_index, user_ids, "User")
+        if len(item_ids_per_user) != u.size:
+            raise ValueError("item_ids_per_user must hold one list per user")
+        if u.size == 0:
+            return []
+        lists = [self._item_id_list_to_index_list(x) for x in item_ids_per_user]
+        return self._explanations(recommender.explain(u, lists, n_top=n_top), u.size, lists)
 
     def similar_users(self, recommender: Any, user_ids: List[UserIdType], cutoff: int = 20
                       ) -> List[List[Tuple[UserIdType, float]]]:
