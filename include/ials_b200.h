@@ -464,6 +464,17 @@ IALS_API int ials_weighted_gram256(const float *Y_host, int64_t n, int64_t K, co
                           const float *w_host, int64_t m, int64_t n_jobs, float bias, int device,
                           float *G_host, float *b_host);
 
+/* Both operators job by job (K <= 256): job j sums the entries [job_begin[j], job_end[j]) of
+ * (idx, w) -- of the rows of Y when idx is NULL (m ignored) -- in one launch of the K <= 128
+ * kernel (row stride 128) or of the 256-column one (128 < K <= 256), and returns its own block
+ *   G_jobs[j][K*K] = W_j + W_j^T,   b_jobs[j][K] = sum_{t in job j} (bias + w[t]) * y_{idx[t]}
+ * Any bounds with 0 <= begin <= end <= m are accepted: empty, overlapping or out-of-order jobs.
+ * n_jobs <= 4096 (K <= 128) or 1024 (K > 128); m <= 2^31 - 64; b_jobs may be NULL. */
+IALS_API int ials_weighted_gram_jobs(const float *Y_host, int64_t n, int64_t K, const int32_t *idx_host,
+                            const float *w_host, int64_t m, const int64_t *job_begin,
+                            const int64_t *job_end, int64_t n_jobs, float bias, int device,
+                            float *G_jobs, float *b_jobs);
+
 /* Device-side phase timing.  When enabled, every epoch enqueued by
  * ials_trainer_step[_async] records CUDA events (on the trainer's stream)
  * around its phases.  ials_trainer_get_timings synchronises, adds up the elapsed

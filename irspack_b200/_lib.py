@@ -98,6 +98,7 @@ def _load() -> ctypes.CDLL:
         "ials_retrieve_recommend": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
         "ials_weighted_gram": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_float, c_int, c_void_p, c_void_p]),
         "ials_weighted_gram256": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_float, c_int, c_void_p, c_void_p]),
+        "ials_weighted_gram_jobs": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_float, c_int, c_void_p, c_void_p]),
         "ials_trainer_set_profiling": (c_int, [H, c_int]),
         "ials_trainer_get_timings": (c_int, [H, POINTER(ctypes.c_double), POINTER(c_int64)]),
         "ials_trainer_plan_stats": (c_int, [H, c_int, POINTER(c_int64)]),

@@ -2,6 +2,7 @@
 // replaces irspack's `_ials_core.IALSTrainer`
 // (/root/reference/cpp_source/als/IALSTrainer.hpp:709-984, wrapper.cpp:130-181).
 #include <algorithm>
+#include <cerrno>
 #include <cmath>
 #include <cstdlib>
 #include <random>
@@ -118,12 +119,22 @@ int64_t env_int(const char *name, int64_t dflt) {
   const char *e = std::getenv(name);
   return e != nullptr && *e ? std::atoll(e) : dflt;
 }
+// A job length of 0 would divide by zero when the plan cuts a row, and a negative one never ends it.
+int64_t heavy_job_len() {
+  const char *e = std::getenv("IALS_HEAVY_JOB_LEN");
+  if (e == nullptr || !*e) return 4096;
+  char *end = nullptr;
+  errno = 0;
+  const long long v = std::strtoll(e, &end, 10);
+  require(*end == '\0' && errno == 0 && v >= 1, "IALS_HEAVY_JOB_LEN must be a positive integer");
+  return v;
+}
 void plan_csr(ials_trainer *t, DeviceCsr &csr) {
   build_row_order(csr, t->stream);
   csr.has_negative = csr_has_negative(csr, t->stream);
   if (t->ld == 128) {
     const int64_t heavy = std::max<int64_t>(env_int("IALS_HEAVY_THRESHOLD", 2048), 1);
-    build_heavy_plan(csr, heavy, env_int("IALS_HEAVY_JOB_LEN", 4096), csr.heavy, t->stream);
+    build_heavy_plan(csr, heavy, heavy_job_len(), csr.heavy, t->stream);
   }
 }
 
@@ -140,7 +151,9 @@ void upload_csr(DeviceCsr &d, int64_t n_rows, int64_t n_cols, const int64_t *ind
     for (int64_t r = 0; r < n_rows; r++) require(indptr[r + 1] >= indptr[r], "indptr must be non-decreasing");
     nnz = indptr[n_rows];
   }
-  require(nnz < (1ll << 31), "nnz must fit int32 (as in the reference's Eigen StorageIndex)");
+  require(nnz <= kMaxGramEntries,
+          "nnz must be at most 2^31 - 64 (int32 offsets, as in the reference's Eigen StorageIndex, with room for "
+          "the tensor-core Gram's last pipeline stage)");
   require(nnz == 0 || (indices != nullptr && data != nullptr), "indices/data are null");
   if (!on_device)
     for (int64_t j = 0; j < nnz; j++)

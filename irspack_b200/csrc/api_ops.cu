@@ -9,13 +9,14 @@ using namespace ials;
 namespace {
 
 // The entries of a weighted Gram operator on the device: gathered row ids (optional), weights
-// (optional) and an even split of the m entries into n_jobs jobs.
+// (optional) and the job bounds.
 struct GramEntries {
   DeviceBuffer<int32_t> idx;
   DeviceBuffer<float> w;
   DeviceBuffer<int64_t> job_begin, job_end;
 
-  void upload(const int32_t *idx_host, const float *w_host, int64_t m, int64_t n_jobs) {
+  void upload(const int32_t *idx_host, const float *w_host, int64_t m, const int64_t *jb, const int64_t *je,
+              int64_t n_jobs) {
     if (idx_host) {
       idx.alloc(std::max<int64_t>(m, 1));
       CUDA_CHECK(cudaMemcpy(idx.get(), idx_host, sizeof(int32_t) * m, cudaMemcpyHostToDevice));
@@ -24,16 +25,21 @@ struct GramEntries {
       w.alloc(std::max<int64_t>(m, 1));
       CUDA_CHECK(cudaMemcpy(w.get(), w_host, sizeof(float) * m, cudaMemcpyHostToDevice));
     }
+    job_begin.alloc(n_jobs);
+    job_end.alloc(n_jobs);
+    CUDA_CHECK(cudaMemcpy(job_begin.get(), jb, sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(job_end.get(), je, sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
+  }
+
+  // An even split of the m entries into n_jobs jobs.
+  void upload_even(const int32_t *idx_host, const float *w_host, int64_t m, int64_t n_jobs) {
     std::vector<int64_t> jb(n_jobs), je(n_jobs);
     const int64_t per = (m + n_jobs - 1) / n_jobs;
     for (int64_t j = 0; j < n_jobs; j++) {
       jb[j] = std::min(j * per, m);
       je[j] = std::min(jb[j] + per, m);
     }
-    job_begin.alloc(n_jobs);
-    job_end.alloc(n_jobs);
-    CUDA_CHECK(cudaMemcpy(job_begin.get(), jb.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
-    CUDA_CHECK(cudaMemcpy(job_end.get(), je.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice));
+    upload(idx_host, w_host, m, jb.data(), je.data(), n_jobs);
   }
 
   WGramArgs args(float bias) const {
@@ -47,6 +53,14 @@ struct GramEntries {
     return a;
   }
 };
+
+void check_entries(int64_t n, const int32_t *idx_host, const float *w_host, int64_t m) {
+  require(m >= 0 && m <= kMaxGramEntries, "m must be in [0, 2^31 - 64]");
+  if (idx_host)
+    for (int64_t i = 0; i < m; i++) require(idx_host[i] >= 0 && idx_host[i] < n, "index out of range");
+  if (w_host)
+    for (int64_t i = 0; i < m; i++) require(w_host[i] >= 0.f, "weights must be non-negative");
+}
 
 }  // namespace
 
@@ -63,11 +77,7 @@ int ials_weighted_gram(const float *Y_host, int64_t n, int64_t K, const int32_t 
     require(n_jobs >= 1 && n_jobs <= 4096, "n_jobs must be in [1, 4096]");
     const bool gathered = idx_host != nullptr;
     if (!gathered) m = n;
-    require(m >= 0, "negative length");
-    if (gathered)
-      for (int64_t i = 0; i < m; i++) require(idx_host[i] >= 0 && idx_host[i] < n, "index out of range");
-    if (w_host)
-      for (int64_t i = 0; i < m; i++) require(w_host[i] >= 0.f, "weights must be non-negative");
+    check_entries(n, idx_host, w_host, m);
     require_device(device);
     DeviceGuard g(device);
     const int ld = 128;
@@ -79,7 +89,7 @@ int ials_weighted_gram(const float *Y_host, int64_t n, int64_t K, const int32_t 
     d_Y.alloc(std::max<int64_t>(n * ld, 1));
     CUDA_CHECK(cudaMemcpy(d_tmp.get(), Y_host, sizeof(float) * n * K, cudaMemcpyHostToDevice));
     launch_pad_copy(d_tmp.get(), n, (int)K, d_Y.get(), ld, s);
-    entries.upload(gathered ? idx_host : nullptr, w_host, m, n_jobs);
+    entries.upload_even(gathered ? idx_host : nullptr, w_host, m, n_jobs);
     WGramArgs a = entries.args(bias);
     a.Y = d_Y.get();
     a.ld = ld;
@@ -112,10 +122,8 @@ int ials_weighted_gram256(const float *Y_host, int64_t n, int64_t K, const int32
   return guarded([&] {
     require(Y_host != nullptr && G_host != nullptr && idx_host != nullptr, "null pointer");
     require(n >= 1 && K > 128 && K <= 256, "K must be in (128, 256]");
-    require(n_jobs >= 1 && n_jobs <= 1024 && m >= 0, "n_jobs must be in [1, 1024]");
-    for (int64_t i = 0; i < m; i++) require(idx_host[i] >= 0 && idx_host[i] < n, "index out of range");
-    if (w_host)
-      for (int64_t i = 0; i < m; i++) require(w_host[i] >= 0.f, "weights must be non-negative");
+    require(n_jobs >= 1 && n_jobs <= 1024, "n_jobs must be in [1, 1024]");
+    check_entries(n, idx_host, w_host, m);
     require_device(device);
     DeviceGuard g(device);
     const int ld = 256;
@@ -126,7 +134,7 @@ int ials_weighted_gram256(const float *Y_host, int64_t n, int64_t K, const int32
     DeviceSyncOnExit sync;
     CUDA_CHECK(cudaMemset(d_Y.alloc(n * ld), 0, sizeof(float) * n * ld));
     rows_to_device(d_Y.get(), ld, Y_host, K, n);
-    entries.upload(idx_host, w_host, m, n_jobs);
+    entries.upload_even(idx_host, w_host, m, n_jobs);
     WGramArgs a = entries.args(bias);
     a.ld = ld;
     a.Y = d_Y.get();
@@ -150,6 +158,64 @@ int ials_weighted_gram256(const float *Y_host, int64_t n, int64_t K, const int32
         for (int64_t q = 0; q < n_jobs * kWGram256BParts; q++) acc += bp[q * 256];
         b_host[k] = (float)acc;
       }
+  });
+}
+
+// The same operators job by job, on explicit job bounds: job j takes the entries
+// [job_begin[j], job_end[j]) of (idx, w) -- of the rows of Y when idx is null -- in one launch of
+// wgram_kernel (K <= 128, row stride 128) or wgram256_kernel (K <= 256, row stride 256), and its own
+// block comes back: G_jobs[j] = W_j + W_j^T (K x K) and b_jobs[j] = the sum of its producers'
+// partials of (bias + w) y.  These are the blocks the trainer's solvers add up per row.
+int ials_weighted_gram_jobs(const float *Y_host, int64_t n, int64_t K, const int32_t *idx_host,
+                            const float *w_host, int64_t m, const int64_t *job_begin, const int64_t *job_end,
+                            int64_t n_jobs, float bias, int device, float *G_jobs, float *b_jobs) {
+  return guarded([&] {
+    require(Y_host != nullptr && job_begin != nullptr && job_end != nullptr && G_jobs != nullptr,
+            "null pointer");
+    require(n >= 0 && K >= 1 && K <= 256, "K must be in [1, 256]");
+    const bool wide = K > 128;
+    require(n_jobs >= 1 && n_jobs <= (wide ? 1024 : 4096),
+            wide ? "n_jobs must be in [1, 1024] for K > 128" : "n_jobs must be in [1, 4096]");
+    if (idx_host == nullptr) m = n;
+    check_entries(n, idx_host, w_host, m);
+    for (int64_t j = 0; j < n_jobs; j++)
+      require(job_begin[j] >= 0 && job_begin[j] <= job_end[j] && job_end[j] <= m,
+              "job bounds must satisfy 0 <= begin <= end <= m");
+    require_device(device);
+    DeviceGuard g(device);
+    const int ld = wide ? 256 : 128, parts = wide ? kWGram256BParts : kWGramBParts;
+    const size_t blk = (size_t)ld * ld;
+    cudaStream_t s = nullptr;
+    DeviceBuffer<float> d_Y, d_W, d_b;
+    GramEntries entries;
+    DeviceSyncOnExit sync;
+    CUDA_CHECK(cudaMemset(d_Y.alloc(std::max<int64_t>(n * ld, 1)), 0, sizeof(float) * std::max<int64_t>(n * ld, 1)));
+    if (n) rows_to_device(d_Y.get(), ld, Y_host, K, n);
+    entries.upload(idx_host, w_host, m, job_begin, job_end, n_jobs);
+    WGramArgs a = entries.args(bias);
+    a.Y = d_Y.get();
+    a.ld = ld;
+    a.W = d_W.alloc(n_jobs * blk);
+    a.bpart = d_b.alloc(n_jobs * parts * ld);
+    if (wide)
+      launch_wgram256(a, s);
+    else
+      launch_wgram(a, s);
+    std::vector<float> hW((size_t)n_jobs * blk), hb((size_t)n_jobs * parts * ld);
+    CUDA_CHECK(cudaMemcpy(hW.data(), d_W.get(), sizeof(float) * hW.size(), cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(hb.data(), d_b.get(), sizeof(float) * hb.size(), cudaMemcpyDeviceToHost));
+    for (int64_t j = 0; j < n_jobs; j++) {
+      const float *W = hW.data() + j * blk;
+      float *G = G_jobs + j * K * K;
+      for (int64_t r = 0; r < K; r++)
+        for (int64_t c = 0; c < K; c++) G[r * K + c] = W[r * ld + c] + W[c * ld + r];
+      if (b_jobs)
+        for (int64_t k = 0; k < K; k++) {
+          double acc = 0.0;
+          for (int p = 0; p < parts; p++) acc += hb[((size_t)j * parts + p) * ld + k];
+          b_jobs[j * K + k] = (float)acc;
+        }
+    }
   });
 }
 

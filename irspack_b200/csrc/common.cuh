@@ -253,6 +253,10 @@ struct WGramArgs {
   float *bpart;
 };
 
+// Entries one operand list of the tensor-core Gram may hold: the producers of wgram.cu step int32
+// offsets up to 32 entries past a job's end and read 31 past a stage's start.
+constexpr int64_t kMaxGramEntries = (1ll << 31) - 64;
+
 // ---- kernels / launchers (one .cu each) ----
 void launch_wgram(const WGramArgs &a, cudaStream_t s);
 void launch_wgram256(const WGramArgs &a, cudaStream_t s);  // whole Gram of 256-column rows: W [256][256] per job

@@ -33,7 +33,7 @@ const JobPlan &all_rows_plan(ials_trainer *t, const DeviceCsr &csr, int side, cu
   JobPlan &plan = t->all_rows[side];
   std::vector<int32_t> &first = t->all_rows_first[side];
   if (first.empty()) {
-    build_heavy_plan(csr, /*threshold=*/0, env_int("IALS_HEAVY_JOB_LEN", 4096), plan, s);
+    build_heavy_plan(csr, /*threshold=*/0, heavy_job_len(), plan, s);
     first.assign((size_t)plan.n_heavy + 1, 0);
     if (plan.n_heavy > 0)
       CUDA_CHECK(cudaMemcpy(first.data(), plan.heavy_first_job.get(), sizeof(int32_t) * (plan.n_heavy + 1),

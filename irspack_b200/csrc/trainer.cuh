@@ -183,6 +183,7 @@ void alloc_common(ials_trainer *t);
 TrainerPtr new_trainer(const ials_model_config *cfg, int64_t U, int64_t I, int device);
 void init_factors(ials_trainer *t, bool on_device);
 int64_t env_int(const char *name, int64_t dflt);
+int64_t heavy_job_len();  // IALS_HEAVY_JOB_LEN (default 4096); anything but a positive integer is rejected
 void plan_csr(ials_trainer *t, DeviceCsr &csr);
 void copy_csr(DeviceCsr &d, int64_t n_rows, int64_t n_cols, int64_t nnz, const int64_t *indptr,
               const int32_t *indices, const float *data, cudaMemcpyKind kind);

@@ -46,6 +46,39 @@ def test_topk_scores_rejects_malformed_mask(indptr, indices):
     assert "mask indptr / indices must both be given" in message
 
 
+GRAM_CALL = r"""
+import ctypes, sys
+sys.path.insert(0, {root!r})
+from irspack_b200 import _lib
+P = ctypes.c_void_p
+Y, G, b = (ctypes.c_float * 256)(), (ctypes.c_float * 65536)(), (ctypes.c_float * 256)()
+idx = (ctypes.c_int32 * 4)()
+jb, je = (ctypes.c_int64 * 1)(0), (ctypes.c_int64 * 1)(0)
+p = lambda a: ctypes.cast(a, P)
+m = 2 ** 31 - 63
+calls = {{
+    "gram": lambda: _lib.lib.ials_weighted_gram(p(Y), m, 1, None, None, 0, 1, 0.0, 0, p(G), p(b)),
+    "gram_gathered": lambda: _lib.lib.ials_weighted_gram(p(Y), 4, 1, p(idx), None, m, 1, 0.0, 0, p(G), p(b)),
+    "gram256": lambda: _lib.lib.ials_weighted_gram256(p(Y), 1, 200, p(idx), None, m, 1, 0.0, 0, p(G), p(b)),
+    "gram_jobs": lambda: _lib.lib.ials_weighted_gram_jobs(p(Y), 4, 1, p(idx), None, m, p(jb), p(je), 1, 0.0, 0,
+                                                          p(G), p(b)),
+}}
+st = calls[{which!r}]()
+print(st, (_lib.lib.ials_last_error() or b"").decode() if st else "")
+"""
+
+
+@pytest.mark.parametrize("which", ["gram", "gram_gathered", "gram256", "gram_jobs"])
+def test_gram_operators_reject_more_than_2_31_minus_64_entries(which):
+    """The producers of the tensor-core Gram keep int32 offsets that run a stage past a job's end: a
+    length that claims 2^31 - 63 entries is rejected before any entry is read."""
+    res = subprocess.run([sys.executable, "-c", GRAM_CALL.format(root=ROOT, which=which)],
+                         capture_output=True, text=True, cwd=ROOT, timeout=300)
+    assert res.returncode == 0, f"process died (rc {res.returncode}): {res.stderr[-2000:]}"
+    status, _, message = res.stdout.strip().partition(" ")
+    assert int(status) == IALS_ERR_INVALID_ARGUMENT and "2^31 - 64" in message, res.stdout
+
+
 @pytest.mark.parametrize("indptr, indices", [
     (None, None),       # no mask
     ([0, 1, 2], [1, 2]),  # a mask with entries
